@@ -2,9 +2,12 @@
 """bench.py -- the SRCNN hot path on B200, BASELINE.json's configurations.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--workloads c3,c2,c4,c5]
+                    [--workloads c3,c2,c4,c5] [--dump-outputs DIR]
 
-Prints ONE JSON line (rank 0).  Workloads (BASELINE.json `configs`):
+Prints ONE JSON line (rank 0).  Every timed loop of `--impl ours` runs exactly K steps.
+`--dump-outputs DIR` writes, after the timed loops, what the last step of each loop returned
+(rank 0's share) as DIR/<workload>_<entry>.npy; see dump_sample.  Workloads (BASELINE.json
+`configs`):
   * c3 (primary: `metric`/`value`/`e2e`/`roofline`): INFERENCE of one 4096x4096 luma image with
     the 9-1-5 n1=64 n2=32 network, halo row-sharded across the N ranks (no collective; strong
     scaling).  A step = one forward pass of the whole image.  MPix/s = input pixels / step time.
@@ -247,6 +250,21 @@ def frames_like(rng, n, h, w):
     return out
 
 
+DUMP_SAMPLE = 1 << 20
+
+
+def dump_sample(a):
+    """An output as it is dumped: whole when it has at most DUMP_SAMPLE values, else the values
+    at DUMP_SAMPLE distinct flat indices drawn by default_rng(0) (sorted), so that two builds
+    given the same arguments are compared at the same positions.  Four sampled outputs of 4 MB
+    keep a dump of every workload far below 64 MB."""
+    a = np.ascontiguousarray(a, np.float32).reshape(-1)
+    if a.size <= DUMP_SAMPLE:
+        return a.copy()
+    idx = np.sort(np.random.default_rng(0).choice(a.size, DUMP_SAMPLE, replace=False))
+    return a[idx]
+
+
 def workload_config(n, wl):
     return {"workload": "C3: SRCNN 9-1-5 n1=64 n2=32 inference, one 4096x4096 luma image, halo "
                         "row bands over %d GPU(s)" % n,
@@ -380,6 +398,8 @@ def run_ours(args, rank, world, local_rank, wl):
         return float(t.item())
 
     res = {}
+    dump = bool(args.dump_outputs) and rank == 0
+    dumps = {}
     with torch.cuda.stream(stream):
         ctx = pkg.Context(local_rank, stream=stream.cuda_stream)
         if world > 1:
@@ -500,7 +520,10 @@ def run_ours(args, rank, world, local_rank, wl):
 
             windows["c3"] = [time.time(), None]      # clocks: samples of the timed loops only
             inf_ms, inf_launches = timed(infer_step, args.steps, args.warmup)
-            e2e_ms, _ = timed(infer_e2e_step, max(2, args.steps // 2), 3)
+            if dump:
+                last = outs[(args.warmup + args.steps - 1) % R]
+                dumps["c3_forward_fused"] = dump_sample(ctx.read(last, (r1 - r0, w3)))
+            e2e_ms, _ = timed(infer_e2e_step, args.steps, 3)
 
             # a STREAM of images through the non-blocking entry: up to two calls in flight, so
             # the download of step i overlaps the upload / first launches of step i+1; every
@@ -525,6 +548,8 @@ def run_ours(args, rank, world, local_rank, wl):
 
             e2e_stream_ms = infer_stream(args.steps, 3)
             assert np.array_equal(out_host.array, out_host2.array)
+            if dump:
+                dumps["c3_infer_rows_host"] = dump_sample(outs_h[(args.steps - 1) % 2].array)
             out_host2.free()
             res["c3"] = dict(ms=inf_ms, launches=inf_launches, e2e_ms=e2e_ms,
                              e2e_stream_ms=e2e_stream_ms, rows=(r0, r1),
@@ -581,10 +606,15 @@ def run_ours(args, rank, world, local_rank, wl):
                         off += cnt
                 ctx.block()
 
-            steps = max(2, 2 * args.steps) if key == "c2" else max(2, args.steps // 10)
             windows[key] = [time.time(), None]
-            ms, launches = timed(train_step, steps, args.warmup)
-            e2e_ms, _ = timed(train_e2e_step, steps, 3)
+            ms, launches = timed(train_step, args.steps, args.warmup)
+            if dump:
+                p = net.params()
+                dumps[key + "_train_chunk_params"] = np.concatenate(
+                    [p["%s%d" % (t, l)] for l in (1, 2, 3) for t in ("w", "b")])
+            e2e_ms, _ = timed(train_e2e_step, args.steps, 3)
+            if dump:
+                dumps[key + "_train_chunks_host_params"] = params_host.array.copy()
             windows[key][1] = time.time()
             # per-kernel-id device time of ONE epoch through a profiling context (not the timed run)
             kern = None
@@ -603,7 +633,7 @@ def run_ours(args, rank, world, local_rank, wl):
                         for k in after if after[k][1] != before[k][1]}
                 kern["_chunk_patches"] = pS
                 pctx.close()
-            out = dict(ms=ms, launches=launches, e2e_ms=e2e_ms, steps=steps, chunk=chunk,
+            out = dict(ms=ms, launches=launches, e2e_ms=e2e_ms, steps=args.steps, chunk=chunk,
                        n_loc=n_loc, n_global=n_global, grad_floats=grad.numel(), kernels=kern,
                        h2d=2 * n_loc * bytes_per, d2h=4 * grad.numel())
             for m in (d_in, d_gt, work):
@@ -647,12 +677,17 @@ def run_ours(args, rank, world, local_rank, wl):
             def frames_e2e_step(i):
                 net.infer_frames_host(fin.array, C5_W, C5_H, fout.array)
 
-            steps = max(2, args.steps // 10)
             windows["c5"] = [time.time(), None]
-            ms, launches = timed(frames_step, steps, args.warmup)
-            e2e_ms, _ = timed(frames_e2e_step, steps, 3)
+            ms, launches = timed(frames_step, args.steps, args.warmup)
+            if dump:
+                # into fout, which the host-buffer loop below overwrites: no second 2 GB array
+                pkg._check(ctx.L.srcnn_read(ctx.h, d_out, 0, fout.nbytes, fout.ptr, 1))
+                dumps["c5_forward_fused"] = dump_sample(fout.array)
+            e2e_ms, _ = timed(frames_e2e_step, args.steps, 3)
+            if dump:
+                dumps["c5_infer_frames_host"] = dump_sample(fout.array)
             windows["c5"][1] = time.time()
-            res["c5"] = dict(ms=ms, launches=launches, e2e_ms=e2e_ms, steps=steps, n_loc=n_loc,
+            res["c5"] = dict(ms=ms, launches=launches, e2e_ms=e2e_ms, steps=args.steps, n_loc=n_loc,
                              h2d=fin.nbytes, d2h=fout.nbytes)
             ctx.release(d_in)
             ctx.release(d_out)
@@ -840,6 +875,11 @@ def run_ours(args, rank, world, local_rank, wl):
                               "d2h_bytes_per_step": c["d2h"],
                               "pcie": pcie_block(c["h2d"], c["d2h"], c["e2e_ms"])}}
 
+    if dump:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dumps.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
+
     if world == 1 and not args.no_cpu_baseline:
         line["cpu_baseline"] = cpu_baseline(args, wl)
     print(json.dumps(line), flush=True)
@@ -882,7 +922,11 @@ def main():
                     help="output rows of C3 the reference arm computes per step (default: all)")
     ap.add_argument("--ref-patches", type=int, default=512)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step of each loop to DIR/*.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs dumps the outputs of --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     wl = [w for w in args.workloads.split(",") if w]
     rank = int(os.environ.get("RANK", "0"))
