@@ -457,6 +457,7 @@ __global__ void __launch_bounds__(Cfg::NT, 1) bwd3_tc_kernel(Args a) {
 }
 
 inline bool supported(int k, int f) { return k == Cfg::N && f == Cfg::F; }
+constexpr int MAX_ROWS = 64;   // out2 rows per sample (see fast::backward3_tc)
 
 // d3 + d2 + gW3/gB3 partials; returns 1 when launched (partials in ctx->splitk_scratch, *count of
 // them), 0 when the shape is not handled.  `mx`: the context's maxima block; out2's maximum must

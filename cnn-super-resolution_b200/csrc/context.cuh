@@ -116,6 +116,7 @@ struct srcnn_ctx {
   const void* c5_l1_max_of = nullptr;   // out1 whose maximum the layer-1-only kernel recorded
   const void* c5_fresh_out2 = nullptr;  // out2 whose maximum the forward of this chunk recorded
   const void* c5_fresh_d2 = nullptr;    // d2 whose maximum the layer-3 backward recorded
+  // (the three pointers above hold inside one training chunk only: cleared when it returns)
   // per-context (= per-device) one-time kernel setup: opt-in dynamic shared memory sizes and
   // occupancy queries, keyed by the kernel's address.  cudaFuncSetAttribute is per DEVICE, so a
   // process-wide flag would leave a second context on another GPU unconfigured.

@@ -415,6 +415,9 @@ __global__ void __launch_bounds__(Cfg::NT, 1) forward_fused_hp_kernel(fused::Arg
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int X0 = blockIdx.x * C::OW3;
+  // out1 / out2 kept (BATCH): a strip stores the columns of its OW3 output columns; the last one
+  // also stores the halo columns to their right, which no strip after it covers
+  const bool last_strip = X0 + C::OW3 >= a.w3;
   const int R0 = blockIdx.y * rpc;
   const float* img = BATCH ? a.in : a.in + (size_t)blockIdx.z * a.w * a.h;
   float* dst = BATCH ? a.out : a.out + (size_t)blockIdx.z * a.w3 * a.h3;
@@ -700,7 +703,7 @@ __global__ void __launch_bounds__(Cfg::NT, 1) forward_fused_hp_kernel(fused::Arg
     if (keep1) {
       const int m = (warp & 3) * 32 + lane, vx = X0 + m, smp = vx / bx.pw, px = vx - smp * bx.pw;
       const int w1 = bx.pw - (C::F1 - 1), h1 = bx.ph - (C::F1 - 1);
-      if (m < C::OW3 && vx < a.w && px < w1) pix1 = (smp * h1 + R0) * w1 + px;
+      if ((m < C::OW3 || last_strip) && vx < a.w && px < w1) pix1 = (smp * h1 + R0) * w1 + px;
     }
     const int w1_row = bx.pw - (C::F1 - 1);
     float* st1 = reinterpret_cast<float*>(smem_raw + C::oS1) +
@@ -803,7 +806,7 @@ __global__ void __launch_bounds__(Cfg::NT, 1) forward_fused_hp_kernel(fused::Arg
     if (keep2) {
       const int m = (warp & 3) * 32 + lane, vx = X0 + m, smp = vx / bx.pw, px = vx - smp * bx.pw;
       const int w2 = bx.pw - (C::F1 - 1), h2 = bx.ph - (C::F1 - 1);
-      if (m < C::OW3 && vx < a.w && px < w2) pix2 = (smp * h2 + R0) * w2 + px;
+      if ((m < C::OW3 || last_strip) && vx < a.w && px < w2) pix2 = (smp * h2 + R0) * w2 + px;
     }
     const int w2_row = bx.pw - (C::F1 - 1);
     float* st2 = reinterpret_cast<float*>(smem_raw + C::oS2) + (warp - C::W_E2) * (32 * C::SP);

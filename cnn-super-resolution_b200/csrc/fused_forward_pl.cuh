@@ -194,6 +194,9 @@ __global__ void __launch_bounds__(Cfg::NT, 1) forward_fused_pl_kernel(fused::Arg
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int X0 = blockIdx.x * C::OW3;
+  // out1 / out2 kept (BATCH): a strip stores the columns of its OW3 output columns; the last one
+  // also stores the halo columns to their right, which no strip after it covers
+  const bool last_strip = X0 + C::OW3 >= a.w3;
   const int R0 = blockIdx.y * rpc;
   const float* img = BATCH ? a.in : a.in + (size_t)blockIdx.z * a.w * a.h;
   float* dst = BATCH ? a.out : a.out + (size_t)blockIdx.z * a.w3 * a.h3;
@@ -442,7 +445,7 @@ __global__ void __launch_bounds__(Cfg::NT, 1) forward_fused_pl_kernel(fused::Arg
     if (BATCH && bx.out1) {
       const int m = (warp & 3) * 32 + lane, vx = X0 + m, smp = vx / bx.pw, px = vx - smp * bx.pw;
       const int w1 = bx.pw - (C::F1 - 1), h1 = bx.ph - (C::F1 - 1);
-      if (m < C::OW3 && vx < a.w && px < w1)
+      if ((m < C::OW3 || last_strip) && vx < a.w && px < w1)
         o1 = bx.out1 + (((size_t)smp * h1 + R0) * w1 + px) * C::N1 + ch0;
     }
     const size_t o1_row = (size_t)(bx.pw - (C::F1 - 1)) * C::N1;
@@ -496,7 +499,7 @@ __global__ void __launch_bounds__(Cfg::NT, 1) forward_fused_pl_kernel(fused::Arg
     if (BATCH && bx.out2) {
       const int m = (warp & 3) * 32 + lane, vx = X0 + m, smp = vx / bx.pw, px = vx - smp * bx.pw;
       const int w2 = bx.pw - (C::F1 - 1), h2 = bx.ph - (C::F1 - 1);
-      if (m < C::OW3 && vx < a.w && px < w2)
+      if ((m < C::OW3 || last_strip) && vx < a.w && px < w2)
         o2 = bx.out2 + (((size_t)smp * h2 + R0) * w2 + px) * C::N2;
     }
     const size_t o2_row = (size_t)(bx.pw - (C::F1 - 1)) * C::N2;

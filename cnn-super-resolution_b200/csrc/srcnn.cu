@@ -1193,9 +1193,15 @@ int train_chunk_on(srcnn_ctx* ctx, const srcnn_net* net, srcnn_mem in, srcnn_mem
   // valid for the layer-2 gradient of the same chunk
   ctx->c5_max_out1_of = ctx->c5_max_d2_of = nullptr;
   ctx->c5_fresh_out2 = ctx->c5_fresh_d2 = nullptr;
+  // the maxima this chunk's producers record describe its buffers only until it returns: a later
+  // standalone call on the same buffers (after new data was written into them, or after another
+  // call overwrote the context's c5::Maxes) must measure them again
   struct KnownScope {
     srcnn_ctx* c;
-    ~KnownScope() { c->c5_maxes_known = false; }
+    ~KnownScope() {
+      c->c5_maxes_known = false;
+      c->c5_fresh_out2 = c->c5_fresh_d2 = c->c5_l1_max_of = nullptr;
+    }
   } known_scope{ctx};
   // forward, keeping the activations (ConfigBasedDataPipeline.cpp:200-241)
   int fused_fwd = 0;
