@@ -26,7 +26,9 @@ NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", 
 
 KERNEL_IDS = ["forward", "squared_err", "last_layer_delta", "deltas", "backpropagate",
               "update_params", "sum", "sub_from_all", "extract_luma", "swap_luma",
-              "forward_fused", "train_fused"]
+              "forward_fused", "train_fused", "resample"]
+
+RESAMPLE_FILTERS = {"bicubic": 0, "lanczos": 1}   # SRCNN_RESAMPLE_BICUBIC / _LANCZOS
 
 
 class SrcnnError(RuntimeError):
@@ -98,6 +100,8 @@ _SIGS = {
     "srcnn_sub_from_all": (_i, [_vp, _u64, _f, _u]),
     "srcnn_extract_luma": (_i, [_vp, _u64, _u64, _i, _i, _i]),
     "srcnn_swap_luma": (_i, [_vp, _u64, _u64, _u64] + [_i] * 4),
+    "srcnn_resample": (_i, [_vp, _u64, _i, _i, _u64, _u64, _i, _i, _i]),
+    "srcnn_upscale_image_host": (_i, [_vp, C.POINTER(CNet), _vp, _i, _i, _i, _i, _i, _vp]),
     "srcnn_forward_fused_supported": (_i, [C.POINTER(CNet)]),
     "srcnn_forward_fused": (_i, [_vp, C.POINTER(CNet), _u64, _u64, _i, _i, _i, _u64, _u64]),
     "srcnn_infer_rows_host": (_i, [_vp, C.POINTER(CNet), _vp, _i, _i, _i, _i, _vp]),
@@ -147,6 +151,12 @@ def lib():
 def _check(rc):
     if rc != 0:
         raise SrcnnError("srcnn error %d: %s" % (rc, lib().srcnn_last_error().decode()))
+
+
+def _filter_id(name):
+    if name not in RESAMPLE_FILTERS:
+        raise ValueError("unknown resample filter %r (have %s)" % (name, sorted(RESAMPLE_FILTERS)))
+    return RESAMPLE_FILTERS[name]
 
 
 def _np_ptr(a):
@@ -357,6 +367,13 @@ class Context:
     def swap_luma(self, rgba, new_luma, target, gt_w, gt_h, luma_w, luma_h):
         _check(self.L.srcnn_swap_luma(self.h, rgba, new_luma, target, gt_w, gt_h, luma_w, luma_h))
 
+    def resample(self, rgba_in, w, h, rgba_out, out_w, out_h, resample="lanczos",
+                 luma_out=NULL_MEM):
+        """Pillow-exact enlargement of a w x h RGBA8 image to out_w x out_h RGBA8 (alpha 255),
+        with its normalized luma in luma_out unless that is NULL_MEM."""
+        _check(self.L.srcnn_resample(self.h, rgba_in, w, h, rgba_out, luma_out, out_w, out_h,
+                                     _filter_id(resample)))
+
 
 class Net:
     """Device-resident parameters, gradient accumulators and momentum state of the three
@@ -421,6 +438,20 @@ class Net:
         fn = self.ctx.L.srcnn_infer_rows_host if block else self.ctx.L.srcnn_infer_rows_host_async
         _check(fn(self.ctx.h, C.byref(self.c), _np_ptr(host_in), w, h, row0, row1,
                   _np_ptr(host_out)))
+
+    def upscale_image_host(self, rgba, out_w, out_h, resample="lanczos", out=None):
+        """rgba: uint8 [h][w][4] (alpha ignored) -> uint8 [out_h][out_w][3]: the image enlarged
+        with Pillow's filter, then the `cnn` forward mode on it (luma through the network,
+        swapped back into the enlarged image).  `out` may be a preallocated (pinned) array."""
+        assert rgba.dtype == np.uint8 and rgba.ndim == 3 and rgba.shape[2] == 4
+        rgba = np.ascontiguousarray(rgba)
+        if out is None:
+            out = np.empty((out_h, out_w, 3), np.uint8)
+        assert out.dtype == np.uint8 and out.shape == (out_h, out_w, 3) and out.flags.c_contiguous
+        _check(self.ctx.L.srcnn_upscale_image_host(self.ctx.h, C.byref(self.c), _np_ptr(rgba),
+                                                   rgba.shape[1], rgba.shape[0], out_w, out_h,
+                                                   _filter_id(resample), _np_ptr(out)))
+        return out
 
     def infer_frames_host(self, host_in, w, h, host_out):
         """host_in: [n][h][w] float32 frames; host_out: [n][h3][w3].  Upload / forward / download

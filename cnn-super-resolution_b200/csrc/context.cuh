@@ -137,9 +137,12 @@ struct srcnn_ctx {
   cudaStream_t copy_in = nullptr, copy_out = nullptr, compute2 = nullptr;
   // the sub-band pipeline of srcnn_infer_rows_host as an instantiated CUDA graph, replayed while
   // the call's arguments (host / device pointers, shape, band, parameters) stay the same
+  // (the sub-band pipelines, srcnn_infer_rows_host and srcnn_upscale_image_host, key their
+  // graphs by kGraphKey words of call arguments)
+  static constexpr int kGraphKey = 32;
   cudaGraphExec_t e2e_graph = nullptr;
-  unsigned long long e2e_key[20] = {};
-  unsigned e2e_graph_launches = 0;
+  unsigned long long e2e_key[kGraphKey] = {};
+  unsigned e2e_graph_launches[SRCNN_K_COUNT] = {};   // launches per kernel id of one replay
   cudaEvent_t ev_join[2] = {};
   // srcnn_infer_rows_host_async: two lanes, each with its own stream, staging and graph, used
   // alternately, so that the tail (download) of one call overlaps the head (upload, first
@@ -150,14 +153,41 @@ struct srcnn_ctx {
     void* out = nullptr;
     size_t in_bytes = 0, out_bytes = 0;
     cudaGraphExec_t graph = nullptr;
-    unsigned long long key[20] = {};
-    unsigned graph_launches = 0;
+    unsigned long long key[kGraphKey] = {};
+    unsigned graph_launches[SRCNN_K_COUNT] = {};
     srcnn_mem params[6] = {};   // the parameter buffers the lane's call in flight reads
   } lanes[2];
   unsigned lane_next = 0;
   bool lanes_busy = false;
 
   cudaEvent_t lane_ev = nullptr;
+  // srcnn_resample weight tables, one per (w, h, W, H, filter); the host copy stays alive
+  // because the upload that reads it is asynchronous
+  struct ResampleKey {
+    int w, h, W, H, filter;
+  };
+  struct ResampleTable {
+    ResampleKey key;
+    std::vector<int> host;
+    int* dev = nullptr;
+    int rows_max = 0;
+  };
+  std::vector<ResampleTable> resample_tables;
+  // srcnn_upscale_image_host: device staging (grown on demand) and its captured pipeline
+  struct UpscaleStaging {
+    void* small = nullptr;   // input RGBA8
+    void* rgba = nullptr;    // enlarged RGBA8
+    void* luma = nullptr;    // enlarged luma, then minus its Q1 mean
+    void* out = nullptr;     // network output
+    void* rgb = nullptr;     // result RGB8
+    void* s1 = nullptr;      // layer 1 / 2 activations of the three-launch route
+    void* s2 = nullptr;
+    size_t small_bytes = 0, rgba_bytes = 0, luma_bytes = 0, out_bytes = 0, rgb_bytes = 0,
+           s1_bytes = 0, s2_bytes = 0;
+    cudaGraphExec_t graph = nullptr;
+    unsigned long long key[kGraphKey] = {};
+    unsigned graph_launches[SRCNN_K_COUNT] = {};
+  } up;
   static constexpr int kEvents = 32;
   cudaEvent_t ev_in[kEvents] = {}, ev_k[kEvents] = {};
   cudaEvent_t ev_d[4] = {};   // download-finished events of srcnn_infer_frames_host's ring

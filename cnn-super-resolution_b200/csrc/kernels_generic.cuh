@@ -323,6 +323,15 @@ __global__ void sub_from_all_kernel(float* data, float value, unsigned len) {
     data[i] = data[i] - value;
 }
 
+// sub_from_all_kernel with value = *sum / (float)len read on the device (the mean never goes
+// through the host): the same float division and subtraction as the host route
+__global__ void sub_mean_kernel(float* data, const float* __restrict__ sum, unsigned len) {
+  const float value = __fdiv_rn(*sum, (float)len);
+  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < len;
+       i += (size_t)gridDim.x * blockDim.x)
+    data[i] = data[i] - value;
+}
+
 __global__ void fill_kernel(float* data, float value, size_t len) {
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < len;
        i += (size_t)gridDim.x * blockDim.x)
@@ -429,25 +438,30 @@ __global__ void gather_kernel(const float* const* __restrict__ src, float* __res
 
 // ------------------------------------------------------------------ luma -------------
 // reference: src/kernel/extract_luma.cl:7-23
-__global__ void extract_luma_kernel(const uchar4* __restrict__ rgba, float* __restrict__ target,
-                                    int count, int normalize) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= count) return;
-  const uchar4 p = rgba[i];
+// the luma of one RGBA8 pixel; every kernel that produces luma from pixels calls this
+__device__ __forceinline__ float luma_of(uchar4 p, int normalize) {
   // explicit round-to-nearest mul/add (never contracted to FMA) in the order of the
   // oracle's dot(): ((R*.299 + G*.587) + B*.114) + A*0
   float y = __fadd_rn(__fmul_rn((float)p.x, 0.299f), __fmul_rn((float)p.y, 0.587f));
   y = __fadd_rn(y, __fmul_rn((float)p.z, 0.114f));
-  target[i] = normalize ? __fdiv_rn(y, 255.0f) : y;
+  return normalize ? __fdiv_rn(y, 255.0f) : y;
 }
 
-// reference: src/kernel/swap_luma.cl:18-69
+__global__ void extract_luma_kernel(const uchar4* __restrict__ rgba, float* __restrict__ target,
+                                    int count, int normalize) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= count) return;
+  target[i] = luma_of(rgba[i], normalize);
+}
+
+// reference: src/kernel/swap_luma.cl:18-69.  Image rows [row0, row1) (the whole image is
+// [0, gt_h)); the grid covers row1 - row0 rows.
 __global__ void swap_luma_kernel(const uchar4* __restrict__ rgba, const float* __restrict__ luma,
-                                 unsigned char* __restrict__ target, int gt_w, int gt_h,
+                                 unsigned char* __restrict__ target, int gt_w, int row0, int row1,
                                  int luma_w, int luma_h) {
   const int x = blockIdx.x * blockDim.x + threadIdx.x;
-  const int y = blockIdx.y * blockDim.y + threadIdx.y;
-  if (x >= gt_w || y >= gt_h) return;
+  const int y = row0 + blockIdx.y * blockDim.y + threadIdx.y;
+  if (x >= gt_w || y >= row1) return;
   const int pad = (gt_w - luma_w) / 2;
   const size_t i = (size_t)y * gt_w + x;
   const uchar4 p = rgba[i];

@@ -12,6 +12,7 @@
 #include "context.cuh"
 #include "kernels_fast.cuh"
 #include "kernels_generic.cuh"
+#include "resample.cuh"
 
 using namespace srcnn;
 
@@ -39,6 +40,19 @@ inline Dims net_dims(const srcnn_net* net, int w, int h) {
 }
 
 inline size_t align256(size_t bytes) { return (bytes + 255) & ~(size_t)255; }
+
+// the enlargements srcnn_resample accepts
+inline int check_resample(int w, int h, int out_w, int out_h, int filter) {
+  SRCNN_REQUIRE(w > 0 && h > 0 && out_w > 0 && out_h > 0, "bad resample size %dx%d -> %dx%d", w, h,
+                out_w, out_h);
+  SRCNN_REQUIRE(out_w >= w && out_h >= h, "resample %dx%d -> %dx%d: only enlargements are supported",
+                w, h, out_w, out_h);
+  SRCNN_REQUIRE((size_t)out_w * out_h < ((size_t)1 << 31), "output of %dx%d pixels is too large",
+                out_w, out_h);
+  SRCNN_REQUIRE(filter == SRCNN_RESAMPLE_BICUBIC || filter == SRCNN_RESAMPLE_LANCZOS,
+                "unknown resample filter %d", filter);
+  return SRCNN_OK;
+}
 
 inline int check_net(const srcnn_net* net) {
   SRCNN_REQUIRE(net != nullptr, "net is null");
@@ -121,6 +135,13 @@ int srcnn_ctx_destroy(srcnn_ctx* ctx) {
     if (l.stream) cudaStreamDestroy(l.stream);
   }
   if (ctx->lane_ev) cudaEventDestroy(ctx->lane_ev);
+  {
+    srcnn_ctx::UpscaleStaging& u = ctx->up;
+    if (u.graph) cudaGraphExecDestroy(u.graph);
+    for (void* p : {u.small, u.rgba, u.luma, u.out, u.rgb, u.s1, u.s2})
+      if (p) cudaFree(p);
+  }
+  for (srcnn_ctx::ResampleTable& t : ctx->resample_tables) cudaFree(t.dev);
   if (ctx->nccl_comm && comm::api()) comm::api()->CommDestroy(ctx->nccl_comm);
   ctx->nccl_comm = nullptr;
   for (Allocation& a : ctx->allocs)
@@ -619,8 +640,32 @@ int srcnn_swap_luma(srcnn_ctx* ctx, srcnn_mem rgba, srcnn_mem new_luma, srcnn_me
   ctx->note_write(target);
   LaunchScope scope(ctx, SRCNN_K_SWAP_LUMA);
   dim3 block(32, 8), grid((gt_w + 31) / 32, (gt_h + 7) / 8);
-  generic::swap_luma_kernel<<<grid, block, 0, ctx->stream>>>(pi, pl, pt, gt_w, gt_h, luma_w, luma_h);
+  generic::swap_luma_kernel<<<grid, block, 0, ctx->stream>>>(pi, pl, pt, gt_w, 0, gt_h, luma_w,
+                                                             luma_h);
   return check_launch("swap_luma");
+}
+
+int srcnn_resample(srcnn_ctx* ctx, srcnn_mem rgba_in, int w, int h, srcnn_mem rgba_out,
+                   srcnn_mem luma_out, int out_w, int out_h, int filter) {
+  SRCNN_ENTER(ctx);
+  SRCNN_TRY(check_resample(w, h, out_w, out_h, filter));
+  const uchar4* pi;
+  uchar4* po;
+  float* pl = nullptr;
+  const size_t npx = (size_t)out_w * out_h;
+  SRCNN_TRY(resolve(ctx, rgba_in, (size_t)w * h * 4, &pi, "rgba input"));
+  SRCNN_TRY(resolve(ctx, rgba_out, npx * 4, &po, "rgba output"));
+  if (luma_out != SRCNN_NULL_MEM) {
+    SRCNN_TRY(resolve(ctx, luma_out, sizeof(float) * npx, &pl, "luma output"));
+    ctx->note_write(luma_out);
+  }
+  ctx->note_write(rgba_out);
+  const int* tab;
+  int rows_max;
+  SRCNN_TRY(resample::table_for(ctx, w, h, out_w, out_h, filter, &tab, &rows_max));
+  LaunchScope scope(ctx, SRCNN_K_RESAMPLE);
+  SRCNN_TRY(resample::launch(ctx, pi, w, po, pl, out_w, out_h, filter, tab, rows_max));
+  return check_launch("resample");
 }
 
 // ======================================================================= fused hot path
@@ -738,6 +783,146 @@ int srcnn_forward_fused(srcnn_ctx* ctx, const srcnn_net* net, srcnn_mem in, srcn
 }
 
 namespace {
+constexpr int kMaxSub = srcnn_ctx::kEvents;
+
+// The sub-band cut of a band of `band_out_h` output rows: sub-band i is the band-relative output
+// rows [sub_r0[i], sub_r0[i + 1]); returns the count (1 below 256 rows).
+int subband_rows(int band_out_h, int sub_r0[kMaxSub + 1]) {
+  // SRCNN_E2E_SUBBANDS=n (2..32) / SRCNN_E2E_RAMPCAP=c override the defaults for experiments.
+  // Measured on C3 (PCIe gen5 x16, 55 GB/s each way, 47.6 with both directions busy), wall
+  // clock of the call with the 0.9 ms kernel: 12 sub-bands 1.84-1.88 ms, 14: 1.78, 16: 1.73-1.78,
+  // 18: 1.78, 20 (cap 3): 1.79, 24: 1.83, 32: 1.96; ramp cap 3 / 5 / 6 at 16: 1.78 / 1.83 / 1.79.
+  static const int kSubDefault = std::getenv("SRCNN_E2E_SUBBANDS") ? std::atoi(std::getenv("SRCNN_E2E_SUBBANDS")) : 16;
+  // bands of a multi-GPU partition are pipelined too (an 8-way split of C3 leaves 511 rows per
+  // rank, and with 8 ranks copying at once each gets ~18 GB/s of the host's pinned-copy rate, so
+  // the copies dominate even more): about one sub-band per 64 output rows, at most the default
+  const int n_sub = band_out_h >= 256
+                  ? std::min(std::min(std::max(kSubDefault, 2), kMaxSub), std::max(2, band_out_h / 64))
+                  : 1;
+  sub_r0[0] = 0;
+  {
+    // shares ramp up from a small first sub-band and down to a small last one: 1,2,3,..,3,2,1
+    // capped at 2 units (round-2 sweep, profiles/r2g_e2e_subband_sweep.txt: cap 2 / 4 / 8 at 16
+    // sub-bands: 1.69 / 1.77 / 1.86 ms); the exposed head upload / tail download shrink with them
+    float unit[kMaxSub], total = 0.f;
+    for (int i = 0; i < n_sub; i++) {
+      static const int kRampCap = std::getenv("SRCNN_E2E_RAMPCAP") ? std::atoi(std::getenv("SRCNN_E2E_RAMPCAP")) : 2;
+      unit[i] = (float)std::min(std::min(i + 1, n_sub - i), std::max(kRampCap, 1));
+      total += unit[i];
+    }
+    float acc = 0.f;
+    for (int i = 0; i < n_sub; i++) {
+      acc += unit[i];
+      sub_r0[i + 1] = i + 1 == n_sub ? band_out_h : std::min((int)(acc / total * band_out_h + 0.5f), band_out_h);
+    }
+    if (n_sub == 1) sub_r0[1] = band_out_h;
+  }
+  return n_sub;
+}
+
+// ---- the captured sub-band pipelines (srcnn_infer_rows_host, srcnn_upscale_image_host) -------
+// The pipelines are ~10 runtime calls per sub-band; issued one by one the host only just stays
+// ahead of the GPU (and falls behind when another thread competes for the CPU), so each is
+// captured once into a CUDA graph and replayed with one launch while the arguments repeat
+// (SRCNN_E2E_GRAPH=0 disables; profile mode times individual launches and never captures).
+bool graphs_enabled(const srcnn_ctx* ctx) {
+  static const bool kGraphs = !(std::getenv("SRCNN_E2E_GRAPH") && std::atoi(std::getenv("SRCNN_E2E_GRAPH")) == 0);
+  return kGraphs && !ctx->profile;
+}
+
+// one route's graph, the arguments it was captured for, and its launches per kernel id
+struct GraphSlot {
+  cudaGraphExec_t* graph;
+  unsigned long long* key;   // [srcnn_ctx::kGraphKey]
+  unsigned* launches;        // [SRCNN_K_COUNT]
+};
+
+// the launch counters when a capture started
+struct LaunchTally {
+  uint64_t per_id[SRCNN_K_COUNT];
+  explicit LaunchTally(const srcnn_ctx* ctx) {
+    for (int i = 0; i < SRCNN_K_COUNT; i++) per_id[i] = ctx->stats[i].launches;
+  }
+};
+
+// true when the slot holds a graph captured for `key`; counts its launches (the caller launches it)
+bool graph_replay(srcnn_ctx* ctx, const GraphSlot& g, const unsigned long long* key) {
+  if (!*g.graph || std::memcmp(key, g.key, sizeof(unsigned long long) * srcnn_ctx::kGraphKey) != 0)
+    return false;
+  for (int i = 0; i < SRCNN_K_COUNT; i++) {
+    ctx->launch_count += g.launches[i];
+    ctx->stats[i].launches += g.launches[i];
+  }
+  return true;
+}
+
+// drops the slot's old graph and starts capturing the context stream
+int graph_begin(srcnn_ctx* ctx, const GraphSlot& g) {
+  if (*g.graph) {
+    SRCNN_CUDA(cudaStreamSynchronize(ctx->stream));   // the old graph may still be running
+    cudaGraphExecDestroy(*g.graph);
+    *g.graph = nullptr;
+  }
+  if (!ctx->ev_join[0])
+    for (int i = 0; i < 2; i++)
+      SRCNN_CUDA(cudaEventCreateWithFlags(&ctx->ev_join[i], cudaEventDisableTiming));
+  {   // everything the launches allocate lazily must exist before the capture starts
+    fused_hp::Scales* s_;
+    unsigned* w_;
+    SRCNN_TRY(fused_hp::scale_slot(ctx, &s_, &w_));
+  }
+  cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+  if (cudaStreamIsCapturing(ctx->stream, &cap) == cudaSuccess && cap != cudaStreamCaptureStatusNone) {
+    cudaGraph_t stale = nullptr;   // a capture an earlier failed call left open
+    cudaStreamEndCapture(ctx->stream, &stale);
+    if (stale) cudaGraphDestroy(stale);
+    cudaGetLastError();
+  }
+  SRCNN_CUDA(cudaStreamSynchronize(ctx->stream));
+  SRCNN_CUDA(cudaStreamBeginCapture(ctx->stream, cudaStreamCaptureModeRelaxed));
+  return SRCNN_OK;
+}
+
+// ends (and discards) an open capture on every early exit, so that a failed call never leaves
+// the context stream and the side streams capturing
+struct CaptureGuard {
+  cudaStream_t s;
+  bool active;
+  ~CaptureGuard() {
+    if (!active) return;
+    cudaGraph_t g = nullptr;
+    cudaStreamEndCapture(s, &g);
+    if (g) cudaGraphDestroy(g);
+    cudaGetLastError();
+  }
+};
+
+// joins the side streams back into the capturing stream, instantiates the graph into the slot
+// and launches it once; `rc` is the status of the captured issue
+int graph_end(srcnn_ctx* ctx, const GraphSlot& g, const unsigned long long* key,
+              const LaunchTally& tally, cudaStream_t main_stream, int rc, CaptureGuard& capture) {
+  cudaGraph_t graph = nullptr;
+  cudaError_t e = cudaEventRecord(ctx->ev_join[0], ctx->copy_out);
+  if (e == cudaSuccess) e = cudaStreamWaitEvent(main_stream, ctx->ev_join[0], 0);
+  if (e == cudaSuccess) e = cudaEventRecord(ctx->ev_join[1], ctx->compute2);
+  if (e == cudaSuccess) e = cudaStreamWaitEvent(main_stream, ctx->ev_join[1], 0);
+  const cudaError_t e2 = cudaStreamEndCapture(main_stream, &graph);
+  capture.active = false;
+  if (e == cudaSuccess) e = e2;
+  if (rc == SRCNN_OK && e == cudaSuccess) e = cudaGraphInstantiate(g.graph, graph, 0);
+  if (graph) cudaGraphDestroy(graph);
+  if (rc != SRCNN_OK) return rc;
+  if (e != cudaSuccess) {
+    *g.graph = nullptr;
+    return fail(SRCNN_ECUDA, "capturing the sub-band pipeline failed: %s", cudaGetErrorString(e));
+  }
+  std::memcpy(g.key, key, sizeof(unsigned long long) * srcnn_ctx::kGraphKey);
+  for (int i = 0; i < SRCNN_K_COUNT; i++)
+    g.launches[i] = (unsigned)(ctx->stats[i].launches - tally.per_id[i]);
+  SRCNN_CUDA(cudaGraphLaunch(*g.graph, main_stream));
+  return SRCNN_OK;
+}
+
 // lane < 0: the blocking call (context stream, returns when host_out is complete);
 // lane 0 / 1: srcnn_infer_rows_host_async (that lane's stream, staging and graph; no wait)
 int infer_rows_host_impl(srcnn_ctx* ctx, const srcnn_net* net, const float* host_in, int in_w,
@@ -758,9 +943,8 @@ int infer_rows_host_impl(srcnn_ctx* ctx, const srcnn_net* net, const float* host
   srcnn_ctx::RowsLane* ln = async ? &ctx->lanes[lane] : nullptr;
   void** st_in = async ? &ln->in : &ctx->band_in;
   void** st_out = async ? &ln->out : &ctx->band_out;
-  cudaGraphExec_t* st_graph = async ? &ln->graph : &ctx->e2e_graph;
-  unsigned long long* st_key = async ? ln->key : ctx->e2e_key;
-  unsigned* st_launches = async ? &ln->graph_launches : &ctx->e2e_graph_launches;
+  const GraphSlot slot = async ? GraphSlot{&ln->graph, ln->key, ln->graph_launches}
+                               : GraphSlot{&ctx->e2e_graph, ctx->e2e_key, ctx->e2e_graph_launches};
   if (!async) SRCNN_CUDA(ctx->drain_lanes());   // "returns when done" covers earlier async calls
   SRCNN_TRY(ensure_scratch(ctx, st_in, async ? &ln->in_bytes : &ctx->band_in_bytes, in_bytes));
   SRCNN_TRY(ensure_scratch(ctx, st_out, async ? &ln->out_bytes : &ctx->band_out_bytes, out_bytes));
@@ -781,36 +965,8 @@ int infer_rows_host_impl(srcnn_ctx* ctx, const srcnn_net* net, const float* host
   // last sub-band are small because their upload / download is exposed.  Every sub-band is the
   // same valid-convolution problem with a halo, so the result is bit-identical to a single
   // launch.
-  constexpr int kMaxSub = srcnn_ctx::kEvents;
-  // SRCNN_E2E_SUBBANDS=n (2..32) / SRCNN_E2E_RAMPCAP=c override the defaults for experiments.
-  // Measured on C3 (PCIe gen5 x16, 55 GB/s each way, 47.6 with both directions busy), wall
-  // clock of the call with the 0.9 ms kernel: 12 sub-bands 1.84-1.88 ms, 14: 1.78, 16: 1.73-1.78,
-  // 18: 1.78, 20 (cap 3): 1.79, 24: 1.83, 32: 1.96; ramp cap 3 / 5 / 6 at 16: 1.78 / 1.83 / 1.79.
-  static const int kSubDefault = std::getenv("SRCNN_E2E_SUBBANDS") ? std::atoi(std::getenv("SRCNN_E2E_SUBBANDS")) : 16;
-  // bands of a multi-GPU partition are pipelined too (an 8-way split of C3 leaves 511 rows per
-  // rank, and with 8 ranks copying at once each gets ~18 GB/s of the host's pinned-copy rate, so
-  // the copies dominate even more): about one sub-band per 64 output rows, at most the default
-  int n_sub = band_out_h >= 256
-                  ? std::min(std::min(std::max(kSubDefault, 2), kMaxSub), std::max(2, band_out_h / 64))
-                  : 1;
-  int sub_r0[kMaxSub + 1] = {0};
-  {
-    // shares ramp up from a small first sub-band and down to a small last one: 1,2,3,..,3,2,1
-    // capped at 2 units (round-2 sweep, profiles/r2g_e2e_subband_sweep.txt: cap 2 / 4 / 8 at 16
-    // sub-bands: 1.69 / 1.77 / 1.86 ms); the exposed head upload / tail download shrink with them
-    float unit[kMaxSub], total = 0.f;
-    for (int i = 0; i < n_sub; i++) {
-      static const int kRampCap = std::getenv("SRCNN_E2E_RAMPCAP") ? std::atoi(std::getenv("SRCNN_E2E_RAMPCAP")) : 2;
-      unit[i] = (float)std::min(std::min(i + 1, n_sub - i), std::max(kRampCap, 1));
-      total += unit[i];
-    }
-    float acc = 0.f;
-    for (int i = 0; i < n_sub; i++) {
-      acc += unit[i];
-      sub_r0[i + 1] = i + 1 == n_sub ? band_out_h : std::min((int)(acc / total * band_out_h + 0.5f), band_out_h);
-    }
-    if (n_sub == 1) sub_r0[1] = band_out_h;
-  }
+  int sub_r0[kMaxSub + 1];
+  const int n_sub = subband_rows(band_out_h, sub_r0);
   if (n_sub > 1) SRCNN_TRY(ensure_side_streams(ctx));
   float* din = (float*)*st_in;
   float* dout = (float*)*st_out;
@@ -854,13 +1010,8 @@ int infer_rows_host_impl(srcnn_ctx* ctx, const srcnn_net* net, const float* host
     if (!async) SRCNN_CUDA(cudaStreamSynchronize(ctx->stream));
     return SRCNN_OK;
   }
-  // The pipeline is ~10 runtime calls per sub-band; issued one by one the host only just stays
-  // ahead of the GPU (and falls behind when another thread competes for the CPU), so it is
-  // captured once into a CUDA graph and replayed with one launch while the arguments repeat
-  // (SRCNN_E2E_GRAPH=0 disables; profile mode times individual launches and never captures).
-  static const bool kGraphs = !(std::getenv("SRCNN_E2E_GRAPH") && std::atoi(std::getenv("SRCNN_E2E_GRAPH")) == 0);
-  const bool use_graph = kGraphs && !ctx->profile;
-  unsigned long long key[20] = {
+  const bool use_graph = graphs_enabled(ctx);
+  unsigned long long key[srcnn_ctx::kGraphKey] = {
       (unsigned long long)(uintptr_t)host_in, (unsigned long long)(uintptr_t)host_out,
       (unsigned long long)(uintptr_t)din, (unsigned long long)(uintptr_t)dout,
       (unsigned long long)in_w, (unsigned long long)in_h, (unsigned long long)out_row0,
@@ -871,51 +1022,14 @@ int infer_rows_host_impl(srcnn_ctx* ctx, const srcnn_net* net, const float* host
       (unsigned long long)(uintptr_t)scales, (unsigned long long)ctx->fused_impl,
       (unsigned long long)net->n1, (unsigned long long)net->n2,
       (unsigned long long)(uintptr_t)ctx->stream};
-  if (use_graph && *st_graph && std::memcmp(key, st_key, sizeof(key)) == 0) {
-    SRCNN_CUDA(cudaGraphLaunch(*st_graph, ctx->stream));
-    ctx->launch_count += *st_launches;
-    ctx->stats[SRCNN_K_FORWARD_FUSED].launches += *st_launches;
+  if (use_graph && graph_replay(ctx, slot, key)) {
+    SRCNN_CUDA(cudaGraphLaunch(*slot.graph, ctx->stream));
     if (!async) SRCNN_CUDA(cudaStreamSynchronize(ctx->stream));
     return SRCNN_OK;
   }
-  if (use_graph) {
-    if (*st_graph) {
-      SRCNN_CUDA(cudaStreamSynchronize(ctx->stream));   // the old graph may still be running
-      cudaGraphExecDestroy(*st_graph);
-      *st_graph = nullptr;
-    }
-    if (!ctx->ev_join[0])
-      for (int i = 0; i < 2; i++)
-        SRCNN_CUDA(cudaEventCreateWithFlags(&ctx->ev_join[i], cudaEventDisableTiming));
-    {   // everything the launches allocate lazily must exist before the capture starts
-      fused_hp::Scales* s_;
-      unsigned* w_;
-      SRCNN_TRY(fused_hp::scale_slot(ctx, &s_, &w_));
-    }
-    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-    if (cudaStreamIsCapturing(ctx->stream, &cap) == cudaSuccess && cap != cudaStreamCaptureStatusNone) {
-      cudaGraph_t stale = nullptr;   // a capture an earlier failed call left open
-      cudaStreamEndCapture(ctx->stream, &stale);
-      if (stale) cudaGraphDestroy(stale);
-      cudaGetLastError();
-    }
-    SRCNN_CUDA(cudaStreamSynchronize(ctx->stream));
-    SRCNN_CUDA(cudaStreamBeginCapture(ctx->stream, cudaStreamCaptureModeRelaxed));
-  }
-  // ends (and discards) the capture on every early exit below, so that a failed call never
-  // leaves the context stream and the side streams capturing
-  struct CaptureGuard {
-    cudaStream_t s;
-    bool active;
-    ~CaptureGuard() {
-      if (!active) return;
-      cudaGraph_t g = nullptr;
-      cudaStreamEndCapture(s, &g);
-      if (g) cudaGraphDestroy(g);
-      cudaGetLastError();
-    }
-  } capture{ctx->stream, use_graph};
-  const uint64_t launches_before = ctx->launch_count;
+  if (use_graph) SRCNN_TRY(graph_begin(ctx, slot));
+  CaptureGuard capture{ctx->stream, use_graph};
+  const LaunchTally tally(ctx);
   // order the side streams after whatever the context stream was doing with the buffers
   SRCNN_CUDA(cudaEventRecord(ctx->ev_k[0], ctx->stream));
   SRCNN_CUDA(cudaStreamWaitEvent(ctx->copy_in, ctx->ev_k[0], 0));
@@ -952,25 +1066,7 @@ int infer_rows_host_impl(srcnn_ctx* ctx, const srcnn_net* net, const float* host
                                ctx->copy_out));
   }
   if (use_graph) {
-    // join the side streams back into the capturing stream, instantiate, replay
-    cudaGraph_t graph = nullptr;
-    cudaError_t e = cudaEventRecord(ctx->ev_join[0], ctx->copy_out);
-    if (e == cudaSuccess) e = cudaStreamWaitEvent(main_stream, ctx->ev_join[0], 0);
-    if (e == cudaSuccess) e = cudaEventRecord(ctx->ev_join[1], ctx->compute2);
-    if (e == cudaSuccess) e = cudaStreamWaitEvent(main_stream, ctx->ev_join[1], 0);
-    const cudaError_t e2 = cudaStreamEndCapture(main_stream, &graph);
-    capture.active = false;
-    if (e == cudaSuccess) e = e2;
-    if (rc == SRCNN_OK && e == cudaSuccess) e = cudaGraphInstantiate(st_graph, graph, 0);
-    if (graph) cudaGraphDestroy(graph);
-    if (rc != SRCNN_OK) return rc;
-    if (e != cudaSuccess) {
-      *st_graph = nullptr;
-      return fail(SRCNN_ECUDA, "capturing the sub-band pipeline failed: %s", cudaGetErrorString(e));
-    }
-    std::memcpy(st_key, key, sizeof(key));
-    *st_launches = (unsigned)(ctx->launch_count - launches_before);
-    SRCNN_CUDA(cudaGraphLaunch(*st_graph, main_stream));
+    SRCNN_TRY(graph_end(ctx, slot, key, tally, main_stream, rc, capture));
     if (!async) SRCNN_CUDA(cudaStreamSynchronize(main_stream));
     return SRCNN_OK;
   }
@@ -995,6 +1091,187 @@ int srcnn_infer_rows_host_async(srcnn_ctx* ctx, const srcnn_net* net, const floa
   return infer_rows_host_impl(ctx, net, host_in, in_w, in_h, out_row0, out_row1, host_out, lane);
 }
 
+
+namespace {
+// wraps context-owned staging under a handle for the handle-based entries (dropped by TableScope)
+srcnn_mem stage_handle(srcnn_ctx* ctx, void* ptr, size_t bytes) {
+  Allocation a;
+  a.ptr = ptr;
+  a.bytes = bytes;
+  a.owned = false;
+  ctx->allocs.push_back(a);
+  return (srcnn_mem)(ctx->allocs.size() - 1);
+}
+}  // namespace
+
+int srcnn_upscale_image_host(srcnn_ctx* ctx, const srcnn_net* net, const unsigned char* host_rgba,
+                             int w, int h, int out_w, int out_h, int filter,
+                             unsigned char* host_rgb) {
+  SRCNN_REQUIRE(ctx && host_rgba && host_rgb, "null argument");
+  SRCNN_ENTER(ctx);
+  SRCNN_TRY(check_net(net));
+  SRCNN_TRY(check_resample(w, h, out_w, out_h, filter));
+  const int pad = net->f1 + net->f2 + net->f3 - 3;
+  SRCNN_REQUIRE(out_w > pad && out_h > pad, "output %dx%d too small for the network (padding %d)",
+                out_w, out_h, pad);
+  const Dims d = net_dims(net, out_w, out_h);
+  const size_t npx = (size_t)out_w * out_h;
+  SRCNN_CUDA(ctx->drain_lanes());
+  srcnn_ctx::UpscaleStaging& st = ctx->up;
+  SRCNN_TRY(ensure_scratch(ctx, &st.small, &st.small_bytes, (size_t)w * h * 4));
+  SRCNN_TRY(ensure_scratch(ctx, &st.rgba, &st.rgba_bytes, npx * 4));
+  SRCNN_TRY(ensure_scratch(ctx, &st.luma, &st.luma_bytes, npx * sizeof(float)));
+  SRCNN_TRY(ensure_scratch(ctx, &st.out, &st.out_bytes, sizeof(float) * (size_t)d.w3 * d.h3));
+  SRCNN_TRY(ensure_scratch(ctx, &st.rgb, &st.rgb_bytes, npx * 3));
+  const bool fused = fast::fused_supported(net->n1, net->n2, net->f1, net->f2, net->f3);
+  if (!fused) {
+    SRCNN_TRY(ensure_scratch(ctx, &st.s1, &st.s1_bytes, sizeof(float) * (size_t)d.w1 * d.h1 * net->n1));
+    SRCNN_TRY(ensure_scratch(ctx, &st.s2, &st.s2_bytes, sizeof(float) * (size_t)d.w2 * d.h2 * net->n2));
+  }
+  const int* tab;
+  int rows_max;
+  SRCNN_TRY(resample::table_for(ctx, w, h, out_w, out_h, filter, &tab, &rows_max));
+  const float *w1, *b1, *w2, *b2, *w3, *b3;
+  SRCNN_TRY(resolve(ctx, net->w[0], sizeof(float) * (size_t)net->f1 * net->f1 * net->n1, &w1, "w1"));
+  SRCNN_TRY(resolve(ctx, net->b[0], sizeof(float) * (size_t)net->n1, &b1, "b1"));
+  SRCNN_TRY(resolve(ctx, net->w[1], sizeof(float) * (size_t)net->f2 * net->f2 * net->n1 * net->n2, &w2, "w2"));
+  SRCNN_TRY(resolve(ctx, net->b[1], sizeof(float) * (size_t)net->n2, &b2, "b2"));
+  SRCNN_TRY(resolve(ctx, net->w[2], sizeof(float) * (size_t)net->f3 * net->f3 * net->n2, &w3, "w3"));
+  SRCNN_TRY(resolve(ctx, net->b[2], sizeof(float), &b3, "b3"));
+  uchar4* rgba = (uchar4*)st.rgba;
+  float* luma = (float*)st.luma;
+  float* out3 = (float*)st.out;
+  unsigned char* rgb = (unsigned char*)st.rgb;
+  // the head, which the forward cannot start before: upload, enlargement + luma, the Q1 "mean"
+  // (sum of squares / count, subtracted on the device: DataPipeline::subtract_mean)
+  auto head = [&]() -> int {
+    SRCNN_CUDA(cudaMemcpyAsync(st.small, host_rgba, (size_t)w * h * 4, cudaMemcpyHostToDevice,
+                               ctx->stream));
+    {
+      LaunchScope scope(ctx, SRCNN_K_RESAMPLE);
+      SRCNN_TRY(resample::launch(ctx, (const uchar4*)st.small, w, rgba, luma, out_w, out_h, filter,
+                                 tab, rows_max));
+      SRCNN_TRY(check_launch("resample"));
+    }
+    // the sum lands in the last word of the reduction scratch (the partials take at most
+    // RED_MAX_BLOCKS doubles at its start)
+    float* sum = (float*)ctx->red_scratch + srcnn_ctx::kRedScratchBytes / sizeof(float) - 1;
+    const int blocks = grid_1d(npx, generic::RED_THREADS, generic::RED_MAX_BLOCKS);
+    {
+      LaunchScope scope(ctx, SRCNN_K_SUM, 2);
+      generic::sum_stage1<<<blocks, generic::RED_THREADS, 0, ctx->stream>>>(
+          luma, (double*)ctx->red_scratch, (unsigned)npx, 1);
+      generic::reduce_stage2<<<1, generic::RED_THREADS, 0, ctx->stream>>>(
+          (const double*)ctx->red_scratch, blocks, sum);
+      SRCNN_TRY(check_launch("sum"));
+    }
+    LaunchScope scope(ctx, SRCNN_K_SUB_FROM_ALL);
+    generic::sub_mean_kernel<<<grid_1d(npx, 256, 8 * ctx->sm_count), 256, 0, ctx->stream>>>(
+        luma, sum, (unsigned)npx);
+    return check_launch("sub_from_all");
+  };
+  // swap_luma over image rows [y0, y1) of the result
+  auto swap_rows = [&](int y0, int y1) -> int {
+    LaunchScope scope(ctx, SRCNN_K_SWAP_LUMA);
+    dim3 block(32, 8), grid((out_w + 31) / 32, (y1 - y0 + 7) / 8);
+    generic::swap_luma_kernel<<<grid, block, 0, ctx->stream>>>(rgba, out3, rgb, out_w, y0, y1,
+                                                               d.w3, d.h3);
+    return check_launch("swap_luma");
+  };
+  if (!fused) {
+    // The whole image through the three-launch path: conv5_tc takes its FP16 operand scale from
+    // the measured maximum of its input, so a sub-band could get another scale (and result) than
+    // the whole image.
+    TableScope handles(ctx);
+    const srcnn_mem m_luma = stage_handle(ctx, st.luma, st.luma_bytes);
+    const srcnn_mem m_out = stage_handle(ctx, st.out, st.out_bytes);
+    const srcnn_mem m_s1 = stage_handle(ctx, st.s1, st.s1_bytes);
+    const srcnn_mem m_s2 = stage_handle(ctx, st.s2, st.s2_bytes);
+    SRCNN_TRY(head());
+    SRCNN_TRY(srcnn_forward_fused(ctx, net, m_luma, m_out, out_w, out_h, 1, m_s1, m_s2));
+    SRCNN_TRY(swap_rows(0, out_h));
+    SRCNN_CUDA(cudaMemcpyAsync(host_rgb, rgb, npx * 3, cudaMemcpyDeviceToHost, ctx->stream));
+    SRCNN_CUDA(cudaStreamSynchronize(ctx->stream));
+    return SRCNN_OK;
+  }
+  // The sub-band pipeline of srcnn_infer_rows_host over the network's output rows: the forward of
+  // each sub-band (alternating compute streams), then swap_luma over its image rows, then their
+  // download (copy-out stream) overlap with the next sub-bands.  The first sub-band also writes
+  // the top border rows, the last one the bottom border rows.
+  int sub_r0[kMaxSub + 1];
+  const int n_sub = subband_rows(d.h3, sub_r0);
+  SRCNN_TRY(ensure_side_streams(ctx));
+  const void* scales = nullptr;
+  SRCNN_TRY(net_prepare(ctx, net, w1, b1, w2, b2, w3, b3, &scales));
+  const bool use_graph = graphs_enabled(ctx);
+  const GraphSlot slot{&st.graph, st.key, st.graph_launches};
+  unsigned long long key[srcnn_ctx::kGraphKey] = {
+      (unsigned long long)(uintptr_t)host_rgba, (unsigned long long)(uintptr_t)host_rgb,
+      (unsigned long long)(uintptr_t)st.small, (unsigned long long)(uintptr_t)st.rgba,
+      (unsigned long long)(uintptr_t)st.luma, (unsigned long long)(uintptr_t)st.out,
+      (unsigned long long)(uintptr_t)st.rgb, (unsigned long long)(uintptr_t)tab,
+      (unsigned long long)w, (unsigned long long)h, (unsigned long long)out_w,
+      (unsigned long long)out_h, (unsigned long long)filter, (unsigned long long)n_sub,
+      (unsigned long long)(uintptr_t)w1, (unsigned long long)(uintptr_t)b1,
+      (unsigned long long)(uintptr_t)w2, (unsigned long long)(uintptr_t)b2,
+      (unsigned long long)(uintptr_t)w3, (unsigned long long)(uintptr_t)b3,
+      (unsigned long long)(uintptr_t)scales, (unsigned long long)ctx->fused_impl,
+      (unsigned long long)net->n1, (unsigned long long)net->n2, (unsigned long long)net->f1,
+      (unsigned long long)net->f2, (unsigned long long)net->f3,
+      (unsigned long long)(uintptr_t)ctx->stream};
+  if (use_graph && graph_replay(ctx, slot, key)) {
+    SRCNN_CUDA(cudaGraphLaunch(*slot.graph, ctx->stream));
+    SRCNN_CUDA(cudaStreamSynchronize(ctx->stream));
+    return SRCNN_OK;
+  }
+  if (use_graph) SRCNN_TRY(graph_begin(ctx, slot));
+  CaptureGuard capture{ctx->stream, use_graph};
+  const LaunchTally tally(ctx);
+  cudaStream_t main_stream = ctx->stream;
+  struct StreamRestore {
+    srcnn_ctx* c;
+    cudaStream_t s;
+    ~StreamRestore() { c->stream = s; }
+  } restore{ctx, main_stream};
+  int rc = head();
+  if (rc == SRCNN_OK) {
+    SRCNN_CUDA(cudaEventRecord(ctx->ev_k[0], main_stream));
+    SRCNN_CUDA(cudaStreamWaitEvent(ctx->copy_out, ctx->ev_k[0], 0));
+    SRCNN_CUDA(cudaStreamWaitEvent(ctx->compute2, ctx->ev_k[0], 0));
+  }
+  for (int i = 0; i < n_sub && rc == SRCNN_OK; i++) {
+    const int r0 = sub_r0[i], r1 = sub_r0[i + 1];   // network output rows
+    if (r1 <= r0) continue;
+    const int y0 = i == 0 ? 0 : pad / 2 + r0;       // image rows of this sub-band's result
+    const int y1 = i + 1 == n_sub ? out_h : pad / 2 + r1;
+    cudaStream_t cs = (i & 1) ? ctx->compute2 : main_stream;
+    ctx->stream = cs;   // the launch helpers (and the profile timers) use the context stream
+    {
+      LaunchScope scope(ctx, SRCNN_K_FORWARD_FUSED, fast::fused_launches(ctx, net->n1, net->n2, net->f1, net->f2, net->f3, scales != nullptr));
+      rc = fast::forward_fused(ctx, net->n1, net->n2, net->f1, net->f2, net->f3,
+                               luma + (size_t)r0 * out_w, out3 + (size_t)r0 * d.w3, w1, b1, w2,
+                               b2, w3, b3, out_w, r1 - r0 + pad, 1, scales);
+      if (rc == SRCNN_OK) rc = check_launch("forward_fused");
+    }
+    if (rc == SRCNN_OK) rc = swap_rows(y0, y1);
+    ctx->stream = main_stream;
+    if (rc != SRCNN_OK) break;
+    SRCNN_CUDA(cudaEventRecord(ctx->ev_k[i], cs));
+    SRCNN_CUDA(cudaStreamWaitEvent(ctx->copy_out, ctx->ev_k[i], 0));
+    SRCNN_CUDA(cudaMemcpyAsync(host_rgb + (size_t)y0 * out_w * 3, rgb + (size_t)y0 * out_w * 3,
+                               (size_t)(y1 - y0) * out_w * 3, cudaMemcpyDeviceToHost,
+                               ctx->copy_out));
+  }
+  if (use_graph) {
+    SRCNN_TRY(graph_end(ctx, slot, key, tally, main_stream, rc, capture));
+    SRCNN_CUDA(cudaStreamSynchronize(main_stream));
+    return SRCNN_OK;
+  }
+  SRCNN_CUDA(cudaStreamSynchronize(ctx->copy_out));
+  SRCNN_CUDA(cudaStreamSynchronize(ctx->compute2));
+  SRCNN_CUDA(cudaStreamSynchronize(main_stream));
+  return rc;
+}
 
 int srcnn_infer_frames_host(srcnn_ctx* ctx, const srcnn_net* net, const float* host_in, int w,
                             int h, int n_frames, float* host_out) {

@@ -513,4 +513,20 @@ void ConfigBasedDataPipeline::write_result_image(const char* const out_path,
   opencl::utils::write_image(out_path, res_img);
 }
 
+void ConfigBasedDataPipeline::upscale_image(LayerAllocationPool& l1, LayerAllocationPool& l2,
+                                            LayerAllocationPool& l3, opencl::utils::ImageData& in,
+                                            size_t out_w, size_t out_h, int filter,
+                                            opencl::utils::ImageData& out) {
+  if (in.bpp != 4 || out.bpp != 3 || (size_t)out.w != out_w || (size_t)out.h != out_h)
+    throw std::runtime_error("upscale_image: RGBA8 input and an RGB8 output of out_w x out_h expected");
+  check_initialized(DataPipeline::LOAD_KERNEL_LUMA | DataPipeline::LOAD_KERNEL_MISC);
+  const srcnn_net net = device_net(l1, l2, l3, false, false);
+  // `profile`: the per-kernel totals of the steps the call runs besides the forward
+  opencl::ProfiledLaunch p1(*resample_kernel()), p2(*_sum_squared_kernel),
+      p3(*_subtract_from_all_kernel), p4(*_swap_luma_kernel);
+  _context->check_status(srcnn_upscale_image_host(_context->c_ctx(), &net, in.data, in.w, in.h,
+                                                  (int)out_w, (int)out_h, filter, out.data),
+                         "upscale_image");
+}
+
 }  // namespace cnn_sr

@@ -51,6 +51,13 @@ class ConfigBasedDataPipeline : public DataPipeline {
                             LayerAllocationPool);
   void write_result_image(const char* const, opencl::utils::ImageData&, SampleAllocationPool&);
 
+  /** the forward mode for an image that must first be enlarged: `in` (RGBA8) is enlarged to
+   * out_w x out_h with `filter` (SRCNN_RESAMPLE_*), its luma goes through the three layers and is
+   * swapped back; `out` receives the RGB8 result (out_w * out_h * 3 bytes, owned by the caller) */
+  void upscale_image(LayerAllocationPool&, LayerAllocationPool&, LayerAllocationPool&,
+                     opencl::utils::ImageData& in, size_t out_w, size_t out_h, int filter,
+                     opencl::utils::ImageData& out);
+
   inline const Config* config() { return _config; }
   inline const LayerData* layer_1() { return &layer_data_1; }
   inline const LayerData* layer_2() { return &layer_data_2; }

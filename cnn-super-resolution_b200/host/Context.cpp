@@ -312,6 +312,7 @@ Kernel* Context::create_kernel(char const* file_path, char const* cmp_opt, char 
       {"sub_from_all", Kernel::Kind::SubFromAll, SRCNN_K_SUB_FROM_ALL},
       {"extract_luma", Kernel::Kind::ExtractLuma, SRCNN_K_EXTRACT_LUMA},
       {"swap_luma", Kernel::Kind::SwapLuma, SRCNN_K_SWAP_LUMA},
+      {"resample", Kernel::Kind::Resample, SRCNN_K_RESAMPLE},
   };
   const Entry* found = nullptr;
   for (const Entry& e : entries)

@@ -86,7 +86,7 @@ class Kernel {
  public:
   enum class Kind {
     Forward, SquaredErr, LastLayerDelta, Deltas, Backpropagate, UpdateParams, Sum, SubFromAll,
-    ExtractLuma, SwapLuma
+    ExtractLuma, SwapLuma, Resample
   };
   Kind kind() const { return _kind; }
   Context* get_context() const { return _context; }

@@ -12,6 +12,7 @@ namespace {
 const std::string kernel_folder = "src/kernel/";
 const char* const luma_kernel_file = "extract_luma.cl";
 const char* const swap_luma_kernel_file = "swap_luma.cl";
+const char* const resample_kernel_file = "resample.cu";   // (new: no reference kernel)
 const char* const squared_error_kernel_file = "squared_error.cl";
 const char* const sum_kernel_file = "sum.cl";
 const char* const layer_kernel_file = "layer_uber_kernel.cl";
@@ -131,6 +132,34 @@ cl_event DataPipeline::extract_luma(opencl::utils::ImageData& img, MemoryHandle&
                                             _context->mem(gpu_buf_luma), img.w, img.h,
                                             normalize ? 1 : 0),
                          "extract_luma");
+  return _context->ticket();
+}
+
+// created on first use, so that `profile` output lists it only for runs that enlarge
+opencl::Kernel* DataPipeline::resample_kernel() {
+  if (!_resample_kernel)
+    _resample_kernel = _context->create_kernel((kernel_folder + resample_kernel_file).c_str(),
+                                               nullptr, "resample");
+  return _resample_kernel;
+}
+
+cl_event DataPipeline::resample(opencl::utils::ImageData& img, MemoryHandle& gpu_buf_raw_img,
+                                size_t out_w, size_t out_h, int filter, MemoryHandle& gpu_buf_out,
+                                MemoryHandle& gpu_buf_luma) {
+  check_initialized(LOAD_KERNEL_LUMA);
+  const size_t px = (size_t)img.w * img.h, out_px = out_w * out_h;
+  if (!ALLOCATION_HAS_RIGHT_SIZE(gpu_buf_raw_img, px * 4))
+    gpu_buf_raw_img = _context->create_image(CL_MEM_READ_WRITE, CL_RGBA, CL_UNSIGNED_INT8, img.w, img.h);
+  _context->write_image(gpu_buf_raw_img, img, true);
+  if (!ALLOCATION_HAS_RIGHT_SIZE(gpu_buf_out, out_px * 4))
+    gpu_buf_out = _context->create_image(CL_MEM_READ_WRITE, CL_RGBA, CL_UNSIGNED_INT8, out_w, out_h);
+  if (!ALLOCATION_HAS_RIGHT_SIZE(gpu_buf_luma, sizeof(float) * out_px))
+    gpu_buf_luma = _context->allocate(CL_MEM_READ_WRITE, sizeof(float) * out_px);
+  ProfiledLaunch pl(*resample_kernel());
+  _context->check_status(srcnn_resample(_context->c_ctx(), _context->mem(gpu_buf_raw_img), img.w,
+                                        img.h, _context->mem(gpu_buf_out),
+                                        _context->mem(gpu_buf_luma), (int)out_w, (int)out_h, filter),
+                         "resample");
   return _context->ticket();
 }
 

@@ -43,6 +43,12 @@ class DataPipeline {
                         opencl::MemoryHandle& gpu_buf_luma, bool normalize,
                         cl_event* ev = nullptr);
 
+  /** uploads the RGBA image and enlarges it to out_w x out_h (Pillow-exact, `filter` =
+   * SRCNN_RESAMPLE_*) into the RGBA8 gpu_buf_out, with its normalized luma in gpu_buf_luma */
+  cl_event resample(opencl::utils::ImageData&, opencl::MemoryHandle& gpu_buf_raw_img,
+                    size_t out_w, size_t out_h, int filter, opencl::MemoryHandle& gpu_buf_out,
+                    opencl::MemoryHandle& gpu_buf_luma);
+
   /** new luma (x255) + chroma of the original image -> RGB8 in `target` */
   cl_event swap_luma(opencl::utils::ImageData&, opencl::MemoryHandle& gpu_buf_org_img,
                      opencl::MemoryHandle gpu_buf_new_luma, opencl::MemoryHandle& target,
@@ -114,6 +120,8 @@ class DataPipeline {
   opencl::Kernel* _luma_kernel_norm = nullptr;
   opencl::Kernel* _luma_kernel_raw = nullptr;
   opencl::Kernel* _swap_luma_kernel = nullptr;
+  opencl::Kernel* _resample_kernel = nullptr;   // see resample_kernel()
+  opencl::Kernel* resample_kernel();
   opencl::Kernel* _squared_error_kernel = nullptr;
   opencl::Kernel* _sum_kernel = nullptr;
   opencl::Kernel* _sum_squared_kernel = nullptr;

@@ -1,12 +1,18 @@
-// `cnn [train] [dry] [profile] --config CFG --in PATH [--out PATH] [--epochs N]`
+// `cnn [train] [dry] [profile] --config CFG --in PATH [--out PATH] [--epochs N]
+//      [--scale N [--resample lanczos|bicubic]]`
 // Same grammar, flow and console output as the reference CLI (src/Main_cl.cpp:40-318):
 // forward mode = one image through the three layers, luma swapped back into the image;
 // training mode = samples `*_large.*` (ground truth) / `*_small.*` (input) from a directory,
 // 80/20 train/validation split re-drawn every epoch, ONE parameter update per epoch.
+// --scale N (forward mode, N >= 2) first enlarges the input N times with Pillow's filter (Lanczos by
+// default, as the reference's sample generator did; bicubic is Pillow's and the SRCNN paper's
+// default), all on the device (srcnn_upscale_image_host); N = 1 is the plain forward mode.
 // Images are binary PPM/PGM (see Context.hpp); `_large.ppm/_small.ppm` as well as the
 // reference's `.jpg` suffix pattern are recognised by name.
 #include <algorithm>
+#include <cerrno>
 #include <cmath>
+#include <cstring>
 #include <cstdlib>
 #include <iostream>
 #include <random>
@@ -43,6 +49,32 @@ static void execute_forward(ConfigBasedDataPipeline& pipeline, GpuAllocationPool
   context->block();
   pipeline.forward(gpu_alloc.layer_1, gpu_alloc.layer_2, gpu_alloc.layer_3, sample);
   if (out_path) pipeline.write_result_image(out_path, input_img, sample);
+}
+
+static void execute_upscale(ConfigBasedDataPipeline& pipeline, GpuAllocationPool& gpu_alloc,
+                            const char* in_path, const char* out_path, size_t scale, int filter) {
+  ImageData input_img;
+  load_image(in_path, input_img);
+  const size_t out_w = scale * (size_t)input_img.w, out_h = scale * (size_t)input_img.h;
+  std::vector<unsigned char> result(out_w * out_h * 3);
+  ImageData res_img((int)out_w, (int)out_h, 3, result.data());
+  pipeline.upscale_image(gpu_alloc.layer_1, gpu_alloc.layer_2, gpu_alloc.layer_3, input_img, out_w,
+                         out_h, filter, res_img);
+  if (out_path) {
+    std::cout << "Saving result image to: '" << out_path << "'" << std::endl;
+    write_image(out_path, res_img);
+  }
+}
+
+// --scale: a whole number >= 1
+static bool parse_scale(const char* text, size_t* scale) {
+  if (!text) return true;
+  char* end = nullptr;
+  errno = 0;
+  const long v = std::strtol(text, &end, 10);
+  if (end == text || *end != '\0' || errno != 0 || v < 1 || v > 65535) return false;
+  *scale = (size_t)v;
+  return true;
 }
 
 static bool ends_with(const std::string& s, const std::string& suffix, size_t* stem_len) {
@@ -112,6 +144,8 @@ int main(int argc, char** argv) {
   argparse.add_argument("-i", "--in").required().help("Image during forward, samples directory during training");
   argparse.add_argument("-o", "--out").help("Output file path (either result image or new parameters)");
   argparse.add_argument("-e", "--epochs").help("Number of epochs during training");
+  argparse.add_argument("-s", "--scale").help("Forward mode: enlarge the image N times first (default 1)");
+  argparse.add_argument("-r", "--resample").help("Enlargement filter: lanczos (default) or bicubic");
   try {
     if (!argparse.parse((size_t)argc, argv)) return EXIT_SUCCESS;
   } catch (const std::exception& e) {
@@ -130,6 +164,24 @@ int main(int argc, char** argv) {
     std::cout << "Either provide out path or do the dry run" << std::endl;
     return EXIT_FAILURE;
   }
+  size_t scale = 1;
+  if (!parse_scale(argparse.value("scale"), &scale)) {
+    std::cout << "--scale must be a whole number >= 1, got '" << argparse.value("scale") << "'"
+              << std::endl;
+    return EXIT_FAILURE;
+  }
+  const char* resample_name = argparse.value("resample") ? argparse.value("resample") : "lanczos";
+  int filter = SRCNN_RESAMPLE_LANCZOS;
+  if (std::strcmp(resample_name, "bicubic") == 0) {
+    filter = SRCNN_RESAMPLE_BICUBIC;
+  } else if (std::strcmp(resample_name, "lanczos") != 0) {
+    std::cout << "--resample must be lanczos or bicubic, got '" << resample_name << "'" << std::endl;
+    return EXIT_FAILURE;
+  }
+  if (train && argparse.value("scale")) {
+    std::cout << "--scale applies to the forward mode only" << std::endl;
+    return EXIT_FAILURE;
+  }
   if (profile)
     std::cout << "!!!!!!!!!!!!!!!!!!!!!!!!!!!!!!!!!" << std::endl
               << "!!! RUNNING IN PROFILING MODE !!!" << std::endl
@@ -142,6 +194,8 @@ int main(int argc, char** argv) {
     std::cout << "Forward mode" << std::endl
               << "Input image: " << in_path << std::endl
               << "Output: " << (out_path ? out_path : "-") << std::endl;
+  if (!train && scale > 1)
+    std::cout << "Scale: " << scale << "x, resample: " << resample_name << std::endl;
 
   const size_t validation_set_percent = 20, mini_batch_count = 2;
   bool error = false;
@@ -157,7 +211,10 @@ int main(int argc, char** argv) {
     GpuAllocationPool gpu_alloc;
 
     if (!train) {
-      execute_forward(data_pipeline, gpu_alloc, in_path, out_path);
+      if (scale > 1)
+        execute_upscale(data_pipeline, gpu_alloc, in_path, out_path, scale, filter);
+      else
+        execute_forward(data_pipeline, gpu_alloc, in_path, out_path);
       context.block();
       return EXIT_SUCCESS;
     }

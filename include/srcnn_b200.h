@@ -60,6 +60,7 @@ enum srcnn_kernel_id {
   SRCNN_K_SWAP_LUMA,         /* swap_luma.cl          `swap_luma`          */
   SRCNN_K_FORWARD_FUSED,     /* (new) layers 1-3 in one launch, inference  */
   SRCNN_K_TRAIN_FUSED,       /* (new) fused pieces of the training step    */
+  SRCNN_K_RESAMPLE,          /* (new) Pillow-exact enlargement             */
   SRCNN_K_COUNT
 };
 
@@ -186,6 +187,17 @@ int srcnn_extract_luma(srcnn_ctx* ctx, srcnn_mem rgba, srcnn_mem target, int w, 
 int srcnn_swap_luma(srcnn_ctx* ctx, srcnn_mem rgba, srcnn_mem new_luma, srcnn_mem target,
                     int gt_w, int gt_h, int luma_w, int luma_h);
 
+/* Image enlargement, byte for byte Pillow's Image.fromarray(rgb, "RGB").resize((out_w, out_h),
+ * BICUBIC | LANCZOS) (libImaging/Resample.c): the step before the reference's forward flow
+ * (src/Main_cl.cpp:217-239), whose input is an already-enlarged image.  rgba_in = w*h*4 bytes
+ * RGBA8 (alpha ignored), rgba_out = out_w*out_h*4 bytes (alpha 255), luma_out = out_w*out_h
+ * floats: the luma of rgba_out exactly as srcnn_extract_luma(normalize = 1) computes it, or
+ * SRCNN_NULL_MEM for none.  Enlargements only (out_w >= w, out_h >= h); an axis whose size does
+ * not change is copied.  One launch. */
+enum { SRCNN_RESAMPLE_BICUBIC = 0, SRCNN_RESAMPLE_LANCZOS = 1 };
+int srcnn_resample(srcnn_ctx* ctx, srcnn_mem rgba_in, int w, int h, srcnn_mem rgba_out,
+                   srcnn_mem luma_out, int out_w, int out_h, int filter);
+
 /* ---------------------------------------------------------------- fused hot path --- */
 
 typedef struct srcnn_net {
@@ -229,6 +241,24 @@ int srcnn_infer_rows_host(srcnn_ctx* ctx, const srcnn_net* net, const float* hos
  * for the calls in flight; in profile mode (and with SRCNN_E2E_GRAPH=0) the call is blocking. */
 int srcnn_infer_rows_host_async(srcnn_ctx* ctx, const srcnn_net* net, const float* host_in,
                                 int in_w, int in_h, int out_row0, int out_row1, float* host_out);
+
+/* The `cnn` forward mode for an image that must first be enlarged, on HOST buffers: host_rgba
+ * (w*h*4 bytes RGBA8) is enlarged to out_w x out_h by srcnn_resample, and host_rgb receives
+ * out_w*out_h*3 bytes: exactly what the forward mode (src/Main_cl.cpp:217-239) returns for the
+ * enlarged image -- luma/255, minus the Q1 "mean" (the mean of the SQUARES, computed and
+ * subtracted on the device), the three layers, swap_luma.  Synchronous; pageable buffers work.
+ * Networks with a fused kernel run the sub-band pipeline of srcnn_infer_rows_host (forward,
+ * swap_luma and download of consecutive sub-bands overlap; captured into a CUDA graph and replayed
+ * while the arguments repeat); the others run the whole image through the three-launch path.
+ * Launches per call: 4 + n_sub * (F + 1) with a fused kernel (F = launches of one
+ * srcnn_forward_fused call with the packed operand image cached, n_sub = 1 below 256 network
+ * output rows, else min(max(S, 2), 32, max(2, h3 / 64)) with h3 = out_h - padding and S = 16 or
+ * SRCNN_E2E_SUBBANDS), 4 + L + 1 without (L = launches of srcnn_forward_fused on the three-launch path),
+ * plus 1 when the network's packed operand image has to be rebuilt (first call, new parameters).
+ * Out of range sizes, an output smaller than padding + 1 or an unknown filter: SRCNN_EINVAL. */
+int srcnn_upscale_image_host(srcnn_ctx* ctx, const srcnn_net* net, const unsigned char* host_rgba,
+                             int w, int h, int out_w, int out_h, int filter,
+                             unsigned char* host_rgb);
 
 /* ConfigBasedDataPipeline::forward(sample) for MANY frames (src/ConfigBasedDataPipeline.cpp:
  * 114-126 is called once per image by src/Main_cl.cpp:217-239): `n_frames` luma frames of
