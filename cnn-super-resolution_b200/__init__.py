@@ -102,6 +102,7 @@ _SIGS = {
     "srcnn_swap_luma": (_i, [_vp, _u64, _u64, _u64] + [_i] * 4),
     "srcnn_resample": (_i, [_vp, _u64, _i, _i, _u64, _u64, _i, _i, _i]),
     "srcnn_upscale_image_host": (_i, [_vp, C.POINTER(CNet), _vp, _i, _i, _i, _i, _i, _vp]),
+    "srcnn_upscale_frames_host": (_i, [_vp, C.POINTER(CNet), _vp, _i, _i, _i, _i, _i, _i, _vp]),
     "srcnn_forward_fused_supported": (_i, [C.POINTER(CNet)]),
     "srcnn_forward_fused": (_i, [_vp, C.POINTER(CNet), _u64, _u64, _i, _i, _i, _u64, _u64]),
     "srcnn_infer_rows_host": (_i, [_vp, C.POINTER(CNet), _vp, _i, _i, _i, _i, _vp]),
@@ -451,6 +452,21 @@ class Net:
         _check(self.ctx.L.srcnn_upscale_image_host(self.ctx.h, C.byref(self.c), _np_ptr(rgba),
                                                    rgba.shape[1], rgba.shape[0], out_w, out_h,
                                                    _filter_id(resample), _np_ptr(out)))
+        return out
+
+    def upscale_frames_host(self, rgba, out_w, out_h, resample="lanczos", out=None):
+        """rgba: uint8 [n][h][w][4] frames (alpha ignored) -> uint8 [n][out_h][out_w][3]: frame i
+        is what upscale_image_host returns for rgba[i]; upload, device work and download of
+        consecutive frame groups overlap.  `out` may be a preallocated (pinned) array."""
+        assert rgba.dtype == np.uint8 and rgba.ndim == 4 and rgba.shape[3] == 4
+        rgba = np.ascontiguousarray(rgba)
+        n = rgba.shape[0]
+        if out is None:
+            out = np.empty((n, out_h, out_w, 3), np.uint8)
+        assert out.dtype == np.uint8 and out.shape == (n, out_h, out_w, 3) and out.flags.c_contiguous
+        _check(self.ctx.L.srcnn_upscale_frames_host(self.ctx.h, C.byref(self.c), _np_ptr(rgba),
+                                                    rgba.shape[2], rgba.shape[1], n, out_w, out_h,
+                                                    _filter_id(resample), _np_ptr(out)))
         return out
 
     def infer_frames_host(self, host_in, w, h, host_out):

@@ -188,9 +188,24 @@ struct srcnn_ctx {
     unsigned long long key[kGraphKey] = {};
     unsigned graph_launches[SRCNN_K_COUNT] = {};
   } up;
+  // srcnn_upscale_frames_host: device staging (grown on demand), apart from `up` so that the two
+  // entries do not resize (and so re-capture) each other's buffers.  small / rgb hold a ring of
+  // frame groups, rgba / luma / out / red one group.
+  struct FramesStaging {
+    void* small = nullptr;   // input RGBA8
+    void* rgba = nullptr;    // enlarged RGBA8
+    void* luma = nullptr;    // enlarged luma, then minus its Q1 mean
+    void* out = nullptr;     // network output
+    void* rgb = nullptr;     // result RGB8
+    void* red = nullptr;     // Q1 reduction partials, then one sum per frame
+    void* s1 = nullptr;      // layer 1 / 2 activations of the three-launch route
+    void* s2 = nullptr;
+    size_t small_bytes = 0, rgba_bytes = 0, luma_bytes = 0, out_bytes = 0, rgb_bytes = 0,
+           red_bytes = 0, s1_bytes = 0, s2_bytes = 0;
+  } frames;
   static constexpr int kEvents = 32;
   cudaEvent_t ev_in[kEvents] = {}, ev_k[kEvents] = {};
-  cudaEvent_t ev_d[4] = {};   // download-finished events of srcnn_infer_frames_host's ring
+  cudaEvent_t ev_d[4] = {};   // download-finished events of the frame entries' rings
   // data-parallel communicator (NCCL, loaded at run time: comm.cuh); null = single GPU
   void* nccl_comm = nullptr;
   int comm_rank = 0, comm_world = 1;

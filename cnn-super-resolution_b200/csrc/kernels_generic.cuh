@@ -324,9 +324,11 @@ __global__ void sub_from_all_kernel(float* data, float value, unsigned len) {
 }
 
 // sub_from_all_kernel with value = *sum / (float)len read on the device (the mean never goes
-// through the host): the same float division and subtraction as the host route
+// through the host): the same float division and subtraction as the host route.  Frame
+// blockIdx.y: data + blockIdx.y * len, its own sum[blockIdx.y].
 __global__ void sub_mean_kernel(float* data, const float* __restrict__ sum, unsigned len) {
-  const float value = __fdiv_rn(*sum, (float)len);
+  data += blockIdx.y * (size_t)len;
+  const float value = __fdiv_rn(sum[blockIdx.y], (float)len);
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < len;
        i += (size_t)gridDim.x * blockDim.x)
     data[i] = data[i] - value;
@@ -361,7 +363,10 @@ __global__ void update_params_kernel(float* w, float* b, const float* __restrict
 // ------------------------------------------------------------------ reductions -------
 // Deterministic two-stage sums in double (the oracle's definition: double sum of float32
 // terms).  Stage 1: fixed grid, fixed per-thread element assignment, fixed-order tree;
-// stage 2: one block folds the partials in index order.
+// stage 2: one block folds the partials in index order.  Several equal-length arrays at once:
+// stage 1 takes array blockIdx.y (data + blockIdx.y * len, partials blockIdx.y * gridDim.x on),
+// stage 2 one block per array (partials blockIdx.x * count on, target[blockIdx.x]); each sum is
+// the one a single-array launch gives.
 constexpr int RED_THREADS = 256;
 constexpr int RED_MAX_BLOCKS = 1024;
 
@@ -406,6 +411,8 @@ __global__ void __launch_bounds__(RED_THREADS)
 sum_stage1(const float* __restrict__ data, double* __restrict__ partial, unsigned len,
            int squared) {
   __shared__ double sh[32];
+  data += blockIdx.y * (size_t)len;
+  partial += blockIdx.y * gridDim.x;
   double acc = 0.0;
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < len;
        i += (size_t)gridDim.x * blockDim.x) {
@@ -420,10 +427,11 @@ sum_stage1(const float* __restrict__ data, double* __restrict__ partial, unsigne
 __global__ void __launch_bounds__(RED_THREADS)
 reduce_stage2(const double* __restrict__ partial, int count, float* __restrict__ target) {
   __shared__ double sh[32];
+  partial += blockIdx.x * (size_t)count;
   double acc = 0.0;
   for (int i = threadIdx.x; i < count; i += blockDim.x) acc += partial[i];
   const double r = block_sum(acc, sh);
-  if (threadIdx.x == 0) *target = (float)r;
+  if (threadIdx.x == 0) target[blockIdx.x] = (float)r;
 }
 
 // batched sample gather: block (x, y) copies a slice of source y into slot y of dst
@@ -455,10 +463,14 @@ __global__ void extract_luma_kernel(const uchar4* __restrict__ rgba, float* __re
 }
 
 // reference: src/kernel/swap_luma.cl:18-69.  Image rows [row0, row1) (the whole image is
-// [0, gt_h)); the grid covers row1 - row0 rows.
+// [0, gt_h)); the grid covers row1 - row0 rows.  Frame blockIdx.z of a set of gt_w x gt_h
+// frames (rgba, target) and luma_w x luma_h results (luma), back to back.
 __global__ void swap_luma_kernel(const uchar4* __restrict__ rgba, const float* __restrict__ luma,
-                                 unsigned char* __restrict__ target, int gt_w, int row0, int row1,
-                                 int luma_w, int luma_h) {
+                                 unsigned char* __restrict__ target, int gt_w, int gt_h, int row0,
+                                 int row1, int luma_w, int luma_h) {
+  rgba += blockIdx.z * (size_t)gt_w * gt_h;
+  target += blockIdx.z * (size_t)gt_w * gt_h * 3;
+  luma += blockIdx.z * (size_t)luma_w * luma_h;
   const int x = blockIdx.x * blockDim.x + threadIdx.x;
   const int y = row0 + blockIdx.y * blockDim.y + threadIdx.y;
   if (x >= gt_w || y >= row1) return;

@@ -18,7 +18,8 @@
 // the input rows its vertical taps need into shared memory, then the vertical pass from there,
 // and writes the enlarged RGBA8 image (alpha 255) and, when asked, its normalized luma with the
 // arithmetic of extract_luma_kernel (generic::luma_of).  Alpha of the input is ignored: this is
-// Pillow's "RGB" path, not its premultiplying "RGBA" one.
+// Pillow's "RGB" path, not its premultiplying "RGBA" one.  A set of equal-sized frames is one
+// launch with the frame in blockIdx.z (frame f reads in + f * in_frame, writes out / luma + f * W * H).
 #pragma once
 #include <cmath>
 #include <cstring>
@@ -113,9 +114,12 @@ inline std::vector<int> tables(int w, int h, int W, int H, int filter, int* rows
 
 template <int TAPS>
 __global__ void __launch_bounds__(kThreads)
-resample_kernel(const uchar4* __restrict__ in, int w, uchar4* __restrict__ out,
+resample_kernel(const uchar4* __restrict__ in, int w, size_t in_frame, uchar4* __restrict__ out,
                 float* __restrict__ luma, int W, int H, const int* __restrict__ tab) {
   extern __shared__ uchar4 mid[];   // [rows][kTX] horizontal-pass result, 8-bit
+  in += blockIdx.z * in_frame;
+  out += blockIdx.z * (size_t)W * H;
+  if (luma) luma += blockIdx.z * (size_t)W * H;
   const int* xb = tab;
   const int* xn = xb + W;
   const int* xk = xn + W;
@@ -206,15 +210,17 @@ inline int table_for(srcnn_ctx* ctx, int w, int h, int W, int H, int filter, con
   return SRCNN_OK;
 }
 
-inline int launch(srcnn_ctx* ctx, const uchar4* in, int w, uchar4* out, float* luma, int W,
-                  int H, int filter, const int* tab, int rows_max) {
-  const dim3 grid((unsigned)((W + kTX - 1) / kTX), (unsigned)((H + kTY - 1) / kTY));
+// `frames` frames of w x h (in) -> W x H (out, luma), back to back
+inline int launch(srcnn_ctx* ctx, const uchar4* in, int w, int h, uchar4* out, float* luma, int W,
+                  int H, int filter, const int* tab, int rows_max, int frames = 1) {
+  const dim3 grid((unsigned)((W + kTX - 1) / kTX), (unsigned)((H + kTY - 1) / kTY), (unsigned)frames);
+  const size_t in_frame = (size_t)w * h;
   const size_t smem = (size_t)rows_max * kTX * sizeof(uchar4);
   // at most (kTY - 1) + 2 * 3 + 1 rows for an enlargement: well under the default 48 KB
   if (filter == SRCNN_RESAMPLE_LANCZOS)
-    resample_kernel<7><<<grid, kThreads, smem, ctx->stream>>>(in, w, out, luma, W, H, tab);
+    resample_kernel<7><<<grid, kThreads, smem, ctx->stream>>>(in, w, in_frame, out, luma, W, H, tab);
   else
-    resample_kernel<5><<<grid, kThreads, smem, ctx->stream>>>(in, w, out, luma, W, H, tab);
+    resample_kernel<5><<<grid, kThreads, smem, ctx->stream>>>(in, w, in_frame, out, luma, W, H, tab);
   return SRCNN_OK;
 }
 

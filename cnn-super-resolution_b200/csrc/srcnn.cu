@@ -141,6 +141,11 @@ int srcnn_ctx_destroy(srcnn_ctx* ctx) {
     for (void* p : {u.small, u.rgba, u.luma, u.out, u.rgb, u.s1, u.s2})
       if (p) cudaFree(p);
   }
+  {
+    srcnn_ctx::FramesStaging& f = ctx->frames;
+    for (void* p : {f.small, f.rgba, f.luma, f.out, f.rgb, f.red, f.s1, f.s2})
+      if (p) cudaFree(p);
+  }
   for (srcnn_ctx::ResampleTable& t : ctx->resample_tables) cudaFree(t.dev);
   if (ctx->nccl_comm && comm::api()) comm::api()->CommDestroy(ctx->nccl_comm);
   ctx->nccl_comm = nullptr;
@@ -640,8 +645,8 @@ int srcnn_swap_luma(srcnn_ctx* ctx, srcnn_mem rgba, srcnn_mem new_luma, srcnn_me
   ctx->note_write(target);
   LaunchScope scope(ctx, SRCNN_K_SWAP_LUMA);
   dim3 block(32, 8), grid((gt_w + 31) / 32, (gt_h + 7) / 8);
-  generic::swap_luma_kernel<<<grid, block, 0, ctx->stream>>>(pi, pl, pt, gt_w, 0, gt_h, luma_w,
-                                                             luma_h);
+  generic::swap_luma_kernel<<<grid, block, 0, ctx->stream>>>(pi, pl, pt, gt_w, gt_h, 0, gt_h,
+                                                             luma_w, luma_h);
   return check_launch("swap_luma");
 }
 
@@ -664,7 +669,7 @@ int srcnn_resample(srcnn_ctx* ctx, srcnn_mem rgba_in, int w, int h, srcnn_mem rg
   int rows_max;
   SRCNN_TRY(resample::table_for(ctx, w, h, out_w, out_h, filter, &tab, &rows_max));
   LaunchScope scope(ctx, SRCNN_K_RESAMPLE);
-  SRCNN_TRY(resample::launch(ctx, pi, w, po, pl, out_w, out_h, filter, tab, rows_max));
+  SRCNN_TRY(resample::launch(ctx, pi, w, h, po, pl, out_w, out_h, filter, tab, rows_max));
   return check_launch("resample");
 }
 
@@ -1102,6 +1107,91 @@ srcnn_mem stage_handle(srcnn_ctx* ctx, void* ptr, size_t bytes) {
   ctx->allocs.push_back(a);
   return (srcnn_mem)(ctx->allocs.size() - 1);
 }
+
+// the arguments srcnn_upscale_image_host and srcnn_upscale_frames_host accept
+int check_upscale(const srcnn_net* net, int w, int h, int out_w, int out_h, int filter) {
+  SRCNN_TRY(check_net(net));
+  SRCNN_TRY(check_resample(w, h, out_w, out_h, filter));
+  const int pad = net->f1 + net->f2 + net->f3 - 3;
+  SRCNN_REQUIRE(out_w > pad && out_h > pad, "output %dx%d too small for the network (padding %d)",
+                out_w, out_h, pad);
+  return SRCNN_OK;
+}
+
+// One enlargement job: `frames` equal frames back to back in each device buffer, enlarged from
+// w x h to out_w x out_h (network output d.w3 x d.h3).
+struct Upscale {
+  int w, h, out_w, out_h, filter, frames;
+  Dims d;
+  const int* tab;             // resample::table_for
+  int rows_max;
+  const uchar4* small;        // input RGBA8
+  uchar4* rgba;               // enlarged RGBA8
+  float* luma;                // enlarged luma, then minus its Q1 mean
+  float* out3;                // network output
+  unsigned char* rgb;         // result RGB8
+  double* partial;            // Q1 reduction partials: red_blocks() per frame
+  float* sums;                // Q1 sums, one per frame
+  size_t npx() const { return (size_t)out_w * out_h; }
+  int red_blocks() const { return grid_1d(npx(), generic::RED_THREADS, generic::RED_MAX_BLOCKS); }
+};
+
+// the device work the forward waits for: enlargement + luma, the Q1 "mean" of every frame (sum
+// of squares / count, subtracted on the device: DataPipeline::subtract_mean).  4 launches.  Each
+// frame's sum takes the block partition a single-frame sum takes, so its float is the same.
+int upscale_head(srcnn_ctx* ctx, const Upscale& u) {
+  const size_t npx = u.npx();
+  {
+    LaunchScope scope(ctx, SRCNN_K_RESAMPLE);
+    SRCNN_TRY(resample::launch(ctx, u.small, u.w, u.h, u.rgba, u.luma, u.out_w, u.out_h, u.filter,
+                               u.tab, u.rows_max, u.frames));
+    SRCNN_TRY(check_launch("resample"));
+  }
+  const int blocks = u.red_blocks();
+  {
+    LaunchScope scope(ctx, SRCNN_K_SUM, 2);
+    generic::sum_stage1<<<dim3(blocks, u.frames), generic::RED_THREADS, 0, ctx->stream>>>(
+        u.luma, u.partial, (unsigned)npx, 1);
+    generic::reduce_stage2<<<u.frames, generic::RED_THREADS, 0, ctx->stream>>>(u.partial, blocks,
+                                                                               u.sums);
+    SRCNN_TRY(check_launch("sum"));
+  }
+  LaunchScope scope(ctx, SRCNN_K_SUB_FROM_ALL);
+  generic::sub_mean_kernel<<<dim3(grid_1d(npx, 256, 8 * ctx->sm_count), u.frames), 256, 0,
+                             ctx->stream>>>(u.luma, u.sums, (unsigned)npx);
+  return check_launch("sub_from_all");
+}
+
+// swap_luma over image rows [y0, y1) of every frame.  1 launch.
+int upscale_swap(srcnn_ctx* ctx, const Upscale& u, int y0, int y1) {
+  LaunchScope scope(ctx, SRCNN_K_SWAP_LUMA);
+  dim3 block(32, 8), grid((u.out_w + 31) / 32, (y1 - y0 + 7) / 8, u.frames);
+  generic::swap_luma_kernel<<<grid, block, 0, ctx->stream>>>(u.rgba, u.out3, u.rgb, u.out_w,
+                                                             u.out_h, y0, y1, u.d.w3, u.d.h3);
+  return check_launch("swap_luma");
+}
+
+// One image (u.frames == 1) through the three-launch path, on the context stream, synchronous:
+// upload, head, forward, swap_luma, download.  conv5_tc takes its FP16 operand scale from the
+// measured maximum of its whole input, so a sub-band -- or a batch of frames -- could get another
+// scale (and result) than the image alone.
+int upscale_three_launch(srcnn_ctx* ctx, const srcnn_net* net, const Upscale& u, void* s1,
+                         void* s2, const unsigned char* host_rgba, unsigned char* host_rgb) {
+  const Dims& d = u.d;
+  TableScope handles(ctx);
+  const srcnn_mem m_luma = stage_handle(ctx, u.luma, sizeof(float) * u.npx());
+  const srcnn_mem m_out = stage_handle(ctx, u.out3, sizeof(float) * (size_t)d.w3 * d.h3);
+  const srcnn_mem m_s1 = stage_handle(ctx, s1, sizeof(float) * (size_t)d.w1 * d.h1 * net->n1);
+  const srcnn_mem m_s2 = stage_handle(ctx, s2, sizeof(float) * (size_t)d.w2 * d.h2 * net->n2);
+  SRCNN_CUDA(cudaMemcpyAsync((void*)u.small, host_rgba, (size_t)u.w * u.h * 4,
+                             cudaMemcpyHostToDevice, ctx->stream));
+  SRCNN_TRY(upscale_head(ctx, u));
+  SRCNN_TRY(srcnn_forward_fused(ctx, net, m_luma, m_out, u.out_w, u.out_h, 1, m_s1, m_s2));
+  SRCNN_TRY(upscale_swap(ctx, u, 0, u.out_h));
+  SRCNN_CUDA(cudaMemcpyAsync(host_rgb, u.rgb, u.npx() * 3, cudaMemcpyDeviceToHost, ctx->stream));
+  SRCNN_CUDA(cudaStreamSynchronize(ctx->stream));
+  return SRCNN_OK;
+}
 }  // namespace
 
 int srcnn_upscale_image_host(srcnn_ctx* ctx, const srcnn_net* net, const unsigned char* host_rgba,
@@ -1109,11 +1199,8 @@ int srcnn_upscale_image_host(srcnn_ctx* ctx, const srcnn_net* net, const unsigne
                              unsigned char* host_rgb) {
   SRCNN_REQUIRE(ctx && host_rgba && host_rgb, "null argument");
   SRCNN_ENTER(ctx);
-  SRCNN_TRY(check_net(net));
-  SRCNN_TRY(check_resample(w, h, out_w, out_h, filter));
+  SRCNN_TRY(check_upscale(net, w, h, out_w, out_h, filter));
   const int pad = net->f1 + net->f2 + net->f3 - 3;
-  SRCNN_REQUIRE(out_w > pad && out_h > pad, "output %dx%d too small for the network (padding %d)",
-                out_w, out_h, pad);
   const Dims d = net_dims(net, out_w, out_h);
   const size_t npx = (size_t)out_w * out_h;
   SRCNN_CUDA(ctx->drain_lanes());
@@ -1128,9 +1215,9 @@ int srcnn_upscale_image_host(srcnn_ctx* ctx, const srcnn_net* net, const unsigne
     SRCNN_TRY(ensure_scratch(ctx, &st.s1, &st.s1_bytes, sizeof(float) * (size_t)d.w1 * d.h1 * net->n1));
     SRCNN_TRY(ensure_scratch(ctx, &st.s2, &st.s2_bytes, sizeof(float) * (size_t)d.w2 * d.h2 * net->n2));
   }
-  const int* tab;
-  int rows_max;
-  SRCNN_TRY(resample::table_for(ctx, w, h, out_w, out_h, filter, &tab, &rows_max));
+  Upscale u{w, h, out_w, out_h, filter, 1, d, nullptr, 0};
+  SRCNN_TRY(resample::table_for(ctx, w, h, out_w, out_h, filter, &u.tab, &u.rows_max));
+  const int* tab = u.tab;
   const float *w1, *b1, *w2, *b2, *w3, *b3;
   SRCNN_TRY(resolve(ctx, net->w[0], sizeof(float) * (size_t)net->f1 * net->f1 * net->n1, &w1, "w1"));
   SRCNN_TRY(resolve(ctx, net->b[0], sizeof(float) * (size_t)net->n1, &b1, "b1"));
@@ -1138,62 +1225,19 @@ int srcnn_upscale_image_host(srcnn_ctx* ctx, const srcnn_net* net, const unsigne
   SRCNN_TRY(resolve(ctx, net->b[1], sizeof(float) * (size_t)net->n2, &b2, "b2"));
   SRCNN_TRY(resolve(ctx, net->w[2], sizeof(float) * (size_t)net->f3 * net->f3 * net->n2, &w3, "w3"));
   SRCNN_TRY(resolve(ctx, net->b[2], sizeof(float), &b3, "b3"));
-  uchar4* rgba = (uchar4*)st.rgba;
-  float* luma = (float*)st.luma;
-  float* out3 = (float*)st.out;
-  unsigned char* rgb = (unsigned char*)st.rgb;
-  // the head, which the forward cannot start before: upload, enlargement + luma, the Q1 "mean"
-  // (sum of squares / count, subtracted on the device: DataPipeline::subtract_mean)
-  auto head = [&]() -> int {
-    SRCNN_CUDA(cudaMemcpyAsync(st.small, host_rgba, (size_t)w * h * 4, cudaMemcpyHostToDevice,
-                               ctx->stream));
-    {
-      LaunchScope scope(ctx, SRCNN_K_RESAMPLE);
-      SRCNN_TRY(resample::launch(ctx, (const uchar4*)st.small, w, rgba, luma, out_w, out_h, filter,
-                                 tab, rows_max));
-      SRCNN_TRY(check_launch("resample"));
-    }
-    // the sum lands in the last word of the reduction scratch (the partials take at most
-    // RED_MAX_BLOCKS doubles at its start)
-    float* sum = (float*)ctx->red_scratch + srcnn_ctx::kRedScratchBytes / sizeof(float) - 1;
-    const int blocks = grid_1d(npx, generic::RED_THREADS, generic::RED_MAX_BLOCKS);
-    {
-      LaunchScope scope(ctx, SRCNN_K_SUM, 2);
-      generic::sum_stage1<<<blocks, generic::RED_THREADS, 0, ctx->stream>>>(
-          luma, (double*)ctx->red_scratch, (unsigned)npx, 1);
-      generic::reduce_stage2<<<1, generic::RED_THREADS, 0, ctx->stream>>>(
-          (const double*)ctx->red_scratch, blocks, sum);
-      SRCNN_TRY(check_launch("sum"));
-    }
-    LaunchScope scope(ctx, SRCNN_K_SUB_FROM_ALL);
-    generic::sub_mean_kernel<<<grid_1d(npx, 256, 8 * ctx->sm_count), 256, 0, ctx->stream>>>(
-        luma, sum, (unsigned)npx);
-    return check_launch("sub_from_all");
-  };
-  // swap_luma over image rows [y0, y1) of the result
-  auto swap_rows = [&](int y0, int y1) -> int {
-    LaunchScope scope(ctx, SRCNN_K_SWAP_LUMA);
-    dim3 block(32, 8), grid((out_w + 31) / 32, (y1 - y0 + 7) / 8);
-    generic::swap_luma_kernel<<<grid, block, 0, ctx->stream>>>(rgba, out3, rgb, out_w, y0, y1,
-                                                               d.w3, d.h3);
-    return check_launch("swap_luma");
-  };
-  if (!fused) {
-    // The whole image through the three-launch path: conv5_tc takes its FP16 operand scale from
-    // the measured maximum of its input, so a sub-band could get another scale (and result) than
-    // the whole image.
-    TableScope handles(ctx);
-    const srcnn_mem m_luma = stage_handle(ctx, st.luma, st.luma_bytes);
-    const srcnn_mem m_out = stage_handle(ctx, st.out, st.out_bytes);
-    const srcnn_mem m_s1 = stage_handle(ctx, st.s1, st.s1_bytes);
-    const srcnn_mem m_s2 = stage_handle(ctx, st.s2, st.s2_bytes);
-    SRCNN_TRY(head());
-    SRCNN_TRY(srcnn_forward_fused(ctx, net, m_luma, m_out, out_w, out_h, 1, m_s1, m_s2));
-    SRCNN_TRY(swap_rows(0, out_h));
-    SRCNN_CUDA(cudaMemcpyAsync(host_rgb, rgb, npx * 3, cudaMemcpyDeviceToHost, ctx->stream));
-    SRCNN_CUDA(cudaStreamSynchronize(ctx->stream));
-    return SRCNN_OK;
-  }
+  u.small = (const uchar4*)st.small;
+  u.rgba = (uchar4*)st.rgba;
+  u.luma = (float*)st.luma;
+  u.out3 = (float*)st.out;
+  u.rgb = (unsigned char*)st.rgb;
+  // the partials take at most RED_MAX_BLOCKS doubles at the start of the reduction scratch, the
+  // sum its last word
+  u.partial = (double*)ctx->red_scratch;
+  u.sums = (float*)ctx->red_scratch + srcnn_ctx::kRedScratchBytes / sizeof(float) - 1;
+  if (!fused) return upscale_three_launch(ctx, net, u, st.s1, st.s2, host_rgba, host_rgb);
+  float* luma = u.luma;
+  float* out3 = u.out3;
+  unsigned char* rgb = u.rgb;
   // The sub-band pipeline of srcnn_infer_rows_host over the network's output rows: the forward of
   // each sub-band (alternating compute streams), then swap_luma over its image rows, then their
   // download (copy-out stream) overlap with the next sub-bands.  The first sub-band also writes
@@ -1233,7 +1277,9 @@ int srcnn_upscale_image_host(srcnn_ctx* ctx, const srcnn_net* net, const unsigne
     cudaStream_t s;
     ~StreamRestore() { c->stream = s; }
   } restore{ctx, main_stream};
-  int rc = head();
+  SRCNN_CUDA(cudaMemcpyAsync(st.small, host_rgba, (size_t)w * h * 4, cudaMemcpyHostToDevice,
+                             ctx->stream));
+  int rc = upscale_head(ctx, u);
   if (rc == SRCNN_OK) {
     SRCNN_CUDA(cudaEventRecord(ctx->ev_k[0], main_stream));
     SRCNN_CUDA(cudaStreamWaitEvent(ctx->copy_out, ctx->ev_k[0], 0));
@@ -1253,7 +1299,7 @@ int srcnn_upscale_image_host(srcnn_ctx* ctx, const srcnn_net* net, const unsigne
                                b2, w3, b3, out_w, r1 - r0 + pad, 1, scales);
       if (rc == SRCNN_OK) rc = check_launch("forward_fused");
     }
-    if (rc == SRCNN_OK) rc = swap_rows(y0, y1);
+    if (rc == SRCNN_OK) rc = upscale_swap(ctx, u, y0, y1);
     ctx->stream = main_stream;
     if (rc != SRCNN_OK) break;
     SRCNN_CUDA(cudaEventRecord(ctx->ev_k[i], cs));
@@ -1271,6 +1317,114 @@ int srcnn_upscale_image_host(srcnn_ctx* ctx, const srcnn_net* net, const unsigne
   SRCNN_CUDA(cudaStreamSynchronize(ctx->compute2));
   SRCNN_CUDA(cudaStreamSynchronize(main_stream));
   return rc;
+}
+
+namespace {
+// the frame entries' ring of device slots: the upload of group g+1 and the download of group g-1
+// overlap the device work of group g
+constexpr int kFrameRing = 3;
+
+// frames per group: SRCNN_FRAMES_GROUP=n when set (read once per process), else as many as fit
+// `target_bytes` of device staging at `frame_bytes` each (at least 1); never more than n_frames
+int frames_group(size_t frame_bytes, size_t target_bytes, int n_frames) {
+  static const int kGroupEnv = std::getenv("SRCNN_FRAMES_GROUP") ? std::atoi(std::getenv("SRCNN_FRAMES_GROUP")) : 0;
+  const size_t g = kGroupEnv > 0 ? (size_t)kGroupEnv : std::max<size_t>(1, target_bytes / frame_bytes);
+  return (int)std::min<size_t>(g, (size_t)n_frames);
+}
+}  // namespace
+
+int srcnn_upscale_frames_host(srcnn_ctx* ctx, const srcnn_net* net, const unsigned char* host_rgba,
+                              int w, int h, int n_frames, int out_w, int out_h, int filter,
+                              unsigned char* host_rgb) {
+  SRCNN_REQUIRE(ctx && host_rgba && host_rgb, "null argument");
+  SRCNN_ENTER(ctx);
+  SRCNN_TRY(check_upscale(net, w, h, out_w, out_h, filter));
+  SRCNN_REQUIRE(n_frames > 0, "bad frame count %d", n_frames);
+  const Dims d = net_dims(net, out_w, out_h);
+  const size_t in_px = (size_t)w * h, npx = (size_t)out_w * out_h, out_px = (size_t)d.w3 * d.h3;
+  SRCNN_CUDA(ctx->drain_lanes());
+  const bool fused = fast::fused_supported(net->n1, net->n2, net->f1, net->f2, net->f3);
+  Upscale u{w, h, out_w, out_h, filter, 1, d, nullptr, 0};
+  const size_t red_frame = sizeof(double) * u.red_blocks() + sizeof(float);
+  // ~128 MB of device staging per group (input, enlarged RGBA8 + luma + RGB8, network output;
+  // 960x540 -> 1920x1080: 4 frames): launches long enough to fill the GPU, a first upload and a
+  // last download short next to a whole call
+  const size_t frame_bytes = in_px * 4 + npx * (4 + 4 + 3) + out_px * 4;
+  // (the frame is a grid dimension of the head and swap launches: at most 65535 a group)
+  const int group = fused ? std::min(frames_group(frame_bytes, (size_t)128 << 20, n_frames), 65535) : 1;
+  const int ring = fused ? kFrameRing : 1;
+  srcnn_ctx::FramesStaging& st = ctx->frames;
+  SRCNN_TRY(ensure_scratch(ctx, &st.small, &st.small_bytes, in_px * 4 * group * ring));
+  SRCNN_TRY(ensure_scratch(ctx, &st.rgba, &st.rgba_bytes, npx * 4 * group));
+  SRCNN_TRY(ensure_scratch(ctx, &st.luma, &st.luma_bytes, npx * sizeof(float) * group));
+  SRCNN_TRY(ensure_scratch(ctx, &st.out, &st.out_bytes, out_px * sizeof(float) * group));
+  SRCNN_TRY(ensure_scratch(ctx, &st.rgb, &st.rgb_bytes, npx * 3 * group * ring));
+  SRCNN_TRY(ensure_scratch(ctx, &st.red, &st.red_bytes, red_frame * group));
+  if (!fused) {
+    SRCNN_TRY(ensure_scratch(ctx, &st.s1, &st.s1_bytes, sizeof(float) * (size_t)d.w1 * d.h1 * net->n1));
+    SRCNN_TRY(ensure_scratch(ctx, &st.s2, &st.s2_bytes, sizeof(float) * (size_t)d.w2 * d.h2 * net->n2));
+  }
+  SRCNN_TRY(resample::table_for(ctx, w, h, out_w, out_h, filter, &u.tab, &u.rows_max));
+  const float *w1, *b1, *w2, *b2, *w3, *b3;
+  SRCNN_TRY(resolve(ctx, net->w[0], sizeof(float) * (size_t)net->f1 * net->f1 * net->n1, &w1, "w1"));
+  SRCNN_TRY(resolve(ctx, net->b[0], sizeof(float) * (size_t)net->n1, &b1, "b1"));
+  SRCNN_TRY(resolve(ctx, net->w[1], sizeof(float) * (size_t)net->f2 * net->f2 * net->n1 * net->n2, &w2, "w2"));
+  SRCNN_TRY(resolve(ctx, net->b[1], sizeof(float) * (size_t)net->n2, &b2, "b2"));
+  SRCNN_TRY(resolve(ctx, net->w[2], sizeof(float) * (size_t)net->f3 * net->f3 * net->n2, &w3, "w3"));
+  SRCNN_TRY(resolve(ctx, net->b[2], sizeof(float), &b3, "b3"));
+  u.rgba = (uchar4*)st.rgba;
+  u.luma = (float*)st.luma;
+  u.out3 = (float*)st.out;
+  u.partial = (double*)st.red;
+  u.sums = (float*)(u.partial + (size_t)u.red_blocks() * group);
+  uchar4* small = (uchar4*)st.small;
+  unsigned char* rgb = (unsigned char*)st.rgb;
+  if (!fused) {
+    // frame by frame, each as the image entry runs it
+    u.small = small;
+    u.rgb = rgb;
+    for (int f = 0; f < n_frames; f++)
+      SRCNN_TRY(upscale_three_launch(ctx, net, u, st.s1, st.s2, host_rgba + (size_t)f * in_px * 4,
+                                     host_rgb + (size_t)f * npx * 3));
+    return SRCNN_OK;
+  }
+  SRCNN_TRY(ensure_side_streams(ctx));
+  const void* scales = nullptr;
+  SRCNN_TRY(net_prepare(ctx, net, w1, b1, w2, b2, w3, b3, &scales));
+  // the side streams start behind whatever the context stream was doing with the staging
+  SRCNN_CUDA(cudaEventRecord(ctx->ev_k[kFrameRing], ctx->stream));
+  SRCNN_CUDA(cudaStreamWaitEvent(ctx->copy_in, ctx->ev_k[kFrameRing], 0));
+  SRCNN_CUDA(cudaStreamWaitEvent(ctx->copy_out, ctx->ev_k[kFrameRing], 0));
+  for (int g = 0, f0 = 0; f0 < n_frames; g++, f0 += group) {
+    const int S = std::min(group, n_frames - f0), r = g % kFrameRing;
+    u.frames = S;
+    u.small = small + (size_t)r * group * in_px;
+    u.rgb = rgb + (size_t)r * group * npx * 3;
+    // input slot r was last read by the device work of group g - kFrameRing
+    if (g >= kFrameRing) SRCNN_CUDA(cudaStreamWaitEvent(ctx->copy_in, ctx->ev_k[r], 0));
+    SRCNN_CUDA(cudaMemcpyAsync((void*)u.small, host_rgba + (size_t)f0 * in_px * 4, in_px * 4 * S,
+                               cudaMemcpyHostToDevice, ctx->copy_in));
+    SRCNN_CUDA(cudaEventRecord(ctx->ev_in[r], ctx->copy_in));
+    SRCNN_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->ev_in[r], 0));
+    // output slot r was last downloaded for group g - kFrameRing
+    if (g >= kFrameRing) SRCNN_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->ev_d[r], 0));
+    SRCNN_TRY(upscale_head(ctx, u));
+    {
+      LaunchScope scope(ctx, SRCNN_K_FORWARD_FUSED, fast::fused_launches(ctx, net->n1, net->n2, net->f1, net->f2, net->f3, scales != nullptr));
+      SRCNN_TRY(fast::forward_fused(ctx, net->n1, net->n2, net->f1, net->f2, net->f3, u.luma,
+                                    u.out3, w1, b1, w2, b2, w3, b3, out_w, out_h, S, scales));
+      SRCNN_TRY(check_launch("forward_fused"));
+    }
+    SRCNN_TRY(upscale_swap(ctx, u, 0, out_h));
+    SRCNN_CUDA(cudaEventRecord(ctx->ev_k[r], ctx->stream));
+    SRCNN_CUDA(cudaStreamWaitEvent(ctx->copy_out, ctx->ev_k[r], 0));
+    SRCNN_CUDA(cudaMemcpyAsync(host_rgb + (size_t)f0 * npx * 3, u.rgb, npx * 3 * S,
+                               cudaMemcpyDeviceToHost, ctx->copy_out));
+    SRCNN_CUDA(cudaEventRecord(ctx->ev_d[r], ctx->copy_out));
+  }
+  SRCNN_CUDA(cudaStreamSynchronize(ctx->copy_out));
+  SRCNN_CUDA(cudaStreamSynchronize(ctx->stream));
+  return SRCNN_OK;
 }
 
 int srcnn_infer_frames_host(srcnn_ctx* ctx, const srcnn_net* net, const float* host_in, int w,
@@ -1292,13 +1446,11 @@ int srcnn_infer_frames_host(srcnn_ctx* ctx, const srcnn_net* net, const float* h
   SRCNN_TRY(resolve(ctx, net->b[2], sizeof(float), &b3, "b3"));
   // groups of frames go through a ring of device slots: the upload of group g+1 and the download
   // of group g-1 overlap the fused forward of group g (one launch per group, frame = gridDim.z)
-  constexpr int kRing = 3;
-  static const int kGroupEnv = std::getenv("SRCNN_FRAMES_GROUP") ? std::atoi(std::getenv("SRCNN_FRAMES_GROUP")) : 0;
+  constexpr int kRing = kFrameRing;
   const size_t in_px = (size_t)w * h, out_px = (size_t)d.w3 * d.h3;
   // ~16 MB of input per group: long enough launches to fill the GPU, short enough that the
   // exposed first upload / last download stay small
-  int group = kGroupEnv > 0 ? kGroupEnv : (int)std::max<size_t>(1, ((size_t)16 << 20) / (in_px * sizeof(float)));
-  group = std::min(group, n_frames);
+  const int group = frames_group(in_px * sizeof(float), (size_t)16 << 20, n_frames);
   SRCNN_TRY(ensure_scratch(ctx, &ctx->band_in, &ctx->band_in_bytes, sizeof(float) * in_px * group * kRing));
   SRCNN_TRY(ensure_scratch(ctx, &ctx->band_out, &ctx->band_out_bytes, sizeof(float) * out_px * group * kRing));
   SRCNN_TRY(ensure_side_streams(ctx));

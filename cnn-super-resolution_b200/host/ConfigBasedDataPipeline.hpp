@@ -57,6 +57,11 @@ class ConfigBasedDataPipeline : public DataPipeline {
   void upscale_image(LayerAllocationPool&, LayerAllocationPool&, LayerAllocationPool&,
                      opencl::utils::ImageData& in, size_t out_w, size_t out_h, int filter,
                      opencl::utils::ImageData& out);
+  /** upscale_image for n_frames frames of w x h RGBA8, back to back in `in_rgba`; `out_rgb`
+   * receives n_frames results of out_w * out_h * 3 bytes (srcnn_upscale_frames_host) */
+  void upscale_frames(LayerAllocationPool&, LayerAllocationPool&, LayerAllocationPool&,
+                      const unsigned char* in_rgba, size_t w, size_t h, size_t n_frames,
+                      size_t out_w, size_t out_h, int filter, unsigned char* out_rgb);
 
   inline const Config* config() { return _config; }
   inline const LayerData* layer_1() { return &layer_data_1; }

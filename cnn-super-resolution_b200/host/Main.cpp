@@ -1,14 +1,20 @@
 // `cnn [train] [dry] [profile] --config CFG --in PATH [--out PATH] [--epochs N]
 //      [--scale N [--resample lanczos|bicubic]]`
 // Same grammar, flow and console output as the reference CLI (src/Main_cl.cpp:40-318):
-// forward mode = one image through the three layers, luma swapped back into the image;
+// forward mode = one image through the three layers, luma swapped back into the image (or every
+// image of a directory, see below);
 // training mode = samples `*_large.*` (ground truth) / `*_small.*` (input) from a directory,
 // 80/20 train/validation split re-drawn every epoch, ONE parameter update per epoch.
 // --scale N (forward mode, N >= 2) first enlarges the input N times with Pillow's filter (Lanczos by
 // default, as the reference's sample generator did; bicubic is Pillow's and the SRCNN paper's
 // default), all on the device (srcnn_upscale_image_host); N = 1 is the plain forward mode.
+// -i DIR (forward mode) runs every `.ppm` / `.pgm` file of DIR, in sorted name order, into
+// OUT_DIR/<stem>.ppm (-o OUT_DIR): consecutive files of equal size go through
+// srcnn_upscale_frames_host together, at most kDirBatch at a time; other files are skipped.
 // Images are binary PPM/PGM (see Context.hpp); `_large.ppm/_small.ppm` as well as the
 // reference's `.jpg` suffix pattern are recognised by name.
+#include <sys/stat.h>
+
 #include <algorithm>
 #include <cerrno>
 #include <cmath>
@@ -84,6 +90,76 @@ static bool ends_with(const std::string& s, const std::string& suffix, size_t* s
   return true;
 }
 
+static bool is_directory(const char* path) {
+  struct stat st;
+  return path && stat(path, &st) == 0 && S_ISDIR(st.st_mode);
+}
+
+// frames per srcnn_upscale_frames_host call in directory mode: bounds the host memory a batch
+// holds (its input RGBA8 and its result RGB8; 64 frames of 960x540 -> 1920x1080: 531 MB)
+static const size_t kDirBatch = 64;
+
+struct DirImage {
+  std::string path, stem;
+};
+
+// the `.ppm` / `.pgm` files of `dir`, in sorted name order; the others are skipped with a message
+static std::vector<DirImage> get_directory_images(const std::string& dir) {
+  std::vector<std::string> files;
+  cnn_sr::utils::list_files(dir.c_str(), files);
+  std::sort(files.begin(), files.end());
+  std::vector<DirImage> images;
+  for (const std::string& f : files) {
+    size_t stem = 0;
+    if (ends_with(f, ".ppm", &stem) || ends_with(f, ".pgm", &stem)) {
+      if (is_directory((dir + "/" + f).c_str()))
+        std::cout << "'" << f << "' is a directory. Skipping" << std::endl;
+      else
+        images.push_back({dir + "/" + f, f.substr(0, stem)});
+    } else if (f != "." && f != "..") {
+      std::cout << "'" << f << "' is not a .ppm/.pgm image. Skipping" << std::endl;
+    }
+  }
+  return images;
+}
+
+// every image of the directory through the frames entry, `scale` times enlarged (1: at its own
+// size); results go to out_dir/<stem>.ppm unless out_dir is null (dry run)
+static void execute_directory(ConfigBasedDataPipeline& pipeline, GpuAllocationPool& gpu_alloc,
+                              const std::vector<DirImage>& images, const char* out_dir,
+                              size_t scale, int filter) {
+  std::vector<unsigned char> in, out;
+  std::vector<const DirImage*> batch;
+  size_t w = 0, h = 0;
+  auto flush = [&]() {
+    if (batch.empty()) return;
+    const size_t out_w = scale * w, out_h = scale * h, out_bytes = out_w * out_h * 3;
+    out.resize(batch.size() * out_bytes);
+    pipeline.upscale_frames(gpu_alloc.layer_1, gpu_alloc.layer_2, gpu_alloc.layer_3, in.data(), w,
+                            h, batch.size(), out_w, out_h, filter, out.data());
+    for (size_t i = 0; i < batch.size() && out_dir; i++) {
+      const std::string path = std::string(out_dir) + "/" + batch[i]->stem + ".ppm";
+      std::cout << "Saving result image to: '" << path << "'" << std::endl;
+      ImageData res_img((int)out_w, (int)out_h, 3, out.data() + i * out_bytes);
+      if (!write_image(path.c_str(), res_img))
+        throw std::runtime_error("Could not write image: " + path);
+    }
+    batch.clear();
+    in.clear();
+  };
+  for (const DirImage& image : images) {
+    ImageData img;
+    load_image(image.path.c_str(), img);
+    if (!batch.empty() && ((size_t)img.w != w || (size_t)img.h != h || batch.size() == kDirBatch))
+      flush();
+    w = (size_t)img.w;
+    h = (size_t)img.h;
+    in.insert(in.end(), img.data, img.data + w * h * 4);
+    batch.push_back(&image);
+  }
+  flush();
+}
+
 static void get_training_samples(const std::string& dir, std::vector<TrainSampleFiles>& target) {
   std::vector<std::string> files;
   cnn_sr::utils::list_files(dir.c_str(), files);
@@ -141,7 +217,7 @@ int main(int argc, char** argv) {
   argparse.add_argument("dry").help("Do not store result");
   argparse.add_argument("profile").help("Print kernel execution times");
   argparse.add_argument("-c", "--config").required().help("CNN configuration");
-  argparse.add_argument("-i", "--in").required().help("Image during forward, samples directory during training");
+  argparse.add_argument("-i", "--in").required().help("Image (or directory of images) during forward, samples directory during training");
   argparse.add_argument("-o", "--out").help("Output file path (either result image or new parameters)");
   argparse.add_argument("-e", "--epochs").help("Number of epochs during training");
   argparse.add_argument("-s", "--scale").help("Forward mode: enlarge the image N times first (default 1)");
@@ -182,6 +258,12 @@ int main(int argc, char** argv) {
     std::cout << "--scale applies to the forward mode only" << std::endl;
     return EXIT_FAILURE;
   }
+  const bool in_dir = !train && is_directory(in_path);
+  if (in_dir && out_path && !is_directory(out_path)) {
+    std::cout << "Output directory '" << out_path << "' does not exist or is not a directory"
+              << std::endl;
+    return EXIT_FAILURE;
+  }
   if (profile)
     std::cout << "!!!!!!!!!!!!!!!!!!!!!!!!!!!!!!!!!" << std::endl
               << "!!! RUNNING IN PROFILING MODE !!!" << std::endl
@@ -192,7 +274,7 @@ int main(int argc, char** argv) {
               << "Output: " << (out_path ? out_path : "-") << std::endl;
   else
     std::cout << "Forward mode" << std::endl
-              << "Input image: " << in_path << std::endl
+              << (in_dir ? "Input directory: " : "Input image: ") << in_path << std::endl
               << "Output: " << (out_path ? out_path : "-") << std::endl;
   if (!train && scale > 1)
     std::cout << "Scale: " << scale << "x, resample: " << resample_name << std::endl;
@@ -210,6 +292,13 @@ int main(int argc, char** argv) {
     data_pipeline.init(DataPipeline::LOAD_KERNEL_ALL);
     GpuAllocationPool gpu_alloc;
 
+    if (in_dir) {
+      const std::vector<DirImage> images = get_directory_images(in_path);
+      if (images.empty()) throw std::runtime_error("No .ppm/.pgm images found");
+      execute_directory(data_pipeline, gpu_alloc, images, out_path, scale, filter);
+      context.block();
+      return EXIT_SUCCESS;
+    }
     if (!train) {
       if (scale > 1)
         execute_upscale(data_pipeline, gpu_alloc, in_path, out_path, scale, filter);

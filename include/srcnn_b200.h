@@ -260,6 +260,29 @@ int srcnn_upscale_image_host(srcnn_ctx* ctx, const srcnn_net* net, const unsigne
                              int w, int h, int out_w, int out_h, int filter,
                              unsigned char* host_rgb);
 
+/* srcnn_upscale_image_host for MANY equal-sized frames (a folder of photos, the frames of a
+ * video): host_rgba holds n_frames frames of w*h*4 bytes RGBA8, host_rgb receives n_frames frames
+ * of out_w*out_h*3 bytes RGB8.  Frame i of the result is byte for byte what
+ * srcnn_upscale_image_host returns for frame i alone.  Synchronous; pageable buffers work, pinned
+ * ones give the overlap.  Waits for srcnn_infer_rows_host_async calls in flight first.
+ * Networks with a fused kernel run groups of frames through a ring of device slots: the upload of
+ * group g+1 (copy-in stream) and the download of group g-1 (copy-out stream) overlap the device
+ * work of group g, which is one launch per step with every frame of the group in the grid:
+ * enlargement + luma, the Q1 sum (per frame, with the block partition of a single frame), minus
+ * the mean, the fused forward, swap_luma.  A group holds as many frames as fit ~128 MB of device
+ * staging (w*h*4 + out_w*out_h*11 + h3*w3*4 bytes a frame; 4 frames of 960x540 -> 1920x1080), or
+ * SRCNN_FRAMES_GROUP frames when that is set (at most 65535).  Networks without a fused kernel run
+ * frame by frame through the image entry's three-launch route: conv5_tc takes its operand scale
+ * from its whole input, so a batch of frames could change a frame's result.
+ * Launches per call: n_groups * (5 + F) with a fused kernel (n_groups = ceil(n_frames / group),
+ * F = launches of one srcnn_forward_fused call with the packed operand image cached),
+ * n_frames * (4 + L + 1) without (L as for srcnn_upscale_image_host), plus 1 when the network's
+ * packed operand image has to be rebuilt.  Everything srcnn_upscale_image_host rejects, n_frames
+ * <= 0 and null pointers: SRCNN_EINVAL before any host buffer is read or written. */
+int srcnn_upscale_frames_host(srcnn_ctx* ctx, const srcnn_net* net, const unsigned char* host_rgba,
+                              int w, int h, int n_frames, int out_w, int out_h, int filter,
+                              unsigned char* host_rgb);
+
 /* ConfigBasedDataPipeline::forward(sample) for MANY frames (src/ConfigBasedDataPipeline.cpp:
  * 114-126 is called once per image by src/Main_cl.cpp:217-239): `n_frames` luma frames of
  * w x h floats in host memory -> n_frames results of w3 x h3 floats in host_out.  Groups of
