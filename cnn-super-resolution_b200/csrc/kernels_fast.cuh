@@ -258,16 +258,23 @@ inline bool fused_supported(int n1, int n2, int f1, int f2, int f3) {
   return fused::supported(n1, n2, f1, f2, f3);
 }
 
+// a network with a fused forward: its shape, its six parameter buffers and the operand image
+// fused_prepare returned for them (null when the selected kernel needs none, or not prepared)
+struct FusedNet {
+  int n1, n2, f1, f2, f3;
+  const float *w1, *b1, *w2, *b2, *w3, *b3;
+  const void* scales;
+};
+
 // prepared operand image for forward_fused launches with these parameters (null when the
 // selected kernel needs none).  `cacheable`: the six buffers are context-owned allocations, so
 // nothing outside the device layer can have changed them since ctx->write_gen was recorded.
-inline int fused_prepare(srcnn_ctx* ctx, int n1, int n2, int f1, int f2, int f3, const float* w1,
-                         const float* b1, const float* w2, const float* b2, const float* w3,
-                         const float* b3, bool cacheable, const void** out) {
+inline int fused_prepare(srcnn_ctx* ctx, const FusedNet& net, bool cacheable, const void** out) {
   *out = nullptr;
+  const int n1 = net.n1, n2 = net.n2, f1 = net.f1, f2 = net.f2, f3 = net.f3;
   const bool wide = fused_hpw::supported(n1, n2, f1, f2, f3);
   if (ctx->fused_impl != 4 || !(wide || fused_hp::supported(n1, n2, f1, f2, f3))) return SRCNN_OK;
-  const void* key[6] = {w1, b1, w2, b2, w3, b3};
+  const void* key[6] = {net.w1, net.b1, net.w2, net.b2, net.w3, net.b3};
   if (cacheable && ctx->hp_cache_valid && ctx->hp_cache_gen == ctx->write_gen &&
       ctx->hp_cache_n1 == n1 && std::memcmp(key, ctx->hp_cache_key, sizeof(key)) == 0) {
     *out = ctx->hp_cache;
@@ -281,7 +288,7 @@ inline int fused_prepare(srcnn_ctx* ctx, int n1, int n2, int f1, int f2, int f3,
                                  ? sizeof(fused_hpw::Scales) : sizeof(fused_hp::Scales);
     SRCNN_CUDA(cudaMalloc(&ctx->hp_cache, bytes));
   }
-  fused::Args a{nullptr, nullptr, w1, b1, w2, b2, w3, b3, 0, 0, 0, 0};
+  fused::Args a{nullptr, nullptr, net.w1, net.b1, net.w2, net.b2, net.w3, net.b3, 0, 0, 0, 0};
   if (wide)
     fused_hpw::prepare(ctx, a, ctx->hp_cache);
   else
@@ -296,12 +303,10 @@ inline int fused_prepare(srcnn_ctx* ctx, int n1, int n2, int f1, int f2, int f3,
   return SRCNN_OK;
 }
 
-// `scales`: the operand image fused_prepare returned for these parameters, shared by a series of
-// launches (or null)
-inline int forward_fused(srcnn_ctx* ctx, int n1, int n2, int f1, int f2, int f3, const float* in,
-                         float* out, const float* w1, const float* b1, const float* w2,
-                         const float* b2, const float* w3, const float* b3, int in_w, int in_h,
-                         int S, const void* scales = nullptr) {
+// one fused forward of `net` (its `scales` shared by a series of launches, or null)
+inline int forward_fused(srcnn_ctx* ctx, const FusedNet& net, const float* in, float* out, int in_w,
+                         int in_h, int S) {
+  const int n1 = net.n1, n2 = net.n2, f1 = net.f1, f2 = net.f2, f3 = net.f3;
   if (!fused::supported(n1, n2, f1, f2, f3))
     return fail(SRCNN_EINVAL, "no fused forward instantiation");
   // the per-image launches put the sample index in gridDim.z (at most 65 535): larger sample
@@ -315,16 +320,17 @@ inline int forward_fused(srcnn_ctx* ctx, int n1, int n2, int f1, int f2, int f3,
     const int pad = f1 + f2 + f3 - 3;
     const size_t in_px = (size_t)in_w * in_h, out_px = (size_t)(in_w - pad) * (in_h - pad);
     for (int s0 = 0; s0 < S; s0 += kMaxZ)
-      SRCNN_TRY(forward_fused(ctx, n1, n2, f1, f2, f3, in + s0 * in_px, out + s0 * out_px, w1, b1,
-                              w2, b2, w3, b3, in_w, in_h, std::min(kMaxZ, S - s0), scales));
+      SRCNN_TRY(forward_fused(ctx, net, in + s0 * in_px, out + s0 * out_px, in_w, in_h,
+                              std::min(kMaxZ, S - s0)));
     return SRCNN_OK;
   }
-  fused::Args a{in, out, w1, b1, w2, b2, w3, b3, in_w, in_h, in_w - (f1 + f2 + f3 - 3),
-                in_h - (f1 + f2 + f3 - 3)};
+  fused::Args a{in, out, net.w1, net.b1, net.w2, net.b2, net.w3, net.b3, in_w, in_h,
+                in_w - (f1 + f2 + f3 - 3), in_h - (f1 + f2 + f3 - 3)};
+  const void* scales = net.scales;
   if (ctx->fused_impl == 4 && fused_hpw::supported(n1, n2, f1, f2, f3)) {
     // the wide network (n1 = 128, n2 = 64)
     const bool as_batch = S > 1 && in_w <= 512 && (long long)S * in_w < (1LL << 30);
-    if (!scales) SRCNN_TRY(fused_prepare(ctx, n1, n2, f1, f2, f3, w1, b1, w2, b2, w3, b3, false, &scales));
+    if (!scales) SRCNN_TRY(fused_prepare(ctx, net, false, &scales));
     fused_hp::Scales* unused;
     unsigned* ws;
     SRCNN_TRY(fused_hp::scale_slot(ctx, &unused, &ws));
@@ -344,13 +350,13 @@ inline int forward_fused(srcnn_ctx* ctx, int n1, int n2, int f1, int f2, int f3,
 }
 
 // kernels one fused forward call launches: the FP16-split path is prepare + main + gated TF32
-inline int fused_launches(srcnn_ctx* ctx, int n1, int n2, int f1, int f2, int f3,
-                          bool shared_scales = false) {
+inline int fused_launches(srcnn_ctx* ctx, const FusedNet& net) {
   if (ctx->fused_impl != 4) return 1;
   // FP16 kernel + gated fallback kernel, + the prepare kernel when the launch packs its own
   // operand image (fused_prepare counts the ones it launches itself)
-  if (fused_hp::supported(n1, n2, f1, f2, f3) || fused_hpw::supported(n1, n2, f1, f2, f3))
-    return shared_scales ? 2 : 3;
+  if (fused_hp::supported(net.n1, net.n2, net.f1, net.f2, net.f3) ||
+      fused_hpw::supported(net.n1, net.n2, net.f1, net.f2, net.f3))
+    return net.scales ? 2 : 3;
   return 1;
 }
 
@@ -360,19 +366,18 @@ inline bool fused_train_supported(srcnn_ctx* ctx, int n1, int n2, int f1, int f2
 
 // forward pass of a training chunk: all three layers in one launch, n1/n2-channel maps kept.
 // returns 1 when it launched, 0 when there is no instantiation for the shape
-inline int forward_train_fused(srcnn_ctx* ctx, int n1, int n2, int f1, int f2, int f3,
-                               const float* in, float* out1, float* out2, float* out3,
-                               const float* w1, const float* b1, const float* w2, const float* b2,
-                               const float* w3, const float* b3, int in_w, int in_h, int S,
-                               const void* scales = nullptr, unsigned* out2_max = nullptr) {
-  if (ctx->fused_impl < 3 || !fused_pl::supported(n1, n2, f1, f2, f3)) return 0;
+inline int forward_train_fused(srcnn_ctx* ctx, const FusedNet& net, const float* in, float* out1,
+                               float* out2, float* out3, int in_w, int in_h, int S,
+                               unsigned* out2_max) {
+  const int pad = net.f1 + net.f2 + net.f3 - 3;
+  if (ctx->fused_impl < 3 || !fused_pl::supported(net.n1, net.n2, net.f1, net.f2, net.f3)) return 0;
   if ((long long)S * in_w >= (1LL << 30)) return 0;
   if ((long long)S * in_w * in_h >= (1LL << 31)) return 0;   // 32-bit pixel indices of out1 / out2
-  fused::Args a{in, out3, w1, b1, w2, b2, w3, b3, in_w, in_h, in_w - (f1 + f2 + f3 - 3),
-                in_h - (f1 + f2 + f3 - 3)};
+  fused::Args a{in, out3, net.w1, net.b1, net.w2, net.b2, net.w3, net.b3, in_w, in_h, in_w - pad,
+                in_h - pad};
   const int rc = ctx->fused_impl == 4
                      ? fused_hp::launch(ctx, a, S, true, out1, out2,
-                                        static_cast<const fused_hp::Scales*>(scales), out2_max)
+                                        static_cast<const fused_hp::Scales*>(net.scales), out2_max)
                      : fused_pl::launch_batch(ctx, a, S, out1, out2, out2_max);
   return rc == SRCNN_OK ? 1 : rc;
 }

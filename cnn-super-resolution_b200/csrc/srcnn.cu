@@ -5,6 +5,7 @@
 
 
 #include <algorithm>
+#include <functional>
 #include <new>
 #include <vector>
 
@@ -59,6 +60,16 @@ inline int check_net(const srcnn_net* net) {
   SRCNN_REQUIRE(net->n1 > 0 && net->n2 > 0, "n1/n2 must be > 0");
   SRCNN_REQUIRE(net->f1 > 0 && net->f2 > 0 && net->f3 > 0, "f1/f2/f3 must be > 0");
   return SRCNN_OK;
+}
+
+// fills `key` with the call arguments (pointers and integers) a captured pipeline depends on
+inline unsigned long long key_word(const void* p) { return (unsigned long long)(uintptr_t)p; }
+inline unsigned long long key_word(long long v) { return (unsigned long long)v; }
+template <class... T>
+void graph_key(unsigned long long (&key)[srcnn_ctx::kGraphKey], T... args) {
+  static_assert(sizeof...(T) <= srcnn_ctx::kGraphKey, "graph key too long");
+  const unsigned long long words[] = {key_word(args)...};
+  std::copy(words, words + sizeof...(T), key);
 }
 
 }  // namespace
@@ -687,19 +698,42 @@ bool params_owned(srcnn_ctx* ctx, const srcnn_net* net) {
   return true;
 }
 
-// the prepared operand image of `net` for the fused kernels (from the context's cache while the
-// six parameter buffers are untouched, context-owned and never exposed; else packed afresh)
-int net_prepare(srcnn_ctx* ctx, const srcnn_net* net, const float* w1, const float* b1,
-                const float* w2, const float* b2, const float* w3, const float* b3,
-                const void** scales) {
-  SRCNN_TRY(fast::fused_prepare(ctx, net->n1, net->n2, net->f1, net->f2, net->f3, w1, b1, w2, b2, w3,
-                                b3, params_owned(ctx, net), scales));
+// `net` for the fused kernels: its six parameter buffers resolved and, when it has a fused
+// forward, their prepared operand image (from the context's cache while the six buffers are
+// untouched, context-owned and never exposed; else packed afresh)
+int fused_net(srcnn_ctx* ctx, const srcnn_net* net, fast::FusedNet* fn) {
+  *fn = fast::FusedNet{net->n1, net->n2, net->f1, net->f2, net->f3};
+  SRCNN_TRY(resolve(ctx, net->w[0], sizeof(float) * (size_t)net->f1 * net->f1 * net->n1, &fn->w1, "w1"));
+  SRCNN_TRY(resolve(ctx, net->b[0], sizeof(float) * (size_t)net->n1, &fn->b1, "b1"));
+  SRCNN_TRY(resolve(ctx, net->w[1], sizeof(float) * (size_t)net->f2 * net->f2 * net->n1 * net->n2, &fn->w2, "w2"));
+  SRCNN_TRY(resolve(ctx, net->b[1], sizeof(float) * (size_t)net->n2, &fn->b2, "b2"));
+  SRCNN_TRY(resolve(ctx, net->w[2], sizeof(float) * (size_t)net->f3 * net->f3 * net->n2, &fn->w3, "w3"));
+  SRCNN_TRY(resolve(ctx, net->b[2], sizeof(float), &fn->b3, "b3"));
+  if (!fast::fused_supported(net->n1, net->n2, net->f1, net->f2, net->f3)) return SRCNN_OK;
+  SRCNN_TRY(fast::fused_prepare(ctx, *fn, params_owned(ctx, net), &fn->scales));
   for (int l = 0; l < 3; l++) {
     ctx->hp_cache_h[2 * l] = net->w[l];
     ctx->hp_cache_h[2 * l + 1] = net->b[l];
   }
   return SRCNN_OK;
 }
+
+// one fused forward on the context stream
+int launch_fused(srcnn_ctx* ctx, const fast::FusedNet& fn, const float* in, float* out, int in_w,
+                 int in_h, int S) {
+  LaunchScope scope(ctx, SRCNN_K_FORWARD_FUSED, fast::fused_launches(ctx, fn));
+  SRCNN_TRY(fast::forward_fused(ctx, fn, in, out, in_w, in_h, S));
+  return check_launch("forward_fused");
+}
+
+// points the context stream (which the launch helpers and the profile timers use) at `s` for the
+// lifetime of the object
+struct StreamSwap {
+  srcnn_ctx* ctx;
+  cudaStream_t saved;
+  StreamSwap(srcnn_ctx* c, cudaStream_t s) : ctx(c), saved(c->stream) { c->stream = s; }
+  ~StreamSwap() { ctx->stream = saved; }
+};
 
 // the copy-in / copy-out / second compute stream and the events of the pipelined host-buffer
 // entries (created on first use)
@@ -758,23 +792,14 @@ int srcnn_forward_fused(srcnn_ctx* ctx, const srcnn_net* net, srcnn_mem in, srcn
   const Dims d = net_dims(net, in_w, in_h);
   SRCNN_REQUIRE(S > 0 && d.w3 > 0 && d.h3 > 0, "image %dx%d too small for the network", in_w, in_h);
   if (fast::fused_supported(net->n1, net->n2, net->f1, net->f2, net->f3)) {
-    const float *pin, *w1, *b1, *w2, *b2, *w3, *b3;
+    const float* pin;
     float* pout;
     SRCNN_TRY(resolve(ctx, in, sizeof(float) * (size_t)S * in_w * in_h, &pin, "input luma"));
     SRCNN_TRY(resolve(ctx, out, sizeof(float) * (size_t)S * d.w3 * d.h3, &pout, "output luma"));
-    SRCNN_TRY(resolve(ctx, net->w[0], sizeof(float) * (size_t)net->f1 * net->f1 * net->n1, &w1, "w1"));
-    SRCNN_TRY(resolve(ctx, net->b[0], sizeof(float) * (size_t)net->n1, &b1, "b1"));
-    SRCNN_TRY(resolve(ctx, net->w[1], sizeof(float) * (size_t)net->f2 * net->f2 * net->n1 * net->n2, &w2, "w2"));
-    SRCNN_TRY(resolve(ctx, net->b[1], sizeof(float) * (size_t)net->n2, &b2, "b2"));
-    SRCNN_TRY(resolve(ctx, net->w[2], sizeof(float) * (size_t)net->f3 * net->f3 * net->n2, &w3, "w3"));
-    SRCNN_TRY(resolve(ctx, net->b[2], sizeof(float), &b3, "b3"));
-    ctx->note_write(out);
-    const void* scales = nullptr;
-    SRCNN_TRY(net_prepare(ctx, net, w1, b1, w2, b2, w3, b3, &scales));
-    LaunchScope scope(ctx, SRCNN_K_FORWARD_FUSED, fast::fused_launches(ctx, net->n1, net->n2, net->f1, net->f2, net->f3, scales != nullptr));
-    SRCNN_TRY(fast::forward_fused(ctx, net->n1, net->n2, net->f1, net->f2, net->f3, pin, pout, w1,
-                                  b1, w2, b2, w3, b3, in_w, in_h, S, scales));
-    return check_launch("forward_fused");
+    ctx->note_write(out);   // before the operand image: `out` may be a parameter buffer
+    fast::FusedNet fn;
+    SRCNN_TRY(fused_net(ctx, net, &fn));
+    return launch_fused(ctx, fn, pin, pout, in_w, in_h, S);
   }
   SRCNN_REQUIRE(scratch1 != SRCNN_NULL_MEM && scratch2 != SRCNN_NULL_MEM,
                 "no fused kernel for %d-%d-%d n1=%d n2=%d and no scratch buffers for the "
@@ -842,25 +867,6 @@ struct GraphSlot {
   unsigned* launches;        // [SRCNN_K_COUNT]
 };
 
-// the launch counters when a capture started
-struct LaunchTally {
-  uint64_t per_id[SRCNN_K_COUNT];
-  explicit LaunchTally(const srcnn_ctx* ctx) {
-    for (int i = 0; i < SRCNN_K_COUNT; i++) per_id[i] = ctx->stats[i].launches;
-  }
-};
-
-// true when the slot holds a graph captured for `key`; counts its launches (the caller launches it)
-bool graph_replay(srcnn_ctx* ctx, const GraphSlot& g, const unsigned long long* key) {
-  if (!*g.graph || std::memcmp(key, g.key, sizeof(unsigned long long) * srcnn_ctx::kGraphKey) != 0)
-    return false;
-  for (int i = 0; i < SRCNN_K_COUNT; i++) {
-    ctx->launch_count += g.launches[i];
-    ctx->stats[i].launches += g.launches[i];
-  }
-  return true;
-}
-
 // drops the slot's old graph and starts capturing the context stream
 int graph_begin(srcnn_ctx* ctx, const GraphSlot& g) {
   if (*g.graph) {
@@ -902,10 +908,70 @@ struct CaptureGuard {
   }
 };
 
-// joins the side streams back into the capturing stream, instantiates the graph into the slot
-// and launches it once; `rc` is the status of the captured issue
-int graph_end(srcnn_ctx* ctx, const GraphSlot& g, const unsigned long long* key,
-              const LaunchTally& tally, cudaStream_t main_stream, int rc, CaptureGuard& capture) {
+// One call of a sub-band pipeline (srcnn_infer_rows_host, srcnn_upscale_image_host): `head`
+// (optional) on the context stream; then for every sub-band i of output rows
+// [sub_r0[i], sub_r0[i + 1]), `upload` (optional) on the copy-in stream, `work` on the context
+// stream or the second compute stream (alternately, so that the tail wave of one sub-band overlaps
+// the head of the next) and `download` on the copy-out stream.  Captured into `slot`'s graph and
+// replayed while `key` repeats.  `block`: return when the downloads are complete (the route
+// without graphs always does: its side streams and events are shared).
+int run_subbands(srcnn_ctx* ctx, const GraphSlot& slot, const unsigned long long* key,
+                 const int* sub_r0, int n_sub, bool block, const std::function<int()>& head,
+                 const std::function<cudaError_t(int i, int r0, int r1)>& upload,
+                 const std::function<int(int i, int r0, int r1)>& work,
+                 const std::function<cudaError_t(int i, int r0, int r1)>& download) {
+  SRCNN_TRY(ensure_side_streams(ctx));
+  const bool use_graph = graphs_enabled(ctx);
+  const size_t key_bytes = sizeof(unsigned long long) * srcnn_ctx::kGraphKey;
+  if (use_graph && *slot.graph && std::memcmp(key, slot.key, key_bytes) == 0) {
+    for (int i = 0; i < SRCNN_K_COUNT; i++) {
+      ctx->launch_count += slot.launches[i];
+      ctx->stats[i].launches += slot.launches[i];
+    }
+    SRCNN_CUDA(cudaGraphLaunch(*slot.graph, ctx->stream));
+    if (block) SRCNN_CUDA(cudaStreamSynchronize(ctx->stream));
+    return SRCNN_OK;
+  }
+  if (use_graph) SRCNN_TRY(graph_begin(ctx, slot));
+  CaptureGuard capture{ctx->stream, use_graph};
+  uint64_t before[SRCNN_K_COUNT];   // the launch counters when the capture started
+  for (int i = 0; i < SRCNN_K_COUNT; i++) before[i] = ctx->stats[i].launches;
+  cudaStream_t main_stream = ctx->stream;
+  int rc = head ? head() : SRCNN_OK;
+  if (rc == SRCNN_OK) {
+    // order the side streams after whatever the context stream was doing with the buffers (the
+    // copy-in stream only when it has work: the capture joins back the other two only)
+    SRCNN_CUDA(cudaEventRecord(ctx->ev_k[0], main_stream));
+    if (upload) SRCNN_CUDA(cudaStreamWaitEvent(ctx->copy_in, ctx->ev_k[0], 0));
+    SRCNN_CUDA(cudaStreamWaitEvent(ctx->copy_out, ctx->ev_k[0], 0));
+    SRCNN_CUDA(cudaStreamWaitEvent(ctx->compute2, ctx->ev_k[0], 0));
+  }
+  for (int i = 0; i < n_sub && rc == SRCNN_OK; i++) {
+    const int r0 = sub_r0[i], r1 = sub_r0[i + 1];
+    if (r1 <= r0) continue;
+    cudaStream_t cs = (i & 1) ? ctx->compute2 : main_stream;
+    if (upload) {
+      SRCNN_CUDA(upload(i, r0, r1));
+      SRCNN_CUDA(cudaEventRecord(ctx->ev_in[i], ctx->copy_in));
+      SRCNN_CUDA(cudaStreamWaitEvent(cs, ctx->ev_in[i], 0));
+    }
+    {
+      StreamSwap on(ctx, cs);
+      rc = work(i, r0, r1);
+    }
+    if (rc != SRCNN_OK) break;
+    SRCNN_CUDA(cudaEventRecord(ctx->ev_k[i], cs));
+    SRCNN_CUDA(cudaStreamWaitEvent(ctx->copy_out, ctx->ev_k[i], 0));
+    SRCNN_CUDA(download(i, r0, r1));
+  }
+  if (!use_graph) {
+    SRCNN_CUDA(cudaStreamSynchronize(ctx->copy_out));
+    SRCNN_CUDA(cudaStreamSynchronize(ctx->compute2));
+    SRCNN_CUDA(cudaStreamSynchronize(main_stream));
+    return rc;
+  }
+  // join the side streams back into the capturing stream, instantiate the graph into the slot
+  // and launch it once
   cudaGraph_t graph = nullptr;
   cudaError_t e = cudaEventRecord(ctx->ev_join[0], ctx->copy_out);
   if (e == cudaSuccess) e = cudaStreamWaitEvent(main_stream, ctx->ev_join[0], 0);
@@ -914,17 +980,18 @@ int graph_end(srcnn_ctx* ctx, const GraphSlot& g, const unsigned long long* key,
   const cudaError_t e2 = cudaStreamEndCapture(main_stream, &graph);
   capture.active = false;
   if (e == cudaSuccess) e = e2;
-  if (rc == SRCNN_OK && e == cudaSuccess) e = cudaGraphInstantiate(g.graph, graph, 0);
+  if (rc == SRCNN_OK && e == cudaSuccess) e = cudaGraphInstantiate(slot.graph, graph, 0);
   if (graph) cudaGraphDestroy(graph);
   if (rc != SRCNN_OK) return rc;
   if (e != cudaSuccess) {
-    *g.graph = nullptr;
+    *slot.graph = nullptr;
     return fail(SRCNN_ECUDA, "capturing the sub-band pipeline failed: %s", cudaGetErrorString(e));
   }
-  std::memcpy(g.key, key, sizeof(unsigned long long) * srcnn_ctx::kGraphKey);
+  std::memcpy(slot.key, key, key_bytes);
   for (int i = 0; i < SRCNN_K_COUNT; i++)
-    g.launches[i] = (unsigned)(ctx->stats[i].launches - tally.per_id[i]);
-  SRCNN_CUDA(cudaGraphLaunch(*g.graph, main_stream));
+    slot.launches[i] = (unsigned)(ctx->stats[i].launches - before[i]);
+  SRCNN_CUDA(cudaGraphLaunch(*slot.graph, main_stream));
+  if (block) SRCNN_CUDA(cudaStreamSynchronize(main_stream));
   return SRCNN_OK;
 }
 
@@ -953,40 +1020,24 @@ int infer_rows_host_impl(srcnn_ctx* ctx, const srcnn_net* net, const float* host
   if (!async) SRCNN_CUDA(ctx->drain_lanes());   // "returns when done" covers earlier async calls
   SRCNN_TRY(ensure_scratch(ctx, st_in, async ? &ln->in_bytes : &ctx->band_in_bytes, in_bytes));
   SRCNN_TRY(ensure_scratch(ctx, st_out, async ? &ln->out_bytes : &ctx->band_out_bytes, out_bytes));
-  const float *w1, *b1, *w2, *b2, *w3, *b3;
-  SRCNN_TRY(resolve(ctx, net->w[0], sizeof(float) * (size_t)net->f1 * net->f1 * net->n1, &w1, "w1"));
-  SRCNN_TRY(resolve(ctx, net->b[0], sizeof(float) * (size_t)net->n1, &b1, "b1"));
-  SRCNN_TRY(resolve(ctx, net->w[1], sizeof(float) * (size_t)net->f2 * net->f2 * net->n1 * net->n2, &w2, "w2"));
-  SRCNN_TRY(resolve(ctx, net->b[1], sizeof(float) * (size_t)net->n2, &b2, "b2"));
-  SRCNN_TRY(resolve(ctx, net->w[2], sizeof(float) * (size_t)net->f3 * net->f3 * net->n2, &w3, "w3"));
-  SRCNN_TRY(resolve(ctx, net->b[2], sizeof(float), &b3, "b3"));
+  // one set of operand scales for all sub-bands (computed on the context stream, before the
+  // event the side streams wait for)
+  fast::FusedNet fn;
+  SRCNN_TRY(fused_net(ctx, net, &fn));
   SRCNN_REQUIRE(fast::fused_supported(net->n1, net->n2, net->f1, net->f2, net->f3),
                 "srcnn_infer_rows_host needs a fused instantiation for %d-%d-%d n1=%d n2=%d",
                 net->f1, net->f2, net->f3, net->n1, net->n2);
-  // The band is cut into sub-bands; upload (copy-in stream), fused forward (two alternating
-  // compute streams, so the tail wave of one sub-band overlaps the head of the next) and
-  // download (copy-out stream) of consecutive sub-bands overlap, so a large image costs
-  // ~max(H2D, compute, D2H) + a short head and tail instead of their sum: the first and the
-  // last sub-band are small because their upload / download is exposed.  Every sub-band is the
-  // same valid-convolution problem with a halo, so the result is bit-identical to a single
-  // launch.
+  // The band is cut into sub-bands; upload, fused forward and download of consecutive sub-bands
+  // overlap, so a large image costs ~max(H2D, compute, D2H) + a short head and tail instead of
+  // their sum: the first and the last sub-band are small because their upload / download is
+  // exposed.  Every sub-band is the same valid-convolution problem with a halo, so the result is
+  // bit-identical to a single launch.
   int sub_r0[kMaxSub + 1];
   const int n_sub = subband_rows(band_out_h, sub_r0);
-  if (n_sub > 1) SRCNN_TRY(ensure_side_streams(ctx));
   float* din = (float*)*st_in;
   float* dout = (float*)*st_out;
-  // one set of operand scales for all sub-bands (computed on the context stream, before the
-  // event the side streams wait for)
-  const void* scales = nullptr;
-  SRCNN_TRY(net_prepare(ctx, net, w1, b1, w2, b2, w3, b3, &scales));
   // an asynchronous call runs on its lane's stream, behind whatever the context stream has
-  // queued so far (the operand image above, parameter updates); the launch helpers take the
-  // stream from the context, so it is swapped for the duration of the call
-  struct StreamSwap {
-    srcnn_ctx* c;
-    cudaStream_t real;
-    ~StreamSwap() { c->stream = real; }
-  } swap{ctx, ctx->stream};
+  // queued so far (the operand image above, parameter updates)
   if (async) {
     if (!ln->stream) SRCNN_CUDA(cudaStreamCreateWithFlags(&ln->stream, cudaStreamNonBlocking));
     if (!ctx->lane_ev) SRCNN_CUDA(cudaEventCreateWithFlags(&ctx->lane_ev, cudaEventDisableTiming));
@@ -995,92 +1046,42 @@ int infer_rows_host_impl(srcnn_ctx* ctx, const srcnn_net* net, const float* host
     // (Ordering the two calls stage by stage -- this call's uploads behind the other lane's last
     // upload, through an external event-record node in the graph -- was measured SLOWER than
     // letting them share the copy engines: 1.83 vs 1.67 ms per 4096x4096 image.)
-    ctx->stream = ln->stream;
     ctx->lanes_busy = true;
     for (int l = 0; l < 3; l++) {
       ln->params[2 * l] = net->w[l];
       ln->params[2 * l + 1] = net->b[l];
     }
   }
+  StreamSwap on_lane(ctx, async ? ln->stream : ctx->stream);
   if (n_sub == 1) {
     SRCNN_CUDA(cudaMemcpyAsync(din, host_in + (size_t)out_row0 * in_w, in_bytes,
                                cudaMemcpyHostToDevice, ctx->stream));
-    {
-      LaunchScope scope(ctx, SRCNN_K_FORWARD_FUSED, fast::fused_launches(ctx, net->n1, net->n2, net->f1, net->f2, net->f3, scales != nullptr));
-      SRCNN_TRY(fast::forward_fused(ctx, net->n1, net->n2, net->f1, net->f2, net->f3, din, dout,
-                                    w1, b1, w2, b2, w3, b3, in_w, band_in_h, 1, scales));
-      SRCNN_TRY(check_launch("forward_fused"));
-    }
+    SRCNN_TRY(launch_fused(ctx, fn, din, dout, in_w, band_in_h, 1));
     SRCNN_CUDA(cudaMemcpyAsync(host_out, dout, out_bytes, cudaMemcpyDeviceToHost, ctx->stream));
     if (!async) SRCNN_CUDA(cudaStreamSynchronize(ctx->stream));
     return SRCNN_OK;
   }
-  const bool use_graph = graphs_enabled(ctx);
-  unsigned long long key[srcnn_ctx::kGraphKey] = {
-      (unsigned long long)(uintptr_t)host_in, (unsigned long long)(uintptr_t)host_out,
-      (unsigned long long)(uintptr_t)din, (unsigned long long)(uintptr_t)dout,
-      (unsigned long long)in_w, (unsigned long long)in_h, (unsigned long long)out_row0,
-      (unsigned long long)out_row1, (unsigned long long)n_sub,
-      (unsigned long long)(uintptr_t)w1, (unsigned long long)(uintptr_t)b1,
-      (unsigned long long)(uintptr_t)w2, (unsigned long long)(uintptr_t)b2,
-      (unsigned long long)(uintptr_t)w3, (unsigned long long)(uintptr_t)b3,
-      (unsigned long long)(uintptr_t)scales, (unsigned long long)ctx->fused_impl,
-      (unsigned long long)net->n1, (unsigned long long)net->n2,
-      (unsigned long long)(uintptr_t)ctx->stream};
-  if (use_graph && graph_replay(ctx, slot, key)) {
-    SRCNN_CUDA(cudaGraphLaunch(*slot.graph, ctx->stream));
-    if (!async) SRCNN_CUDA(cudaStreamSynchronize(ctx->stream));
-    return SRCNN_OK;
-  }
-  if (use_graph) SRCNN_TRY(graph_begin(ctx, slot));
-  CaptureGuard capture{ctx->stream, use_graph};
-  const LaunchTally tally(ctx);
-  // order the side streams after whatever the context stream was doing with the buffers
-  SRCNN_CUDA(cudaEventRecord(ctx->ev_k[0], ctx->stream));
-  SRCNN_CUDA(cudaStreamWaitEvent(ctx->copy_in, ctx->ev_k[0], 0));
-  SRCNN_CUDA(cudaStreamWaitEvent(ctx->copy_out, ctx->ev_k[0], 0));
-  SRCNN_CUDA(cudaStreamWaitEvent(ctx->compute2, ctx->ev_k[0], 0));
-  cudaStream_t main_stream = ctx->stream;
-  int rc = SRCNN_OK;
-  for (int i = 0; i < n_sub && rc == SRCNN_OK; i++) {
-    const int r0 = sub_r0[i], r1 = sub_r0[i + 1];   // band-relative output rows
-    if (r1 <= r0) continue;
-    // input rows [r0 + (i ? halo : 0), r1 + halo): disjoint pieces that tile the band
-    const int in0 = r0 + (i ? halo : 0), in1 = r1 + halo;
-    SRCNN_CUDA(cudaMemcpyAsync(din + (size_t)in0 * in_w,
-                               host_in + ((size_t)out_row0 + in0) * in_w,
+  unsigned long long key[srcnn_ctx::kGraphKey] = {};
+  graph_key(key, host_in, host_out, din, dout, in_w, in_h, out_row0, out_row1, n_sub, fn.w1, fn.b1,
+            fn.w2, fn.b2, fn.w3, fn.b3, fn.scales, ctx->fused_impl, net->n1, net->n2, ctx->stream);
+  return run_subbands(
+      ctx, slot, key, sub_r0, n_sub, !async, nullptr,
+      [&](int i, int r0, int r1) {
+        // input rows [r0 + (i ? halo : 0), r1 + halo): disjoint pieces that tile the band
+        const int in0 = r0 + (i ? halo : 0), in1 = r1 + halo;
+        return cudaMemcpyAsync(din + (size_t)in0 * in_w, host_in + ((size_t)out_row0 + in0) * in_w,
                                sizeof(float) * (size_t)(in1 - in0) * in_w, cudaMemcpyHostToDevice,
-                               ctx->copy_in));
-    SRCNN_CUDA(cudaEventRecord(ctx->ev_in[i], ctx->copy_in));
-    cudaStream_t cs = (i & 1) ? ctx->compute2 : main_stream;
-    SRCNN_CUDA(cudaStreamWaitEvent(cs, ctx->ev_in[i], 0));
-    ctx->stream = cs;   // the launch helpers (and the profile timers) use the context stream
-    {
-      LaunchScope scope(ctx, SRCNN_K_FORWARD_FUSED, fast::fused_launches(ctx, net->n1, net->n2, net->f1, net->f2, net->f3, scales != nullptr));
-      rc = fast::forward_fused(ctx, net->n1, net->n2, net->f1, net->f2, net->f3,
-                               din + (size_t)r0 * in_w, dout + (size_t)r0 * d.w3, w1, b1, w2, b2,
-                               w3, b3, in_w, r1 - r0 + halo, 1, scales);
-      if (rc == SRCNN_OK) rc = check_launch("forward_fused");
-    }
-    ctx->stream = main_stream;
-    if (rc != SRCNN_OK) break;
-    SRCNN_CUDA(cudaEventRecord(ctx->ev_k[i], cs));
-    SRCNN_CUDA(cudaStreamWaitEvent(ctx->copy_out, ctx->ev_k[i], 0));
-    SRCNN_CUDA(cudaMemcpyAsync(host_out + (size_t)r0 * d.w3, dout + (size_t)r0 * d.w3,
+                               ctx->copy_in);
+      },
+      [&](int, int r0, int r1) {
+        return launch_fused(ctx, fn, din + (size_t)r0 * in_w, dout + (size_t)r0 * d.w3, in_w,
+                            r1 - r0 + halo, 1);
+      },
+      [&](int, int r0, int r1) {
+        return cudaMemcpyAsync(host_out + (size_t)r0 * d.w3, dout + (size_t)r0 * d.w3,
                                sizeof(float) * (size_t)(r1 - r0) * d.w3, cudaMemcpyDeviceToHost,
-                               ctx->copy_out));
-  }
-  if (use_graph) {
-    SRCNN_TRY(graph_end(ctx, slot, key, tally, main_stream, rc, capture));
-    if (!async) SRCNN_CUDA(cudaStreamSynchronize(main_stream));
-    return SRCNN_OK;
-  }
-  // issued call by call (profile mode, SRCNN_E2E_GRAPH=0): the side streams and their events are
-  // shared, so this route always completes before it returns
-  SRCNN_CUDA(cudaStreamSynchronize(ctx->copy_out));
-  SRCNN_CUDA(cudaStreamSynchronize(ctx->compute2));
-  SRCNN_CUDA(cudaStreamSynchronize(ctx->stream));
-  return rc;
+                               ctx->copy_out);
+      });
 }
 }  // namespace
 
@@ -1217,14 +1218,8 @@ int srcnn_upscale_image_host(srcnn_ctx* ctx, const srcnn_net* net, const unsigne
   }
   Upscale u{w, h, out_w, out_h, filter, 1, d, nullptr, 0};
   SRCNN_TRY(resample::table_for(ctx, w, h, out_w, out_h, filter, &u.tab, &u.rows_max));
-  const int* tab = u.tab;
-  const float *w1, *b1, *w2, *b2, *w3, *b3;
-  SRCNN_TRY(resolve(ctx, net->w[0], sizeof(float) * (size_t)net->f1 * net->f1 * net->n1, &w1, "w1"));
-  SRCNN_TRY(resolve(ctx, net->b[0], sizeof(float) * (size_t)net->n1, &b1, "b1"));
-  SRCNN_TRY(resolve(ctx, net->w[1], sizeof(float) * (size_t)net->f2 * net->f2 * net->n1 * net->n2, &w2, "w2"));
-  SRCNN_TRY(resolve(ctx, net->b[1], sizeof(float) * (size_t)net->n2, &b2, "b2"));
-  SRCNN_TRY(resolve(ctx, net->w[2], sizeof(float) * (size_t)net->f3 * net->f3 * net->n2, &w3, "w3"));
-  SRCNN_TRY(resolve(ctx, net->b[2], sizeof(float), &b3, "b3"));
+  fast::FusedNet fn;
+  SRCNN_TRY(fused_net(ctx, net, &fn));
   u.small = (const uchar4*)st.small;
   u.rgba = (uchar4*)st.rgba;
   u.luma = (float*)st.luma;
@@ -1235,88 +1230,40 @@ int srcnn_upscale_image_host(srcnn_ctx* ctx, const srcnn_net* net, const unsigne
   u.partial = (double*)ctx->red_scratch;
   u.sums = (float*)ctx->red_scratch + srcnn_ctx::kRedScratchBytes / sizeof(float) - 1;
   if (!fused) return upscale_three_launch(ctx, net, u, st.s1, st.s2, host_rgba, host_rgb);
-  float* luma = u.luma;
-  float* out3 = u.out3;
-  unsigned char* rgb = u.rgb;
-  // The sub-band pipeline of srcnn_infer_rows_host over the network's output rows: the forward of
-  // each sub-band (alternating compute streams), then swap_luma over its image rows, then their
-  // download (copy-out stream) overlap with the next sub-bands.  The first sub-band also writes
-  // the top border rows, the last one the bottom border rows.
+  // The sub-band pipeline of srcnn_infer_rows_host over the network's output rows, behind the
+  // upload and the head: the forward of each sub-band, then swap_luma over its image rows, then
+  // their download.  The first sub-band also writes the top border rows, the last one the bottom
+  // border rows.
   int sub_r0[kMaxSub + 1];
   const int n_sub = subband_rows(d.h3, sub_r0);
-  SRCNN_TRY(ensure_side_streams(ctx));
-  const void* scales = nullptr;
-  SRCNN_TRY(net_prepare(ctx, net, w1, b1, w2, b2, w3, b3, &scales));
-  const bool use_graph = graphs_enabled(ctx);
-  const GraphSlot slot{&st.graph, st.key, st.graph_launches};
-  unsigned long long key[srcnn_ctx::kGraphKey] = {
-      (unsigned long long)(uintptr_t)host_rgba, (unsigned long long)(uintptr_t)host_rgb,
-      (unsigned long long)(uintptr_t)st.small, (unsigned long long)(uintptr_t)st.rgba,
-      (unsigned long long)(uintptr_t)st.luma, (unsigned long long)(uintptr_t)st.out,
-      (unsigned long long)(uintptr_t)st.rgb, (unsigned long long)(uintptr_t)tab,
-      (unsigned long long)w, (unsigned long long)h, (unsigned long long)out_w,
-      (unsigned long long)out_h, (unsigned long long)filter, (unsigned long long)n_sub,
-      (unsigned long long)(uintptr_t)w1, (unsigned long long)(uintptr_t)b1,
-      (unsigned long long)(uintptr_t)w2, (unsigned long long)(uintptr_t)b2,
-      (unsigned long long)(uintptr_t)w3, (unsigned long long)(uintptr_t)b3,
-      (unsigned long long)(uintptr_t)scales, (unsigned long long)ctx->fused_impl,
-      (unsigned long long)net->n1, (unsigned long long)net->n2, (unsigned long long)net->f1,
-      (unsigned long long)net->f2, (unsigned long long)net->f3,
-      (unsigned long long)(uintptr_t)ctx->stream};
-  if (use_graph && graph_replay(ctx, slot, key)) {
-    SRCNN_CUDA(cudaGraphLaunch(*slot.graph, ctx->stream));
-    SRCNN_CUDA(cudaStreamSynchronize(ctx->stream));
-    return SRCNN_OK;
-  }
-  if (use_graph) SRCNN_TRY(graph_begin(ctx, slot));
-  CaptureGuard capture{ctx->stream, use_graph};
-  const LaunchTally tally(ctx);
-  cudaStream_t main_stream = ctx->stream;
-  struct StreamRestore {
-    srcnn_ctx* c;
-    cudaStream_t s;
-    ~StreamRestore() { c->stream = s; }
-  } restore{ctx, main_stream};
-  SRCNN_CUDA(cudaMemcpyAsync(st.small, host_rgba, (size_t)w * h * 4, cudaMemcpyHostToDevice,
-                             ctx->stream));
-  int rc = upscale_head(ctx, u);
-  if (rc == SRCNN_OK) {
-    SRCNN_CUDA(cudaEventRecord(ctx->ev_k[0], main_stream));
-    SRCNN_CUDA(cudaStreamWaitEvent(ctx->copy_out, ctx->ev_k[0], 0));
-    SRCNN_CUDA(cudaStreamWaitEvent(ctx->compute2, ctx->ev_k[0], 0));
-  }
-  for (int i = 0; i < n_sub && rc == SRCNN_OK; i++) {
-    const int r0 = sub_r0[i], r1 = sub_r0[i + 1];   // network output rows
-    if (r1 <= r0) continue;
-    const int y0 = i == 0 ? 0 : pad / 2 + r0;       // image rows of this sub-band's result
-    const int y1 = i + 1 == n_sub ? out_h : pad / 2 + r1;
-    cudaStream_t cs = (i & 1) ? ctx->compute2 : main_stream;
-    ctx->stream = cs;   // the launch helpers (and the profile timers) use the context stream
-    {
-      LaunchScope scope(ctx, SRCNN_K_FORWARD_FUSED, fast::fused_launches(ctx, net->n1, net->n2, net->f1, net->f2, net->f3, scales != nullptr));
-      rc = fast::forward_fused(ctx, net->n1, net->n2, net->f1, net->f2, net->f3,
-                               luma + (size_t)r0 * out_w, out3 + (size_t)r0 * d.w3, w1, b1, w2,
-                               b2, w3, b3, out_w, r1 - r0 + pad, 1, scales);
-      if (rc == SRCNN_OK) rc = check_launch("forward_fused");
-    }
-    if (rc == SRCNN_OK) rc = upscale_swap(ctx, u, y0, y1);
-    ctx->stream = main_stream;
-    if (rc != SRCNN_OK) break;
-    SRCNN_CUDA(cudaEventRecord(ctx->ev_k[i], cs));
-    SRCNN_CUDA(cudaStreamWaitEvent(ctx->copy_out, ctx->ev_k[i], 0));
-    SRCNN_CUDA(cudaMemcpyAsync(host_rgb + (size_t)y0 * out_w * 3, rgb + (size_t)y0 * out_w * 3,
-                               (size_t)(y1 - y0) * out_w * 3, cudaMemcpyDeviceToHost,
-                               ctx->copy_out));
-  }
-  if (use_graph) {
-    SRCNN_TRY(graph_end(ctx, slot, key, tally, main_stream, rc, capture));
-    SRCNN_CUDA(cudaStreamSynchronize(main_stream));
-    return SRCNN_OK;
-  }
-  SRCNN_CUDA(cudaStreamSynchronize(ctx->copy_out));
-  SRCNN_CUDA(cudaStreamSynchronize(ctx->compute2));
-  SRCNN_CUDA(cudaStreamSynchronize(main_stream));
-  return rc;
+  const auto image_rows = [&](int i, int r0, int r1) {
+    return std::make_pair(i == 0 ? 0 : pad / 2 + r0, i + 1 == n_sub ? out_h : pad / 2 + r1);
+  };
+  unsigned long long key[srcnn_ctx::kGraphKey] = {};
+  graph_key(key, host_rgba, host_rgb, st.small, st.rgba, st.luma, st.out, st.rgb, u.tab, w, h, out_w,
+            out_h, filter, n_sub, fn.w1, fn.b1, fn.w2, fn.b2, fn.w3, fn.b3, fn.scales, ctx->fused_impl,
+            net->n1, net->n2, net->f1, net->f2, net->f3, ctx->stream);
+  return run_subbands(
+      ctx, GraphSlot{&st.graph, st.key, st.graph_launches}, key, sub_r0, n_sub, true,
+      [&] {
+        SRCNN_CUDA(cudaMemcpyAsync(st.small, host_rgba, (size_t)w * h * 4, cudaMemcpyHostToDevice,
+                                   ctx->stream));
+        return upscale_head(ctx, u);
+      },
+      nullptr,
+      [&](int i, int r0, int r1) {
+        SRCNN_TRY(launch_fused(ctx, fn, u.luma + (size_t)r0 * out_w, u.out3 + (size_t)r0 * d.w3,
+                               out_w, r1 - r0 + pad, 1));
+        const auto y = image_rows(i, r0, r1);
+        return upscale_swap(ctx, u, y.first, y.second);
+      },
+      [&](int i, int r0, int r1) {
+        const auto y = image_rows(i, r0, r1);
+        return cudaMemcpyAsync(host_rgb + (size_t)y.first * out_w * 3,
+                               u.rgb + (size_t)y.first * out_w * 3,
+                               (size_t)(y.second - y.first) * out_w * 3, cudaMemcpyDeviceToHost,
+                               ctx->copy_out);
+      });
 }
 
 namespace {
@@ -1330,6 +1277,40 @@ int frames_group(size_t frame_bytes, size_t target_bytes, int n_frames) {
   static const int kGroupEnv = std::getenv("SRCNN_FRAMES_GROUP") ? std::atoi(std::getenv("SRCNN_FRAMES_GROUP")) : 0;
   const size_t g = kGroupEnv > 0 ? (size_t)kGroupEnv : std::max<size_t>(1, target_bytes / frame_bytes);
   return (int)std::min<size_t>(g, (size_t)n_frames);
+}
+
+// Runs n_frames frames in groups of `group` through the ring: the upload of a group's frames
+// (`in_frame` bytes each) from host_in into device slot r of dev_in (copy-in stream), then
+// work(S frames, r) on the context stream, then the download of the slot's results (`out_frame`
+// bytes each) from dev_out to host_out (copy-out stream).  Returns when the downloads are done.
+int run_frame_ring(srcnn_ctx* ctx, int n_frames, int group, const void* host_in, void* dev_in,
+                   size_t in_frame, void* host_out, const void* dev_out, size_t out_frame,
+                   const std::function<int(int S, int r)>& work) {
+  SRCNN_TRY(ensure_side_streams(ctx));
+  // the side streams start behind whatever the context stream was doing with the staging
+  SRCNN_CUDA(cudaEventRecord(ctx->ev_k[kFrameRing], ctx->stream));
+  SRCNN_CUDA(cudaStreamWaitEvent(ctx->copy_in, ctx->ev_k[kFrameRing], 0));
+  SRCNN_CUDA(cudaStreamWaitEvent(ctx->copy_out, ctx->ev_k[kFrameRing], 0));
+  for (int g = 0, f0 = 0; f0 < n_frames; g++, f0 += group) {
+    const int S = std::min(group, n_frames - f0), r = g % kFrameRing;
+    // input slot r was last read by the device work of group g - kFrameRing
+    if (g >= kFrameRing) SRCNN_CUDA(cudaStreamWaitEvent(ctx->copy_in, ctx->ev_k[r], 0));
+    SRCNN_CUDA(cudaMemcpyAsync((char*)dev_in + in_frame * group * r, (const char*)host_in + in_frame * f0,
+                               in_frame * S, cudaMemcpyHostToDevice, ctx->copy_in));
+    SRCNN_CUDA(cudaEventRecord(ctx->ev_in[r], ctx->copy_in));
+    SRCNN_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->ev_in[r], 0));
+    // output slot r was last downloaded for group g - kFrameRing
+    if (g >= kFrameRing) SRCNN_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->ev_d[r], 0));
+    SRCNN_TRY(work(S, r));
+    SRCNN_CUDA(cudaEventRecord(ctx->ev_k[r], ctx->stream));
+    SRCNN_CUDA(cudaStreamWaitEvent(ctx->copy_out, ctx->ev_k[r], 0));
+    SRCNN_CUDA(cudaMemcpyAsync((char*)host_out + out_frame * f0, (const char*)dev_out + out_frame * group * r,
+                               out_frame * S, cudaMemcpyDeviceToHost, ctx->copy_out));
+    SRCNN_CUDA(cudaEventRecord(ctx->ev_d[r], ctx->copy_out));
+  }
+  SRCNN_CUDA(cudaStreamSynchronize(ctx->copy_out));
+  SRCNN_CUDA(cudaStreamSynchronize(ctx->stream));
+  return SRCNN_OK;
 }
 }  // namespace
 
@@ -1365,13 +1346,8 @@ int srcnn_upscale_frames_host(srcnn_ctx* ctx, const srcnn_net* net, const unsign
     SRCNN_TRY(ensure_scratch(ctx, &st.s2, &st.s2_bytes, sizeof(float) * (size_t)d.w2 * d.h2 * net->n2));
   }
   SRCNN_TRY(resample::table_for(ctx, w, h, out_w, out_h, filter, &u.tab, &u.rows_max));
-  const float *w1, *b1, *w2, *b2, *w3, *b3;
-  SRCNN_TRY(resolve(ctx, net->w[0], sizeof(float) * (size_t)net->f1 * net->f1 * net->n1, &w1, "w1"));
-  SRCNN_TRY(resolve(ctx, net->b[0], sizeof(float) * (size_t)net->n1, &b1, "b1"));
-  SRCNN_TRY(resolve(ctx, net->w[1], sizeof(float) * (size_t)net->f2 * net->f2 * net->n1 * net->n2, &w2, "w2"));
-  SRCNN_TRY(resolve(ctx, net->b[1], sizeof(float) * (size_t)net->n2, &b2, "b2"));
-  SRCNN_TRY(resolve(ctx, net->w[2], sizeof(float) * (size_t)net->f3 * net->f3 * net->n2, &w3, "w3"));
-  SRCNN_TRY(resolve(ctx, net->b[2], sizeof(float), &b3, "b3"));
+  fast::FusedNet fn;
+  SRCNN_TRY(fused_net(ctx, net, &fn));
   u.rgba = (uchar4*)st.rgba;
   u.luma = (float*)st.luma;
   u.out3 = (float*)st.out;
@@ -1388,43 +1364,15 @@ int srcnn_upscale_frames_host(srcnn_ctx* ctx, const srcnn_net* net, const unsign
                                      host_rgb + (size_t)f * npx * 3));
     return SRCNN_OK;
   }
-  SRCNN_TRY(ensure_side_streams(ctx));
-  const void* scales = nullptr;
-  SRCNN_TRY(net_prepare(ctx, net, w1, b1, w2, b2, w3, b3, &scales));
-  // the side streams start behind whatever the context stream was doing with the staging
-  SRCNN_CUDA(cudaEventRecord(ctx->ev_k[kFrameRing], ctx->stream));
-  SRCNN_CUDA(cudaStreamWaitEvent(ctx->copy_in, ctx->ev_k[kFrameRing], 0));
-  SRCNN_CUDA(cudaStreamWaitEvent(ctx->copy_out, ctx->ev_k[kFrameRing], 0));
-  for (int g = 0, f0 = 0; f0 < n_frames; g++, f0 += group) {
-    const int S = std::min(group, n_frames - f0), r = g % kFrameRing;
-    u.frames = S;
-    u.small = small + (size_t)r * group * in_px;
-    u.rgb = rgb + (size_t)r * group * npx * 3;
-    // input slot r was last read by the device work of group g - kFrameRing
-    if (g >= kFrameRing) SRCNN_CUDA(cudaStreamWaitEvent(ctx->copy_in, ctx->ev_k[r], 0));
-    SRCNN_CUDA(cudaMemcpyAsync((void*)u.small, host_rgba + (size_t)f0 * in_px * 4, in_px * 4 * S,
-                               cudaMemcpyHostToDevice, ctx->copy_in));
-    SRCNN_CUDA(cudaEventRecord(ctx->ev_in[r], ctx->copy_in));
-    SRCNN_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->ev_in[r], 0));
-    // output slot r was last downloaded for group g - kFrameRing
-    if (g >= kFrameRing) SRCNN_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->ev_d[r], 0));
-    SRCNN_TRY(upscale_head(ctx, u));
-    {
-      LaunchScope scope(ctx, SRCNN_K_FORWARD_FUSED, fast::fused_launches(ctx, net->n1, net->n2, net->f1, net->f2, net->f3, scales != nullptr));
-      SRCNN_TRY(fast::forward_fused(ctx, net->n1, net->n2, net->f1, net->f2, net->f3, u.luma,
-                                    u.out3, w1, b1, w2, b2, w3, b3, out_w, out_h, S, scales));
-      SRCNN_TRY(check_launch("forward_fused"));
-    }
-    SRCNN_TRY(upscale_swap(ctx, u, 0, out_h));
-    SRCNN_CUDA(cudaEventRecord(ctx->ev_k[r], ctx->stream));
-    SRCNN_CUDA(cudaStreamWaitEvent(ctx->copy_out, ctx->ev_k[r], 0));
-    SRCNN_CUDA(cudaMemcpyAsync(host_rgb + (size_t)f0 * npx * 3, u.rgb, npx * 3 * S,
-                               cudaMemcpyDeviceToHost, ctx->copy_out));
-    SRCNN_CUDA(cudaEventRecord(ctx->ev_d[r], ctx->copy_out));
-  }
-  SRCNN_CUDA(cudaStreamSynchronize(ctx->copy_out));
-  SRCNN_CUDA(cudaStreamSynchronize(ctx->stream));
-  return SRCNN_OK;
+  return run_frame_ring(ctx, n_frames, group, host_rgba, small, in_px * 4, host_rgb, rgb, npx * 3,
+                        [&](int S, int r) {
+                          u.frames = S;
+                          u.small = small + (size_t)r * group * in_px;
+                          u.rgb = rgb + (size_t)r * group * npx * 3;
+                          SRCNN_TRY(upscale_head(ctx, u));
+                          SRCNN_TRY(launch_fused(ctx, fn, u.luma, u.out3, out_w, out_h, S));
+                          return upscale_swap(ctx, u, 0, out_h);
+                        });
 }
 
 int srcnn_infer_frames_host(srcnn_ctx* ctx, const srcnn_net* net, const float* host_in, int w,
@@ -1437,58 +1385,22 @@ int srcnn_infer_frames_host(srcnn_ctx* ctx, const srcnn_net* net, const float* h
   SRCNN_REQUIRE(fast::fused_supported(net->n1, net->n2, net->f1, net->f2, net->f3),
                 "srcnn_infer_frames_host needs a fused instantiation for %d-%d-%d n1=%d n2=%d",
                 net->f1, net->f2, net->f3, net->n1, net->n2);
-  const float *w1, *b1, *w2, *b2, *w3, *b3;
-  SRCNN_TRY(resolve(ctx, net->w[0], sizeof(float) * (size_t)net->f1 * net->f1 * net->n1, &w1, "w1"));
-  SRCNN_TRY(resolve(ctx, net->b[0], sizeof(float) * (size_t)net->n1, &b1, "b1"));
-  SRCNN_TRY(resolve(ctx, net->w[1], sizeof(float) * (size_t)net->f2 * net->f2 * net->n1 * net->n2, &w2, "w2"));
-  SRCNN_TRY(resolve(ctx, net->b[1], sizeof(float) * (size_t)net->n2, &b2, "b2"));
-  SRCNN_TRY(resolve(ctx, net->w[2], sizeof(float) * (size_t)net->f3 * net->f3 * net->n2, &w3, "w3"));
-  SRCNN_TRY(resolve(ctx, net->b[2], sizeof(float), &b3, "b3"));
-  // groups of frames go through a ring of device slots: the upload of group g+1 and the download
-  // of group g-1 overlap the fused forward of group g (one launch per group, frame = gridDim.z)
-  constexpr int kRing = kFrameRing;
+  fast::FusedNet fn;
+  SRCNN_TRY(fused_net(ctx, net, &fn));
+  // groups of frames go through the ring (one fused forward per group, frame = gridDim.z)
   const size_t in_px = (size_t)w * h, out_px = (size_t)d.w3 * d.h3;
   // ~16 MB of input per group: long enough launches to fill the GPU, short enough that the
   // exposed first upload / last download stay small
   const int group = frames_group(in_px * sizeof(float), (size_t)16 << 20, n_frames);
-  SRCNN_TRY(ensure_scratch(ctx, &ctx->band_in, &ctx->band_in_bytes, sizeof(float) * in_px * group * kRing));
-  SRCNN_TRY(ensure_scratch(ctx, &ctx->band_out, &ctx->band_out_bytes, sizeof(float) * out_px * group * kRing));
-  SRCNN_TRY(ensure_side_streams(ctx));
-  const void* scales = nullptr;
-  SRCNN_TRY(net_prepare(ctx, net, w1, b1, w2, b2, w3, b3, &scales));
-  // the side streams start behind whatever the context stream was doing with the staging
-  SRCNN_CUDA(cudaEventRecord(ctx->ev_k[kRing], ctx->stream));
-  SRCNN_CUDA(cudaStreamWaitEvent(ctx->copy_in, ctx->ev_k[kRing], 0));
-  SRCNN_CUDA(cudaStreamWaitEvent(ctx->copy_out, ctx->ev_k[kRing], 0));
+  SRCNN_TRY(ensure_scratch(ctx, &ctx->band_in, &ctx->band_in_bytes, sizeof(float) * in_px * group * kFrameRing));
+  SRCNN_TRY(ensure_scratch(ctx, &ctx->band_out, &ctx->band_out_bytes, sizeof(float) * out_px * group * kFrameRing));
   float* din = (float*)ctx->band_in;
   float* dout = (float*)ctx->band_out;
-  for (int g = 0, f0 = 0; f0 < n_frames; g++, f0 += group) {
-    const int S = std::min(group, n_frames - f0), r = g % kRing;
-    float* si = din + (size_t)r * group * in_px;
-    float* so = dout + (size_t)r * group * out_px;
-    // input slot r was last read by the forward of group g - kRing
-    if (g >= kRing) SRCNN_CUDA(cudaStreamWaitEvent(ctx->copy_in, ctx->ev_k[r], 0));
-    SRCNN_CUDA(cudaMemcpyAsync(si, host_in + (size_t)f0 * in_px, sizeof(float) * in_px * S,
-                               cudaMemcpyHostToDevice, ctx->copy_in));
-    SRCNN_CUDA(cudaEventRecord(ctx->ev_in[r], ctx->copy_in));
-    SRCNN_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->ev_in[r], 0));
-    // output slot r was last downloaded for group g - kRing
-    if (g >= kRing) SRCNN_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->ev_d[r], 0));
-    {
-      LaunchScope scope(ctx, SRCNN_K_FORWARD_FUSED, fast::fused_launches(ctx, net->n1, net->n2, net->f1, net->f2, net->f3, scales != nullptr));
-      SRCNN_TRY(fast::forward_fused(ctx, net->n1, net->n2, net->f1, net->f2, net->f3, si, so, w1, b1,
-                                    w2, b2, w3, b3, w, h, S, scales));
-      SRCNN_TRY(check_launch("forward_fused"));
-    }
-    SRCNN_CUDA(cudaEventRecord(ctx->ev_k[r], ctx->stream));
-    SRCNN_CUDA(cudaStreamWaitEvent(ctx->copy_out, ctx->ev_k[r], 0));
-    SRCNN_CUDA(cudaMemcpyAsync(host_out + (size_t)f0 * out_px, so, sizeof(float) * out_px * S,
-                               cudaMemcpyDeviceToHost, ctx->copy_out));
-    SRCNN_CUDA(cudaEventRecord(ctx->ev_d[r], ctx->copy_out));
-  }
-  SRCNN_CUDA(cudaStreamSynchronize(ctx->copy_out));
-  SRCNN_CUDA(cudaStreamSynchronize(ctx->stream));
-  return SRCNN_OK;
+  return run_frame_ring(ctx, n_frames, group, host_in, din, sizeof(float) * in_px, host_out, dout,
+                        sizeof(float) * out_px, [&](int S, int r) {
+                          return launch_fused(ctx, fn, din + (size_t)r * group * in_px,
+                                              dout + (size_t)r * group * out_px, w, h, S);
+                        });
 }
 
 size_t srcnn_train_workspace_bytes(const srcnn_net* net, int w, int h, int S) {
@@ -1582,28 +1494,20 @@ int backward1_fused_entry(srcnn_ctx* ctx, const srcnn_net* net, srcnn_mem in, co
 int forward_train_fused_entry(srcnn_ctx* ctx, const srcnn_net* net, srcnn_mem in, const Work& wk,
                               int w, int h, int S, int* launched) {
   const Dims d = net_dims(net, w, h);
-  const float *pin, *w1, *b1, *w2, *b2, *w3, *b3;
+  const float* pin;
   float *o1, *o2, *o3;
   SRCNN_TRY(resolve(ctx, in, sizeof(float) * (size_t)S * w * h, &pin, "input luma"));
   SRCNN_TRY(resolve(ctx, wk.out1, sizeof(float) * (size_t)S * d.w1 * d.h1 * net->n1, &o1, "out1"));
   SRCNN_TRY(resolve(ctx, wk.out2, sizeof(float) * (size_t)S * d.w2 * d.h2 * net->n2, &o2, "out2"));
   SRCNN_TRY(resolve(ctx, wk.out3, sizeof(float) * (size_t)S * d.w3 * d.h3, &o3, "out3"));
-  SRCNN_TRY(resolve(ctx, net->w[0], sizeof(float) * (size_t)net->f1 * net->f1 * net->n1, &w1, "w1"));
-  SRCNN_TRY(resolve(ctx, net->b[0], sizeof(float) * (size_t)net->n1, &b1, "b1"));
-  SRCNN_TRY(resolve(ctx, net->w[1], sizeof(float) * (size_t)net->f2 * net->f2 * net->n1 * net->n2, &w2, "w2"));
-  SRCNN_TRY(resolve(ctx, net->b[1], sizeof(float) * (size_t)net->n2, &b2, "b2"));
-  SRCNN_TRY(resolve(ctx, net->w[2], sizeof(float) * (size_t)net->f3 * net->f3 * net->n2, &w3, "w3"));
-  SRCNN_TRY(resolve(ctx, net->b[2], sizeof(float), &b3, "b3"));
   // the operand image only changes when the parameters do (srcnn_update_all, srcnn_write ...):
   // the chunks of an epoch share the context's cached copy
-  const void* scales = nullptr;
-  SRCNN_TRY(net_prepare(ctx, net, w1, b1, w2, b2, w3, b3, &scales));
-  LaunchScope scope(ctx, SRCNN_K_FORWARD_FUSED, fast::fused_launches(ctx, net->n1, net->n2, net->f1, net->f2, net->f3, scales != nullptr));
+  fast::FusedNet fn;
+  SRCNN_TRY(fused_net(ctx, net, &fn));
+  LaunchScope scope(ctx, SRCNN_K_FORWARD_FUSED, fast::fused_launches(ctx, fn));
   c5::Maxes* mx;
   SRCNN_TRY(fast::conv5_maxes(ctx, &mx));
-  const int rc = fast::forward_train_fused(ctx, net->n1, net->n2, net->f1, net->f2, net->f3, pin,
-                                           o1, o2, o3, w1, b1, w2, b2, w3, b3, w, h, S, scales,
-                                           &mx->out2);
+  const int rc = fast::forward_train_fused(ctx, fn, pin, o1, o2, o3, w, h, S, &mx->out2);
   if (rc < 0) return rc;
   if (rc > 0) ctx->c5_fresh_out2 = o2;   // max |out2| recorded for the layer-3 backward
   *launched = rc;
