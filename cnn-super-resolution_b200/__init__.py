@@ -26,7 +26,7 @@ NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", 
 
 KERNEL_IDS = ["forward", "squared_err", "last_layer_delta", "deltas", "backpropagate",
               "update_params", "sum", "sub_from_all", "extract_luma", "swap_luma",
-              "forward_fused", "train_fused", "resample"]
+              "forward_fused", "train_fused", "resample", "quality"]
 
 RESAMPLE_FILTERS = {"bicubic": 0, "lanczos": 1}   # SRCNN_RESAMPLE_BICUBIC / _LANCZOS
 
@@ -103,6 +103,9 @@ _SIGS = {
     "srcnn_resample": (_i, [_vp, _u64, _i, _i, _u64, _u64, _i, _i, _i]),
     "srcnn_upscale_image_host": (_i, [_vp, C.POINTER(CNet), _vp, _i, _i, _i, _i, _i, _vp]),
     "srcnn_upscale_frames_host": (_i, [_vp, C.POINTER(CNet), _vp, _i, _i, _i, _i, _i, _i, _vp]),
+    "srcnn_image_quality": (_i, [_vp, _u64, _i, _u64, _i, _i, _i, _i, _u64]),
+    "srcnn_evaluate_frames_host": (_i, [_vp, C.POINTER(CNet), _vp, _i, _i, _i, _i, _i, _i, _vp,
+                                        _i, _vp, _vp]),
     "srcnn_forward_fused_supported": (_i, [C.POINTER(CNet)]),
     "srcnn_forward_fused": (_i, [_vp, C.POINTER(CNet), _u64, _u64, _i, _i, _i, _u64, _u64]),
     "srcnn_infer_rows_host": (_i, [_vp, C.POINTER(CNet), _vp, _i, _i, _i, _i, _vp]),
@@ -375,6 +378,18 @@ class Context:
         _check(self.L.srcnn_resample(self.h, rgba_in, w, h, rgba_out, luma_out, out_w, out_h,
                                      _filter_id(resample)))
 
+    def image_quality(self, result_mem, reference_mem, w, h, S, border, result_bpp=3):
+        """{mse, ssim} of S w x h result frames (RGB8, or RGBA8 with result_bpp=4) against S RGBA8
+        reference frames on the device, over [border, w-border) x [border, h-border) of the
+        normalized luma: float64 [S, 2].  PSNR = 10 log10(1 / mse)."""
+        out = self.alloc(16 * S)
+        try:
+            _check(self.L.srcnn_image_quality(self.h, result_mem, result_bpp, reference_mem, w, h,
+                                              S, border, out))
+            return self.read(out, (S, 2), np.float64)
+        finally:
+            self.release(out)
+
 
 class Net:
     """Device-resident parameters, gradient accumulators and momentum state of the three
@@ -468,6 +483,26 @@ class Net:
                                                     rgba.shape[2], rgba.shape[1], n, out_w, out_h,
                                                     _filter_id(resample), _np_ptr(out)))
         return out
+
+    def evaluate_frames_host(self, rgba, reference, out_w, out_h, resample="lanczos", border=None,
+                             out=None):
+        """upscale_frames_host plus the quality of every frame against its reference (uint8
+        [n][out_h][out_w][4] RGBA8): returns (rgb [n][out_h][out_w][3], metrics float64 [n][4]),
+        metrics[i] = {mse, ssim} of the network's result, then {mse, ssim} of the plain
+        enlargement, over the region `border` pixels in from each edge (None: (f1+f2+f3-3)/2)."""
+        assert rgba.dtype == np.uint8 and rgba.ndim == 4 and rgba.shape[3] == 4
+        n = rgba.shape[0]
+        assert reference.dtype == np.uint8 and reference.shape == (n, out_h, out_w, 4)
+        rgba, reference = np.ascontiguousarray(rgba), np.ascontiguousarray(reference)
+        if out is None:
+            out = np.empty((n, out_h, out_w, 3), np.uint8)
+        assert out.dtype == np.uint8 and out.shape == (n, out_h, out_w, 3) and out.flags.c_contiguous
+        metrics = np.empty((n, 4), np.float64)
+        _check(self.ctx.L.srcnn_evaluate_frames_host(
+            self.ctx.h, C.byref(self.c), _np_ptr(rgba), rgba.shape[2], rgba.shape[1], n, out_w,
+            out_h, _filter_id(resample), _np_ptr(reference), -1 if border is None else int(border),
+            _np_ptr(out), _np_ptr(metrics)))
+        return out, metrics
 
     def infer_frames_host(self, host_in, w, h, host_out):
         """host_in: [n][h][w] float32 frames; host_out: [n][h3][w3].  Upload / forward / download

@@ -188,9 +188,10 @@ struct srcnn_ctx {
     unsigned long long key[kGraphKey] = {};
     unsigned graph_launches[SRCNN_K_COUNT] = {};
   } up;
-  // srcnn_upscale_frames_host: device staging (grown on demand), apart from `up` so that the two
-  // entries do not resize (and so re-capture) each other's buffers.  small / rgb hold a ring of
-  // frame groups, rgba / luma / out / red one group.
+  // srcnn_upscale_frames_host (`frames`) and srcnn_evaluate_frames_host (`eval`): device staging
+  // (grown on demand), apart from `up` and from each other so that the entries do not resize (and
+  // so re-capture) each other's buffers.  small / rgb / ref hold a ring of frame groups, rgba /
+  // luma / out / red / qred one group.
   struct FramesStaging {
     void* small = nullptr;   // input RGBA8
     void* rgba = nullptr;    // enlarged RGBA8
@@ -200,9 +201,16 @@ struct srcnn_ctx {
     void* red = nullptr;     // Q1 reduction partials, then one sum per frame
     void* s1 = nullptr;      // layer 1 / 2 activations of the three-launch route
     void* s2 = nullptr;
+    void* ref = nullptr;     // reference RGBA8 (evaluate entry)
+    void* qred = nullptr;    // quality reduction partials (evaluate entry)
+    void* metrics = nullptr; // 4 doubles a frame of the whole call (evaluate entry)
     size_t small_bytes = 0, rgba_bytes = 0, luma_bytes = 0, out_bytes = 0, rgb_bytes = 0,
-           red_bytes = 0, s1_bytes = 0, s2_bytes = 0;
-  } frames;
+           red_bytes = 0, s1_bytes = 0, s2_bytes = 0, ref_bytes = 0, qred_bytes = 0,
+           metrics_bytes = 0;
+  } frames, eval;
+  // srcnn_image_quality's reduction partials (grown on demand)
+  void* quality_red = nullptr;
+  size_t quality_red_bytes = 0;
   static constexpr int kEvents = 32;
   cudaEvent_t ev_in[kEvents] = {}, ev_k[kEvents] = {};
   cudaEvent_t ev_d[4] = {};   // download-finished events of the frame entries' rings

@@ -13,6 +13,7 @@
 #include "context.cuh"
 #include "kernels_fast.cuh"
 #include "kernels_generic.cuh"
+#include "quality.cuh"
 #include "resample.cuh"
 
 using namespace srcnn;
@@ -52,6 +53,15 @@ inline int check_resample(int w, int h, int out_w, int out_h, int filter) {
                 out_w, out_h);
   SRCNN_REQUIRE(filter == SRCNN_RESAMPLE_BICUBIC || filter == SRCNN_RESAMPLE_LANCZOS,
                 "unknown resample filter %d", filter);
+  return SRCNN_OK;
+}
+
+// the region srcnn_image_quality measures: at least one SSIM window
+inline int check_quality_region(int w, int h, int border) {
+  SRCNN_REQUIRE(border >= 0 && w - 2 * (long long)border >= quality::kWin &&
+                    h - 2 * (long long)border >= quality::kWin,
+                "border %d leaves less than %dx%d pixels of a %dx%d image", border, quality::kWin,
+                quality::kWin, w, h);
   return SRCNN_OK;
 }
 
@@ -152,11 +162,11 @@ int srcnn_ctx_destroy(srcnn_ctx* ctx) {
     for (void* p : {u.small, u.rgba, u.luma, u.out, u.rgb, u.s1, u.s2})
       if (p) cudaFree(p);
   }
-  {
-    srcnn_ctx::FramesStaging& f = ctx->frames;
-    for (void* p : {f.small, f.rgba, f.luma, f.out, f.rgb, f.red, f.s1, f.s2})
+  for (srcnn_ctx::FramesStaging* f : {&ctx->frames, &ctx->eval})
+    for (void* p : {f->small, f->rgba, f->luma, f->out, f->rgb, f->red, f->s1, f->s2, f->ref,
+                    f->qred, f->metrics})
       if (p) cudaFree(p);
-  }
+  if (ctx->quality_red) cudaFree(ctx->quality_red);
   for (srcnn_ctx::ResampleTable& t : ctx->resample_tables) cudaFree(t.dev);
   if (ctx->nccl_comm && comm::api()) comm::api()->CommDestroy(ctx->nccl_comm);
   ctx->nccl_comm = nullptr;
@@ -682,6 +692,27 @@ int srcnn_resample(srcnn_ctx* ctx, srcnn_mem rgba_in, int w, int h, srcnn_mem rg
   LaunchScope scope(ctx, SRCNN_K_RESAMPLE);
   SRCNN_TRY(resample::launch(ctx, pi, w, h, po, pl, out_w, out_h, filter, tab, rows_max));
   return check_launch("resample");
+}
+
+int srcnn_image_quality(srcnn_ctx* ctx, srcnn_mem result, int result_bpp, srcnn_mem reference,
+                        int w, int h, int S, int border, srcnn_mem out) {
+  SRCNN_ENTER(ctx);
+  SRCNN_REQUIRE(w > 0 && h > 0 && S > 0 && S <= 65535, "bad image set: %d frames of %dx%d", S, w, h);
+  SRCNN_REQUIRE(result_bpp == 3 || result_bpp == 4, "result_bpp must be 3 or 4, got %d", result_bpp);
+  SRCNN_TRY(check_quality_region(w, h, border));
+  const size_t npx = (size_t)w * h * S;
+  const unsigned char* pr;
+  const uchar4* pref;
+  double* po;
+  SRCNN_TRY(resolve(ctx, result, npx * result_bpp, &pr, "result images"));
+  SRCNN_TRY(resolve(ctx, reference, npx * 4, &pref, "reference images"));
+  SRCNN_TRY(resolve(ctx, out, sizeof(double) * 2 * (size_t)S, &po, "quality output"));
+  ctx->note_write(out);
+  SRCNN_TRY(ensure_scratch(ctx, &ctx->quality_red, &ctx->quality_red_bytes,
+                           quality::partial_bytes(w, h, border, S)));
+  LaunchScope scope(ctx, SRCNN_K_QUALITY, 2);
+  quality::launch(ctx, pr, result_bpp, pref, w, h, S, border, (double2*)ctx->quality_red, po, 2);
+  return check_launch("image_quality");
 }
 
 // ======================================================================= fused hot path
@@ -1283,9 +1314,12 @@ int frames_group(size_t frame_bytes, size_t target_bytes, int n_frames) {
 // (`in_frame` bytes each) from host_in into device slot r of dev_in (copy-in stream), then
 // work(S frames, r) on the context stream, then the download of the slot's results (`out_frame`
 // bytes each) from dev_out to host_out (copy-out stream).  Returns when the downloads are done.
+// With host_in2, a second input (`in2_frame` bytes a frame) goes up the same way into slot r of
+// dev_in2, right behind the first.
 int run_frame_ring(srcnn_ctx* ctx, int n_frames, int group, const void* host_in, void* dev_in,
                    size_t in_frame, void* host_out, const void* dev_out, size_t out_frame,
-                   const std::function<int(int S, int r)>& work) {
+                   const std::function<int(int S, int r)>& work, const void* host_in2 = nullptr,
+                   void* dev_in2 = nullptr, size_t in2_frame = 0) {
   SRCNN_TRY(ensure_side_streams(ctx));
   // the side streams start behind whatever the context stream was doing with the staging
   SRCNN_CUDA(cudaEventRecord(ctx->ev_k[kFrameRing], ctx->stream));
@@ -1297,6 +1331,10 @@ int run_frame_ring(srcnn_ctx* ctx, int n_frames, int group, const void* host_in,
     if (g >= kFrameRing) SRCNN_CUDA(cudaStreamWaitEvent(ctx->copy_in, ctx->ev_k[r], 0));
     SRCNN_CUDA(cudaMemcpyAsync((char*)dev_in + in_frame * group * r, (const char*)host_in + in_frame * f0,
                                in_frame * S, cudaMemcpyHostToDevice, ctx->copy_in));
+    if (host_in2)
+      SRCNN_CUDA(cudaMemcpyAsync((char*)dev_in2 + in2_frame * group * r,
+                                 (const char*)host_in2 + in2_frame * f0, in2_frame * S,
+                                 cudaMemcpyHostToDevice, ctx->copy_in));
     SRCNN_CUDA(cudaEventRecord(ctx->ev_in[r], ctx->copy_in));
     SRCNN_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->ev_in[r], 0));
     // output slot r was last downloaded for group g - kFrameRing
@@ -1314,13 +1352,24 @@ int run_frame_ring(srcnn_ctx* ctx, int n_frames, int group, const void* host_in,
 }
 }  // namespace
 
-int srcnn_upscale_frames_host(srcnn_ctx* ctx, const srcnn_net* net, const unsigned char* host_rgba,
-                              int w, int h, int n_frames, int out_w, int out_h, int filter,
-                              unsigned char* host_rgb) {
-  SRCNN_REQUIRE(ctx && host_rgba && host_rgb, "null argument");
-  SRCNN_ENTER(ctx);
-  SRCNN_TRY(check_upscale(net, w, h, out_w, out_h, filter));
-  SRCNN_REQUIRE(n_frames > 0, "bad frame count %d", n_frames);
+namespace {
+// A call of the frames entries: its enlargement job (u.frames, u.small and u.rgb are set per
+// group), its network, its group size and where the ring of inputs and results lives.
+struct FramesCall {
+  Upscale u;
+  fast::FusedNet fn;
+  int group;
+  bool fused;
+  uchar4* small;          // ring of input groups (one frame without a fused kernel)
+  unsigned char* rgb;     // ring of result groups
+};
+
+// staging in `st`, the resample table and the prepared network of a frames call whose arguments
+// have been checked; `extra_frame` more device bytes a frame enter the group size and the caller
+// allocates them
+int frames_prepare(srcnn_ctx* ctx, const srcnn_net* net, srcnn_ctx::FramesStaging& st, int w, int h,
+                   int n_frames, int out_w, int out_h, int filter, size_t extra_frame,
+                   FramesCall* fc) {
   const Dims d = net_dims(net, out_w, out_h);
   const size_t in_px = (size_t)w * h, npx = (size_t)out_w * out_h, out_px = (size_t)d.w3 * d.h3;
   SRCNN_CUDA(ctx->drain_lanes());
@@ -1330,11 +1379,10 @@ int srcnn_upscale_frames_host(srcnn_ctx* ctx, const srcnn_net* net, const unsign
   // ~128 MB of device staging per group (input, enlarged RGBA8 + luma + RGB8, network output;
   // 960x540 -> 1920x1080: 4 frames): launches long enough to fill the GPU, a first upload and a
   // last download short next to a whole call
-  const size_t frame_bytes = in_px * 4 + npx * (4 + 4 + 3) + out_px * 4;
+  const size_t frame_bytes = in_px * 4 + npx * (4 + 4 + 3) + out_px * 4 + extra_frame;
   // (the frame is a grid dimension of the head and swap launches: at most 65535 a group)
   const int group = fused ? std::min(frames_group(frame_bytes, (size_t)128 << 20, n_frames), 65535) : 1;
   const int ring = fused ? kFrameRing : 1;
-  srcnn_ctx::FramesStaging& st = ctx->frames;
   SRCNN_TRY(ensure_scratch(ctx, &st.small, &st.small_bytes, in_px * 4 * group * ring));
   SRCNN_TRY(ensure_scratch(ctx, &st.rgba, &st.rgba_bytes, npx * 4 * group));
   SRCNN_TRY(ensure_scratch(ctx, &st.luma, &st.luma_bytes, npx * sizeof(float) * group));
@@ -1346,33 +1394,118 @@ int srcnn_upscale_frames_host(srcnn_ctx* ctx, const srcnn_net* net, const unsign
     SRCNN_TRY(ensure_scratch(ctx, &st.s2, &st.s2_bytes, sizeof(float) * (size_t)d.w2 * d.h2 * net->n2));
   }
   SRCNN_TRY(resample::table_for(ctx, w, h, out_w, out_h, filter, &u.tab, &u.rows_max));
-  fast::FusedNet fn;
-  SRCNN_TRY(fused_net(ctx, net, &fn));
+  SRCNN_TRY(fused_net(ctx, net, &fc->fn));
   u.rgba = (uchar4*)st.rgba;
   u.luma = (float*)st.luma;
   u.out3 = (float*)st.out;
   u.partial = (double*)st.red;
   u.sums = (float*)(u.partial + (size_t)u.red_blocks() * group);
-  uchar4* small = (uchar4*)st.small;
-  unsigned char* rgb = (unsigned char*)st.rgb;
-  if (!fused) {
+  u.small = (uchar4*)st.small;
+  u.rgb = (unsigned char*)st.rgb;
+  fc->u = u;
+  fc->group = group;
+  fc->fused = fused;
+  fc->small = (uchar4*)st.small;
+  fc->rgb = (unsigned char*)st.rgb;
+  return SRCNN_OK;
+}
+
+// the device work of one group of the frames entry in ring slot r: enlargement, Q1 mean, fused
+// forward, swap_luma.  5 + F launches.
+int frames_group_work(srcnn_ctx* ctx, FramesCall& fc, int S, int r) {
+  Upscale& u = fc.u;
+  const size_t in_px = (size_t)u.w * u.h, npx = u.npx();
+  u.frames = S;
+  u.small = fc.small + (size_t)r * fc.group * in_px;
+  u.rgb = fc.rgb + (size_t)r * fc.group * npx * 3;
+  SRCNN_TRY(upscale_head(ctx, u));
+  SRCNN_TRY(launch_fused(ctx, fc.fn, u.luma, u.out3, u.out_w, u.out_h, S));
+  return upscale_swap(ctx, u, 0, u.out_h);
+}
+
+// the quality of u's frames against `ref`: the RGB8 result into m[4 s + 0, 1], the enlarged
+// RGBA8 into m[4 s + 2, 3].  4 launches.
+int quality_pair(srcnn_ctx* ctx, const Upscale& u, const uchar4* ref, int border, double2* partial,
+                 double* m) {
+  LaunchScope scope(ctx, SRCNN_K_QUALITY, 4);
+  quality::launch(ctx, u.rgb, 3, ref, u.out_w, u.out_h, u.frames, border, partial, m, 4);
+  quality::launch(ctx, (const unsigned char*)u.rgba, 4, ref, u.out_w, u.out_h, u.frames, border,
+                  partial, m + 2, 4);
+  return check_launch("image_quality");
+}
+}  // namespace
+
+int srcnn_upscale_frames_host(srcnn_ctx* ctx, const srcnn_net* net, const unsigned char* host_rgba,
+                              int w, int h, int n_frames, int out_w, int out_h, int filter,
+                              unsigned char* host_rgb) {
+  SRCNN_REQUIRE(ctx && host_rgba && host_rgb, "null argument");
+  SRCNN_ENTER(ctx);
+  SRCNN_TRY(check_upscale(net, w, h, out_w, out_h, filter));
+  SRCNN_REQUIRE(n_frames > 0, "bad frame count %d", n_frames);
+  srcnn_ctx::FramesStaging& st = ctx->frames;
+  FramesCall fc;
+  SRCNN_TRY(frames_prepare(ctx, net, st, w, h, n_frames, out_w, out_h, filter, 0, &fc));
+  const size_t in_px = (size_t)w * h, npx = (size_t)out_w * out_h;
+  if (!fc.fused) {
     // frame by frame, each as the image entry runs it
-    u.small = small;
-    u.rgb = rgb;
     for (int f = 0; f < n_frames; f++)
-      SRCNN_TRY(upscale_three_launch(ctx, net, u, st.s1, st.s2, host_rgba + (size_t)f * in_px * 4,
+      SRCNN_TRY(upscale_three_launch(ctx, net, fc.u, st.s1, st.s2, host_rgba + (size_t)f * in_px * 4,
                                      host_rgb + (size_t)f * npx * 3));
     return SRCNN_OK;
   }
-  return run_frame_ring(ctx, n_frames, group, host_rgba, small, in_px * 4, host_rgb, rgb, npx * 3,
-                        [&](int S, int r) {
-                          u.frames = S;
-                          u.small = small + (size_t)r * group * in_px;
-                          u.rgb = rgb + (size_t)r * group * npx * 3;
-                          SRCNN_TRY(upscale_head(ctx, u));
-                          SRCNN_TRY(launch_fused(ctx, fn, u.luma, u.out3, out_w, out_h, S));
-                          return upscale_swap(ctx, u, 0, out_h);
-                        });
+  return run_frame_ring(ctx, n_frames, fc.group, host_rgba, fc.small, in_px * 4, host_rgb, fc.rgb,
+                        npx * 3, [&](int S, int r) { return frames_group_work(ctx, fc, S, r); });
+}
+
+int srcnn_evaluate_frames_host(srcnn_ctx* ctx, const srcnn_net* net, const unsigned char* host_rgba,
+                               int w, int h, int n_frames, int out_w, int out_h, int filter,
+                               const unsigned char* host_ref, int border, unsigned char* host_rgb,
+                               double* host_metrics) {
+  SRCNN_REQUIRE(ctx && host_rgba && host_rgb && host_ref && host_metrics, "null argument");
+  SRCNN_ENTER(ctx);
+  SRCNN_TRY(check_upscale(net, w, h, out_w, out_h, filter));
+  SRCNN_REQUIRE(n_frames > 0, "bad frame count %d", n_frames);
+  if (border < 0) border = (net->f1 + net->f2 + net->f3 - 3) / 2;
+  SRCNN_TRY(check_quality_region(out_w, out_h, border));
+  srcnn_ctx::FramesStaging& st = ctx->eval;
+  const size_t in_px = (size_t)w * h, npx = (size_t)out_w * out_h;
+  FramesCall fc;
+  SRCNN_TRY(frames_prepare(ctx, net, st, w, h, n_frames, out_w, out_h, filter, npx * 4, &fc));
+  const int ring = fc.fused ? kFrameRing : 1;
+  SRCNN_TRY(ensure_scratch(ctx, &st.ref, &st.ref_bytes, npx * 4 * fc.group * ring));
+  SRCNN_TRY(ensure_scratch(ctx, &st.qred, &st.qred_bytes,
+                           quality::partial_bytes(out_w, out_h, border, fc.group)));
+  SRCNN_TRY(ensure_scratch(ctx, &st.metrics, &st.metrics_bytes, sizeof(double) * 4 * (size_t)n_frames));
+  uchar4* refs = (uchar4*)st.ref;
+  double2* qred = (double2*)st.qred;
+  double* metrics = (double*)st.metrics;
+  if (!fc.fused) {
+    // frame by frame through the image entry's route, the reference uploaded ahead of it and the
+    // quality measured behind it on the context stream
+    for (int f = 0; f < n_frames; f++) {
+      SRCNN_CUDA(cudaMemcpyAsync(refs, host_ref + (size_t)f * npx * 4, npx * 4,
+                                 cudaMemcpyHostToDevice, ctx->stream));
+      SRCNN_TRY(upscale_three_launch(ctx, net, fc.u, st.s1, st.s2, host_rgba + (size_t)f * in_px * 4,
+                                     host_rgb + (size_t)f * npx * 3));
+      SRCNN_TRY(quality_pair(ctx, fc.u, refs, border, qred, metrics + (size_t)f * 4));
+    }
+  } else {
+    int f0 = 0;   // first frame of the group the ring hands out next (groups come in order)
+    SRCNN_TRY(run_frame_ring(
+        ctx, n_frames, fc.group, host_rgba, fc.small, in_px * 4, host_rgb, fc.rgb, npx * 3,
+        [&](int S, int r) {
+          SRCNN_TRY(frames_group_work(ctx, fc, S, r));
+          const uchar4* ref = refs + (size_t)r * fc.group * npx;
+          double* m = metrics + (size_t)f0 * 4;
+          f0 += S;
+          return quality_pair(ctx, fc.u, ref, border, qred, m);
+        },
+        host_ref, refs, npx * 4));
+  }
+  SRCNN_CUDA(cudaMemcpyAsync(host_metrics, metrics, sizeof(double) * 4 * (size_t)n_frames,
+                             cudaMemcpyDeviceToHost, ctx->stream));
+  SRCNN_CUDA(cudaStreamSynchronize(ctx->stream));
+  return SRCNN_OK;
 }
 
 int srcnn_infer_frames_host(srcnn_ctx* ctx, const srcnn_net* net, const float* host_in, int w,

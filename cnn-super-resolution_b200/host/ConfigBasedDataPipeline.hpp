@@ -62,6 +62,14 @@ class ConfigBasedDataPipeline : public DataPipeline {
   void upscale_frames(LayerAllocationPool&, LayerAllocationPool&, LayerAllocationPool&,
                       const unsigned char* in_rgba, size_t w, size_t h, size_t n_frames,
                       size_t out_w, size_t out_h, int filter, unsigned char* out_rgb);
+  /** upscale_frames plus the quality of every result against its reference (n_frames frames of
+   * out_w x out_h RGBA8 in `ref_rgba`): `metrics` receives 4 doubles a frame, {mse, ssim} of the
+   * network's result and of the plain enlargement, over the region `border` pixels in from each
+   * edge (< 0: half the network's padding) (srcnn_evaluate_frames_host) */
+  void evaluate_frames(LayerAllocationPool&, LayerAllocationPool&, LayerAllocationPool&,
+                       const unsigned char* in_rgba, size_t w, size_t h, size_t n_frames,
+                       size_t out_w, size_t out_h, int filter, const unsigned char* ref_rgba,
+                       int border, unsigned char* out_rgb, double* metrics);
 
   inline const Config* config() { return _config; }
   inline const LayerData* layer_1() { return &layer_data_1; }

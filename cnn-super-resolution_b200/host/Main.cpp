@@ -1,4 +1,4 @@
-// `cnn [train] [dry] [profile] --config CFG --in PATH [--out PATH] [--epochs N]
+// `cnn [train | eval] [dry] [profile] --config CFG --in PATH [--out PATH] [--epochs N]
 //      [--scale N [--resample lanczos|bicubic]]`
 // Same grammar, flow and console output as the reference CLI (src/Main_cl.cpp:40-318):
 // forward mode = one image through the three layers, luma swapped back into the image (or every
@@ -11,6 +11,11 @@
 // -i DIR (forward mode) runs every `.ppm` / `.pgm` file of DIR, in sorted name order, into
 // OUT_DIR/<stem>.ppm (-o OUT_DIR): consecutive files of equal size go through
 // srcnn_upscale_frames_host together, at most kDirBatch at a time; other files are skipped.
+// eval -i SAMPLES_DIR measures the network on the training mode's sample pairs: every `_small`
+// image, enlarged N times (--scale, default 1: the reference's `_small` images are already
+// enlarged), against its `_large` image, which must be exactly N times its size.  One line a pair
+// (PSNR / SSIM of the network's result and of the plain enlargement, and the PSNR gain), then
+// their means; -o OUT_DIR also writes OUT_DIR/<name>.ppm (srcnn_evaluate_frames_host).
 // Images are binary PPM/PGM (see Context.hpp); `_large.ppm/_small.ppm` as well as the
 // reference's `.jpg` suffix pattern are recognised by name.
 #include <sys/stat.h>
@@ -18,6 +23,7 @@
 #include <algorithm>
 #include <cerrno>
 #include <cmath>
+#include <cstdio>
 #include <cstring>
 #include <cstdlib>
 #include <iostream>
@@ -192,6 +198,93 @@ static void get_training_samples(const std::string& dir, std::vector<TrainSample
   }
 }
 
+// PSNR for data range 1 (+inf for identical images)
+static double psnr_db(double mse) { return mse > 0.0 ? 10.0 * std::log10(1.0 / mse) : INFINITY; }
+
+static std::string quality_line(double net_mse, double net_ssim, double base_mse, double base_ssim) {
+  char buf[256];
+  const double net = psnr_db(net_mse), base = psnr_db(base_mse);
+  std::snprintf(buf, sizeof(buf),
+                "network PSNR %.4f dB SSIM %.6f | baseline PSNR %.4f dB SSIM %.6f | gain %.4f dB",
+                net, net_ssim, base, base_ssim, net - base);
+  return buf;
+}
+
+// `eval`: every sample pair through the evaluate entry, consecutive pairs of equal size together
+// (at most kDirBatch); per pair and mean PSNR / SSIM lines, results to out_dir/<name>.ppm unless
+// out_dir is null (dry run)
+static void execute_eval(ConfigBasedDataPipeline& pipeline, GpuAllocationPool& gpu_alloc,
+                         const std::vector<TrainSampleFiles>& files, const char* out_dir,
+                         size_t scale, int filter) {
+  const int border = (int)pipeline.config()->total_padding() / 2;
+  std::vector<unsigned char> in, ref, out;
+  std::vector<double> metrics;
+  std::vector<std::string> batch;
+  double sum[5] = {};
+  size_t n_done = 0, w = 0, h = 0;
+  auto flush = [&]() {
+    if (batch.empty()) return;
+    const size_t out_w = scale * w, out_h = scale * h, out_bytes = out_w * out_h * 3;
+    out.resize(batch.size() * out_bytes);
+    metrics.resize(batch.size() * 4);
+    pipeline.evaluate_frames(gpu_alloc.layer_1, gpu_alloc.layer_2, gpu_alloc.layer_3, in.data(), w,
+                             h, batch.size(), out_w, out_h, filter, ref.data(), border, out.data(),
+                             metrics.data());
+    for (size_t i = 0; i < batch.size(); i++) {
+      const double* m = metrics.data() + 4 * i;
+      std::cout << batch[i] << ": " << quality_line(m[0], m[1], m[2], m[3]) << std::endl;
+      const double v[5] = {psnr_db(m[0]), m[1], psnr_db(m[2]), m[3], psnr_db(m[0]) - psnr_db(m[2])};
+      for (int k = 0; k < 5; k++) sum[k] += v[k];
+      n_done++;
+      if (!out_dir) continue;
+      const std::string path = std::string(out_dir) + "/" + batch[i] + ".ppm";
+      std::cout << "Saving result image to: '" << path << "'" << std::endl;
+      ImageData res_img((int)out_w, (int)out_h, 3, out.data() + i * out_bytes);
+      if (!write_image(path.c_str(), res_img))
+        throw std::runtime_error("Could not write image: " + path);
+    }
+    batch.clear();
+    in.clear();
+    ref.clear();
+  };
+  for (const TrainSampleFiles& pair : files) {
+    // the pair's name: the file name of its small image before "_small"
+    const size_t slash = pair.second.find_last_of('/');
+    std::string name = pair.second.substr(slash == std::string::npos ? 0 : slash + 1);
+    name = name.substr(0, name.rfind("_small"));
+    ImageData small, large;
+    load_image(pair.second.c_str(), small);
+    load_image(pair.first.c_str(), large);
+    if ((size_t)large.w != scale * small.w || (size_t)large.h != scale * small.h) {
+      std::cout << "'" << name << "': reference is " << large.w << "x" << large.h << ", not " << scale
+                << " x " << small.w << "x" << small.h << ". Skipping sample" << std::endl;
+      continue;
+    }
+    if (large.w - 2 * border < 11 || large.h - 2 * border < 11) {
+      std::cout << "'" << name << "': " << large.w << "x" << large.h
+                << " leaves less than 11x11 pixels inside the border of " << border
+                << ". Skipping sample" << std::endl;
+      continue;
+    }
+    if (!batch.empty() && ((size_t)small.w != w || (size_t)small.h != h || batch.size() == kDirBatch))
+      flush();
+    w = (size_t)small.w;
+    h = (size_t)small.h;
+    in.insert(in.end(), small.data, small.data + w * h * 4);
+    ref.insert(ref.end(), large.data, large.data + (size_t)large.w * large.h * 4);
+    batch.push_back(name);
+  }
+  flush();
+  if (n_done == 0) throw std::runtime_error("No sample pairs of matching sizes found");
+  const double n = (double)n_done;
+  char buf[256];
+  std::snprintf(buf, sizeof(buf),
+                "mean over %zu pairs: network PSNR %.4f dB SSIM %.6f | baseline PSNR %.4f dB SSIM "
+                "%.6f | gain %.4f dB",
+                n_done, sum[0] / n, sum[1] / n, sum[2] / n, sum[3] / n, sum[4] / n);
+  std::cout << buf << std::endl;
+}
+
 static void divide_samples(size_t validation_set_size, GpuAllocationPool& pool,
                            std::vector<SampleAllocationPool*>& train_set,
                            std::vector<SampleAllocationPool*>& validation_set, std::mt19937& rng) {
@@ -214,6 +307,7 @@ static std::vector<SampleAllocationPool*> shard(const std::vector<SampleAllocati
 int main(int argc, char** argv) {
   cnn_sr::utils::Argparse argparse("cnn", "SRCNN super-resolution (B200 CUDA build)");
   argparse.add_argument("train").help("Train mode");
+  argparse.add_argument("eval").help("Measure PSNR / SSIM of the samples of a directory against their references");
   argparse.add_argument("dry").help("Do not store result");
   argparse.add_argument("profile").help("Print kernel execution times");
   argparse.add_argument("-c", "--config").required().help("CNN configuration");
@@ -229,8 +323,8 @@ int main(int argc, char** argv) {
     return EXIT_FAILURE;
   }
 
-  const bool train = argparse.has_arg("train"), dry = argparse.has_arg("dry"),
-             profile = argparse.has_arg("profile");
+  const bool train = argparse.has_arg("train"), eval = argparse.has_arg("eval"),
+             dry = argparse.has_arg("dry"), profile = argparse.has_arg("profile");
   const char* config_path = argparse.value("config");
   const char* in_path = argparse.value("in");
   const char* out_path = dry ? nullptr : argparse.value("out");
@@ -254,12 +348,16 @@ int main(int argc, char** argv) {
     std::cout << "--resample must be lanczos or bicubic, got '" << resample_name << "'" << std::endl;
     return EXIT_FAILURE;
   }
+  if (train && eval) {
+    std::cout << "eval and train exclude each other" << std::endl;
+    return EXIT_FAILURE;
+  }
   if (train && argparse.value("scale")) {
     std::cout << "--scale applies to the forward mode only" << std::endl;
     return EXIT_FAILURE;
   }
-  const bool in_dir = !train && is_directory(in_path);
-  if (in_dir && out_path && !is_directory(out_path)) {
+  const bool in_dir = !train && !eval && is_directory(in_path);
+  if ((in_dir || eval) && out_path && !is_directory(out_path)) {
     std::cout << "Output directory '" << out_path << "' does not exist or is not a directory"
               << std::endl;
     return EXIT_FAILURE;
@@ -271,6 +369,10 @@ int main(int argc, char** argv) {
   if (train)
     std::cout << "Training mode, epochs: " << epochs << std::endl
               << "Training samples directory: " << in_path << std::endl
+              << "Output: " << (out_path ? out_path : "-") << std::endl;
+  else if (eval)
+    std::cout << "Evaluation mode" << std::endl
+              << "Samples directory: " << in_path << std::endl
               << "Output: " << (out_path ? out_path : "-") << std::endl;
   else
     std::cout << "Forward mode" << std::endl
@@ -292,6 +394,14 @@ int main(int argc, char** argv) {
     data_pipeline.init(DataPipeline::LOAD_KERNEL_ALL);
     GpuAllocationPool gpu_alloc;
 
+    if (eval) {
+      std::vector<TrainSampleFiles> files;
+      get_training_samples(in_path, files);
+      if (files.empty()) throw std::runtime_error("No samples found");
+      execute_eval(data_pipeline, gpu_alloc, files, out_path, scale, filter);
+      context.block();
+      return EXIT_SUCCESS;
+    }
     if (in_dir) {
       const std::vector<DirImage> images = get_directory_images(in_path);
       if (images.empty()) throw std::runtime_error("No .ppm/.pgm images found");

@@ -61,6 +61,7 @@ enum srcnn_kernel_id {
   SRCNN_K_FORWARD_FUSED,     /* (new) layers 1-3 in one launch, inference  */
   SRCNN_K_TRAIN_FUSED,       /* (new) fused pieces of the training step    */
   SRCNN_K_RESAMPLE,          /* (new) Pillow-exact enlargement             */
+  SRCNN_K_QUALITY,           /* (new) PSNR / SSIM of image pairs           */
   SRCNN_K_COUNT
 };
 
@@ -198,6 +199,22 @@ enum { SRCNN_RESAMPLE_BICUBIC = 0, SRCNN_RESAMPLE_LANCZOS = 1 };
 int srcnn_resample(srcnn_ctx* ctx, srcnn_mem rgba_in, int w, int h, srcnn_mem rgba_out,
                    srcnn_mem luma_out, int out_w, int out_h, int filter);
 
+/* Enlargement quality: the PSNR / SSIM inputs of S image pairs on the device.  result holds S
+ * frames of w*h*result_bpp bytes (result_bpp = 3: RGB8 as srcnn_swap_luma writes it, 4: RGBA8),
+ * reference S frames of w*h RGBA8; out receives 2*S doubles, {mse, ssim} per frame, over the
+ * region [border, w-border) x [border, h-border).  Both are taken on the luma srcnn_extract_luma
+ * computes with normalize = 1 (data range 1):
+ *   mse  = mean over the region of d^2, d = Y_result - Y_reference in float, d^2 and the sum in
+ *          double; PSNR = 10 log10(1 / mse) (+inf for mse = 0) is the caller's;
+ *   ssim = Wang et al. 2004 (`ssim_index`): the mean over every 11x11 window wholly inside the
+ *          region of the SSIM of the window, Gaussian weights (sigma 1.5, sum 1), C1 = 0.01^2,
+ *          C2 = 0.03^2, population (co)variances E[xy] - mx*my.
+ * A frame's result does not depend on S or on the other frames, and repeats bit for bit.  A
+ * region smaller than 11x11, a negative border, S outside [1, 65535] or result_bpp other than 3
+ * or 4: SRCNN_EINVAL.  2 launches. */
+int srcnn_image_quality(srcnn_ctx* ctx, srcnn_mem result, int result_bpp, srcnn_mem reference,
+                        int w, int h, int S, int border, srcnn_mem out);
+
 /* ---------------------------------------------------------------- fused hot path --- */
 
 typedef struct srcnn_net {
@@ -282,6 +299,28 @@ int srcnn_upscale_image_host(srcnn_ctx* ctx, const srcnn_net* net, const unsigne
 int srcnn_upscale_frames_host(srcnn_ctx* ctx, const srcnn_net* net, const unsigned char* host_rgba,
                               int w, int h, int n_frames, int out_w, int out_h, int filter,
                               unsigned char* host_rgb);
+
+/* srcnn_upscale_frames_host plus the quality of its results: host_ref holds n_frames reference
+ * frames of out_w*out_h*4 bytes RGBA8 (the ground truth the small frames were made from).
+ * host_rgb receives what srcnn_upscale_frames_host returns for the same arguments, byte for byte;
+ * host_metrics receives 4 doubles a frame: {mse, ssim} of the network's result and {mse, ssim}
+ * of the plain enlargement (the resampled RGBA8 alone, the baseline the network starts from),
+ * both against the reference as srcnn_image_quality measures them, over the region border from
+ * each edge (border < 0: (f1+f2+f3-3)/2, the rows and columns swap_luma leaves as enlarged).
+ * Synchronous; pinned host buffers give the overlap.  The reference frames go up on the copy-in
+ * stream into ring slots of their own; the metrics of all frames stay on the device and come
+ * down once, after the last group.  Staging is the context's and apart from the frames entry's.
+ * Groups hold as many frames as fit ~128 MB (the frames entry's bytes + out_w*out_h*4 a frame),
+ * or SRCNN_FRAMES_GROUP frames.
+ * Launches per call: n_groups * (5 + F + 4) with a fused kernel, n_frames * (4 + L + 1 + 4)
+ * without (F, L as for srcnn_upscale_frames_host), plus 1 when the network's packed operand image
+ * has to be rebuilt.  Everything srcnn_upscale_frames_host rejects, a null host_ref or
+ * host_metrics and a border that leaves less than 11x11 pixels: SRCNN_EINVAL before any host
+ * buffer is read or written. */
+int srcnn_evaluate_frames_host(srcnn_ctx* ctx, const srcnn_net* net, const unsigned char* host_rgba,
+                               int w, int h, int n_frames, int out_w, int out_h, int filter,
+                               const unsigned char* host_ref, int border, unsigned char* host_rgb,
+                               double* host_metrics);
 
 /* ConfigBasedDataPipeline::forward(sample) for MANY frames (src/ConfigBasedDataPipeline.cpp:
  * 114-126 is called once per image by src/Main_cl.cpp:217-239): `n_frames` luma frames of
