@@ -34,8 +34,6 @@
 
 #include "context.cuh"
 #include "conv5_tc.cuh"
-#include "fused_forward_hp.cuh"
-#include "fused_forward_pl.cuh"
 #include "tc_common.cuh"
 
 namespace srcnn {
@@ -99,15 +97,6 @@ struct Args {
 __global__ void __launch_bounds__(Cfg::NT, 1) bwd3_tc_kernel(Args a) {
   using C = Cfg;
   using namespace tc;
-  using fused_hp::kmajor16;
-  using fused_hp::make_idesc_f16;
-  using fused_hp::mma_f16_ss;
-  using fused_hp::pack2;
-  using fused_hp::split_h;
-  using fused_hp::split_h2;
-  using fused_pl::elect_one;
-  using fused_pl::tmem_ld16_nowait;
-  using fused_pl::tmem_ld_wait;
   extern __shared__ __align__(128) uint8_t smem_raw[];
   __shared__ __align__(8) uint64_t pfull[C::RP], pfree[C::RP], qfull[C::RQ], qfree[C::RQ],
       d2_done[2], d2_free[2], gw_done;

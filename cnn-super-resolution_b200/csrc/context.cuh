@@ -83,7 +83,8 @@ struct srcnn_ctx {
   uint64_t launch_count = 0;
   // fused inference implementation: tensor cores (tcgen05, 3xTF32) where instantiated, unless
   // SRCNN_FUSED_IMPL=simt asks for the FP32 SIMT kernel (A/B measurements)
-  // 0 simt, 3 planes (3xTF32), 4 planes (FP16 split); earlier generations live in exp/superseded
+  // 0 simt, 3 planes (3xTF32), 4 planes (FP16 split); the two earlier generations are in the
+  // git history (tools/superseded/ at 99b7bf0)
   int fused_impl = 4;
   bool deltas_tc = true;              // f=1 deltas on the tensor cores (deltas_tc.cuh)
   bool wgrad_tc = true;               // layer-1 weight gradient on the tensor cores (wgrad_tc.cuh)

@@ -23,7 +23,7 @@
 // and one shared-memory copy.  The 5 output rows an input row contributes to (dy = 0..4) each
 // have their own accumulator in tensor memory, side by side in a ring of 16 (forward) / 8
 // (deltas) slots (row rho in slot rho % NACC), so that ONE instruction A x [W(dy=4); ...; W(dy=0)] feeds all five (N = 5 * C_out
-// = 160 forward; deltas 4 + 1 rows of 64): "dy-stacked" MMAs, see Cfg::DYS.  A row leaves
+// = 160 forward; deltas 4 + 1 rows of 64): "dy-stacked" MMAs, see Cfg.  A row leaves
 // through the epilogue when its last input row has been issued.  W (hi | lo, 204 800 bytes)
 // stays resident in shared memory, stored [hi | lo][dx][slice][(4 - dy) * C_out + n][16] so that
 // a range of filter rows is one B operand.
@@ -36,20 +36,16 @@
 // weights likewise.
 //
 //   P  (5 warps)  input row slice -> split -> planes (loads two slices ahead)  -> full[slot]
-//   I0 [, I1]     MMA issuers: per (slice, dx) one instruction per product and piece of the
+//   I  (1 warp)   MMA issuer: per (slice, dx) one instruction per product and piece of the
 //                 row range (pieces: where the ring wraps, and <= 256 / C_out rows)
 //                                                                            -> empty[slot], done[acc]
 //   E  (4 warps)  accumulator -> bias + relu / relu' mask -> global          -> acc_free[acc]
 //                 (deltas: 16x256b fragments, mask loaded before the accumulator wait)
-// C5_DYS=0 builds the earlier scheme: one accumulator per row, instructions per (dy, dx), three
-// issuers by output row, A_hi x [W_hi; W_lo] stacked where tensor memory allows.
 #pragma once
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
 
 #include "context.cuh"
-#include "fused_forward_hp.cuh"
-#include "fused_forward_pl.cuh"
 #include "tc_common.cuh"
 
 namespace srcnn {
@@ -102,73 +98,30 @@ struct Cfg {
   static constexpr int PW = 136;                      // plane entries (>= M + F - 1)
   static constexpr int PB = PW * 16;                  // bytes per plane
   static constexpr int SLOT_BYTES = 4 * PB;           // hi chunk 0, hi chunk 1, lo chunk 0, lo chunk 1
-  // DYS ("dy-stacked", MODE 0): the five filter rows dy of an input row slice use the SAME A tile
-  // (same input row, same dx shift) and only differ in the output row they feed.  With the
+  // dy-stacked MMAs: the five filter rows dy of an input row slice use the SAME A tile (same
+  // input row, same dx shift) and only differ in the output row they feed.  With the
   // accumulators of consecutive output rows side by side in tensor memory, ONE instruction
   // A x [W(dy=4); W(dy=3); ... ; W(dy=0)] (N = 5 * COUT = 160) serves all five: 3 instructions per
-  // (slice, dx) -- hi.hi and lo.hi into region H, hi.lo into region L -- instead of 10, and each
-  // is math-bound (80 cycles of tensor math against 72 of operand fetch) where the per-dy
-  // instructions were fetch-bound (94 cycles per 48 of math: the kernel's tensor pipe was 74 %
-  // busy at 39 % math, profiles/r3j_ncu_summary.txt).  Output row rho lives in slot rho % 8 of
-  // both regions; a range of rows that wraps around the ring is issued as two instructions.
-#ifndef C5_DYS
-#define C5_DYS 1
-#endif
-#ifndef C5_TWO
-#define C5_TWO 0
-#endif
-  static constexpr bool DYS = C5_DYS != 0;
-  // two regions (hi.w_lo apart from the rest, one issuer each) where 2 * 8 rows fit tensor memory
-  // (MODE 0); else all three products of a row share one accumulator and one issuer (MODE 1,
-  // where an instruction carries at most 256 / COUT = 4 rows)
-  static constexpr bool TWO = C5_TWO != 0 && DYS && 2 * 8 * COUT_ <= 512;
-  // Forward (C_out = 32): ONE region of 16 slots and one issuer with all three products in a
-  // row's accumulator, like the deltas: a range of 5 rows wraps in 4 of 16 input rows instead
-  // of 4 of 8 (chunk of 3 028 patches 2.229 -> 2.207 ms).  C5_TWO=1: two regions of 8 slots, H
-  // (hi.w_hi + lo.w_hi) and L (hi.w_lo), one issuer each, added by the epilogue.
-  static constexpr int NSLOT = 3, NACC = DYS ? ((C5_TWO == 0 && COUT_ * 16 <= 512) ? 16 : 8) : 7;
-  // HALVES (MODE 1, C_out = 64; experiment, default off): two issuers that each own 32 output
-  // channels -- all three products into their own region, N = 5 * 32 = 160 per instruction like
-  // the forward -- instead of one issuer carrying every instruction.  Same results, same speed
-  // (2.302 ms per chunk of 3 028 either way: the deltas kernel is not issue-bound), twice the A
-  // fetches: not used.
-#ifndef C5_HALVES
-#define C5_HALVES 0
-#endif
-  static constexpr bool HALVES = C5_HALVES != 0 && DYS && !TWO && COUT_ == 64;
-  static constexpr int CI = HALVES ? 32 : COUT_;      // DYS: output channels per issuer and region
-  static constexpr int NH = HALVES ? 2 : 1;
-  static constexpr int REGION = 256;                  // DYS: columns of a region (TWO: H, L; HALVES)
-  static constexpr int BLK_BYTES = F * CI * 32;       // DYS: image block of one (dx, slice[, half])
-  static constexpr int IMG_L = F * NSLICE * NH * BLK_BYTES;   // DYS: byte offset of the W_lo blocks
-  // STACK: A_hi x [W_hi ; W_lo] as ONE N = 2*COUT instruction (its two halves land in separate
-  // accumulator columns, the epilogue adds them) + A_lo x W_hi: two A-tile fetches per K-step
-  // instead of three.  The A tile (128 rows at a 16-byte shifted base: every 128-byte core matrix
-  // straddles two shared-memory lines) is the expensive operand.  Needs 2*COUT columns per row.
-  static constexpr bool STACK = !DYS && 2 * NACC * COUT <= 512;
-  static constexpr int ACCW = STACK ? 2 * COUT : COUT;
-  static constexpr int W_BYTES = 2 * COUT * KT * 2;   // [W_hi rows ; W_lo rows][KT] halves
-  static constexpr int W_SBO = 128 * (KT / 8);        // bytes between 8-row groups of the image
+  // (slice, dx), one per product, instead of 10, and each is math-bound (80 cycles of tensor math
+  // against 72 of operand fetch) where the per-dy instructions were fetch-bound (94 cycles per 48
+  // of math: the kernel's tensor pipe was 74 % busy at 39 % math, profiles/r3j_ncu_summary.txt).
+  // Output row rho lives in slot rho % NACC; a range of rows that wraps around the ring is issued
+  // as two instructions.  All three products of a row go into its one accumulator, issued by one
+  // warp (the summation order is fixed).  The forward (C_out = 32) has 16 slots: a range of 5 rows
+  // wraps in 4 of 16 input rows instead of 4 of 8 (chunk of 3 028 patches 2.229 -> 2.207 ms); the
+  // deltas (C_out = 64) fill tensor memory with 8.
+  static constexpr int NSLOT = 3, NACC = COUT_ * 16 <= 512 ? 16 : 8;
+  static constexpr int BLK_BYTES = F * COUT * 32;     // image block of one (dx, slice)
+  static constexpr int IMG_L = F * NSLICE * BLK_BYTES;   // byte offset of the W_lo blocks
+  static constexpr int W_BYTES = 2 * COUT * KT * 2;   // [W_hi blocks ; W_lo blocks] halves
   static constexpr int oW = 0, oSlots = W_BYTES, oBias = oSlots + NSLOT * SLOT_BYTES;
   static constexpr size_t SMEM_BYTES = (size_t)oBias + COUT * 4;
-  // MMA issuer warps: output rows split modulo N_I (3 instead of 2: forward of a 3 028-patch
-  // chunk 0.99 -> 0.94 ms; 4: no further gain)
-  // (DYS: issuer 0 owns region H, issuer 1 region L -- no accumulator has two writers)
-  static constexpr int N_I = DYS ? ((TWO || HALVES) ? 2 : 1) : 3;
-#ifndef C5_NP
-#define C5_NP 5
-#endif
-  static constexpr int W_E = 0, W_P = 4, N_P = C5_NP, W_I = W_P + N_P, NT = (W_I + N_I) * 32;
+  // warps: epilogue, plane producers, the MMA issuer
+  static constexpr int W_E = 0, W_P = 4, N_P = 5, W_I = W_P + N_P, NT = (W_I + 1) * 32;
   static constexpr int ITEMS = (2 * PW + N_P * 32 - 1) / (N_P * 32);   // plane items per producer thread
-  static constexpr uint32_t TMEM_COLS = DYS ? 512 : (NACC * ACCW <= 256 ? 256 : 512);
-  static_assert(DYS ? ((TWO || HALVES) ? NACC * CI <= REGION : NACC * COUT <= 512) : NACC * ACCW <= 512,
-                "accumulators must fit tensor memory");
-#ifndef C5_FRAG_EPI
-#define C5_FRAG_EPI 1
-#endif
-  static constexpr bool FRAG_EPI = C5_FRAG_EPI != 0 && DYS && !TWO && MODE_ == 1;   // fragment-layout epilogue
-  static_assert(!HALVES || FRAG_EPI, "the per-pixel epilogue reads one region only");
-  static constexpr int MAXROWS = 256 / CI;            // DYS: output rows per instruction (N <= 256)
+  static constexpr uint32_t TMEM_COLS = 512;
+  static_assert(NACC * COUT <= 512, "accumulators must fit tensor memory");
+  static constexpr int MAXROWS = 256 / COUT;          // output rows per instruction (N <= 256)
   static_assert(CIN % 16 == 0 && COUT % 16 == 0, "channel counts");
   static_assert(SMEM_BYTES + 1024 <= 232448, "shared memory");
 };
@@ -178,10 +131,10 @@ struct Cfg {
 struct Images {
   float sw, inv_sw;        // weights were multiplied by sw
   float pad_[2];
-  // DYS layout: [hi | lo][dx][slice][row = (4 - dy) * 32 + n2][16 ci], every block canonical K-major
-  // (8-row groups 256 bytes apart); otherwise rows = n2 (hi 0..31, lo 32..63), k = tap*64 + ci
+  // [hi | lo][dx][slice][row = (4 - dy) * C_out + n][16 ci], every block canonical K-major
+  // (8-row groups 256 bytes apart); n = n2 (forward) / n1 (deltas)
   unsigned char fwd[Cfg<64, 32, 0>::W_BYTES];
-  unsigned char d1[Cfg<32, 64, 1>::W_BYTES];    // rows = n1 (hi 0..63, lo 64..127), k = tap*32 + ci
+  unsigned char d1[Cfg<32, 64, 1>::W_BYTES];
 };
 static_assert(offsetof(Images, fwd) % 16 == 0 && offsetof(Images, d1) % 16 == 0, "uint4 copies");
 
@@ -216,19 +169,14 @@ __global__ void __launch_bounds__(256) prepare_kernel(const float* __restrict__ 
     for (int i = gtid; i < N2 * KT; i += gn) {
       const int n = i / KT, k = i % KT;            // k = t*64 + ci
       unsigned short hi, lo;
-      fused_hp::split_h(__ldg(w2 + (size_t)k * N2 + n) * sw, hi, lo);
+      tc::split_h(__ldg(w2 + (size_t)k * N2 + n) * sw, hi, lo);
       using FC = Cfg<64, 32, 0>;
-      if (FC::DYS) {
-        const int t = k / N1, ci = k % N1, dy = t / F, dx = t % F, c = ci / 16, kk = ci % 16;
-        const int row = (F - 1 - dy) * N2 + n;
-        const int off = ((dx * FC::NSLICE + c) * FC::BLK_BYTES) / 2 + (row >> 3) * 128 + (kk >> 3) * 64 +
-                        (row & 7) * 8 + (kk & 7);
-        f[off] = __ushort_as_half(hi);
-        f[FC::IMG_L / 2 + off] = __ushort_as_half(lo);
-      } else {
-        f[fused_hp::kmajor16(n, k, KT)] = __ushort_as_half(hi);
-        f[fused_hp::kmajor16(N2 + n, k, KT)] = __ushort_as_half(lo);
-      }
+      const int t = k / N1, ci = k % N1, dy = t / F, dx = t % F, c = ci / 16, kk = ci % 16;
+      const int row = (F - 1 - dy) * N2 + n;
+      const int off = ((dx * FC::NSLICE + c) * FC::BLK_BYTES) / 2 + (row >> 3) * 128 + (kk >> 3) * 64 +
+                      (row & 7) * 8 + (kk & 7);
+      f[off] = __ushort_as_half(hi);
+      f[FC::IMG_L / 2 + off] = __ushort_as_half(lo);
     }
   }
   {   // deltas image: Wg[t][ci = k2][co = n1] = W2[24 - t][n1][k2]
@@ -237,19 +185,14 @@ __global__ void __launch_bounds__(256) prepare_kernel(const float* __restrict__ 
       const int n = i / KT, k = i % KT;            // k = t*32 + ci
       const int t = k / N2, ci = k % N2;
       unsigned short hi, lo;
-      fused_hp::split_h(__ldg(w2 + ((size_t)(T - 1 - t) * N1 + n) * N2 + ci) * sw, hi, lo);
+      tc::split_h(__ldg(w2 + ((size_t)(T - 1 - t) * N1 + n) * N2 + ci) * sw, hi, lo);
       using DC = Cfg<32, 64, 1>;
-      if (DC::DYS) {
-        const int dy = t / F, dx = t % F, c = ci / 16, kk = ci % 16;
-        const int row = (F - 1 - dy) * DC::CI + n % DC::CI, half = n / DC::CI;
-        const int off = (((dx * DC::NSLICE + c) * DC::NH + half) * DC::BLK_BYTES) / 2 + (row >> 3) * 128 +
-                        (kk >> 3) * 64 + (row & 7) * 8 + (kk & 7);
-        d[off] = __ushort_as_half(hi);
-        d[DC::IMG_L / 2 + off] = __ushort_as_half(lo);
-      } else {
-        d[fused_hp::kmajor16(n, k, KT)] = __ushort_as_half(hi);
-        d[fused_hp::kmajor16(N1 + n, k, KT)] = __ushort_as_half(lo);
-      }
+      const int dy = t / F, dx = t % F, c = ci / 16, kk = ci % 16;
+      const int row = (F - 1 - dy) * N1 + n;
+      const int off = ((dx * DC::NSLICE + c) * DC::BLK_BYTES) / 2 + (row >> 3) * 128 + (kk >> 3) * 64 +
+                      (row & 7) * 8 + (kk & 7);
+      d[off] = __ushort_as_half(hi);
+      d[DC::IMG_L / 2 + off] = __ushort_as_half(lo);
     }
   }
 }
@@ -268,12 +211,6 @@ struct Args {
 template <class C>
 __global__ void __launch_bounds__(C::NT, 1) conv5_tc_kernel(Args a) {
   using namespace tc;
-  using fused_hp::make_idesc_f16;
-  using fused_hp::mma_f16_ss;
-  using fused_hp::split_h2;
-  using fused_pl::elect_one;
-  using fused_pl::tmem_ld16_nowait;
-  using fused_pl::tmem_ld_wait;
   extern __shared__ __align__(128) uint8_t smem_raw[];
   __shared__ __align__(8) uint64_t full[C::NSLOT], empty[C::NSLOT], done[C::NACC], acc_free[C::NACC];
   __shared__ uint32_t tmem_slot;
@@ -307,10 +244,10 @@ __global__ void __launch_bounds__(C::NT, 1) conv5_tc_kernel(Args a) {
     if (smem_u32(smem_raw) & 127u) __trap();
     for (int i = 0; i < C::NSLOT; i++) {
       mbar_init(&full[i], C::N_P * 32);
-      mbar_init(&empty[i], C::N_I);
+      mbar_init(&empty[i], 1);
     }
     for (int i = 0; i < C::NACC; i++) {
-      mbar_init(&done[i], C::DYS ? C::N_I : 1);
+      mbar_init(&done[i], 1);
       mbar_init(&acc_free[i], 128);
     }
   }
@@ -322,10 +259,6 @@ __global__ void __launch_bounds__(C::NT, 1) conv5_tc_kernel(Args a) {
 
   const float s_in = scale_for(__uint_as_float(__ldg(a.in_max)));
   const float sw = __ldg(a.sw);
-
-  // first / last input row that contributes to output row rho (rho = r - dy + P)
-  auto r_first = [&](int rho) { return max(rho - P, 0); };
-  auto r_last = [&](int rho) { return min(rho - P + (F - 1), ih - 1); };
 
   if (warp >= C::W_P && warp < C::W_P + C::N_P) {
     // ============================ P: plane producers ==========================================
@@ -399,246 +332,167 @@ __global__ void __launch_bounds__(C::NT, 1) conv5_tc_kernel(Args a) {
       }
     }
   } else if (warp >= C::W_I) {
-    // ============================ I0 / I1: MMA issuers ========================================
-    const int me = warp - C::W_I;                       // owns output rows rho % N_I == me
-    const uint32_t idesc = make_idesc_f16(C::M, C::COUT);
-    const uint32_t idesc2 = make_idesc_f16(C::M, 2 * C::COUT);   // stacked [W_hi ; W_lo]
+    // ============================ I: MMA issuer ===============================================
+    // Input row r feeds output rows rho = r - dy + P; a row is first touched at input row
+    // max(rho - P, 0) (slice 0, dx = 0) and complete after input row min(rho - P + 4, ih - 1).
     const uint32_t sW = smem_u32(smem_raw + C::oW);
     const uint32_t sS = smem_u32(smem_raw + C::oSlots);
     auto adesc = [](uint32_t addr) -> uint64_t {        // K-major, LBO = plane stride, SBO = 128
       return (uint64_t)((addr >> 4) & 0x3FFF) | ((uint64_t)((C::PB >> 4) & 0x3FFF) << 16) |
              ((uint64_t)(128 >> 4) << 32) | ((uint64_t)1 << 46);
     };
-    auto wdesc = [](uint32_t addr) -> uint64_t {        // canonical K-major image
+    auto bdesc = [](uint32_t addr) -> uint64_t {        // image block: LBO = 128, SBO = 256
       return (uint64_t)((addr >> 4) & 0x3FFF) | ((uint64_t)(128 >> 4) << 16) |
-             ((uint64_t)((C::W_SBO >> 4) & 0x3FFF) << 32) | ((uint64_t)1 << 46);
+             ((uint64_t)(256 >> 4) << 32) | ((uint64_t)1 << 46);
     };
-    constexpr uint32_t W_LO = (uint32_t)(C::COUT / 8) * C::W_SBO;   // first W_lo row group
+    constexpr uint64_t kImgL = (uint64_t)(C::IMG_L >> 4);             // descriptor address units
+    constexpr uint64_t kDx = (uint64_t)((C::NSLICE * C::BLK_BYTES) >> 4);
     int it = 0;
-    if (C::DYS) {
-      // ---- dy-stacked issue.  Input row r feeds output rows rho = r - dy + P; a row is first
-      // touched at input row max(rho - P, 0) (slice 0, dx = 0) and complete after input row
-      // min(rho - P + 4, ih - 1).  TWO: me = 0 issues region H (hi.w_hi + lo.w_hi), me = 1 region L
-      // (hi.w_lo); else the one issuer puts all three products into the row's accumulator.
-      auto bdesc = [](uint32_t addr) -> uint64_t {      // image block: LBO = 128, SBO = 256
-        return (uint64_t)((addr >> 4) & 0x3FFF) | ((uint64_t)(128 >> 4) << 16) |
-               ((uint64_t)(256 >> 4) << 32) | ((uint64_t)1 << 46);
-      };
-      const uint32_t region = tmem + (uint32_t)((C::TWO || C::HALVES) ? me * C::REGION : 0);
-      const uint32_t imgH = sW + (uint32_t)((C::TWO && me == 1) ? C::IMG_L : 0) +
-                            (uint32_t)(C::HALVES ? me * C::BLK_BYTES : 0);
-      constexpr uint64_t kImgL = (uint64_t)(C::IMG_L >> 4);             // descriptor address units
-      constexpr uint64_t kDx = (uint64_t)((C::NSLICE * C::NH * C::BLK_BYTES) >> 4);
-      for (int r = 0; r < ih; r++) {
-        const int dy_lo = max(0, r + P - (oh - 1)), dy_hi = min(F - 1, r + P);
-        // the instructions of one (slice, dx) step of this input row: rows of dy = dy_hi .. dy_lo
-        // (rho ascending) -> slots (r - dy + P) % NACC, cut where the ring wraps and at MAXROWS
-        // rows.  At most 3 pieces; computed once per input row, the issue loop only adds offsets.
-        uint32_t seg_d[3], seg_i[3];
-        uint64_t seg_b[3];
-        int nseg = 0;
-        auto cut = [&](int a0, int b0, uint32_t (&sd)[3], uint64_t (&sb)[3], uint32_t (&si)[3]) {
-          int n_out = 0, b = b0;
-#pragma unroll
-          for (int q = 0; q < 3; q++)      // static indices: the tables stay in registers
-            if (b >= a0) {
-              const int s0 = (r - b + P) % C::NACC;
-              const int n = min(min(b - a0 + 1, C::NACC - s0), C::MAXROWS);
-              sd[q] = (uint32_t)(s0 * C::CI);
-              sb[q] = (uint64_t)(((F - 1 - b) * C::CI * 32) >> 4);
-              si[q] = make_idesc_f16(C::M, n * C::CI);
-              n_out = q + 1;
-              b -= n;
-            }
-          return n_out;
-        };
-        nseg = cut(dy_lo, dy_hi, seg_d, seg_b, seg_i);
-        for (int c = 0; c < C::NSLICE; c++, it++) {
-          const int slot = it % C::NSLOT;
-          mbar_wait(&full[slot], (uint32_t)((it / C::NSLOT) & 1));
-          if (c == 0 && dy_lo == 0 && r + P >= C::NACC)   // row r + P starts: its slot's last row has left
-            mbar_wait(&acc_free[(r + P) % C::NACC], (uint32_t)((((r + P) / C::NACC) - 1) & 1));
-          tcgen05_fence_after();
-          const uint32_t ah = sS + slot * C::SLOT_BYTES, al = ah + 2 * C::PB;
-          if (elect_one()) {
-            const uint64_t dah0 = adesc(ah), dal0 = adesc(al);
-            const uint64_t blk0 = bdesc(imgH + (uint32_t)(c * C::NH * C::BLK_BYTES));
-            // all products of the pieces, in a fixed order
-            auto step = [&](uint64_t dah, uint64_t dal, uint64_t blk, int ns, const uint32_t (&sd)[3],
-                            const uint64_t (&sb)[3], const uint32_t (&si)[3], uint32_t acc_flag) {
-#pragma unroll
-              for (int q = 0; q < 3; q++)
-                if (q < ns) {
-                  mma_f16_ss(region + sd[q], dah, blk + sb[q], si[q], acc_flag);          // hi.w_hi (me = 1: hi.w_lo)
-                  if (!C::TWO) mma_f16_ss(region + sd[q], dah, blk + kImgL + sb[q], si[q], 1u);   // hi.w_lo
-                  if (!C::TWO || me == 0) mma_f16_ss(region + sd[q], dal, blk + sb[q], si[q], 1u);   // lo.w_hi
-                }
-            };
-            int dx0 = 0;
-            if (c == 0 && (r == 0 || dy_lo == 0)) {      // rows start here: their first product overwrites
-              uint32_t fd[3], fi[3];
-              uint64_t fb[3];
-              const int f_hi = r == 0 ? dy_hi : 0;       // at r = 0 every row is new, later only dy = 0
-              int nf = cut(dy_lo, f_hi, fd, fb, fi);
-              step(dah0, dal0, blk0, nf, fd, fb, fi, 0u);
-              if (f_hi < dy_hi) {
-                nf = cut(f_hi + 1, dy_hi, fd, fb, fi);
-                step(dah0, dal0, blk0, nf, fd, fb, fi, 1u);
-              }
-              dx0 = 1;
-            }
-            if (dx0 == 0) step(dah0, dal0, blk0, nseg, seg_d, seg_b, seg_i, 1u);
-#pragma unroll
-            for (int dx = 1; dx < F; dx++)
-              step(dah0 + dx, dal0 + dx, blk0 + dx * kDx, nseg, seg_d, seg_b, seg_i, 1u);
-            if (c == C::NSLICE - 1)
-              for (int dy = dy_lo; dy <= dy_hi; dy++) {
-                const int rho = r - dy + P;
-                if (r == min(rho - P + (F - 1), ih - 1)) mma_commit(&done[rho % C::NACC]);
-              }
-            mma_commit(&empty[slot]);
-          }
-          __syncwarp();
-        }
-      }
-    } else
     for (int r = 0; r < ih; r++) {
+      const int dy_lo = max(0, r + P - (oh - 1)), dy_hi = min(F - 1, r + P);
+      // the instructions of one (slice, dx) step of this input row: rows of dy = dy_hi .. dy_lo
+      // (rho ascending) -> slots (r - dy + P) % NACC, cut where the ring wraps and at MAXROWS
+      // rows.  At most 3 pieces; computed once per input row, the issue loop only adds offsets.
+      uint32_t seg_d[3], seg_i[3];
+      uint64_t seg_b[3];
+      int nseg = 0;
+      auto cut = [&](int a0, int b0, uint32_t (&sd)[3], uint64_t (&sb)[3], uint32_t (&si)[3]) {
+        int n_out = 0, b = b0;
+#pragma unroll
+        for (int q = 0; q < 3; q++)      // static indices: the tables stay in registers
+          if (b >= a0) {
+            const int s0 = (r - b + P) % C::NACC;
+            const int n = min(min(b - a0 + 1, C::NACC - s0), C::MAXROWS);
+            sd[q] = (uint32_t)(s0 * C::COUT);
+            sb[q] = (uint64_t)(((F - 1 - b) * C::COUT * 32) >> 4);
+            si[q] = make_idesc_f16(C::M, n * C::COUT);
+            n_out = q + 1;
+            b -= n;
+          }
+        return n_out;
+      };
+      nseg = cut(dy_lo, dy_hi, seg_d, seg_b, seg_i);
       for (int c = 0; c < C::NSLICE; c++, it++) {
         const int slot = it % C::NSLOT;
         mbar_wait(&full[slot], (uint32_t)((it / C::NSLOT) & 1));
+        if (c == 0 && dy_lo == 0 && r + P >= C::NACC)   // row r + P starts: its slot's last row has left
+          mbar_wait(&acc_free[(r + P) % C::NACC], (uint32_t)((((r + P) / C::NACC) - 1) & 1));
         tcgen05_fence_after();
         const uint32_t ah = sS + slot * C::SLOT_BYTES, al = ah + 2 * C::PB;
-        // MMAs into one accumulator stay consecutive: interleaving the rows of a slice across
-        // accumulators measured 30-40 % SLOWER (r2c: 829 vs 599 us forward, 580 vs 475 us deltas)
-        bool issued = false;
-#pragma unroll 1
-        for (int dy = 0; dy < F; dy++) {
-          const int rho = r - dy + P;
-          if (rho < 0 || rho >= oh || (rho % C::N_I) != me) continue;
-          const int acc = rho % C::NACC;
-          const bool first = (r == r_first(rho)) && c == 0;
-          if (first && rho >= C::NACC) {                 // the accumulator's previous row has left
-            mbar_wait(&acc_free[acc], (uint32_t)(((rho / C::NACC) - 1) & 1));
-            tcgen05_fence_after();
-          }
-          const uint32_t d = tmem + (uint32_t)(acc * C::ACCW);
-          if (elect_one()) {
-#pragma unroll
-            for (int dx = 0; dx < F; dx++) {
-              // K-step (tap, slice): 16 halves = 2 core matrices of the image
-              const uint32_t wk = sW + (uint32_t)(((dy * F + dx) * C::CIN + c * 16) / 8) * 128u;
-              const uint64_t dah = adesc(ah + dx * 16), dal = adesc(al + dx * 16);
-              const uint64_t dwh = wdesc(wk), dwl = wdesc(wk + W_LO);
-              const uint32_t fresh = (first && dx == 0) ? 0u : 1u;
-              if (C::STACK) {
-                mma_f16_ss(d, dah, dwh, idesc2, fresh);       // [hi.w_hi | hi.w_lo]
-                mma_f16_ss(d, dal, dwh, idesc, 1u);           // + lo.w_hi
-              } else {
-                mma_f16_ss(d, dah, dwh, idesc, fresh);
-                mma_f16_ss(d, dah, dwl, idesc, 1u);
-                mma_f16_ss(d, dal, dwh, idesc, 1u);
-              }
-            }
-            if (r == r_last(rho) && c == C::NSLICE - 1) mma_commit(&done[acc]);
-          }
-          __syncwarp();
-          issued = true;
-        }
         if (elect_one()) {
-          if (issued) mma_commit(&empty[slot]);
-          else mbar_arrive(&empty[slot]);
+          const uint64_t dah0 = adesc(ah), dal0 = adesc(al);
+          const uint64_t blk0 = bdesc(sW + (uint32_t)(c * C::BLK_BYTES));
+          // all products of the pieces, in a fixed order
+          auto step = [&](uint64_t dah, uint64_t dal, uint64_t blk, int ns, const uint32_t (&sd)[3],
+                          const uint64_t (&sb)[3], const uint32_t (&si)[3], uint32_t acc_flag) {
+#pragma unroll
+            for (int q = 0; q < 3; q++)
+              if (q < ns) {
+                mma_f16_ss(tmem + sd[q], dah, blk + sb[q], si[q], acc_flag);      // hi.w_hi
+                mma_f16_ss(tmem + sd[q], dah, blk + kImgL + sb[q], si[q], 1u);    // hi.w_lo
+                mma_f16_ss(tmem + sd[q], dal, blk + sb[q], si[q], 1u);            // lo.w_hi
+              }
+          };
+          int dx0 = 0;
+          if (c == 0 && (r == 0 || dy_lo == 0)) {      // rows start here: their first product overwrites
+            uint32_t fd[3], fi[3];
+            uint64_t fb[3];
+            const int f_hi = r == 0 ? dy_hi : 0;       // at r = 0 every row is new, later only dy = 0
+            int nf = cut(dy_lo, f_hi, fd, fb, fi);
+            step(dah0, dal0, blk0, nf, fd, fb, fi, 0u);
+            if (f_hi < dy_hi) {
+              nf = cut(f_hi + 1, dy_hi, fd, fb, fi);
+              step(dah0, dal0, blk0, nf, fd, fb, fi, 1u);
+            }
+            dx0 = 1;
+          }
+          if (dx0 == 0) step(dah0, dal0, blk0, nseg, seg_d, seg_b, seg_i, 1u);
+#pragma unroll
+          for (int dx = 1; dx < F; dx++)
+            step(dah0 + dx, dal0 + dx, blk0 + dx * kDx, nseg, seg_d, seg_b, seg_i, 1u);
+          if (c == C::NSLICE - 1)
+            for (int dy = dy_lo; dy <= dy_hi; dy++) {
+              const int rho = r - dy + P;
+              if (r == min(rho - P + (F - 1), ih - 1)) mma_commit(&done[rho % C::NACC]);
+            }
+          mma_commit(&empty[slot]);
         }
         __syncwarp();
       }
     }
-  } else {
-    // ============================ E: epilogue =================================================
-    if (C::FRAG_EPI) {
-      // MODE 1 with the accumulator read as 16x256b fragments (the layout of an mma accumulator:
-      // a thread holds 2 adjacent channels of rows lane/4 and lane/4 + 8 of a 16-lane half, for
-      // every group of 8 channels), so that 4 lanes cover 32 contiguous bytes of a pixel and an
-      // 8-byte access per lane touches 8 lines per instruction.  With one pixel per lane (64
-      // channels = 256 bytes apart) every 16-byte access of a warp touched 32 lines, and the L1
-      // pipe -- mask loads and d1 stores of the epilogue -- was what bound the kernel (81 % busy
-      // at 53 % tensor-pipe activity, profiles/r3l_ncu_summary.txt).
-      const int q4 = lane >> 2, l4 = lane & 3;
-      long long ob[4];   // pixels (warp & 3) * 32 + j * 8 + lane / 4
+  } else if (C::MODE == 1) {
+    // ============================ E: epilogue of the deltas ===================================
+    // The accumulator is read as 16x256b fragments (the layout of an mma accumulator:
+    // a thread holds 2 adjacent channels of rows lane/4 and lane/4 + 8 of a 16-lane half, for
+    // every group of 8 channels), so that 4 lanes cover 32 contiguous bytes of a pixel and an
+    // 8-byte access per lane touches 8 lines per instruction.  With one pixel per lane (64
+    // channels = 256 bytes apart) every 16-byte access of a warp touched 32 lines, and the L1
+    // pipe -- mask loads and d1 stores of the epilogue -- was what bound the kernel (81 % busy
+    // at 53 % tensor-pipe activity, profiles/r3l_ncu_summary.txt).
+    const int q4 = lane >> 2, l4 = lane & 3;
+    long long ob[4];   // pixels (warp & 3) * 32 + j * 8 + lane / 4
+#pragma unroll
+    for (int j = 0; j < 4; j++) {
+      const long long vo = X0 + (warp & 3) * 32 + j * 8 + q4;
+      ob[j] = -1;
+      if (vo < vw) {
+        const int smp = (int)(vo / slot_w), x = (int)(vo - (long long)smp * slot_w);
+        if (x < ow) ob[j] = (((long long)smp * oh) * ow + x) * C::COUT + 2 * l4;
+      }
+    }
+    const long long orow_f = (long long)ow * C::COUT;
+    const float csf = 1.f / (s_in * sw);
+    for (int rho = 0; rho < oh; rho++) {
+      const int acc = rho % C::NACC;
+      // the relu' mask of this row does not depend on the accumulator: all its loads are in
+      // flight while the row's MMAs finish (issued after the wait, their HBM round trips --
+      // several dependent batches per row -- were the row period)
+      float2 gm[4][C::COUT / 8];
+#pragma unroll
+      for (int j = 0; j < 4; j++)
+#pragma unroll
+        for (int g = 0; g < C::COUT / 8; g++)
+          gm[j][g] = ob[j] >= 0 ? __ldg(reinterpret_cast<const float2*>(a.aux + ob[j] + rho * orow_f + 8 * g))
+                                : make_float2(0.f, 0.f);
+      mbar_wait(&done[acc], (uint32_t)((rho / C::NACC) & 1));
+      tcgen05_fence_after();
+      uint32_t f[2][32];
+#pragma unroll
+      for (int h = 0; h < 2; h++) {
+        const uint32_t tl = tmem + ((uint32_t)((warp & 3) * 32 + h * 16) << 16);
+        const uint32_t ta = tl + (uint32_t)(acc * C::COUT);
+        asm volatile(
+            "tcgen05.ld.sync.aligned.16x256b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, "
+            "%13, %14, %15, %16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, "
+            "[%32];"
+            : "=r"(f[h][0]), "=r"(f[h][1]), "=r"(f[h][2]), "=r"(f[h][3]), "=r"(f[h][4]), "=r"(f[h][5]),
+              "=r"(f[h][6]), "=r"(f[h][7]), "=r"(f[h][8]), "=r"(f[h][9]), "=r"(f[h][10]), "=r"(f[h][11]),
+              "=r"(f[h][12]), "=r"(f[h][13]), "=r"(f[h][14]), "=r"(f[h][15]), "=r"(f[h][16]),
+              "=r"(f[h][17]), "=r"(f[h][18]), "=r"(f[h][19]), "=r"(f[h][20]), "=r"(f[h][21]),
+              "=r"(f[h][22]), "=r"(f[h][23]), "=r"(f[h][24]), "=r"(f[h][25]), "=r"(f[h][26]),
+              "=r"(f[h][27]), "=r"(f[h][28]), "=r"(f[h][29]), "=r"(f[h][30]), "=r"(f[h][31])
+            : "r"(ta));
+      }
+      tmem_ld_wait();
+      tcgen05_fence_before();
+      mbar_arrive(&acc_free[acc]);
+      // f[h][4 g + 2 s + e] = D[row h*16 + s*8 + lane/4][channel 8 g + 2 (lane%4) + e]
 #pragma unroll
       for (int j = 0; j < 4; j++) {
-        const long long vo = X0 + (warp & 3) * 32 + j * 8 + q4;
-        ob[j] = -1;
-        if (vo < vw) {
-          const int smp = (int)(vo / slot_w), x = (int)(vo - (long long)smp * slot_w);
-          if (x < ow) ob[j] = (((long long)smp * oh) * ow + x) * C::COUT + 2 * l4;
+        if (ob[j] < 0) continue;
+        const int h = j >> 1, sidx = j & 1;
+        float* o = a.out + ob[j] + rho * orow_f;
+#pragma unroll
+        for (int g = 0; g < C::COUT / 8; g++) {
+          const float x0 = __uint_as_float(f[h][4 * g + 2 * sidx]) * csf;
+          const float x1 = __uint_as_float(f[h][4 * g + 2 * sidx + 1]) * csf;
+          *reinterpret_cast<float2*>(o + 8 * g) =
+              make_float2(gm[j][g].x > 0.f ? x0 : 0.f, gm[j][g].y > 0.f ? x1 : 0.f);
         }
       }
-      const long long orow_f = (long long)ow * C::COUT;
-      const float csf = 1.f / (s_in * sw);
-      for (int rho = 0; rho < oh; rho++) {
-        const int acc = rho % C::NACC;
-        // the relu' mask of this row does not depend on the accumulator: all its loads are in
-        // flight while the row's MMAs finish (issued after the wait, their HBM round trips --
-        // several dependent batches per row -- were the row period)
-        float2 gm[4][C::COUT / 8];
-#pragma unroll
-        for (int j = 0; j < 4; j++)
-#pragma unroll
-          for (int g = 0; g < C::COUT / 8; g++)
-            gm[j][g] = ob[j] >= 0 ? __ldg(reinterpret_cast<const float2*>(a.aux + ob[j] + rho * orow_f + 8 * g))
-                                  : make_float2(0.f, 0.f);
-        mbar_wait(&done[acc], (uint32_t)((rho / C::NACC) & 1));
-        tcgen05_fence_after();
-        uint32_t f[2][32];
-#pragma unroll
-        for (int h = 0; h < 2; h++) {
-          const uint32_t tl = tmem + ((uint32_t)((warp & 3) * 32 + h * 16) << 16);
-          if (C::HALVES) {
-            // channels 0..31 in region 0, 32..63 in region 1 (slot = 32 columns in each)
-#pragma unroll
-            for (int hf = 0; hf < 2; hf++) {
-              uint32_t* ff = f[h] + 16 * hf;
-              asm volatile(
-                  "tcgen05.ld.sync.aligned.16x256b.x4.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, "
-                  "%13, %14, %15}, [%16];"
-                  : "=r"(ff[0]), "=r"(ff[1]), "=r"(ff[2]), "=r"(ff[3]), "=r"(ff[4]), "=r"(ff[5]), "=r"(ff[6]),
-                    "=r"(ff[7]), "=r"(ff[8]), "=r"(ff[9]), "=r"(ff[10]), "=r"(ff[11]), "=r"(ff[12]),
-                    "=r"(ff[13]), "=r"(ff[14]), "=r"(ff[15])
-                  : "r"(tl + (uint32_t)(hf * C::REGION + acc * C::CI)));
-            }
-            continue;
-          }
-          const uint32_t ta = tl + (uint32_t)(acc * C::COUT);
-          asm volatile(
-              "tcgen05.ld.sync.aligned.16x256b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, "
-              "%13, %14, %15, %16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, "
-              "[%32];"
-              : "=r"(f[h][0]), "=r"(f[h][1]), "=r"(f[h][2]), "=r"(f[h][3]), "=r"(f[h][4]), "=r"(f[h][5]),
-                "=r"(f[h][6]), "=r"(f[h][7]), "=r"(f[h][8]), "=r"(f[h][9]), "=r"(f[h][10]), "=r"(f[h][11]),
-                "=r"(f[h][12]), "=r"(f[h][13]), "=r"(f[h][14]), "=r"(f[h][15]), "=r"(f[h][16]),
-                "=r"(f[h][17]), "=r"(f[h][18]), "=r"(f[h][19]), "=r"(f[h][20]), "=r"(f[h][21]),
-                "=r"(f[h][22]), "=r"(f[h][23]), "=r"(f[h][24]), "=r"(f[h][25]), "=r"(f[h][26]),
-                "=r"(f[h][27]), "=r"(f[h][28]), "=r"(f[h][29]), "=r"(f[h][30]), "=r"(f[h][31])
-              : "r"(ta));
-        }
-        tmem_ld_wait();
-        tcgen05_fence_before();
-        mbar_arrive(&acc_free[acc]);
-        // f[h][4 g + 2 s + e] = D[row h*16 + s*8 + lane/4][channel 8 g + 2 (lane%4) + e]
-#pragma unroll
-        for (int j = 0; j < 4; j++) {
-          if (ob[j] < 0) continue;
-          const int h = j >> 1, sidx = j & 1;
-          float* o = a.out + ob[j] + rho * orow_f;
-#pragma unroll
-          for (int g = 0; g < C::COUT / 8; g++) {
-            const float x0 = __uint_as_float(f[h][4 * g + 2 * sidx]) * csf;
-            const float x1 = __uint_as_float(f[h][4 * g + 2 * sidx + 1]) * csf;
-            *reinterpret_cast<float2*>(o + 8 * g) =
-                make_float2(gm[j][g].x > 0.f ? x0 : 0.f, gm[j][g].y > 0.f ? x1 : 0.f);
-          }
-        }
-      }
-    } else {
+    }
+  } else {
+    // ============================ E: epilogue of the forward ==================================
     const uint32_t lane_base = (uint32_t)((warp & 3) * 32) << 16;
     const int m = (warp & 3) * 32 + lane;
     const long long vout = X0 + m;
@@ -656,50 +510,29 @@ __global__ void __launch_bounds__(C::NT, 1) conv5_tc_kernel(Args a) {
       mbar_wait(&done[acc], (uint32_t)((rho / C::NACC) & 1));
       tcgen05_fence_after();
       float v[C::COUT];
-      const uint32_t c0 = C::DYS ? (uint32_t)(acc * C::COUT) : (uint32_t)(acc * C::ACCW);
-      const uint32_t c1 = C::DYS ? (uint32_t)(C::REGION + acc * C::COUT) : (uint32_t)(acc * C::ACCW + C::COUT);
+      const uint32_t c0 = (uint32_t)(acc * C::COUT);
 #pragma unroll
       for (int g = 0; g < C::COUT / 16; g++)
         tmem_ld16_nowait(tmem + lane_base + c0 + g * 16, v + g * 16);
-      if (C::STACK || C::TWO) {
-        float v2[C::COUT];
-#pragma unroll
-        for (int g = 0; g < C::COUT / 16; g++)
-          tmem_ld16_nowait(tmem + lane_base + c1 + g * 16, v2 + g * 16);
-        tmem_ld_wait();
-#pragma unroll
-        for (int j = 0; j < C::COUT; j++) v[j] += v2[j];
-      }
       tmem_ld_wait();
       tcgen05_fence_before();
       mbar_arrive(&acc_free[acc]);
       if (obase < 0) continue;
       float4* o = reinterpret_cast<float4*>(a.out + obase + rho * orow);
-      if (C::MODE == 0) {
 #pragma unroll
-        for (int j = 0; j < C::COUT / 4; j++) {
-          const float4 r = make_float4(fmaxf(fmaf(v[4 * j], cs, sB[4 * j]), 0.f),
-                                       fmaxf(fmaf(v[4 * j + 1], cs, sB[4 * j + 1]), 0.f),
-                                       fmaxf(fmaf(v[4 * j + 2], cs, sB[4 * j + 2]), 0.f),
-                                       fmaxf(fmaf(v[4 * j + 3], cs, sB[4 * j + 3]), 0.f));
-          o[j] = r;
-          omax = fmaxf(fmaxf(omax, fmaxf(r.x, r.y)), fmaxf(r.z, r.w));
-        }
-      } else {
-        const float4* mk = reinterpret_cast<const float4*>(a.aux + obase + rho * orow);
-#pragma unroll
-        for (int j = 0; j < C::COUT / 4; j++) {
-          const float4 g = __ldg(mk + j);
-          o[j] = make_float4(g.x > 0.f ? v[4 * j] * cs : 0.f, g.y > 0.f ? v[4 * j + 1] * cs : 0.f,
-                             g.z > 0.f ? v[4 * j + 2] * cs : 0.f, g.w > 0.f ? v[4 * j + 3] * cs : 0.f);
-        }
+      for (int j = 0; j < C::COUT / 4; j++) {
+        const float4 r = make_float4(fmaxf(fmaf(v[4 * j], cs, sB[4 * j]), 0.f),
+                                     fmaxf(fmaf(v[4 * j + 1], cs, sB[4 * j + 1]), 0.f),
+                                     fmaxf(fmaf(v[4 * j + 2], cs, sB[4 * j + 2]), 0.f),
+                                     fmaxf(fmaf(v[4 * j + 3], cs, sB[4 * j + 3]), 0.f));
+        o[j] = r;
+        omax = fmaxf(fmaxf(omax, fmaxf(r.x, r.y)), fmaxf(r.z, r.w));
       }
     }
-    if (C::MODE == 0 && a.out_max) {
+    if (a.out_max) {
 #pragma unroll
       for (int o = 16; o > 0; o >>= 1) omax = fmaxf(omax, __shfl_xor_sync(0xffffffffu, omax, o));
       if (lane == 0 && omax > 0.f) atomicMax(a.out_max, __float_as_uint(omax));
-    }
     }
   }
 

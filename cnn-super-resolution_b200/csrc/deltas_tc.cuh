@@ -16,7 +16,6 @@
 #include <cuda_runtime.h>
 
 #include "context.cuh"
-#include "fused_forward_pl.cuh"
 #include "tc_common.cuh"
 
 namespace srcnn {
@@ -37,9 +36,6 @@ __global__ void __launch_bounds__(Cfg::NT, 1) f1_deltas_tc_kernel(const float* _
                                                                   long long P, int n_tiles_total) {
   using C = Cfg;
   using namespace tc;
-  using fused_pl::elect_one;
-  using fused_pl::tmem_ld16_nowait;
-  using fused_pl::tmem_ld_wait;
   using tc::mbar_arrive;
   __shared__ __align__(128) float sW[2 * C::N * C::K];   // [128][K]: rows 0..63 hi, 64..127 lo
   __shared__ __align__(8) uint64_t a_full[2], mma_done[2], d_free[2];

@@ -49,23 +49,10 @@ struct Cfg {
   static constexpr int PW = 144;                 // plane entries (16 bytes = 8 halves each)
   static constexpr int PB = PW * 16;             // bytes per plane
   static constexpr int RO = 4, RH = 4;           // ring slots: oct planes, H8 planes
-#ifndef HP_N_E1
-#define HP_N_E1 8
-#endif
   // role -> warp ids.  Every E role needs warp % 4 = its TMEM lane quarter, so E blocks start at
-  // multiples of 4; the plane producers are 4 + 1 warps (IMA: columns 0..127, IMB: 128..143).
-#ifndef HP_ORDER
-#define HP_ORDER 0
-#endif
-  static constexpr int N_E1 = HP_N_E1, N_IM = 5;
-#if HP_ORDER == 0
-  static constexpr int W_E1 = 0, W_E2 = N_E1, W_E3 = W_E2 + 4, W_IM = W_E3 + 4, N_IMA = 5, W_IMB = -1;
-#elif HP_ORDER == 1
-  static constexpr int W_IM = 0, N_IMA = 4, W_E1 = 4, W_E2 = W_E1 + N_E1, W_E3 = W_E2 + 4, W_IMB = W_E3 + 4;
-#else
-  static constexpr int W_IM = 0, N_IMA = 4, W_E3 = 4, W_E2 = 8, W_E1 = 12, W_IMB = W_E1 + N_E1;
-#endif
-  static constexpr int W_I1 = N_E1 + 8 + N_IM, W_I2 = W_I1 + 1, W_I3 = W_I2 + 1;
+  // multiples of 4.
+  static constexpr int W_E1 = 0, N_E1 = 8, W_E2 = N_E1, W_E3 = W_E2 + 4, W_IM = W_E3 + 4,
+                       N_IM = 5, W_I1 = W_IM + N_IM, W_I2 = W_I1 + 1, W_I3 = W_I2 + 1;
   static constexpr int NT = (W_I3 + 1) * 32;
   static constexpr int E1_CHUNKS = (N1 / 16) / (N_E1 / 4);   // 16-channel chunks per E1 warp
   static constexpr int IM_THREADS = N_IM * 32;
@@ -93,7 +80,7 @@ struct Cfg {
   // tensor memory columns (+ size * (b & 1)):
   //   D1: [0,64) hi.w_hi, [64,128) corrections  ->  A2: hi pairs of channels 16g..16g+15 at
   //       a2col(g) = 32*(g/2) + 8*(g%2), lo pairs at 64 + a2col(g): inside the columns the SAME
-  //       E1 warp has already read, whether 4 or 8 warps share the 64 channels
+  //       E1 warp has already read
   //   D2: [0,32), [32,64)                       ->  A3: [0,16) hi pairs, [32,48) lo pairs
   //   D3: [0,32), [32,64) (25 taps of 32 used)
   static constexpr uint32_t cD1 = 0, cD2 = 256, cD3 = 384;
@@ -148,11 +135,6 @@ struct Scales {
 };
 static_assert(offsetof(Scales, wimg) % 16 == 0 && sizeof(Scales) % 16 == 0, "uint4 copies");
 
-// K-major canonical layout for 16-bit elements: core matrix = 8 rows x 16 bytes (8 halves);
-// returns the offset in halves of (row r, element k) of a [rows][K] operand
-__host__ __device__ __forceinline__ int kmajor16(int r, int k, int K) {
-  return (r >> 3) * (64 * (K >> 3)) + (k >> 3) * 64 + (r & 7) * 8 + (k & 7);
-}
 // (K-step s, 16-byte chunk j, element e) of the layer-1 contraction -> filter tap, or -1.
 // chunks 0..8: O at dx = chunk (taps dy = e); chunk 9: H8 at dx' = 0 (taps (8, e));
 // chunk 10: H8 at dx' = 8 (tap (8,8) + 7 pads); chunk 11: pad
@@ -163,77 +145,13 @@ __host__ __device__ __forceinline__ int tap16(int s, int j, int e) {
   if (c == 10) return e == 0 ? 8 * Cfg::F1 + 8 : -1;
   return -1;
 }
-__host__ __device__ __forceinline__ uint32_t make_idesc_f16(int Mm, int Nn) {
-  // c_format = F32, a_format = b_format = F16, both K-major
-  return (1u << 4) | ((uint32_t)(Nn >> 3) << 17) | ((uint32_t)(Mm >> 4) << 24);
-}
-__device__ __forceinline__ void mma_f16_ss(uint32_t d, uint64_t a, uint64_t b, uint32_t idesc,
-                                           uint32_t acc) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}\n" ::"r"(d),
-      "l"(a), "l"(b), "r"(idesc), "r"(acc)
-      : "memory");
-}
-__device__ __forceinline__ void mma_f16_ts(uint32_t d, uint32_t a, uint64_t b, uint32_t idesc,
-                                           uint32_t acc) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}\n" ::"r"(d),
-      "r"(a), "l"(b), "r"(idesc), "r"(acc)
-      : "memory");
-}
-// xs = hi + lo (raw half bits)
-__device__ __forceinline__ void split_h(float xs, unsigned short& hi, unsigned short& lo) {
-  const __half h = __float2half_rn(xs);
-  hi = __half_as_ushort(h);
-  lo = __half_as_ushort(__float2half_rn(xs - __half2float(h)));
-}
-// two values -> packed pairs (element 0 in the low half: K index order)
-__device__ __forceinline__ void split_h2(float a, float b, uint32_t& hi, uint32_t& lo) {
-  const __half2 h = __floats2half2_rn(a, b);
-  const float2 hf = __half22float2(h);
-  const __half2 l = __floats2half2_rn(a - hf.x, b - hf.y);
-  hi = *reinterpret_cast<const uint32_t*>(&h);
-  lo = *reinterpret_cast<const uint32_t*>(&l);
-}
-__device__ __forceinline__ uint32_t pack2(unsigned short a, unsigned short b) {
-  return (uint32_t)a | ((uint32_t)b << 16);
-}
-__device__ __forceinline__ void tmem_st8u(uint32_t taddr, const uint32_t v[8]) {
-  asm volatile(
-      "tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"r"(taddr),
-      "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7])
-      : "memory");
-}
 
 #ifdef PL_TRACE
 using fused_pl::pl_trace;
 #endif
 using fused_pl::BatchExt;
-using fused_pl::elect_one;
-using fused_pl::tmem_ld16_nowait;
-using fused_pl::tmem_ld_wait;
 using tc::mbar_arrive;
 using tc::named_bar_sync;
-
-// HP_L1WIDE (experiment, default off): in the layer-1-only launch the warps of the idle E2 / E3
-// roles take channel chunks too -- 16 warps of one 16-channel chunk each instead of 8 of two.
-// Same results; a C4 chunk of 3 028 patches takes 2.226 ms instead of 2.200 (64-byte runs per
-// pixel in the out1 stores instead of 128): E1's arithmetic is not that launch's bound.
-#ifndef HP_L1WIDE
-#define HP_L1WIDE 0
-#endif
-// HP_SPIN (experiment): bit 0 -- the three MMA issuers poll their barriers (test_wait, never
-// parked) instead of try_wait with a suspend hint; bit 1 -- E1 polls bar1 likewise
-#ifndef HP_SPIN
-#define HP_SPIN 0
-#endif
-__device__ __forceinline__ void mbar_poll(uint64_t* bar, uint32_t parity) {
-  while (!tc::mbar_test(bar, parity)) {}
-}
-#define HP_IWAIT(bar, par) { if (HP_SPIN & 1) mbar_poll(bar, par); else tc::mbar_wait(bar, par); }
-#define HP_EWAIT(bar, par) { if (HP_SPIN & 2) mbar_poll(bar, par); else tc::mbar_wait(bar, par); }
 
 #ifdef HP_PROF
 // kernel-development aid: per-warp cycles spent blocked at each hand-off of CTA (1,1,0), read
@@ -250,17 +168,12 @@ __device__ unsigned hp_prof[32][4];
 // the plane producers of the main kernel, which see every pixel anyway: the first |x| >= 64 (or
 // NaN) clears `ok`, and the TF32 kernel launched behind redoes the launch.
 constexpr float kInMax = 64.f;
-__device__ __forceinline__ float pow2_scale(float bound) {   // 2^14 / pow2ceil(bound)
-  if (!(bound > 0.f) || !(bound < 1e30f)) return 1.f;
-  int e;
-  frexpf(bound, &e);                 // bound = f * 2^e, f in [0.5, 1)
-  return ldexpf(1.f, 14 - e);
-}
 // `in_max` (may be null): bit pattern of the largest |input| of the launch, measured on the
 // device -- the input scale then follows the data (no domain restriction, no fallback); used by
 // the layer-1-only launches, where a.pw2 / a.pw3 are null.
 __global__ void __launch_bounds__(256) hp_prepare_kernel(fused::Args a, Scales* sc,
                                                          const unsigned* in_max = nullptr) {
+  using namespace tc;
   // the parameters are staged in shared memory with coalesced loads first: the column sums
   // below would otherwise be chains of dependent global loads (13 us instead of ~3)
   __shared__ float sw1[Cfg::F1 * Cfg::F1 * Cfg::N1];   // |W1| [tap][n]
@@ -443,8 +356,8 @@ __global__ void __launch_bounds__(Cfg::NT, 1) forward_fused_hp_kernel(fused::Arg
     for (int i = 0; i < 2; i++) {
       mbar_init(&bar1[i], 1);
       mbar_init(&a2_full[i], C::N_E1 * 32);
-      mbar_init(&bar2[i], (L1ONLY && !C::A2SEP) ? (HP_L1WIDE ? 16 : C::N_E1) * 32 : 1);
-      mbar_init(&d1_free[i], ((L1ONLY && HP_L1WIDE) ? 16 : C::N_E1) * 32);
+      mbar_init(&bar2[i], (L1ONLY && !C::A2SEP) ? C::N_E1 * 32 : 1);
+      mbar_init(&d1_free[i], C::N_E1 * 32);
       mbar_init(&a3_full[i], 128);
       mbar_init(&bar3[i], 1);
       mbar_init(&d3_free[i], 128);
@@ -463,7 +376,7 @@ __global__ void __launch_bounds__(Cfg::NT, 1) forward_fused_hp_kernel(fused::Arg
   const unsigned _hstart = (unsigned)clock();
 #endif
 
-  const bool is_im = (warp >= C::W_IM && warp < C::W_IM + C::N_IMA) || warp == C::W_IMB;
+  const bool is_im = warp >= C::W_IM && warp < C::W_IM + C::N_IM;
   const bool is_e1 = warp >= C::W_E1 && warp < C::W_E1 + C::N_E1;
   const bool is_e2 = warp >= C::W_E2 && warp < C::W_E2 + 4;
   const bool is_e3 = warp >= C::W_E3 && warp < C::W_E3 + 4;
@@ -472,7 +385,7 @@ __global__ void __launch_bounds__(Cfg::NT, 1) forward_fused_hp_kernel(fused::Arg
     // thread c owns plane column c (image column X0+c): per input row r it writes
     // H8(r)[c] = in[r][c..c+7] and O(r-7)[c] = (in[r-7..r][c]); the 7 older rows of the column
     // live in registers as halves.
-    const int c = warp == C::W_IMB ? C::N_IMA * 32 + lane : tid - C::W_IM * 32;
+    const int c = tid - C::W_IM * 32;
     const bool active = c < C::PW;
     const int gx = X0 + c;
     uint8_t* pOh = smem_raw + C::oOh + c * 16;
@@ -574,9 +487,9 @@ __global__ void __launch_bounds__(Cfg::NT, 1) forward_fused_hp_kernel(fused::Arg
              ((uint64_t)(128 >> 4) << 32) | ((uint64_t)1 << 46);
     };
     for (int t = 0; t < n_tiles; t++) {
-      HPW(0, HP_IWAIT(&p_full[t & 3], (uint32_t)((t >> 2) & 1)))
+      HPW(0, mbar_wait(&p_full[t & 3], (uint32_t)((t >> 2) & 1)))
       // D1[t&1] still holds A2(t-2) until MMA-2(t-2) has read it
-      if (t >= 2) HPW(1, HP_IWAIT(C::A2SEP ? &d1_free[t & 1] : &bar2[t & 1], (uint32_t)(((t - 2) >> 1) & 1)))
+      if (t >= 2) HPW(1, mbar_wait(C::A2SEP ? &d1_free[t & 1] : &bar2[t & 1], (uint32_t)(((t - 2) >> 1) & 1)))
       tcgen05_fence_after();
       const uint32_t d1 = tmem + C::cD1 + 128u * (uint32_t)(t & 1);
       const uint32_t so = (uint32_t)(t & (C::RO - 1)) * C::PB;
@@ -607,7 +520,7 @@ __global__ void __launch_bounds__(Cfg::NT, 1) forward_fused_hp_kernel(fused::Arg
 #endif
       PL_EV(t, 1)
     }
-  } else if (L1ONLY && !is_e1 && !(HP_L1WIDE && (is_e2 || is_e3))) {
+  } else if (L1ONLY && !is_e1) {
     // layer-1-only launch: the layer-2 / layer-3 roles have nothing to do
   } else if (warp == C::W_I2) {
     // ============================ I2: layer-2 MMA issuer (A2 in TMEM) ======================
@@ -615,9 +528,9 @@ __global__ void __launch_bounds__(Cfg::NT, 1) forward_fused_hp_kernel(fused::Arg
     const uint32_t idesc_lo = make_idesc_f16(C::M, C::N2);
     const uint64_t wdesc = make_desc_kmajor(sW2, 0, 128, 128 * (C::K2 / 8));
     for (int t = 0; t < n_tiles; t++) {
-      HPW(0, HP_IWAIT(&a2_full[t & 1], (uint32_t)((t >> 1) & 1)))
+      HPW(0, mbar_wait(&a2_full[t & 1], (uint32_t)((t >> 1) & 1)))
       // D2[t&1] still holds A3(t-2) until MMA-3(t-2) has read it
-      if (t >= 2) HPW(1, HP_IWAIT(&bar3[t & 1], (uint32_t)(((t - 2) >> 1) & 1)))
+      if (t >= 2) HPW(1, mbar_wait(&bar3[t & 1], (uint32_t)(((t - 2) >> 1) & 1)))
       tcgen05_fence_after();
       const uint32_t a2 = tmem + C::cA2 + C::sA2 * (uint32_t)(t & 1);
       const uint32_t d2 = tmem + C::cD2x + C::sD2 * (uint32_t)(t & 1);
@@ -654,8 +567,8 @@ __global__ void __launch_bounds__(Cfg::NT, 1) forward_fused_hp_kernel(fused::Arg
     const uint32_t idesc_lo = make_idesc_f16(C::M, C::NT3);
     const uint64_t wdesc = make_desc_kmajor(sW3, 0, 128, 128 * (C::K3 / 8));
     for (int t = 0; t < n_tiles; t++) {
-      HPW(0, HP_IWAIT(&a3_full[t & 1], (uint32_t)((t >> 1) & 1)))
-      if (t >= 2) HPW(1, HP_IWAIT(&d3_free[t & 1], (uint32_t)(((t - 2) >> 1) & 1)))
+      HPW(0, mbar_wait(&a3_full[t & 1], (uint32_t)((t >> 1) & 1)))
+      if (t >= 2) HPW(1, mbar_wait(&d3_free[t & 1], (uint32_t)(((t - 2) >> 1) & 1)))
       tcgen05_fence_after();
       const uint32_t a3 = tmem + C::cD2x + C::sD2 * (uint32_t)(t & 1);
       const uint32_t d3 = tmem + C::cD3x + C::sD3 * (uint32_t)(t & 1);
@@ -684,19 +597,13 @@ __global__ void __launch_bounds__(Cfg::NT, 1) forward_fused_hp_kernel(fused::Arg
 #endif
       PL_EV(t, 9)
     }
-  } else if (is_e1 || (L1ONLY && HP_L1WIDE && (is_e2 || is_e3))) {
+  } else if (is_e1) {
     // ============================ E1: A2 = split(relu(out1) * s1), in place ================
     // warp w: TMEM lane quarter w&3, chunks g0 .. g0+E1_CHUNKS-1 of 16 channels.  Chunk g reads
     // D1 columns [16g,16g+16) and [64+16g, ..), then writes its hi pairs to a2col(g) and its lo
     // pairs to 64 + a2col(g): columns this warp has consumed
     const uint32_t lane_base = (uint32_t)((warp & 3) * 32) << 16;
-    // (wide layer-1-only launch: warp group wg = E1 first half, E1 second half, E2, E3 owns chunk wg)
-    constexpr bool WIDE = L1ONLY && HP_L1WIDE != 0;
-    constexpr int NCH = WIDE ? 1 : C::E1_CHUNKS;       // chunks per warp
-    constexpr int SPX = WIDE ? 20 : C::SP;             // floats per staged pixel
-    constexpr int LPP = WIDE ? 4 : 8;                  // lanes per pixel in the store loop
-    const int wg = is_e1 ? (warp - C::W_E1) >> 2 : (is_e2 ? 2 : 3);
-    const int g0 = WIDE ? wg : wg * C::E1_CHUNKS;
+    const int g0 = ((warp - C::W_E1) >> 2) * C::E1_CHUNKS;
     // out1 (training): pixel index of this lane's pixel in tile 0, -1 = not an out1 pixel
     int pix1 = -1;
     const bool keep1 = BATCH && bx.out1 != nullptr;
@@ -706,21 +613,20 @@ __global__ void __launch_bounds__(Cfg::NT, 1) forward_fused_hp_kernel(fused::Arg
       if ((m < C::OW3 || last_strip) && vx < a.w && px < w1) pix1 = (smp * h1 + R0) * w1 + px;
     }
     const int w1_row = bx.pw - (C::F1 - 1);
-    float* st1 = reinterpret_cast<float*>(smem_raw + C::oS1) +
-                 (WIDE ? (wg * 4 + (warp & 3)) * (32 * SPX) : (warp - C::W_E1) * (32 * C::SP));
+    float* st1 = reinterpret_cast<float*>(smem_raw + C::oS1) + (warp - C::W_E1) * (32 * C::SP);
     float act_max = 0.f;   // L1ONLY: largest scaled activation this thread stored
     for (int b = 0; b < n_tiles; b++) {
-      HPW(0, HP_EWAIT(&bar1[b & 1], (uint32_t)((b >> 1) & 1)))       // MMA-1(b) done
+      HPW(0, mbar_wait(&bar1[b & 1], (uint32_t)((b >> 1) & 1)))       // MMA-1(b) done
       if (warp == C::W_E1) PL_EV(b, 2)
       tcgen05_fence_after();
       const uint32_t d1 = tmem + lane_base + C::cD1 + 128u * (uint32_t)(b & 1);
       // all loads of this warp's chunks first (one TMEM round trip), then the conversions
-      float va[NCH][16], vb[NCH][16];
+      float va[C::E1_CHUNKS][16], vb[C::E1_CHUNKS][16];
 #ifdef HP_PROF
       const unsigned _tl = (unsigned)clock();
 #endif
 #pragma unroll
-      for (int gl = 0; gl < NCH; gl++) {
+      for (int gl = 0; gl < C::E1_CHUNKS; gl++) {
         tmem_ld16_nowait(d1 + (g0 + gl) * 16, va[gl]);
         tmem_ld16_nowait(d1 + C::N1 + (g0 + gl) * 16, vb[gl]);
       }
@@ -738,7 +644,7 @@ __global__ void __launch_bounds__(Cfg::NT, 1) forward_fused_hp_kernel(fused::Arg
       }
       const uint32_t a2w = tmem + lane_base + C::cA2 + C::sA2 * (uint32_t)(b & 1);
 #pragma unroll
-      for (int gl = 0; gl < NCH; gl++) {
+      for (int gl = 0; gl < C::E1_CHUNKS; gl++) {
         const int g = g0 + gl;
         uint32_t hi[8], lo[8];
         float act[16];
@@ -758,7 +664,7 @@ __global__ void __launch_bounds__(Cfg::NT, 1) forward_fused_hp_kernel(fused::Arg
           tmem_st8u(a2w + C::A2LO + col, lo);
         }
         if (keep1) {
-          float4* q = reinterpret_cast<float4*>(st1 + lane * SPX + gl * 16);
+          float4* q = reinterpret_cast<float4*>(st1 + lane * C::SP + gl * 16);
 #pragma unroll
           for (int j = 0; j < 4; j++)
             q[j] = make_float4(act[4 * j] * sc.inv_s1, act[4 * j + 1] * sc.inv_s1,
@@ -781,10 +687,10 @@ __global__ void __launch_bounds__(Cfg::NT, 1) forward_fused_hp_kernel(fused::Arg
         // 64-byte run per thread touched 32 lines per instruction and bound the whole kernel)
         __syncwarp();
 #pragma unroll
-        for (int it = 0; it < LPP; it++) {
-          const int pp = it * (32 / LPP) + lane / LPP, ck = lane % LPP;
+        for (int it = 0; it < 8; it++) {
+          const int pp = it * 4 + (lane >> 3), ck = lane & 7;
           const int pidx = __shfl_sync(0xffffffffu, pix1, pp);
-          const float4 v = *reinterpret_cast<const float4*>(st1 + pp * SPX + ck * 4);
+          const float4 v = *reinterpret_cast<const float4*>(st1 + pp * C::SP + ck * 4);
           if (pidx >= 0)
             *reinterpret_cast<float4*>(bx.out1 + ((size_t)pidx + (size_t)b * w1_row) * C::N1 +
                                        g0 * 16 + ck * 4) = v;

@@ -24,6 +24,7 @@
 
 #include "context.cuh"
 #include "fused_forward.cuh"
+#include "fused_forward_hp.cuh"
 #include "fused_forward_pl.cuh"
 #include "tc_common.cuh"
 
@@ -85,73 +86,12 @@ struct Scales {
   unsigned char wimg[Cfg::oQs - Cfg::oW1];
 };
 static_assert(offsetof(Scales, wimg) % 16 == 0 && sizeof(Scales) % 16 == 0, "uint4 copies");
-
-// K-major canonical layout for 16-bit elements: core matrix = 8 rows x 16 bytes (8 halves);
-// returns the offset in halves of (row r, element k) of a [rows][K] operand
-__host__ __device__ __forceinline__ int kmajor16(int r, int k, int K) {
-  return (r >> 3) * (64 * (K >> 3)) + (k >> 3) * 64 + (r & 7) * 8 + (k & 7);
-}
-// (K-step s, 16-byte chunk j, element e) of the layer-1 contraction -> filter tap, or -1.
-// chunks 0..8: O at dx = chunk (taps dy = e); chunk 9: H8 at dx' = 0 (taps (8, e));
-// chunk 10: H8 at dx' = 8 (tap (8,8) + 7 pads); chunk 11: pad
-__host__ __device__ __forceinline__ int tap16(int s, int j, int e) {
-  const int c = 2 * s + j;
-  if (c < 9) return e * Cfg::F1 + c;
-  if (c == 9) return 8 * Cfg::F1 + e;
-  if (c == 10) return e == 0 ? 8 * Cfg::F1 + 8 : -1;
-  return -1;
-}
-__host__ __device__ __forceinline__ uint32_t make_idesc_f16(int Mm, int Nn) {
-  // c_format = F32, a_format = b_format = F16, both K-major
-  return (1u << 4) | ((uint32_t)(Nn >> 3) << 17) | ((uint32_t)(Mm >> 4) << 24);
-}
-__device__ __forceinline__ void mma_f16_ss(uint32_t d, uint64_t a, uint64_t b, uint32_t idesc,
-                                           uint32_t acc) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}\n" ::"r"(d),
-      "l"(a), "l"(b), "r"(idesc), "r"(acc)
-      : "memory");
-}
-__device__ __forceinline__ void mma_f16_ts(uint32_t d, uint32_t a, uint64_t b, uint32_t idesc,
-                                           uint32_t acc) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}\n" ::"r"(d),
-      "r"(a), "l"(b), "r"(idesc), "r"(acc)
-      : "memory");
-}
-// xs = hi + lo (raw half bits)
-__device__ __forceinline__ void split_h(float xs, unsigned short& hi, unsigned short& lo) {
-  const __half h = __float2half_rn(xs);
-  hi = __half_as_ushort(h);
-  lo = __half_as_ushort(__float2half_rn(xs - __half2float(h)));
-}
-// two values -> packed pairs (element 0 in the low half: K index order)
-__device__ __forceinline__ void split_h2(float a, float b, uint32_t& hi, uint32_t& lo) {
-  const __half2 h = __floats2half2_rn(a, b);
-  const float2 hf = __half22float2(h);
-  const __half2 l = __floats2half2_rn(a - hf.x, b - hf.y);
-  hi = *reinterpret_cast<const uint32_t*>(&h);
-  lo = *reinterpret_cast<const uint32_t*>(&l);
-}
-__device__ __forceinline__ uint32_t pack2(unsigned short a, unsigned short b) {
-  return (uint32_t)a | ((uint32_t)b << 16);
-}
-__device__ __forceinline__ void tmem_st8u(uint32_t taddr, const uint32_t v[8]) {
-  asm volatile(
-      "tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"r"(taddr),
-      "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7])
-      : "memory");
-}
+static_assert(Cfg::F1 == fused_hp::Cfg::F1, "layer 1 uses the 9x9 tap layout of fused_hp::tap16");
 
 #ifdef PL_TRACE
 using fused_pl::pl_trace;
 #endif
 using fused_pl::BatchExt;
-using fused_pl::elect_one;
-using fused_pl::tmem_ld16_nowait;
-using fused_pl::tmem_ld_wait;
 using tc::mbar_arrive;
 using tc::named_bar_sync;
 
@@ -161,13 +101,8 @@ using tc::named_bar_sync;
 // the plane producers of the main kernel, which see every pixel anyway: the first |x| >= 64 (or
 // NaN) clears `ok`, and the TF32 kernel launched behind redoes the launch.
 constexpr float kInMax = 64.f;
-__device__ __forceinline__ float pow2_scale(float bound) {   // 2^14 / pow2ceil(bound)
-  if (!(bound > 0.f) || !(bound < 1e30f)) return 1.f;
-  int e;
-  frexpf(bound, &e);                 // bound = f * 2^e, f in [0.5, 1)
-  return ldexpf(1.f, 14 - e);
-}
 __global__ void __launch_bounds__(256) hpw_prepare_kernel(fused::Args a, Scales* sc) {
+  using namespace tc;
   __shared__ float red_f[8];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   auto block_max = [&](float v) -> float {
@@ -243,7 +178,7 @@ __global__ void __launch_bounds__(256) hpw_prepare_kernel(fused::Args a, Scales*
   const int gtid = blockIdx.x * 256 + tid, gn = gridDim.x * 256;
   for (int i = gtid; i < 2 * C::N1 * C::K1; i += gn) {
     const int n = i / C::K1, k = i % C::K1;
-    const int t = tap16(k >> 4, (k >> 3) & 1, k & 7);
+    const int t = fused_hp::tap16(k >> 4, (k >> 3) & 1, k & 7);
     unsigned short hi, lo;
     split_h(t >= 0 ? __ldg(a.pw1 + t * C::N1 + (n & (C::N1 - 1))) * sv.sw1 : 0.f, hi, lo);
     gW1[kmajor16(n, k, C::K1)] = __ushort_as_half(n < C::N1 ? hi : lo);

@@ -50,10 +50,7 @@ struct Cfg {
   static constexpr int PW = 144;                 // plane entries (16 bytes each)
   static constexpr int PF = PW * 4;              // floats per plane
   static constexpr int RQ = 8, RH = 4;           // ring slots: quad planes, H planes
-#ifndef PL_N_E1
-#define PL_N_E1 4
-#endif
-  static constexpr int W_E1 = 0, N_E1 = PL_N_E1, W_E2 = N_E1, W_E3 = W_E2 + 4, W_IM = W_E3 + 4,
+  static constexpr int W_E1 = 0, N_E1 = 4, W_E2 = N_E1, W_E3 = W_E2 + 4, W_IM = W_E3 + 4,
                        N_IM = 5, W_I1 = W_IM + N_IM, W_I2 = W_I1 + 1, W_I3 = W_I2 + 1;
   static constexpr int NT = (W_I3 + 1) * 32;
   static constexpr int E1_CH = N1 / (N_E1 / 4);  // channels per E1 warp
@@ -108,48 +105,9 @@ __device__ long long pl_trace[8][16];
 #else
 #define PL_EV(t, e) {}
 #endif
-#ifdef PL_TIMING
-#define PL_T0 long long _tw[4] = {0, 0, 0, 0}; const long long _tstart = clock64();
-#define PL_WAIT(i, ...) { const long long _t = clock64(); __VA_ARGS__; _tw[i] += clock64() - _t; }
-#define PL_REPORT(name) if (blockIdx.x == 0 && blockIdx.y == 0 && blockIdx.z == 0 && lane == 0) \
-    printf("%-3s warp %2d: total %8lld  wait0 %8lld  wait1 %8lld  wait2 %8lld  tiles %d\n", name, warp, \
-           clock64() - _tstart, _tw[0], _tw[1], _tw[2], n_tiles);
-#else
-#define PL_T0
-#define PL_WAIT(i, ...) __VA_ARGS__;
-#define PL_REPORT(name)
-#endif
 
 using tc::mbar_arrive;
 using tc::named_bar_sync;
-
-__device__ __forceinline__ void tmem_ld16_nowait(uint32_t taddr, float v[16]) {
-  uint32_t* r = reinterpret_cast<uint32_t*>(v);
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, "
-      "%12, %13, %14, %15}, [%16];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]),
-        "=r"(r[7]), "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]),
-        "=r"(r[14]), "=r"(r[15])
-      : "r"(taddr));
-}
-// one lane of the (converged) warp; ptxas then knows the guarded tcgen05.mma sequence is
-// executed by a single thread and does not wrap every instruction in an ELECT/branch loop
-__device__ __forceinline__ bool elect_one() {
-  uint32_t pred = 0;
-  asm volatile(
-      "{\n\t"
-      ".reg .b32 rx;\n\t"
-      ".reg .pred px;\n\t"
-      "elect.sync rx|px, 0xffffffff;\n\t"
-      "@px mov.s32 %0, 1;\n\t"
-      "}\n"
-      : "+r"(pred));
-  return pred != 0;
-}
-__device__ __forceinline__ void tmem_ld_wait() {
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
 
 // BATCH = true: the input is a batch of S small samples [S][ph][pw] (training patches).  The
 // kernel then works on the VIRTUAL image [ph][S*pw] made of the samples laid side by side, so
@@ -301,7 +259,6 @@ __global__ void __launch_bounds__(Cfg::NT, 1) forward_fused_pl_kernel(fused::Arg
     float v[4];
 #pragma unroll
     for (int e = 0; e < 4; e++) v[e] = ld(C::F1 - 1, e);
-    PL_T0
     for (int b = 0; b < n_tiles; b++) {
       float nv[4];
 #pragma unroll
@@ -310,7 +267,7 @@ __global__ void __launch_bounds__(Cfg::NT, 1) forward_fused_pl_kernel(fused::Arg
 #pragma unroll
       for (int e = 0; e < 4; e++) split_tf32(v[e], h[e], l[e]);
       // H(b+8) replaces H(b+4) (last read by MMA-1(b-4)), Qd(b+5) replaces Qd(b-3) (MMA-1(b-3))
-      if (b >= 3) PL_WAIT(0, mbar_wait(&p_free[(b - 3) & 3], (uint32_t)(((b - 3) >> 2) & 1)))
+      if (b >= 3) mbar_wait(&p_free[(b - 3) & 3], (uint32_t)(((b - 3) >> 2) & 1));
       if (active) {
         const int sh = b & (C::RH - 1), sq = (b + 5) & (C::RQ - 1);
         *reinterpret_cast<float4*>(sHh + sh * C::PF) = make_float4(h[0], h[1], h[2], h[3]);
@@ -326,7 +283,6 @@ __global__ void __launch_bounds__(Cfg::NT, 1) forward_fused_pl_kernel(fused::Arg
 #pragma unroll
       for (int e = 0; e < 4; e++) v[e] = nv[e];
     }
-    PL_REPORT("IM")
   } else if (warp == C::W_I1) {
     // ============================ I1: layer-1 MMA issuer ===================================
     {
@@ -341,11 +297,10 @@ __global__ void __launch_bounds__(Cfg::NT, 1) forward_fused_pl_kernel(fused::Arg
         return (uint64_t)((addr >> 4) & 0x3FFF) | ((uint64_t)((lbo >> 4) & 0x3FFF) << 16) |
                ((uint64_t)(128 >> 4) << 32) | ((uint64_t)1 << 46);
       };
-      PL_T0
       for (int t = 0; t < n_tiles; t++) {
-        PL_WAIT(0, mbar_wait(&p_full[t & 3], (uint32_t)((t >> 2) & 1)))
+        mbar_wait(&p_full[t & 3], (uint32_t)((t >> 2) & 1));
         // D1[t&1] still holds A2(t-2) until MMA-2(t-2) has read it
-        if (t >= 2) PL_WAIT(1, mbar_wait(&bar2[t & 1], (uint32_t)(((t - 2) >> 1) & 1)))
+        if (t >= 2) mbar_wait(&bar2[t & 1], (uint32_t)(((t - 2) >> 1) & 1));
         tcgen05_fence_after();
         const uint32_t d1 = tmem + C::cD1 + 128u * (uint32_t)(t & 1);
         const uint32_t sh = (uint32_t)(t & (C::RH - 1)) * PB;
@@ -373,7 +328,6 @@ __global__ void __launch_bounds__(Cfg::NT, 1) forward_fused_pl_kernel(fused::Arg
         __syncwarp();
         PL_EV(t, 1)
       }
-      PL_REPORT("I1")
     }
   } else if (warp == C::W_I2) {
     // ============================ I2: layer-2 MMA issuer (A2 in TMEM) ======================
@@ -381,11 +335,10 @@ __global__ void __launch_bounds__(Cfg::NT, 1) forward_fused_pl_kernel(fused::Arg
       const uint32_t idesc_hi = make_idesc_tf32(C::M, 2 * C::N2);   // A2_hi x [W2_hi; W2_lo]
       const uint32_t idesc_lo = make_idesc_tf32(C::M, C::N2);       // A2_lo x W2_hi
       const uint64_t wdesc = make_desc_kmajor(sW2, 0, 128, 128 * (C::K2 / 4));
-      PL_T0
       for (int t = 0; t < n_tiles; t++) {
-        PL_WAIT(0, mbar_wait(&a2_full[t & 1], (uint32_t)((t >> 1) & 1)))
+        mbar_wait(&a2_full[t & 1], (uint32_t)((t >> 1) & 1));
         // D2[t&1] still holds A3(t-2) until MMA-3(t-2) has read it
-        if (t >= 2) PL_WAIT(1, mbar_wait(&bar3[t & 1], (uint32_t)(((t - 2) >> 1) & 1)))
+        if (t >= 2) mbar_wait(&bar3[t & 1], (uint32_t)(((t - 2) >> 1) & 1));
         tcgen05_fence_after();
         const uint32_t a2 = tmem + C::cD1 + 128u * (uint32_t)(t & 1);
         const uint32_t d2 = tmem + C::cD2 + 64u * (uint32_t)(t & 1);
@@ -401,7 +354,6 @@ __global__ void __launch_bounds__(Cfg::NT, 1) forward_fused_pl_kernel(fused::Arg
         __syncwarp();
         PL_EV(t, 5)
       }
-      PL_REPORT("I2")
     }
   } else if (warp == C::W_I3) {
     // ============================ I3: layer-3 tap-GEMM issuer (A3 in TMEM) =================
@@ -409,10 +361,9 @@ __global__ void __launch_bounds__(Cfg::NT, 1) forward_fused_pl_kernel(fused::Arg
       const uint32_t idesc_hi = make_idesc_tf32(C::M, 2 * C::NT3);
       const uint32_t idesc_lo = make_idesc_tf32(C::M, C::NT3);
       const uint64_t wdesc = make_desc_kmajor(sW3, 0, 128, 128 * (C::N2 / 4));
-      PL_T0
       for (int t = 0; t < n_tiles; t++) {
-        PL_WAIT(0, mbar_wait(&a3_full[t & 1], (uint32_t)((t >> 1) & 1)))
-        if (t >= 2) PL_WAIT(1, mbar_wait(&d3_free[t & 1], (uint32_t)(((t - 2) >> 1) & 1)))
+        mbar_wait(&a3_full[t & 1], (uint32_t)((t >> 1) & 1));
+        if (t >= 2) mbar_wait(&d3_free[t & 1], (uint32_t)(((t - 2) >> 1) & 1));
         tcgen05_fence_after();
         const uint32_t a3 = tmem + C::cD2 + 64u * (uint32_t)(t & 1);
         const uint32_t d3 = tmem + C::cD3 + 64u * (uint32_t)(t & 1);
@@ -428,7 +379,6 @@ __global__ void __launch_bounds__(Cfg::NT, 1) forward_fused_pl_kernel(fused::Arg
         __syncwarp();
         PL_EV(t, 9)
       }
-      PL_REPORT("I3")
     }
   } else if (warp < C::W_E1 + C::N_E1) {
     // ============================ E1: A2 = split(relu(D1 + b1)), in place ==================
@@ -449,14 +399,10 @@ __global__ void __launch_bounds__(Cfg::NT, 1) forward_fused_pl_kernel(fused::Arg
         o1 = bx.out1 + (((size_t)smp * h1 + R0) * w1 + px) * C::N1 + ch0;
     }
     const size_t o1_row = (size_t)(bx.pw - (C::F1 - 1)) * C::N1;
-    PL_T0
     for (int b = 0; b < n_tiles; b++) {
-      PL_WAIT(0, mbar_wait(&bar1[b & 1], (uint32_t)((b >> 1) & 1)))       // MMA-1(b) done
+      mbar_wait(&bar1[b & 1], (uint32_t)((b >> 1) & 1));       // MMA-1(b) done
       if (warp == 0) PL_EV(b, 2)
       tcgen05_fence_after();
-#ifdef EXP_NO_E1
-      if (b < 0)
-#endif
 #pragma unroll 1
       for (int c16 = 0; c16 < C::E1_CH; c16 += 16) {
         const uint32_t d1 = tmem + lane_base + C::cD1 + 128u * (uint32_t)(b & 1) + ch0 + c16;
@@ -491,7 +437,6 @@ __global__ void __launch_bounds__(Cfg::NT, 1) forward_fused_pl_kernel(fused::Arg
       mbar_arrive(&a2_full[b & 1]);
       if (warp == 0) PL_EV(b, 3)
     }
-    PL_REPORT("E1")
   } else if (warp < C::W_E3) {
     // ============================ E2: A3 = split(relu(D2 + b2)), in place ==================
     const uint32_t lane_base = (uint32_t)((warp & 3) * 32) << 16;
@@ -504,15 +449,11 @@ __global__ void __launch_bounds__(Cfg::NT, 1) forward_fused_pl_kernel(fused::Arg
     }
     const size_t o2_row = (size_t)(bx.pw - (C::F1 - 1)) * C::N2;
     float act2_max = 0.f;   // largest out2 value this thread stored (training forward)
-    PL_T0
     for (int b = 0; b < n_tiles; b++) {
-      PL_WAIT(0, mbar_wait(&bar2[b & 1], (uint32_t)((b >> 1) & 1)))       // MMA-2(b) done
+      mbar_wait(&bar2[b & 1], (uint32_t)((b >> 1) & 1));       // MMA-2(b) done
       if (warp == C::W_E2) PL_EV(b, 6)
       tcgen05_fence_after();
       const uint32_t d2 = tmem + lane_base + C::cD2 + 64u * (uint32_t)(b & 1);
-#ifdef EXP_NO_E2
-      if (b < 0)
-#endif
 #pragma unroll
       for (int g = 0; g < 2; g++) {
         float va[16], vb[16];
@@ -549,7 +490,6 @@ __global__ void __launch_bounds__(Cfg::NT, 1) forward_fused_pl_kernel(fused::Arg
       for (int o = 16; o > 0; o >>= 1) act2_max = fmaxf(act2_max, __shfl_xor_sync(0xffffffffu, act2_max, o));
       if (lane == 0 && act2_max > 0.f) atomicMax(bx.out2_max, __float_as_uint(act2_max));
     }
-    PL_REPORT("E2")
   } else if (warp < C::W_IM) {
     // ============================ E3: Q row -> smem, 25-term gather -> out3 ================
     // thread x owns output column X0+x; the partial sums of the four output rows that still
@@ -567,9 +507,8 @@ __global__ void __launch_bounds__(Cfg::NT, 1) forward_fused_pl_kernel(fused::Arg
       o3_row = (size_t)w3;
     }
     float acc0 = 0.f, acc1 = 0.f, acc2 = 0.f, acc3 = 0.f;
-    PL_T0
     for (int b = 0; b < n_tiles; b++) {
-      PL_WAIT(0, mbar_wait(&bar3[b & 1], (uint32_t)((b >> 1) & 1)))       // MMA-3(b) done
+      mbar_wait(&bar3[b & 1], (uint32_t)((b >> 1) & 1));       // MMA-3(b) done
       if (warp == C::W_E3) PL_EV(b, 10)
       tcgen05_fence_after();
       const uint32_t d3 = tmem + lane_base + C::cD3 + 64u * (uint32_t)(b & 1);
@@ -582,18 +521,11 @@ __global__ void __launch_bounds__(Cfg::NT, 1) forward_fused_pl_kernel(fused::Arg
       tcgen05_fence_before();
       mbar_arrive(&d3_free[b & 1]);                            // D3[b&1] may be overwritten
       float* qs = sQs + (b & 1) * (C::M * C::QP);
-#ifdef EXP_NO_E3
-      if (b < 0)
-#endif
 #pragma unroll
       for (int j = 0; j < C::QP; j++) qs[x * C::QP + j] = v[j] + w[j];
-      PL_WAIT(1, named_bar_sync(C::BAR_E3, 128))               // Q row visible to its neighbours
+      named_bar_sync(C::BAR_E3, 128);                          // Q row visible to its neighbours
       float r[C::F3];
-#ifdef EXP_NO_E3
-      if (b < 0) {
-#else
       if (x < C::OW3) {
-#endif
 #pragma unroll
         for (int dy = 0; dy < C::F3; dy++) {
           float s0 = 0.f, s1 = 0.f;
@@ -618,7 +550,6 @@ __global__ void __launch_bounds__(Cfg::NT, 1) forward_fused_pl_kernel(fused::Arg
         dst[o3 + (size_t)(b - (C::F3 - 1)) * o3_row] = done + b3;
       if (warp == C::W_E3) PL_EV(b, 11)
     }
-    PL_REPORT("E3")
   }
 
   tcgen05_fence_before();

@@ -1,9 +1,10 @@
-// tcgen05 / TMEM / mbarrier building blocks (sm_100a inline PTX) for the tensor-core path of
-// the dense contractions (layers 1 and 2).  Operands are FP32 values split into two TF32
-// terms (hi + lo); a product is evaluated as hi*hi + hi*lo + lo*hi ("3xTF32") with FP32
+// tcgen05 / TMEM / mbarrier building blocks (sm_100a inline PTX) shared by the tensor-core
+// kernels.  Operands are FP32 values split into two terms (hi + lo), either two TF32 values or
+// two scaled FP16 values; a product is evaluated as hi*hi + hi*lo + lo*hi with FP32
 // accumulation in TMEM, which keeps the result within ~1e-6 relative of the FP32 reference --
-// plain TF32 (10-bit mantissa) cannot meet the 1e-4 tolerance of the path.
+// a plain TF32 or FP16 operand (10-bit mantissa) cannot meet the 1e-4 tolerance of the path.
 #pragma once
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 
 #include <cstdint>
@@ -28,12 +29,42 @@ __device__ __forceinline__ void split_tf32(float x, float& hi, float& lo) {
   lo = x - hi;
 }
 
+// FP16 split: x*s = hi + lo with s a power of two that puts the operand range at ~2^14
+__device__ __forceinline__ float pow2_scale(float bound) {   // 2^14 / pow2ceil(bound)
+  if (!(bound > 0.f) || !(bound < 1e30f)) return 1.f;
+  int e;
+  frexpf(bound, &e);                 // bound = f * 2^e, f in [0.5, 1)
+  return ldexpf(1.f, 14 - e);
+}
+// xs = hi + lo (raw half bits)
+__device__ __forceinline__ void split_h(float xs, unsigned short& hi, unsigned short& lo) {
+  const __half h = __float2half_rn(xs);
+  hi = __half_as_ushort(h);
+  lo = __half_as_ushort(__float2half_rn(xs - __half2float(h)));
+}
+// two values -> packed pairs (element 0 in the low half: K index order)
+__device__ __forceinline__ void split_h2(float a, float b, uint32_t& hi, uint32_t& lo) {
+  const __half2 h = __floats2half2_rn(a, b);
+  const float2 hf = __half22float2(h);
+  const __half2 l = __floats2half2_rn(a - hf.x, b - hf.y);
+  hi = *reinterpret_cast<const uint32_t*>(&h);
+  lo = *reinterpret_cast<const uint32_t*>(&l);
+}
+__device__ __forceinline__ uint32_t pack2(unsigned short a, unsigned short b) {
+  return (uint32_t)a | ((uint32_t)b << 16);
+}
+
 // ---- canonical K-major, no-swizzle operand layout ------------------------------------------
 // A [rows][K] operand (K = reduction dim, 32-bit elements) is stored as 8-row x 16-byte core
 // matrices (128 contiguous bytes each).  Core matrices that are neighbours along K are 128 B
 // apart (LBO), 8-row groups are 128*K/4 bytes apart (SBO).  Returns the FLOAT offset of (r,k).
 __host__ __device__ __forceinline__ int kmajor_offset(int r, int k, int K) {
   return (r >> 3) * (32 * (K >> 2)) + (k >> 2) * 32 + (r & 7) * 4 + (k & 3);
+}
+// K-major canonical layout for 16-bit elements: core matrix = 8 rows x 16 bytes (8 halves);
+// returns the offset in halves of (row r, element k) of a [rows][K] operand
+__host__ __device__ __forceinline__ int kmajor16(int r, int k, int K) {
+  return (r >> 3) * (64 * (K >> 3)) + (k >> 3) * 64 + (r & 7) * 8 + (k & 7);
 }
 
 // shared-memory matrix descriptor (cute::UMMA::SmemDescriptor): start address, LBO, SBO in
@@ -59,6 +90,10 @@ __host__ __device__ __forceinline__ uint32_t make_idesc_tf32(int M, int N) {
   d |= (uint32_t)(N >> 3) << 17;   // n_dim
   d |= (uint32_t)(M >> 4) << 24;   // m_dim
   return d;
+}
+__host__ __device__ __forceinline__ uint32_t make_idesc_f16(int Mm, int Nn) {
+  // c_format = F32, a_format = b_format = F16, both K-major
+  return (1u << 4) | ((uint32_t)(Nn >> 3) << 17) | ((uint32_t)(Mm >> 4) << 24);
 }
 
 // ---- TMEM ------------------------------------------------------------------------------------
@@ -103,6 +138,20 @@ __device__ __forceinline__ void tmem_ld16(uint32_t taddr, float v[16]) {
 #pragma unroll
   for (int i = 0; i < 16; i++) v[i] = __uint_as_float(r[i]);
 }
+// the same without the wait: several loads in flight, then one tmem_ld_wait
+__device__ __forceinline__ void tmem_ld16_nowait(uint32_t taddr, float v[16]) {
+  uint32_t* r = reinterpret_cast<uint32_t*>(v);
+  asm volatile(
+      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, "
+      "%12, %13, %14, %15}, [%16];"
+      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]),
+        "=r"(r[7]), "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]),
+        "=r"(r[14]), "=r"(r[15])
+      : "r"(taddr));
+}
+__device__ __forceinline__ void tmem_ld_wait() {
+  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+}
 
 // warp-collective: lane i writes 8 consecutive columns of TMEM lane (lane_base + i)
 __device__ __forceinline__ void tmem_st8(uint32_t taddr, const float v[8]) {
@@ -111,6 +160,13 @@ __device__ __forceinline__ void tmem_st8(uint32_t taddr, const float v[8]) {
       "r"(__float_as_uint(v[0])), "r"(__float_as_uint(v[1])), "r"(__float_as_uint(v[2])),
       "r"(__float_as_uint(v[3])), "r"(__float_as_uint(v[4])), "r"(__float_as_uint(v[5])),
       "r"(__float_as_uint(v[6])), "r"(__float_as_uint(v[7]))
+      : "memory");
+}
+// the same for 32-bit payloads (packed half pairs)
+__device__ __forceinline__ void tmem_st8u(uint32_t taddr, const uint32_t v[8]) {
+  asm volatile(
+      "tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"r"(taddr),
+      "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7])
       : "memory");
 }
 __device__ __forceinline__ void tmem_st_wait() {
@@ -153,6 +209,39 @@ __device__ __forceinline__ void mma_tf32_ts(uint32_t tmem_d, uint32_t tmem_a, ui
       "}\n" ::"r"(tmem_d),
       "r"(tmem_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
       : "memory");
+}
+
+// kind::f16 versions: A in shared memory (ss) or in TMEM (ts)
+__device__ __forceinline__ void mma_f16_ss(uint32_t d, uint64_t a, uint64_t b, uint32_t idesc,
+                                           uint32_t acc) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}\n" ::"r"(d),
+      "l"(a), "l"(b), "r"(idesc), "r"(acc)
+      : "memory");
+}
+__device__ __forceinline__ void mma_f16_ts(uint32_t d, uint32_t a, uint64_t b, uint32_t idesc,
+                                           uint32_t acc) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}\n" ::"r"(d),
+      "r"(a), "l"(b), "r"(idesc), "r"(acc)
+      : "memory");
+}
+
+// one lane of the (converged) warp; ptxas then knows the guarded tcgen05.mma sequence is
+// executed by a single thread and does not wrap every instruction in an ELECT/branch loop
+__device__ __forceinline__ bool elect_one() {
+  uint32_t pred = 0;
+  asm volatile(
+      "{\n\t"
+      ".reg .b32 rx;\n\t"
+      ".reg .pred px;\n\t"
+      "elect.sync rx|px, 0xffffffff;\n\t"
+      "@px mov.s32 %0, 1;\n\t"
+      "}\n"
+      : "+r"(pred));
+  return pred != 0;
 }
 
 // arrives on the mbarrier when all previously issued MMAs of this thread have completed

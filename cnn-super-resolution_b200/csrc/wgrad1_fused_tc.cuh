@@ -37,7 +37,6 @@
 #include <cuda_runtime.h>
 
 #include "context.cuh"
-#include "fused_forward_pl.cuh"
 #include "tc_common.cuh"
 #include "wgrad_tc.cuh"
 
@@ -94,9 +93,6 @@ __global__ void __launch_bounds__(Cfg::NT, 1)
                            int n_tiles_total) {
   using C = Cfg;
   using namespace tc;
-  using fused_pl::elect_one;
-  using fused_pl::tmem_ld16_nowait;
-  using fused_pl::tmem_ld_wait;
   using tc::mbar_arrive;
   using tc::named_bar_sync;
   extern __shared__ __align__(128) float wg_smem[];

@@ -33,8 +33,6 @@
 
 #include "context.cuh"
 #include "conv5_tc.cuh"
-#include "fused_forward_hp.cuh"
-#include "fused_forward_pl.cuh"
 #include "tc_common.cuh"
 
 namespace srcnn {
@@ -81,11 +79,6 @@ struct Args {
 __global__ void __launch_bounds__(Cfg::NT, 1) wgrad5_tc_kernel(Args a) {
   using C = Cfg;
   using namespace tc;
-  using fused_hp::mma_f16_ss;
-  using fused_hp::split_h2;
-  using fused_pl::elect_one;
-  using fused_pl::tmem_ld16_nowait;
-  using fused_pl::tmem_ld_wait;
   extern __shared__ __align__(128) uint8_t smem_raw[];
   __shared__ __align__(8) uint64_t full_a[C::NSTAGE], empty_a[C::NSTAGE], bfull[C::RBN],
       bempty[C::RBN], done;

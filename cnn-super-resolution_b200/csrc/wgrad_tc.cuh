@@ -22,7 +22,6 @@
 #include <cuda_runtime.h>
 
 #include "context.cuh"
-#include "fused_forward_pl.cuh"
 #include "tc_common.cuh"
 
 namespace srcnn {
@@ -62,9 +61,6 @@ __global__ void __launch_bounds__(Cfg::NT, 1) wgrad1_tc_kernel(const float* __re
                                                                int n_tiles_total) {
   using C = Cfg;
   using namespace tc;
-  using fused_pl::elect_one;
-  using fused_pl::tmem_ld16_nowait;
-  using fused_pl::tmem_ld_wait;
   using tc::mbar_arrive;
   using tc::named_bar_sync;
   extern __shared__ __align__(128) float wg_smem[];
@@ -356,9 +352,6 @@ __global__ void __launch_bounds__(Cfg2::NT, 1) wgrad2_tc_kernel(const float* __r
                                                                 long long P, int n_tiles_total) {
   using C = Cfg2;
   using namespace tc;
-  using fused_pl::elect_one;
-  using fused_pl::tmem_ld16_nowait;
-  using fused_pl::tmem_ld_wait;
   using tc::mbar_arrive;
   extern __shared__ __align__(128) float wg_smem[];
   float* sX = wg_smem + C::oX;
