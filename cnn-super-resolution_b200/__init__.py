@@ -103,6 +103,8 @@ _SIGS = {
     "srcnn_resample": (_i, [_vp, _u64, _i, _i, _u64, _u64, _i, _i, _i]),
     "srcnn_upscale_image_host": (_i, [_vp, C.POINTER(CNet), _vp, _i, _i, _i, _i, _i, _vp]),
     "srcnn_upscale_frames_host": (_i, [_vp, C.POINTER(CNet), _vp, _i, _i, _i, _i, _i, _i, _vp]),
+    "srcnn_upscale_yuv420_frames_host": (_i, [_vp, C.POINTER(CNet), _vp, _i, _i, _i, _i, _i, _i,
+                                              _vp]),
     "srcnn_image_quality": (_i, [_vp, _u64, _i, _u64, _i, _i, _i, _i, _u64]),
     "srcnn_evaluate_frames_host": (_i, [_vp, C.POINTER(CNet), _vp, _i, _i, _i, _i, _i, _i, _vp,
                                         _i, _vp, _vp]),
@@ -482,6 +484,23 @@ class Net:
         _check(self.ctx.L.srcnn_upscale_frames_host(self.ctx.h, C.byref(self.c), _np_ptr(rgba),
                                                     rgba.shape[2], rgba.shape[1], n, out_w, out_h,
                                                     _filter_id(resample), _np_ptr(out)))
+        return out
+
+    def upscale_yuv420_frames_host(self, frames, w, h, out_w, out_h, resample="lanczos", out=None):
+        """frames: uint8 [n][w*h*3//2] planar Y'CbCr 4:2:0 (I420: Y, then Cb, then Cr; w and h
+        even) -> uint8 [n][out_w*out_h*3//2] I420: Y enlarged with Pillow's filter and its interior
+        replaced by the network's luma, Cb and Cr enlarged with the same filter (centre-sited
+        chroma).  `out` may be a preallocated (pinned) array."""
+        n = frames.shape[0]
+        assert frames.dtype == np.uint8 and frames.ndim == 2 and frames.shape[1] == w * h * 3 // 2
+        frames = np.ascontiguousarray(frames)
+        if out is None:
+            out = np.empty((n, out_w * out_h * 3 // 2), np.uint8)
+        assert out.dtype == np.uint8 and out.shape == (n, out_w * out_h * 3 // 2)
+        assert out.flags.c_contiguous
+        _check(self.ctx.L.srcnn_upscale_yuv420_frames_host(self.ctx.h, C.byref(self.c),
+                                                           _np_ptr(frames), w, h, n, out_w, out_h,
+                                                           _filter_id(resample), _np_ptr(out)))
         return out
 
     def evaluate_frames_host(self, rgba, reference, out_w, out_h, resample="lanczos", border=None,

@@ -189,16 +189,16 @@ struct srcnn_ctx {
     unsigned long long key[kGraphKey] = {};
     unsigned graph_launches[SRCNN_K_COUNT] = {};
   } up;
-  // srcnn_upscale_frames_host (`frames`) and srcnn_evaluate_frames_host (`eval`): device staging
-  // (grown on demand), apart from `up` and from each other so that the entries do not resize (and
-  // so re-capture) each other's buffers.  small / rgb / ref hold a ring of frame groups, rgba /
-  // luma / out / red / qred one group.
+  // srcnn_upscale_frames_host (`frames`), srcnn_evaluate_frames_host (`eval`) and
+  // srcnn_upscale_yuv420_frames_host (`yuv`): device staging (grown on demand), apart from `up` and
+  // from each other so that the entries do not resize (and so re-capture) each other's buffers.
+  // small / rgb / ref hold a ring of frame groups, rgba / luma / out / red / qred one group.
   struct FramesStaging {
-    void* small = nullptr;   // input RGBA8
-    void* rgba = nullptr;    // enlarged RGBA8
+    void* small = nullptr;   // input RGBA8 (yuv: input I420)
+    void* rgba = nullptr;    // enlarged RGBA8 (not used by yuv)
     void* luma = nullptr;    // enlarged luma, then minus its Q1 mean
     void* out = nullptr;     // network output
-    void* rgb = nullptr;     // result RGB8
+    void* rgb = nullptr;     // result RGB8 (yuv: result I420)
     void* red = nullptr;     // Q1 reduction partials, then one sum per frame
     void* s1 = nullptr;      // layer 1 / 2 activations of the three-launch route
     void* s2 = nullptr;
@@ -208,7 +208,7 @@ struct srcnn_ctx {
     size_t small_bytes = 0, rgba_bytes = 0, luma_bytes = 0, out_bytes = 0, rgb_bytes = 0,
            red_bytes = 0, s1_bytes = 0, s2_bytes = 0, ref_bytes = 0, qred_bytes = 0,
            metrics_bytes = 0;
-  } frames, eval;
+  } frames, eval, yuv;
   // srcnn_image_quality's reduction partials (grown on demand)
   void* quality_red = nullptr;
   size_t quality_red_bytes = 0;

@@ -20,7 +20,11 @@
 // arithmetic of extract_luma_kernel (generic::luma_of).  Alpha of the input is ignored: this is
 // Pillow's "RGB" path, not its premultiplying "RGBA" one.  A set of equal-sized frames is one
 // launch with the frame in blockIdx.z (frame f reads in + f * in_frame, writes out / luma + f * W * H).
+// The same kernel with one byte a pixel enlarges the planes of Y'CbCr 4:2:0 frames: Pillow's "L"
+// path, and for the Y plane the luma Y' / 255.  Pillow maps pixel centres onto pixel centres, so the
+// chroma planes come out right for centre-sited ("jpeg") chroma.
 #pragma once
+#include <algorithm>
 #include <cmath>
 #include <cstring>
 #include <vector>
@@ -112,21 +116,75 @@ inline std::vector<int> tables(int w, int h, int W, int H, int filter, int* rows
   return t;
 }
 
-template <int TAPS>
-__global__ void __launch_bounds__(kThreads)
-resample_kernel(const uchar4* __restrict__ in, int w, size_t in_frame, uchar4* __restrict__ out,
-                float* __restrict__ luma, int W, int H, const int* __restrict__ tab) {
-  extern __shared__ uchar4 mid[];   // [rows][kTX] horizontal-pass result, 8-bit
-  in += blockIdx.z * in_frame;
-  out += blockIdx.z * (size_t)W * H;
-  if (luma) luma += blockIdx.z * (size_t)W * H;
-  const int* xb = tab;
+// one plane of a launch: frame f reads in + f * in_frame and writes out + f * out_frame (pixels)
+// and, with luma, luma + f * W * H; tab = table_for(w, h, W, H)
+template <class Pix>
+struct Plane {
+  const Pix* in;
+  int w;
+  size_t in_frame;
+  Pix* out;
+  size_t out_frame;
+  float* luma;
+  int W, H;
+  const int* tab;
+};
+// up to three planes of every frame in one launch: blockIdx.z = frame * n + plane; a CTA past the
+// edge of its (smaller) plane returns at once
+template <class Pix>
+struct Planes {
+  Plane<Pix> p[3];
+  int n;
+};
+
+// the per-tap sum of one output pixel: three channels of RGBA8 (alpha written as 255), or one
+__device__ __forceinline__ unsigned char clip8(int s) {
+  return (unsigned char)min(max(s >> kPrecisionBits, 0), 255);
+}
+template <class Pix>
+struct Acc;
+template <>
+struct Acc<uchar4> {
+  int s0 = 1 << (kPrecisionBits - 1), s1 = s0, s2 = s0;
+  __device__ __forceinline__ void add(uchar4 p, int k) {
+    s0 += (int)p.x * k;
+    s1 += (int)p.y * k;
+    s2 += (int)p.z * k;
+  }
+  __device__ __forceinline__ uchar4 pixel() const {
+    return make_uchar4(clip8(s0), clip8(s1), clip8(s2), 255);
+  }
+};
+template <>
+struct Acc<unsigned char> {
+  int s = 1 << (kPrecisionBits - 1);
+  __device__ __forceinline__ void add(unsigned char p, int k) { s += (int)p * k; }
+  __device__ __forceinline__ unsigned char pixel() const { return clip8(s); }
+};
+// the normalized luma of an enlarged pixel: extract_luma_kernel's of RGBA8, Y' / 255 of a Y plane
+__device__ __forceinline__ float luma_from(uchar4 p) { return generic::luma_of(p, 1); }
+__device__ __forceinline__ float luma_from(unsigned char y) { return __fdiv_rn((float)y, 255.0f); }
+
+template <int TAPS, class Pix>
+__global__ void __launch_bounds__(kThreads) resample_kernel(const Planes<Pix> planes) {
+  extern __shared__ __align__(16) unsigned char smem[];
+  Pix* mid = reinterpret_cast<Pix*>(smem);   // [rows][kTX] horizontal-pass result, 8-bit
+  const unsigned pl = blockIdx.z % planes.n, f = blockIdx.z / planes.n;
+  // (selected, not indexed: a dynamic index would copy the parameters to local memory)
+  const Plane<Pix>& P = pl == 0 ? planes.p[0] : pl == 1 ? planes.p[1] : planes.p[2];
+  const int W = P.W, H = P.H;
+  const int x0 = blockIdx.x * kTX, y0 = blockIdx.y * kTY;
+  if (x0 >= W || y0 >= H) return;
+  const Pix* __restrict__ in = P.in + f * P.in_frame;
+  Pix* __restrict__ out = P.out + f * P.out_frame;
+  float* __restrict__ luma = P.luma ? P.luma + f * (size_t)W * H : nullptr;
+  const int w = P.w;
+  const int* xb = P.tab;
   const int* xn = xb + W;
   const int* xk = xn + W;
-  const int* yb = tab + (size_t)W * (2 + TAPS);
+  const int* yb = P.tab + (size_t)W * (2 + TAPS);
   const int* yn = yb + H;
   const int* yk = yn + H;
-  const int x0 = blockIdx.x * kTX, y0 = blockIdx.y * kTY;
   const int ylast = min(y0 + kTY, H) - 1;
   const int row0 = __ldg(yb + y0);
   const int rows = __ldg(yb + ylast) + __ldg(yn + ylast) - row0;
@@ -137,21 +195,12 @@ resample_kernel(const uchar4* __restrict__ in, int w, size_t in_frame, uchar4* _
     if (c >= nx) continue;
     const int x = x0 + c;
     const int b = __ldg(xb + x), n = __ldg(xn + x);
-    const uchar4* src = in + (size_t)(row0 + r) * w + b;
-    int s0 = 1 << (kPrecisionBits - 1), s1 = s0, s2 = s0;
+    const Pix* src = in + (size_t)(row0 + r) * w + b;
+    Acc<Pix> acc;
 #pragma unroll
-    for (int j = 0; j < TAPS; j++) {
-      if (j < n) {
-        const uchar4 p = src[j];
-        const int k = __ldg(xk + (size_t)x * TAPS + j);
-        s0 += (int)p.x * k;
-        s1 += (int)p.y * k;
-        s2 += (int)p.z * k;
-      }
-    }
-    mid[i] = make_uchar4((unsigned char)min(max(s0 >> kPrecisionBits, 0), 255),
-                         (unsigned char)min(max(s1 >> kPrecisionBits, 0), 255),
-                         (unsigned char)min(max(s2 >> kPrecisionBits, 0), 255), 255);
+    for (int j = 0; j < TAPS; j++)
+      if (j < n) acc.add(src[j], __ldg(xk + (size_t)x * TAPS + j));
+    mid[i] = acc.pixel();
   }
   __syncthreads();
   // vertical pass from shared memory
@@ -161,23 +210,14 @@ resample_kernel(const uchar4* __restrict__ in, int w, size_t in_frame, uchar4* _
     if (c >= nx) continue;
     const int y = y0 + r, x = x0 + c;
     const int b = __ldg(yb + y) - row0, n = __ldg(yn + y);
-    int s0 = 1 << (kPrecisionBits - 1), s1 = s0, s2 = s0;
+    Acc<Pix> acc;
 #pragma unroll
-    for (int j = 0; j < TAPS; j++) {
-      if (j < n) {
-        const uchar4 p = mid[(b + j) * kTX + c];
-        const int k = __ldg(yk + (size_t)y * TAPS + j);
-        s0 += (int)p.x * k;
-        s1 += (int)p.y * k;
-        s2 += (int)p.z * k;
-      }
-    }
-    const uchar4 o = make_uchar4((unsigned char)min(max(s0 >> kPrecisionBits, 0), 255),
-                                 (unsigned char)min(max(s1 >> kPrecisionBits, 0), 255),
-                                 (unsigned char)min(max(s2 >> kPrecisionBits, 0), 255), 255);
+    for (int j = 0; j < TAPS; j++)
+      if (j < n) acc.add(mid[(b + j) * kTX + c], __ldg(yk + (size_t)y * TAPS + j));
+    const Pix o = acc.pixel();
     const size_t o_i = (size_t)y * W + x;
     out[o_i] = o;
-    if (luma) luma[o_i] = generic::luma_of(o, 1);
+    if (luma) luma[o_i] = luma_from(o);
   }
 }
 
@@ -210,18 +250,51 @@ inline int table_for(srcnn_ctx* ctx, int w, int h, int W, int H, int filter, con
   return SRCNN_OK;
 }
 
-// `frames` frames of w x h (in) -> W x H (out, luma), back to back
-inline int launch(srcnn_ctx* ctx, const uchar4* in, int w, int h, uchar4* out, float* luma, int W,
-                  int H, int filter, const int* tab, int rows_max, int frames = 1) {
-  const dim3 grid((unsigned)((W + kTX - 1) / kTX), (unsigned)((H + kTY - 1) / kTY), (unsigned)frames);
-  const size_t in_frame = (size_t)w * h;
-  const size_t smem = (size_t)rows_max * kTX * sizeof(uchar4);
+// `frames` frames of every plane in one launch; rows_max: the most of the planes' table_for
+template <class Pix>
+inline int launch_planes(srcnn_ctx* ctx, const Planes<Pix>& planes, int filter, int rows_max,
+                         int frames) {
+  int W = 0, H = 0;
+  for (int i = 0; i < planes.n; i++) {
+    W = std::max(W, planes.p[i].W);
+    H = std::max(H, planes.p[i].H);
+  }
+  const dim3 grid((unsigned)((W + kTX - 1) / kTX), (unsigned)((H + kTY - 1) / kTY),
+                  (unsigned)(frames * planes.n));
+  const size_t smem = (size_t)rows_max * kTX * sizeof(Pix);
   // at most (kTY - 1) + 2 * 3 + 1 rows for an enlargement: well under the default 48 KB
   if (filter == SRCNN_RESAMPLE_LANCZOS)
-    resample_kernel<7><<<grid, kThreads, smem, ctx->stream>>>(in, w, in_frame, out, luma, W, H, tab);
+    resample_kernel<7, Pix><<<grid, kThreads, smem, ctx->stream>>>(planes);
   else
-    resample_kernel<5><<<grid, kThreads, smem, ctx->stream>>>(in, w, in_frame, out, luma, W, H, tab);
+    resample_kernel<5, Pix><<<grid, kThreads, smem, ctx->stream>>>(planes);
   return SRCNN_OK;
+}
+
+// `frames` RGBA8 frames of w x h (in) -> W x H (out, luma), back to back
+inline int launch(srcnn_ctx* ctx, const uchar4* in, int w, int h, uchar4* out, float* luma, int W,
+                  int H, int filter, const int* tab, int rows_max, int frames = 1) {
+  Planes<uchar4> p{};
+  p.p[0] = Plane<uchar4>{in, w, (size_t)w * h, out, (size_t)W * H, luma, W, H, tab};
+  p.n = 1;
+  return launch_planes(ctx, p, filter, rows_max, frames);
+}
+
+// `frames` planar Y'CbCr 4:2:0 (I420) frames of w x h (in) -> W x H (out), whole frames back to
+// back: Y through tab_y (w x h -> W x H, its luma into `luma`), Cb and Cr through tab_c
+// (w/2 x h/2 -> W/2 x H/2).  w, h, W and H are even.
+inline int launch_yuv420(srcnn_ctx* ctx, const unsigned char* in, int w, int h, unsigned char* out,
+                         float* luma, int W, int H, int filter, const int* tab_y, int rows_y,
+                         const int* tab_c, int rows_c, int frames) {
+  const size_t in_y = (size_t)w * h, in_c = in_y / 4, out_y = (size_t)W * H, out_c = out_y / 4;
+  const size_t in_frame = in_y + 2 * in_c, out_frame = out_y + 2 * out_c;
+  Planes<unsigned char> p{};
+  p.p[0] = Plane<unsigned char>{in, w, in_frame, out, out_frame, luma, W, H, tab_y};
+  p.p[1] = Plane<unsigned char>{in + in_y, w / 2, in_frame, out + out_y, out_frame, nullptr,
+                                W / 2, H / 2, tab_c};
+  p.p[2] = Plane<unsigned char>{in + in_y + in_c, w / 2, in_frame, out + out_y + out_c, out_frame,
+                                nullptr, W / 2, H / 2, tab_c};
+  p.n = 3;
+  return launch_planes(ctx, p, filter, std::max(rows_y, rows_c), frames);
 }
 
 }  // namespace resample

@@ -162,7 +162,7 @@ int srcnn_ctx_destroy(srcnn_ctx* ctx) {
     for (void* p : {u.small, u.rgba, u.luma, u.out, u.rgb, u.s1, u.s2})
       if (p) cudaFree(p);
   }
-  for (srcnn_ctx::FramesStaging* f : {&ctx->frames, &ctx->eval})
+  for (srcnn_ctx::FramesStaging* f : {&ctx->frames, &ctx->eval, &ctx->yuv})
     for (void* p : {f->small, f->rgba, f->luma, f->out, f->rgb, f->red, f->s1, f->s2, f->ref,
                     f->qred, f->metrics})
       if (p) cudaFree(p);
@@ -1168,17 +1168,11 @@ struct Upscale {
   int red_blocks() const { return grid_1d(npx(), generic::RED_THREADS, generic::RED_MAX_BLOCKS); }
 };
 
-// the device work the forward waits for: enlargement + luma, the Q1 "mean" of every frame (sum
-// of squares / count, subtracted on the device: DataPipeline::subtract_mean).  4 launches.  Each
-// frame's sum takes the block partition a single-frame sum takes, so its float is the same.
-int upscale_head(srcnn_ctx* ctx, const Upscale& u) {
+// the Q1 "mean" of every frame's u.luma (sum of squares / count, subtracted on the device:
+// DataPipeline::subtract_mean).  3 launches.  Each frame's sum takes the block partition a
+// single-frame sum takes, so its float is the same.
+int q1_mean(srcnn_ctx* ctx, const Upscale& u) {
   const size_t npx = u.npx();
-  {
-    LaunchScope scope(ctx, SRCNN_K_RESAMPLE);
-    SRCNN_TRY(resample::launch(ctx, u.small, u.w, u.h, u.rgba, u.luma, u.out_w, u.out_h, u.filter,
-                               u.tab, u.rows_max, u.frames));
-    SRCNN_TRY(check_launch("resample"));
-  }
   const int blocks = u.red_blocks();
   {
     LaunchScope scope(ctx, SRCNN_K_SUM, 2);
@@ -1194,6 +1188,17 @@ int upscale_head(srcnn_ctx* ctx, const Upscale& u) {
   return check_launch("sub_from_all");
 }
 
+// the device work the forward waits for: enlargement + luma, the Q1 mean.  4 launches.
+int upscale_head(srcnn_ctx* ctx, const Upscale& u) {
+  {
+    LaunchScope scope(ctx, SRCNN_K_RESAMPLE);
+    SRCNN_TRY(resample::launch(ctx, u.small, u.w, u.h, u.rgba, u.luma, u.out_w, u.out_h, u.filter,
+                               u.tab, u.rows_max, u.frames));
+    SRCNN_TRY(check_launch("resample"));
+  }
+  return q1_mean(ctx, u);
+}
+
 // swap_luma over image rows [y0, y1) of every frame.  1 launch.
 int upscale_swap(srcnn_ctx* ctx, const Upscale& u, int y0, int y1) {
   LaunchScope scope(ctx, SRCNN_K_SWAP_LUMA);
@@ -1203,22 +1208,28 @@ int upscale_swap(srcnn_ctx* ctx, const Upscale& u, int y0, int y1) {
   return check_launch("swap_luma");
 }
 
-// One image (u.frames == 1) through the three-launch path, on the context stream, synchronous:
-// upload, head, forward, swap_luma, download.  conv5_tc takes its FP16 operand scale from the
+// The forward of one image (u.frames == 1) on the three-launch path, u.luma -> u.out3 through the
+// layer activations s1 and s2.  L launches.  conv5_tc takes its FP16 operand scale from the
 // measured maximum of its whole input, so a sub-band -- or a batch of frames -- could get another
 // scale (and result) than the image alone.
-int upscale_three_launch(srcnn_ctx* ctx, const srcnn_net* net, const Upscale& u, void* s1,
-                         void* s2, const unsigned char* host_rgba, unsigned char* host_rgb) {
+int forward_three_launch(srcnn_ctx* ctx, const srcnn_net* net, const Upscale& u, void* s1, void* s2) {
   const Dims& d = u.d;
   TableScope handles(ctx);
   const srcnn_mem m_luma = stage_handle(ctx, u.luma, sizeof(float) * u.npx());
   const srcnn_mem m_out = stage_handle(ctx, u.out3, sizeof(float) * (size_t)d.w3 * d.h3);
   const srcnn_mem m_s1 = stage_handle(ctx, s1, sizeof(float) * (size_t)d.w1 * d.h1 * net->n1);
   const srcnn_mem m_s2 = stage_handle(ctx, s2, sizeof(float) * (size_t)d.w2 * d.h2 * net->n2);
+  return srcnn_forward_fused(ctx, net, m_luma, m_out, u.out_w, u.out_h, 1, m_s1, m_s2);
+}
+
+// One image (u.frames == 1) through the three-launch path, on the context stream, synchronous:
+// upload, head, forward, swap_luma, download.
+int upscale_three_launch(srcnn_ctx* ctx, const srcnn_net* net, const Upscale& u, void* s1,
+                         void* s2, const unsigned char* host_rgba, unsigned char* host_rgb) {
   SRCNN_CUDA(cudaMemcpyAsync((void*)u.small, host_rgba, (size_t)u.w * u.h * 4,
                              cudaMemcpyHostToDevice, ctx->stream));
   SRCNN_TRY(upscale_head(ctx, u));
-  SRCNN_TRY(srcnn_forward_fused(ctx, net, m_luma, m_out, u.out_w, u.out_h, 1, m_s1, m_s2));
+  SRCNN_TRY(forward_three_launch(ctx, net, u, s1, s2));
   SRCNN_TRY(upscale_swap(ctx, u, 0, u.out_h));
   SRCNN_CUDA(cudaMemcpyAsync(host_rgb, u.rgb, u.npx() * 3, cudaMemcpyDeviceToHost, ctx->stream));
   SRCNN_CUDA(cudaStreamSynchronize(ctx->stream));
@@ -1364,30 +1375,45 @@ struct FramesCall {
   unsigned char* rgb;     // ring of result groups
 };
 
-// staging in `st`, the resample table and the prepared network of a frames call whose arguments
-// have been checked; `extra_frame` more device bytes a frame enter the group size and the caller
-// allocates them
-int frames_prepare(srcnn_ctx* ctx, const srcnn_net* net, srcnn_ctx::FramesStaging& st, int w, int h,
-                   int n_frames, int out_w, int out_h, int filter, size_t extra_frame,
-                   FramesCall* fc) {
+// A frames call's bytes a frame: its input (`in`, ring slots `small`), its enlarged RGBA8 (`rgba`,
+// 0 when the call has none) and its result (`out`, ring slots `rgb`); `group` of them a frame set
+// the group size, `max_group` caps it (the frame is a grid dimension of the group's launches).
+struct FrameBytes {
+  size_t in, rgba, out, group;
+  int max_group;
+};
+
+// the RGBA8-in, RGB8-out frame of srcnn_upscale_frames_host, plus `extra` device bytes a frame
+// that enter the group size (the caller allocates them): ~128 MB of device staging per group
+// (input, enlarged RGBA8 + luma + RGB8, network output; 960x540 -> 1920x1080: 4 frames) --
+// launches long enough to fill the GPU, a first upload and a last download short next to a whole
+// call
+FrameBytes rgba_frame_bytes(const srcnn_net* net, int w, int h, int out_w, int out_h, size_t extra) {
   const Dims d = net_dims(net, out_w, out_h);
   const size_t in_px = (size_t)w * h, npx = (size_t)out_w * out_h, out_px = (size_t)d.w3 * d.h3;
+  return FrameBytes{in_px * 4, npx * 4, npx * 3, in_px * 4 + npx * (4 + 4 + 3) + out_px * 4 + extra,
+                    65535};
+}
+
+// staging in `st`, the resample table and the prepared network of a frames call whose arguments
+// have been checked
+int frames_prepare(srcnn_ctx* ctx, const srcnn_net* net, srcnn_ctx::FramesStaging& st, int w, int h,
+                   int n_frames, int out_w, int out_h, int filter, const FrameBytes& fb,
+                   FramesCall* fc) {
+  const Dims d = net_dims(net, out_w, out_h);
+  const size_t npx = (size_t)out_w * out_h, out_px = (size_t)d.w3 * d.h3;
   SRCNN_CUDA(ctx->drain_lanes());
   const bool fused = fast::fused_supported(net->n1, net->n2, net->f1, net->f2, net->f3);
   Upscale u{w, h, out_w, out_h, filter, 1, d, nullptr, 0};
   const size_t red_frame = sizeof(double) * u.red_blocks() + sizeof(float);
-  // ~128 MB of device staging per group (input, enlarged RGBA8 + luma + RGB8, network output;
-  // 960x540 -> 1920x1080: 4 frames): launches long enough to fill the GPU, a first upload and a
-  // last download short next to a whole call
-  const size_t frame_bytes = in_px * 4 + npx * (4 + 4 + 3) + out_px * 4 + extra_frame;
-  // (the frame is a grid dimension of the head and swap launches: at most 65535 a group)
-  const int group = fused ? std::min(frames_group(frame_bytes, (size_t)128 << 20, n_frames), 65535) : 1;
+  const int group =
+      fused ? std::min(frames_group(fb.group, (size_t)128 << 20, n_frames), fb.max_group) : 1;
   const int ring = fused ? kFrameRing : 1;
-  SRCNN_TRY(ensure_scratch(ctx, &st.small, &st.small_bytes, in_px * 4 * group * ring));
-  SRCNN_TRY(ensure_scratch(ctx, &st.rgba, &st.rgba_bytes, npx * 4 * group));
+  SRCNN_TRY(ensure_scratch(ctx, &st.small, &st.small_bytes, fb.in * group * ring));
+  if (fb.rgba) SRCNN_TRY(ensure_scratch(ctx, &st.rgba, &st.rgba_bytes, fb.rgba * group));
   SRCNN_TRY(ensure_scratch(ctx, &st.luma, &st.luma_bytes, npx * sizeof(float) * group));
   SRCNN_TRY(ensure_scratch(ctx, &st.out, &st.out_bytes, out_px * sizeof(float) * group));
-  SRCNN_TRY(ensure_scratch(ctx, &st.rgb, &st.rgb_bytes, npx * 3 * group * ring));
+  SRCNN_TRY(ensure_scratch(ctx, &st.rgb, &st.rgb_bytes, fb.out * group * ring));
   SRCNN_TRY(ensure_scratch(ctx, &st.red, &st.red_bytes, red_frame * group));
   if (!fused) {
     SRCNN_TRY(ensure_scratch(ctx, &st.s1, &st.s1_bytes, sizeof(float) * (size_t)d.w1 * d.h1 * net->n1));
@@ -1444,7 +1470,8 @@ int srcnn_upscale_frames_host(srcnn_ctx* ctx, const srcnn_net* net, const unsign
   SRCNN_REQUIRE(n_frames > 0, "bad frame count %d", n_frames);
   srcnn_ctx::FramesStaging& st = ctx->frames;
   FramesCall fc;
-  SRCNN_TRY(frames_prepare(ctx, net, st, w, h, n_frames, out_w, out_h, filter, 0, &fc));
+  SRCNN_TRY(frames_prepare(ctx, net, st, w, h, n_frames, out_w, out_h, filter,
+                           rgba_frame_bytes(net, w, h, out_w, out_h, 0), &fc));
   const size_t in_px = (size_t)w * h, npx = (size_t)out_w * out_h;
   if (!fc.fused) {
     // frame by frame, each as the image entry runs it
@@ -1470,7 +1497,8 @@ int srcnn_evaluate_frames_host(srcnn_ctx* ctx, const srcnn_net* net, const unsig
   srcnn_ctx::FramesStaging& st = ctx->eval;
   const size_t in_px = (size_t)w * h, npx = (size_t)out_w * out_h;
   FramesCall fc;
-  SRCNN_TRY(frames_prepare(ctx, net, st, w, h, n_frames, out_w, out_h, filter, npx * 4, &fc));
+  SRCNN_TRY(frames_prepare(ctx, net, st, w, h, n_frames, out_w, out_h, filter,
+                           rgba_frame_bytes(net, w, h, out_w, out_h, npx * 4), &fc));
   const int ring = fc.fused ? kFrameRing : 1;
   SRCNN_TRY(ensure_scratch(ctx, &st.ref, &st.ref_bytes, npx * 4 * fc.group * ring));
   SRCNN_TRY(ensure_scratch(ctx, &st.qred, &st.qred_bytes,
@@ -1506,6 +1534,95 @@ int srcnn_evaluate_frames_host(srcnn_ctx* ctx, const srcnn_net* net, const unsig
                              cudaMemcpyDeviceToHost, ctx->stream));
   SRCNN_CUDA(cudaStreamSynchronize(ctx->stream));
   return SRCNN_OK;
+}
+
+namespace {
+// A group of Y'CbCr 4:2:0 (I420) frames of an Upscale job (its u.small, u.rgba and u.rgb unused):
+// whole frames back to back in `in` and `out`, the chroma planes enlarged through tab_c.
+struct Yuv420 {
+  const int* tab_c;
+  int rows_max_c;
+  const unsigned char* in;
+  unsigned char* out;
+};
+
+size_t yuv420_frame(int w, int h) { return (size_t)w * h * 3 / 2; }
+
+// the device work the forward waits for: the three planes enlarged straight into the result
+// frames, the luma of the Y plane, its Q1 mean.  4 launches.
+int yuv420_head(srcnn_ctx* ctx, const Upscale& u, const Yuv420& y) {
+  {
+    LaunchScope scope(ctx, SRCNN_K_RESAMPLE);
+    SRCNN_TRY(resample::launch_yuv420(ctx, y.in, u.w, u.h, y.out, u.luma, u.out_w, u.out_h,
+                                      u.filter, u.tab, u.rows_max, y.tab_c, y.rows_max_c, u.frames));
+    SRCNN_TRY(check_launch("resample"));
+  }
+  return q1_mean(ctx, u);
+}
+
+// the network's luma over the interior of every frame's Y plane.  1 launch.
+int yuv420_swap(srcnn_ctx* ctx, const Upscale& u, const Yuv420& y) {
+  LaunchScope scope(ctx, SRCNN_K_SWAP_LUMA);
+  dim3 block(32, 8), grid((u.d.w3 + 31) / 32, (u.d.h3 + 7) / 8, u.frames);
+  generic::swap_luma_plane_kernel<<<grid, block, 0, ctx->stream>>>(
+      u.out3, y.out, u.out_w, yuv420_frame(u.out_w, u.out_h), u.d.w3, u.d.h3);
+  return check_launch("swap_luma");
+}
+}  // namespace
+
+int srcnn_upscale_yuv420_frames_host(srcnn_ctx* ctx, const srcnn_net* net,
+                                     const unsigned char* host_in, int w, int h, int n_frames,
+                                     int out_w, int out_h, int filter, unsigned char* host_out) {
+  SRCNN_REQUIRE(ctx && host_in && host_out, "null argument");
+  SRCNN_ENTER(ctx);
+  SRCNN_TRY(check_upscale(net, w, h, out_w, out_h, filter));
+  SRCNN_REQUIRE(w % 2 == 0 && h % 2 == 0 && out_w % 2 == 0 && out_h % 2 == 0,
+                "4:2:0 frames need even sizes, got %dx%d -> %dx%d", w, h, out_w, out_h);
+  SRCNN_REQUIRE(n_frames > 0, "bad frame count %d", n_frames);
+  srcnn_ctx::FramesStaging& st = ctx->yuv;
+  const Dims d = net_dims(net, out_w, out_h);
+  const size_t in_frame = yuv420_frame(w, h), out_frame = yuv420_frame(out_w, out_h);
+  // the device bytes a frame of a group holds: its input and result in each ring slot, its luma
+  // and its network output (960x540 -> 1920x1080: 4 frames in ~128 MB); the frame and the plane
+  // share the grid dimension of the resampling launch
+  const FrameBytes fb{in_frame, 0, out_frame,
+                      (in_frame + out_frame) * kFrameRing + (size_t)out_w * out_h * 4 +
+                          (size_t)d.w3 * d.h3 * 4,
+                      65535 / 3};
+  FramesCall fc;
+  SRCNN_TRY(frames_prepare(ctx, net, st, w, h, n_frames, out_w, out_h, filter, fb, &fc));
+  Yuv420 y{nullptr, 0, nullptr, nullptr};
+  SRCNN_TRY(resample::table_for(ctx, w / 2, h / 2, out_w / 2, out_h / 2, filter, &y.tab_c,
+                                &y.rows_max_c));
+  unsigned char* ring_in = (unsigned char*)st.small;
+  unsigned char* ring_out = (unsigned char*)st.rgb;
+  Upscale& u = fc.u;
+  if (!fc.fused) {
+    // frame by frame, for the reason forward_three_launch gives
+    y.in = ring_in;
+    y.out = ring_out;
+    for (int f = 0; f < n_frames; f++) {
+      SRCNN_CUDA(cudaMemcpyAsync(ring_in, host_in + (size_t)f * in_frame, in_frame,
+                                 cudaMemcpyHostToDevice, ctx->stream));
+      SRCNN_TRY(yuv420_head(ctx, u, y));
+      SRCNN_TRY(forward_three_launch(ctx, net, u, st.s1, st.s2));
+      SRCNN_TRY(yuv420_swap(ctx, u, y));
+      SRCNN_CUDA(cudaMemcpyAsync(host_out + (size_t)f * out_frame, ring_out, out_frame,
+                                 cudaMemcpyDeviceToHost, ctx->stream));
+      SRCNN_CUDA(cudaStreamSynchronize(ctx->stream));
+    }
+    return SRCNN_OK;
+  }
+  // a group's device work: enlargement + luma, Q1 mean, fused forward, Y write.  5 + F launches.
+  return run_frame_ring(ctx, n_frames, fc.group, host_in, ring_in, in_frame, host_out, ring_out,
+                        out_frame, [&](int S, int r) {
+                          u.frames = S;
+                          y.in = ring_in + (size_t)r * fc.group * in_frame;
+                          y.out = ring_out + (size_t)r * fc.group * out_frame;
+                          SRCNN_TRY(yuv420_head(ctx, u, y));
+                          SRCNN_TRY(launch_fused(ctx, fc.fn, u.luma, u.out3, u.out_w, u.out_h, S));
+                          return yuv420_swap(ctx, u, y);
+                        });
 }
 
 int srcnn_infer_frames_host(srcnn_ctx* ctx, const srcnn_net* net, const float* host_in, int w,

@@ -92,6 +92,126 @@ void write_image(const char* path, float* luma, size_t w, size_t h) {
   }
 }
 
+// ------------------------------------------------------------------ video (Y4M) ---------
+static std::runtime_error y4m_error(const std::string& path, const std::string& what) {
+  return std::runtime_error("Y4M '" + path + "': " + what);
+}
+
+Y4mReader::Y4mReader(const char* path) : _path(path), _f(path, std::ios::binary) {
+  if (!_f.is_open()) throw y4m_error(_path, "could not open");
+  std::string line;
+  if (!std::getline(_f, line) || line.compare(0, 10, "YUV4MPEG2 ") != 0)
+    throw y4m_error(_path, "not a YUV4MPEG2 stream");
+  std::istringstream tags(line.substr(10));
+  std::string t;
+  bool has_w = false, has_h = false;
+  while (std::getline(tags, t, ' ')) {
+    if (t.empty()) continue;
+    const std::string v = t.substr(1);
+    switch (t[0]) {
+      case 'W':
+      case 'H': {
+        char* end = nullptr;
+        const long n = std::strtol(v.c_str(), &end, 10);
+        if (v.empty() || *end != '\0' || n <= 0 || n > 65535)
+          throw y4m_error(_path, "bad frame size tag '" + t + "'");
+        (t[0] == 'W' ? _header.w : _header.h) = (int)n;
+        (t[0] == 'W' ? has_w : has_h) = true;
+        break;
+      }
+      case 'C':
+        if (v == "420mpeg2" || v == "420paldv")
+          throw y4m_error(_path, "chroma siting '" + t + "' is left-sited; only centre-sited 4:2:0 "
+                                 "(C420jpeg, C420) is supported");
+        if (v != "420jpeg" && v != "420")
+          throw y4m_error(_path, "colourspace '" + t + "' is not supported; only 8-bit 4:2:0 "
+                                 "(C420jpeg, C420) is");
+        break;
+      case 'I':
+        if (v != "p")
+          throw y4m_error(_path, "interlacing '" + t + "' is not supported; only progressive "
+                                 "frames (Ip) are");
+        break;
+      case 'F':
+      case 'A':
+      case 'X':
+        break;
+      default:
+        throw y4m_error(_path, "unknown header tag '" + t + "'");
+    }
+    _header.tags.push_back(t);
+  }
+  if (!has_w || !has_h) throw y4m_error(_path, "the header gives no W or no H");
+  if (_header.w % 2 || _header.h % 2)
+    throw y4m_error(_path, "frame size " + std::to_string(_header.w) + "x" +
+                               std::to_string(_header.h) + " is odd; 4:2:0 needs even sizes");
+  _first = _f.tellg();
+}
+
+// reads "FRAME[ params]\n"; false at the end of the stream
+bool Y4mReader::read_marker(size_t frame) {
+  if (_f.peek() == std::char_traits<char>::eof()) return false;
+  std::string line;
+  const bool full = (bool)std::getline(_f, line) && !_f.eof();
+  if (line.compare(0, 5, "FRAME") != 0 || (line.size() > 5 && line[5] != ' '))
+    throw y4m_error(_path, "frame " + std::to_string(frame) + " does not start with FRAME");
+  if (!full) throw y4m_error(_path, "frame " + std::to_string(frame) + " is truncated");
+  return true;
+}
+
+size_t Y4mReader::check_frames() {
+  _f.clear();
+  _f.seekg(0, std::ios::end);
+  const std::streamoff size = _f.tellg();
+  _f.seekg(_first);
+  size_t n = 0;
+  while (read_marker(n)) {
+    if (size - (std::streamoff)_f.tellg() < (std::streamoff)_header.frame_bytes())
+      throw y4m_error(_path, "frame " + std::to_string(n) + " is truncated");
+    _f.seekg((std::streamoff)_header.frame_bytes(), std::ios::cur);
+    n++;
+  }
+  _f.clear();
+  _f.seekg(_first);
+  _next = 0;
+  return n;
+}
+
+size_t Y4mReader::read_frames(size_t max, std::vector<unsigned char>& out) {
+  const size_t bytes = _header.frame_bytes();
+  size_t n = 0;
+  while (n < max && read_marker(_next)) {
+    const size_t at = out.size();
+    out.resize(at + bytes);
+    _f.read(reinterpret_cast<char*>(out.data() + at), (std::streamsize)bytes);
+    if ((size_t)_f.gcount() != bytes)
+      throw y4m_error(_path, "frame " + std::to_string(_next) + " is truncated");
+    n++;
+    _next++;
+  }
+  return n;
+}
+
+void write_y4m_header(std::ostream& f, const Y4mHeader& in, int out_w, int out_h) {
+  f << "YUV4MPEG2";
+  for (const std::string& t : in.tags) {
+    if (t[0] == 'W')
+      f << " W" << out_w;
+    else if (t[0] == 'H')
+      f << " H" << out_h;
+    else
+      f << " " << t;
+  }
+  f << "\n";
+}
+
+void write_y4m_frames(std::ostream& f, const unsigned char* frames, size_t n, size_t frame_bytes) {
+  for (size_t i = 0; i < n; i++) {
+    f << "FRAME\n";
+    f.write(reinterpret_cast<const char*>(frames + i * frame_bytes), (std::streamsize)frame_bytes);
+  }
+}
+
 }  // namespace utils
 
 // ------------------------------------------------------------------ RawMemoryHandle ----

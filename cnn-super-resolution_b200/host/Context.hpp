@@ -12,6 +12,7 @@
 #include <cstddef>
 #include <cstdint>
 #include <deque>
+#include <fstream>
 #include <iostream>
 #include <string>
 #include <vector>
@@ -59,6 +60,39 @@ void load_image(const char* path, ImageData&);
 int write_image(const char* path, ImageData&);
 /** luma in [0,1] -> 8-bit binary PGM (reference: UtilsOpenCL.cpp write_image(float*)) */
 void write_image(const char* path, float* luma, size_t w, size_t h);
+
+/** The header of a YUV4MPEG2 (Y4M) stream: "YUV4MPEG2" and space-separated tags.  Only 8-bit
+ * progressive 4:2:0 with centre-sited chroma (C420jpeg, the format's default, or C420) of even
+ * size is accepted: the device layer resamples chroma by pixel centres. */
+struct Y4mHeader {
+  int w = 0, h = 0;
+  std::vector<std::string> tags;   // every tag as read, in order ("W960", "F30000:1001", ...)
+  size_t frame_bytes() const { return (size_t)w * h * 3 / 2; }
+};
+/** Reads the frames of a Y4M file.  Every check throws std::runtime_error with a one-line
+ * message: the constructor checks the header, check_frames() every frame marker and frame size. */
+class Y4mReader {
+ public:
+  explicit Y4mReader(const char* path);
+  const Y4mHeader& header() const { return _header; }
+  /** the number of frames; every frame starts with "FRAME[ params]\n" and is complete.  Leaves
+   * the reader at the first frame. */
+  size_t check_frames();
+  /** up to `max` next frames (I420, their parameters dropped) into `out`; returns how many */
+  size_t read_frames(size_t max, std::vector<unsigned char>& out);
+
+ private:
+  bool read_marker(size_t frame);
+  std::string _path;
+  std::ifstream _f;
+  std::streampos _first;
+  size_t _next = 0;
+  Y4mHeader _header;
+};
+/** `in`'s header with W and H set to out_w x out_h and every other tag copied */
+void write_y4m_header(std::ostream&, const Y4mHeader& in, int out_w, int out_h);
+/** n frames of `frame_bytes` bytes, each behind a bare "FRAME\n" */
+void write_y4m_frames(std::ostream&, const unsigned char* frames, size_t n, size_t frame_bytes);
 }  // namespace utils
 
 /** One allocation of the context (reference: RawMemoryHandle, Context.hpp:53-66) */

@@ -11,6 +11,11 @@
 // -i DIR (forward mode) runs every `.ppm` / `.pgm` file of DIR, in sorted name order, into
 // OUT_DIR/<stem>.ppm (-o OUT_DIR): consecutive files of equal size go through
 // srcnn_upscale_frames_host together, at most kDirBatch at a time; other files are skipped.
+// -i IN.y4m (forward mode) enlarges every frame of a YUV4MPEG2 video, 8-bit progressive 4:2:0 with
+// centre-sited chroma (C420jpeg / C420), into OUT.y4m (-o OUT.y4m): the header's W and H times
+// --scale, its other tags copied, kDirBatch frames per srcnn_upscale_yuv420_frames_host call; the
+// network replaces the luma, the chroma is only enlarged.  The header and every frame marker are
+// checked before any device work.
 // eval -i SAMPLES_DIR measures the network on the training mode's sample pairs: every `_small`
 // image, enlarged N times (--scale, default 1: the reference's `_small` images are already
 // enlarged), against its `_large` image, which must be exactly N times its size.  One line a pair
@@ -26,7 +31,9 @@
 #include <cstdio>
 #include <cstring>
 #include <cstdlib>
+#include <fstream>
 #include <iostream>
+#include <memory>
 #include <random>
 #include <stdexcept>
 #include <unordered_map>
@@ -164,6 +171,32 @@ static void execute_directory(ConfigBasedDataPipeline& pipeline, GpuAllocationPo
     batch.push_back(&image);
   }
   flush();
+}
+
+// every frame of a Y4M video through the I420 frames entry, `scale` times enlarged, kDirBatch
+// frames at a time; the result goes to out_path unless it is null (dry run)
+static void execute_y4m(ConfigBasedDataPipeline& pipeline, GpuAllocationPool& gpu_alloc,
+                        Y4mReader& video, const char* out_path, size_t scale, int filter) {
+  const Y4mHeader& hd = video.header();
+  const size_t w = (size_t)hd.w, h = (size_t)hd.h, out_w = scale * w, out_h = scale * h;
+  const size_t out_bytes = out_w * out_h * 3 / 2;
+  std::ofstream out;
+  if (out_path) {
+    std::cout << "Saving result video to: '" << out_path << "'" << std::endl;
+    out.open(out_path, std::ios::binary);
+    if (!out.is_open()) throw std::runtime_error(std::string("Could not write video: ") + out_path);
+    write_y4m_header(out, hd, (int)out_w, (int)out_h);
+  }
+  std::vector<unsigned char> in, result;
+  size_t n;
+  while ((n = video.read_frames(kDirBatch, in)) > 0) {
+    result.resize(n * out_bytes);
+    pipeline.upscale_yuv420_frames(gpu_alloc.layer_1, gpu_alloc.layer_2, gpu_alloc.layer_3,
+                                   in.data(), w, h, n, out_w, out_h, filter, result.data());
+    if (out_path) write_y4m_frames(out, result.data(), n, out_bytes);
+    in.clear();
+  }
+  if (out_path && !out.good()) throw std::runtime_error(std::string("Could not write video: ") + out_path);
 }
 
 static void get_training_samples(const std::string& dir, std::vector<TrainSampleFiles>& target) {
@@ -356,7 +389,13 @@ int main(int argc, char** argv) {
     std::cout << "--scale applies to the forward mode only" << std::endl;
     return EXIT_FAILURE;
   }
-  const bool in_dir = !train && !eval && is_directory(in_path);
+  size_t stem_len = 0;
+  const bool in_y4m = ends_with(in_path, ".y4m", &stem_len);
+  if ((train || eval) && in_y4m) {
+    std::cout << "A .y4m input applies to the forward mode only" << std::endl;
+    return EXIT_FAILURE;
+  }
+  const bool in_dir = !train && !eval && !in_y4m && is_directory(in_path);
   if ((in_dir || eval) && out_path && !is_directory(out_path)) {
     std::cout << "Output directory '" << out_path << "' does not exist or is not a directory"
               << std::endl;
@@ -376,7 +415,8 @@ int main(int argc, char** argv) {
               << "Output: " << (out_path ? out_path : "-") << std::endl;
   else
     std::cout << "Forward mode" << std::endl
-              << (in_dir ? "Input directory: " : "Input image: ") << in_path << std::endl
+              << (in_dir ? "Input directory: " : in_y4m ? "Input video: " : "Input image: ")
+              << in_path << std::endl
               << "Output: " << (out_path ? out_path : "-") << std::endl;
   if (!train && scale > 1)
     std::cout << "Scale: " << scale << "x, resample: " << resample_name << std::endl;
@@ -387,6 +427,14 @@ int main(int argc, char** argv) {
     ConfigReader reader;
     Config cfg = reader.read(config_path);
     std::cout << cfg << std::endl;
+    // a video is checked whole before the context exists
+    std::unique_ptr<Y4mReader> video;
+    if (in_y4m) {
+      video.reset(new Y4mReader(in_path));
+      const size_t n_frames = video->check_frames();
+      std::cout << "Video: " << video->header().w << "x" << video->header().h << ", " << n_frames
+                << " frames" << std::endl;
+    }
 
     opencl::Context context;
     context.init(profile);
@@ -399,6 +447,11 @@ int main(int argc, char** argv) {
       get_training_samples(in_path, files);
       if (files.empty()) throw std::runtime_error("No samples found");
       execute_eval(data_pipeline, gpu_alloc, files, out_path, scale, filter);
+      context.block();
+      return EXIT_SUCCESS;
+    }
+    if (video) {
+      execute_y4m(data_pipeline, gpu_alloc, *video, out_path, scale, filter);
       context.block();
       return EXIT_SUCCESS;
     }

@@ -300,6 +300,40 @@ int srcnn_upscale_frames_host(srcnn_ctx* ctx, const srcnn_net* net, const unsign
                               int w, int h, int n_frames, int out_w, int out_h, int filter,
                               unsigned char* host_rgb);
 
+/* srcnn_upscale_frames_host for video as decoders hand it out and encoders take it: planar
+ * Y'CbCr 4:2:0 (I420, `yuv420p`, the frames of a Y4M file) in and out.  A frame is its Y plane
+ * (w*h bytes), then Cb, then Cr ((w/2)*(h/2) bytes each): host_in holds n_frames frames of
+ * w*h*3/2 bytes, host_out receives n_frames frames of out_w*out_h*3/2 bytes.  Per frame:
+ *   - Y is enlarged to out_w x out_h with Pillow's 8-bit filter (its "L" mode, the arithmetic of
+ *     srcnn_resample on one channel); its luma Y'/255, minus the Q1 "mean" (the mean of the
+ *     squares), goes through the three layers; inside the network's output region the result is
+ *     clamp(luma * 255, 0, 255) truncated -- the byte swap_luma writes for a pixel with zero
+ *     chroma -- and the border of (f1+f2+f3-3)/2 rows and columns keeps the enlarged Y, as
+ *     swap_luma leaves it.
+ *   - Cb and Cr are each enlarged (w/2, h/2) -> (out_w/2, out_h/2) with the same filter.  Pillow
+ *     maps pixel centres onto pixel centres, which is right for centre-sited ("jpeg", Y4M's
+ *     default 420jpeg) chroma; left-sited chroma (MPEG-2 and later codecs' default) would shift.
+ *   - The network sees the Y plane as stored: there is no range conversion, full or limited.
+ * A frame's bytes do not depend on the other frames of the call or on the group size.
+ * Synchronous; pageable buffers work, pinned ones give the overlap.  Waits for
+ * srcnn_infer_rows_host_async calls in flight first.  Staging is the context's and apart from the
+ * other entries'.  Networks with a fused kernel run groups of frames through the ring of
+ * srcnn_upscale_frames_host; the device work of a group is one launch per step with every frame
+ * in the grid: the enlargement of all three planes straight into the result slot + the luma, the
+ * Q1 sum (2), minus the mean, the fused forward, the Y write.  A group holds as many frames as fit
+ * ~128 MB of device staging (3 * (w*h*3/2 + out_w*out_h*3/2) + out_w*out_h*4 + h3*w3*4 bytes a
+ * frame: input and result in each of the 3 ring slots, luma, network output; 4 frames of 960x540
+ * -> 1920x1080), or SRCNN_FRAMES_GROUP frames when that is set (at most 21845).  Networks without
+ * a fused kernel run frame by frame (upload, head, forward, Y write, download), for the reason
+ * srcnn_upscale_frames_host gives.
+ * Launches per call: n_groups * (5 + F) with a fused kernel, n_frames * (4 + L + 1) without (F, L
+ * as for srcnn_upscale_frames_host), plus 1 when the network's packed operand image has to be
+ * rebuilt.  Everything srcnn_upscale_image_host rejects, an odd w, h, out_w or out_h, n_frames <= 0
+ * and null pointers: SRCNN_EINVAL before any host buffer is read or written. */
+int srcnn_upscale_yuv420_frames_host(srcnn_ctx* ctx, const srcnn_net* net,
+                                     const unsigned char* host_in, int w, int h, int n_frames,
+                                     int out_w, int out_h, int filter, unsigned char* host_out);
+
 /* srcnn_upscale_frames_host plus the quality of its results: host_ref holds n_frames reference
  * frames of out_w*out_h*4 bytes RGBA8 (the ground truth the small frames were made from).
  * host_rgb receives what srcnn_upscale_frames_host returns for the same arguments, byte for byte;
