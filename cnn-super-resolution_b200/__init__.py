@@ -66,6 +66,32 @@ class CNet(C.Structure):
                 ("prev_dw", _u64 * 3), ("prev_db", _u64 * 3)]
 
 
+YUV420_FORMATS = {"i420": 0, "nv12": 1}   # SRCNN_YUV_I420 / _NV12
+
+
+class CYuv420Layout(C.Structure):
+    """struct srcnn_yuv420_layout of include/srcnn_b200.h"""
+    _fields_ = [("format", _i), ("frame_stride", _sz), ("y_pitch", _sz), ("c_pitch", _sz),
+                ("cb_offset", _sz), ("cr_offset", _sz)]
+
+
+def yuv420_layout(fmt, w, h, y_pitch=None, c_pitch=None, cb_offset=None, frame_stride=None):
+    """Where the planes of w x h 4:2:0 frames ("i420" or "nv12") lie in a buffer, in bytes.  The
+    defaults are the dense layout; otherwise the chroma follows Y at cb_offset (default: right after
+    the Y plane's h rows), an I420 Cr plane follows Cb right after its h/2 rows, and a frame spans
+    frame_stride bytes (default: to the end of its last plane's last pitched row)."""
+    if fmt not in YUV420_FORMATS:
+        raise ValueError("unknown 4:2:0 format %r (have %s)" % (fmt, sorted(YUV420_FORMATS)))
+    nv12 = fmt == "nv12"
+    y_pitch = w if y_pitch is None else y_pitch
+    c_pitch = (w if nv12 else w // 2) if c_pitch is None else c_pitch
+    cb_offset = h * y_pitch if cb_offset is None else cb_offset
+    cr_offset = 0 if nv12 else cb_offset + (h // 2) * c_pitch
+    end = (cb_offset if nv12 else cr_offset) + (h // 2) * c_pitch
+    return CYuv420Layout(YUV420_FORMATS[fmt], end if frame_stride is None else frame_stride,
+                         y_pitch, c_pitch, cb_offset, cr_offset)
+
+
 _SIGS = {
     "srcnn_ctx_create": (_i, [_i, _i, C.POINTER(_vp)]),
     "srcnn_ctx_create_on_stream": (_i, [_i, _vp, _i, C.POINTER(_vp)]),
@@ -105,6 +131,8 @@ _SIGS = {
     "srcnn_upscale_frames_host": (_i, [_vp, C.POINTER(CNet), _vp, _i, _i, _i, _i, _i, _i, _vp]),
     "srcnn_upscale_yuv420_frames_host": (_i, [_vp, C.POINTER(CNet), _vp, _i, _i, _i, _i, _i, _i,
                                               _vp]),
+    "srcnn_upscale_yuv420_frames": (_i, [_vp, C.POINTER(CNet), _u64, C.POINTER(CYuv420Layout), _i,
+                                         _i, _i, _u64, C.POINTER(CYuv420Layout), _i, _i, _i]),
     "srcnn_image_quality": (_i, [_vp, _u64, _i, _u64, _i, _i, _i, _i, _u64]),
     "srcnn_evaluate_frames_host": (_i, [_vp, C.POINTER(CNet), _vp, _i, _i, _i, _i, _i, _i, _vp,
                                         _i, _vp, _vp]),
@@ -502,6 +530,20 @@ class Net:
                                                            _np_ptr(frames), w, h, n, out_w, out_h,
                                                            _filter_id(resample), _np_ptr(out)))
         return out
+
+    def upscale_yuv420_frames(self, in_mem, w, h, n_frames, out_mem, out_w, out_h,
+                              resample="lanczos", fmt="i420", in_layout=None, out_layout=None):
+        """upscale_yuv420_frames_host on device memory handles (Context.alloc, or Context.wrap of
+        e.g. a torch CUDA tensor's data_ptr()): n_frames frames of w x h in in_mem -> out_w x out_h
+        in out_mem, both in `fmt` ("i420" or "nv12") and laid out as in_layout / out_layout
+        (yuv420_layout; default: dense).  Enqueued on the context stream; returns at once, without a
+        copy or a host synchronisation."""
+        li = yuv420_layout(fmt, w, h) if in_layout is None else in_layout
+        lo = yuv420_layout(fmt, out_w, out_h) if out_layout is None else out_layout
+        _check(self.ctx.L.srcnn_upscale_yuv420_frames(self.ctx.h, C.byref(self.c), in_mem,
+                                                      C.byref(li), w, h, n_frames, out_mem,
+                                                      C.byref(lo), out_w, out_h,
+                                                      _filter_id(resample)))
 
     def evaluate_frames_host(self, rgba, reference, out_w, out_h, resample="lanczos", border=None,
                              out=None):

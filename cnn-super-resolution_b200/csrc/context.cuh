@@ -189,8 +189,9 @@ struct srcnn_ctx {
     unsigned long long key[kGraphKey] = {};
     unsigned graph_launches[SRCNN_K_COUNT] = {};
   } up;
-  // srcnn_upscale_frames_host (`frames`), srcnn_evaluate_frames_host (`eval`) and
-  // srcnn_upscale_yuv420_frames_host (`yuv`): device staging (grown on demand), apart from `up` and
+  // srcnn_upscale_frames_host (`frames`), srcnn_evaluate_frames_host (`eval`),
+  // srcnn_upscale_yuv420_frames_host (`yuv`) and srcnn_upscale_yuv420_frames (`yuv_dev`, which
+  // uses luma / out / red / s1 / s2 only): device staging (grown on demand), apart from `up` and
   // from each other so that the entries do not resize (and so re-capture) each other's buffers.
   // small / rgb / ref hold a ring of frame groups, rgba / luma / out / red / qred one group.
   struct FramesStaging {
@@ -208,7 +209,7 @@ struct srcnn_ctx {
     size_t small_bytes = 0, rgba_bytes = 0, luma_bytes = 0, out_bytes = 0, rgb_bytes = 0,
            red_bytes = 0, s1_bytes = 0, s2_bytes = 0, ref_bytes = 0, qred_bytes = 0,
            metrics_bytes = 0;
-  } frames, eval, yuv;
+  } frames, eval, yuv, yuv_dev;
   // srcnn_image_quality's reduction partials (grown on demand)
   void* quality_red = nullptr;
   size_t quality_red_bytes = 0;

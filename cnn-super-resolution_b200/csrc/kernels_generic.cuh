@@ -504,10 +504,10 @@ __global__ void swap_luma_kernel(const uchar4* __restrict__ rgba, const float* _
 // swap_luma_kernel for the Y plane of Y'CbCr 4:2:0 frames: the network's luma becomes the byte
 // swap_luma_kernel writes for a pixel with zero chroma, clamp(luma * 255) truncated.  The grid
 // covers the luma_w x luma_h interior, written (gt_w - luma_w) / 2 pixels in from the left and top
-// edges of the gt_w-wide plane; the border keeps the enlarged Y.  Frame blockIdx.z: target +
-// blockIdx.z * frame_bytes (whole frames back to back), luma + blockIdx.z * luma_w * luma_h.
+// edges of the gt_w-wide plane, whose rows are `pitch` bytes apart; the border keeps the enlarged
+// Y.  Frame blockIdx.z: target + blockIdx.z * frame_bytes, luma + blockIdx.z * luma_w * luma_h.
 __global__ void swap_luma_plane_kernel(const float* __restrict__ luma,
-                                       unsigned char* __restrict__ target, int gt_w,
+                                       unsigned char* __restrict__ target, int gt_w, size_t pitch,
                                        size_t frame_bytes, int luma_w, int luma_h) {
   luma += blockIdx.z * (size_t)luma_w * luma_h;
   target += blockIdx.z * frame_bytes;
@@ -516,7 +516,7 @@ __global__ void swap_luma_plane_kernel(const float* __restrict__ luma,
   if (x >= luma_w || y >= luma_h) return;
   const int pad = (gt_w - luma_w) / 2;
   const float Y = __fmul_rn(luma[(size_t)y * luma_w + x], 255.0f);
-  target[(size_t)(y + pad) * gt_w + x + pad] = (unsigned char)(unsigned int)fminf(fmaxf(Y, 0.f), 255.f);
+  target[(size_t)(y + pad) * pitch + x + pad] = (unsigned char)(unsigned int)fminf(fmaxf(Y, 0.f), 255.f);
 }
 
 }  // namespace generic

@@ -21,12 +21,15 @@
 // Pillow's "RGB" path, not its premultiplying "RGBA" one.  A set of equal-sized frames is one
 // launch with the frame in blockIdx.z (frame f reads in + f * in_frame, writes out / luma + f * W * H).
 // The same kernel with one byte a pixel enlarges the planes of Y'CbCr 4:2:0 frames: Pillow's "L"
-// path, and for the Y plane the luma Y' / 255.  Pillow maps pixel centres onto pixel centres, so the
-// chroma planes come out right for centre-sited ("jpeg") chroma.
+// path, and for the Y plane the luma Y' / 255; with two bytes a pixel NV12's interleaved CbCr plane,
+// each byte as its own "L" plane.  Plane rows may be pitched (the luma stays dense).  Pillow maps
+// pixel centres onto pixel centres, so the chroma planes come out right for centre-sited ("jpeg")
+// chroma.
 #pragma once
 #include <algorithm>
 #include <cmath>
 #include <cstring>
+#include <type_traits>
 #include <vector>
 
 #include "context.cuh"
@@ -116,14 +119,16 @@ inline std::vector<int> tables(int w, int h, int W, int H, int filter, int* rows
   return t;
 }
 
-// one plane of a launch: frame f reads in + f * in_frame and writes out + f * out_frame (pixels)
-// and, with luma, luma + f * W * H; tab = table_for(w, h, W, H)
+// one plane of a launch: frame f reads in + f * in_frame and writes out + f * out_frame (pixels),
+// rows in_pitch and out_pitch pixels apart, and, with luma, the dense luma + f * W * H;
+// tab = table_for(w, h, W, H)
 template <class Pix>
 struct Plane {
   const Pix* in;
-  int w;
+  int in_pitch;
   size_t in_frame;
   Pix* out;
+  int out_pitch;
   size_t out_frame;
   float* luma;
   int W, H;
@@ -161,6 +166,16 @@ struct Acc<unsigned char> {
   __device__ __forceinline__ void add(unsigned char p, int k) { s += (int)p * k; }
   __device__ __forceinline__ unsigned char pixel() const { return clip8(s); }
 };
+// two interleaved planes (NV12's CbCr): Acc<unsigned char> on each
+template <>
+struct Acc<uchar2> {
+  int s0 = 1 << (kPrecisionBits - 1), s1 = s0;
+  __device__ __forceinline__ void add(uchar2 p, int k) {
+    s0 += (int)p.x * k;
+    s1 += (int)p.y * k;
+  }
+  __device__ __forceinline__ uchar2 pixel() const { return make_uchar2(clip8(s0), clip8(s1)); }
+};
 // the normalized luma of an enlarged pixel: extract_luma_kernel's of RGBA8, Y' / 255 of a Y plane
 __device__ __forceinline__ float luma_from(uchar4 p) { return generic::luma_of(p, 1); }
 __device__ __forceinline__ float luma_from(unsigned char y) { return __fdiv_rn((float)y, 255.0f); }
@@ -178,7 +193,6 @@ __global__ void __launch_bounds__(kThreads) resample_kernel(const Planes<Pix> pl
   const Pix* __restrict__ in = P.in + f * P.in_frame;
   Pix* __restrict__ out = P.out + f * P.out_frame;
   float* __restrict__ luma = P.luma ? P.luma + f * (size_t)W * H : nullptr;
-  const int w = P.w;
   const int* xb = P.tab;
   const int* xn = xb + W;
   const int* xk = xn + W;
@@ -195,7 +209,7 @@ __global__ void __launch_bounds__(kThreads) resample_kernel(const Planes<Pix> pl
     if (c >= nx) continue;
     const int x = x0 + c;
     const int b = __ldg(xb + x), n = __ldg(xn + x);
-    const Pix* src = in + (size_t)(row0 + r) * w + b;
+    const Pix* src = in + (size_t)(row0 + r) * P.in_pitch + b;
     Acc<Pix> acc;
 #pragma unroll
     for (int j = 0; j < TAPS; j++)
@@ -215,9 +229,9 @@ __global__ void __launch_bounds__(kThreads) resample_kernel(const Planes<Pix> pl
     for (int j = 0; j < TAPS; j++)
       if (j < n) acc.add(mid[(b + j) * kTX + c], __ldg(yk + (size_t)y * TAPS + j));
     const Pix o = acc.pixel();
-    const size_t o_i = (size_t)y * W + x;
-    out[o_i] = o;
-    if (luma) luma[o_i] = luma_from(o);
+    out[(size_t)y * P.out_pitch + x] = o;
+    if constexpr (!std::is_same<Pix, uchar2>::value)
+      if (luma) luma[(size_t)y * W + x] = luma_from(o);
   }
 }
 
@@ -274,27 +288,52 @@ inline int launch_planes(srcnn_ctx* ctx, const Planes<Pix>& planes, int filter, 
 inline int launch(srcnn_ctx* ctx, const uchar4* in, int w, int h, uchar4* out, float* luma, int W,
                   int H, int filter, const int* tab, int rows_max, int frames = 1) {
   Planes<uchar4> p{};
-  p.p[0] = Plane<uchar4>{in, w, (size_t)w * h, out, (size_t)W * H, luma, W, H, tab};
+  p.p[0] = Plane<uchar4>{in, w, (size_t)w * h, out, W, (size_t)W * H, luma, W, H, tab};
   p.n = 1;
   return launch_planes(ctx, p, filter, rows_max, frames);
 }
 
-// `frames` planar Y'CbCr 4:2:0 (I420) frames of w x h (in) -> W x H (out), whole frames back to
-// back: Y through tab_y (w x h -> W x H, its luma into `luma`), Cb and Cr through tab_c
-// (w/2 x h/2 -> W/2 x H/2).  w, h, W and H are even.
-inline int launch_yuv420(srcnn_ctx* ctx, const unsigned char* in, int w, int h, unsigned char* out,
+// `frames` Y'CbCr 4:2:0 frames of w x h (in, layout li) -> W x H (out, layout lo), I420: Y through
+// tab_y (w x h -> W x H, its luma into the dense `luma`), Cb and Cr through tab_c (w/2 x h/2 ->
+// W/2 x H/2), one launch.  w, h, W and H are even; the layouts are I420 and hold the planes (the
+// entries check both).
+inline int launch_yuv420(srcnn_ctx* ctx, const unsigned char* in, const srcnn_yuv420_layout& li,
+                         int w, int h, unsigned char* out, const srcnn_yuv420_layout& lo,
                          float* luma, int W, int H, int filter, const int* tab_y, int rows_y,
                          const int* tab_c, int rows_c, int frames) {
-  const size_t in_y = (size_t)w * h, in_c = in_y / 4, out_y = (size_t)W * H, out_c = out_y / 4;
-  const size_t in_frame = in_y + 2 * in_c, out_frame = out_y + 2 * out_c;
   Planes<unsigned char> p{};
-  p.p[0] = Plane<unsigned char>{in, w, in_frame, out, out_frame, luma, W, H, tab_y};
-  p.p[1] = Plane<unsigned char>{in + in_y, w / 2, in_frame, out + out_y, out_frame, nullptr,
+  p.p[0] = Plane<unsigned char>{in, (int)li.y_pitch, li.frame_stride, out, (int)lo.y_pitch,
+                                lo.frame_stride, luma, W, H, tab_y};
+  p.p[1] = Plane<unsigned char>{in + li.cb_offset, (int)li.c_pitch, li.frame_stride,
+                                out + lo.cb_offset, (int)lo.c_pitch, lo.frame_stride, nullptr,
                                 W / 2, H / 2, tab_c};
-  p.p[2] = Plane<unsigned char>{in + in_y + in_c, w / 2, in_frame, out + out_y + out_c, out_frame,
-                                nullptr, W / 2, H / 2, tab_c};
+  p.p[2] = Plane<unsigned char>{in + li.cr_offset, (int)li.c_pitch, li.frame_stride,
+                                out + lo.cr_offset, (int)lo.c_pitch, lo.frame_stride, nullptr,
+                                W / 2, H / 2, tab_c};
   p.n = 3;
   return launch_planes(ctx, p, filter, std::max(rows_y, rows_c), frames);
+}
+
+// launch_yuv420 for NV12 layouts, whose chroma is one plane of interleaved Cb, Cr pairs: the Y
+// plane, then the CbCr plane as (w/2 x h/2 uchar2 pixels), each byte of a pair as launch_yuv420
+// computes its plane.  Two launches (a launch has one pixel type).  The CbCr planes, their pitches
+// and the frame strides are even (the entry checks them).
+inline int launch_nv12(srcnn_ctx* ctx, const unsigned char* in, const srcnn_yuv420_layout& li,
+                       int w, int h, unsigned char* out, const srcnn_yuv420_layout& lo,
+                       float* luma, int W, int H, int filter, const int* tab_y, int rows_y,
+                       const int* tab_c, int rows_c, int frames) {
+  Planes<unsigned char> y{};
+  y.p[0] = Plane<unsigned char>{in, (int)li.y_pitch, li.frame_stride, out, (int)lo.y_pitch,
+                                lo.frame_stride, luma, W, H, tab_y};
+  y.n = 1;
+  SRCNN_TRY(launch_planes(ctx, y, filter, rows_y, frames));
+  Planes<uchar2> c{};
+  c.p[0] = Plane<uchar2>{reinterpret_cast<const uchar2*>(in + li.cb_offset), (int)(li.c_pitch / 2),
+                         li.frame_stride / 2,
+                         reinterpret_cast<uchar2*>(out + lo.cb_offset), (int)(lo.c_pitch / 2),
+                         lo.frame_stride / 2, nullptr, W / 2, H / 2, tab_c};
+  c.n = 1;
+  return launch_planes(ctx, c, filter, rows_c, frames);
 }
 
 }  // namespace resample

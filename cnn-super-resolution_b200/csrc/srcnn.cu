@@ -162,7 +162,7 @@ int srcnn_ctx_destroy(srcnn_ctx* ctx) {
     for (void* p : {u.small, u.rgba, u.luma, u.out, u.rgb, u.s1, u.s2})
       if (p) cudaFree(p);
   }
-  for (srcnn_ctx::FramesStaging* f : {&ctx->frames, &ctx->eval, &ctx->yuv})
+  for (srcnn_ctx::FramesStaging* f : {&ctx->frames, &ctx->eval, &ctx->yuv, &ctx->yuv_dev})
     for (void* p : {f->small, f->rgba, f->luma, f->out, f->rgb, f->red, f->s1, f->s2, f->ref,
                     f->qred, f->metrics})
       if (p) cudaFree(p);
@@ -1166,6 +1166,8 @@ struct Upscale {
   float* sums;                // Q1 sums, one per frame
   size_t npx() const { return (size_t)out_w * out_h; }
   int red_blocks() const { return grid_1d(npx(), generic::RED_THREADS, generic::RED_MAX_BLOCKS); }
+  // the Q1 reduction bytes of one frame: its partials and its sum
+  size_t red_frame() const { return sizeof(double) * red_blocks() + sizeof(float); }
 };
 
 // the Q1 "mean" of every frame's u.luma (sum of squares / count, subtracted on the device:
@@ -1405,7 +1407,6 @@ int frames_prepare(srcnn_ctx* ctx, const srcnn_net* net, srcnn_ctx::FramesStagin
   SRCNN_CUDA(ctx->drain_lanes());
   const bool fused = fast::fused_supported(net->n1, net->n2, net->f1, net->f2, net->f3);
   Upscale u{w, h, out_w, out_h, filter, 1, d, nullptr, 0};
-  const size_t red_frame = sizeof(double) * u.red_blocks() + sizeof(float);
   const int group =
       fused ? std::min(frames_group(fb.group, (size_t)128 << 20, n_frames), fb.max_group) : 1;
   const int ring = fused ? kFrameRing : 1;
@@ -1414,7 +1415,7 @@ int frames_prepare(srcnn_ctx* ctx, const srcnn_net* net, srcnn_ctx::FramesStagin
   SRCNN_TRY(ensure_scratch(ctx, &st.luma, &st.luma_bytes, npx * sizeof(float) * group));
   SRCNN_TRY(ensure_scratch(ctx, &st.out, &st.out_bytes, out_px * sizeof(float) * group));
   SRCNN_TRY(ensure_scratch(ctx, &st.rgb, &st.rgb_bytes, fb.out * group * ring));
-  SRCNN_TRY(ensure_scratch(ctx, &st.red, &st.red_bytes, red_frame * group));
+  SRCNN_TRY(ensure_scratch(ctx, &st.red, &st.red_bytes, u.red_frame() * group));
   if (!fused) {
     SRCNN_TRY(ensure_scratch(ctx, &st.s1, &st.s1_bytes, sizeof(float) * (size_t)d.w1 * d.h1 * net->n1));
     SRCNN_TRY(ensure_scratch(ctx, &st.s2, &st.s2_bytes, sizeof(float) * (size_t)d.w2 * d.h2 * net->n2));
@@ -1537,24 +1538,78 @@ int srcnn_evaluate_frames_host(srcnn_ctx* ctx, const srcnn_net* net, const unsig
 }
 
 namespace {
-// A group of Y'CbCr 4:2:0 (I420) frames of an Upscale job (its u.small, u.rgba and u.rgb unused):
-// whole frames back to back in `in` and `out`, the chroma planes enlarged through tab_c.
+// the arguments srcnn_upscale_yuv420_frames_host and srcnn_upscale_yuv420_frames accept
+int check_yuv420(const srcnn_net* net, int w, int h, int n_frames, int out_w, int out_h,
+                 int filter) {
+  SRCNN_TRY(check_upscale(net, w, h, out_w, out_h, filter));
+  SRCNN_REQUIRE(w % 2 == 0 && h % 2 == 0 && out_w % 2 == 0 && out_h % 2 == 0,
+                "4:2:0 frames need even sizes, got %dx%d -> %dx%d", w, h, out_w, out_h);
+  SRCNN_REQUIRE(n_frames > 0, "bad frame count %d", n_frames);
+  return SRCNN_OK;
+}
+
+// whole I420 frames of w x h back to back: the frames of srcnn_upscale_yuv420_frames_host
+srcnn_yuv420_layout i420_dense(int w, int h) {
+  const size_t y = (size_t)w * h, c = y / 4;
+  return srcnn_yuv420_layout{SRCNN_YUV_I420, y + 2 * c, (size_t)w, (size_t)w / 2, y, y + c};
+}
+
+// the layout of n_frames frames of w x h (w, h even and > 0) holds them: *need = the bytes from
+// the first frame's start to the end of the last frame's last plane
+int check_layout(const srcnn_yuv420_layout& l, int w, int h, int n_frames, size_t* need,
+                 const char* what) {
+  const bool nv12 = l.format == SRCNN_YUV_NV12;
+  const size_t big = (size_t)1 << 31, c_row = nv12 ? (size_t)w : (size_t)w / 2;
+  SRCNN_REQUIRE(l.frame_stride < big && l.y_pitch < big && l.c_pitch < big && l.cb_offset < big &&
+                    l.cr_offset < big,
+                "%s layout: a pitch, offset or stride of 2^31 bytes or more", what);
+  SRCNN_REQUIRE(l.y_pitch >= (size_t)w && l.c_pitch >= c_row,
+                "%s layout: pitches %zu (Y) and %zu (chroma) below the rows' %d and %zu bytes", what,
+                l.y_pitch, l.c_pitch, w, c_row);
+  // the planes' byte ranges from the frame start: Y [0, y_end), chroma [offset, offset + c_len)
+  const size_t y_end = (size_t)(h - 1) * l.y_pitch + w;
+  const size_t c_len = (size_t)(h / 2 - 1) * l.c_pitch + c_row;
+  size_t extent = std::max(y_end, l.cb_offset + c_len);
+  SRCNN_REQUIRE(l.cb_offset >= y_end, "%s layout: the %s plane at %zu intersects the Y plane [0, %zu)",
+                what, nv12 ? "CbCr" : "Cb", l.cb_offset, y_end);
+  if (nv12) {
+    SRCNN_REQUIRE(l.cr_offset == 0, "%s layout: NV12 needs cr_offset 0, got %zu", what, l.cr_offset);
+    SRCNN_REQUIRE(l.c_pitch % 2 == 0, "%s layout: NV12 needs an even c_pitch, got %zu", what,
+                  l.c_pitch);
+  } else {
+    SRCNN_REQUIRE(l.cr_offset >= y_end &&
+                      (l.cr_offset >= l.cb_offset + c_len || l.cb_offset >= l.cr_offset + c_len),
+                  "%s layout: the Cr plane at %zu intersects the Y plane [0, %zu) or the Cb plane "
+                  "[%zu, %zu)", what, l.cr_offset, y_end, l.cb_offset, l.cb_offset + c_len);
+    extent = std::max(extent, l.cr_offset + c_len);
+  }
+  SRCNN_REQUIRE(n_frames == 1 || l.frame_stride >= extent,
+                "%s layout: frame_stride %zu below the frame's extent %zu", what, l.frame_stride,
+                extent);
+  *need = (size_t)(n_frames - 1) * l.frame_stride + extent;
+  return SRCNN_OK;
+}
+
+// A group of Y'CbCr 4:2:0 frames of an Upscale job (its u.small, u.rgba and u.rgb unused): frame
+// f at in + f * li.frame_stride and out + f * lo.frame_stride, the chroma planes enlarged through
+// tab_c.
 struct Yuv420 {
   const int* tab_c;
   int rows_max_c;
   const unsigned char* in;
   unsigned char* out;
+  srcnn_yuv420_layout li, lo;
 };
 
-size_t yuv420_frame(int w, int h) { return (size_t)w * h * 3 / 2; }
-
-// the device work the forward waits for: the three planes enlarged straight into the result
-// frames, the luma of the Y plane, its Q1 mean.  4 launches.
+// the device work the forward waits for: the planes enlarged straight into the result frames,
+// the luma of the Y plane, its Q1 mean.  4 launches (I420), 5 (NV12).
 int yuv420_head(srcnn_ctx* ctx, const Upscale& u, const Yuv420& y) {
   {
-    LaunchScope scope(ctx, SRCNN_K_RESAMPLE);
-    SRCNN_TRY(resample::launch_yuv420(ctx, y.in, u.w, u.h, y.out, u.luma, u.out_w, u.out_h,
-                                      u.filter, u.tab, u.rows_max, y.tab_c, y.rows_max_c, u.frames));
+    const bool nv12 = y.li.format == SRCNN_YUV_NV12;
+    LaunchScope scope(ctx, SRCNN_K_RESAMPLE, nv12 ? 2 : 1);
+    SRCNN_TRY((nv12 ? resample::launch_nv12 : resample::launch_yuv420)(
+        ctx, y.in, y.li, u.w, u.h, y.out, y.lo, u.luma, u.out_w, u.out_h, u.filter, u.tab,
+        u.rows_max, y.tab_c, y.rows_max_c, u.frames));
     SRCNN_TRY(check_launch("resample"));
   }
   return q1_mean(ctx, u);
@@ -1565,7 +1620,7 @@ int yuv420_swap(srcnn_ctx* ctx, const Upscale& u, const Yuv420& y) {
   LaunchScope scope(ctx, SRCNN_K_SWAP_LUMA);
   dim3 block(32, 8), grid((u.d.w3 + 31) / 32, (u.d.h3 + 7) / 8, u.frames);
   generic::swap_luma_plane_kernel<<<grid, block, 0, ctx->stream>>>(
-      u.out3, y.out, u.out_w, yuv420_frame(u.out_w, u.out_h), u.d.w3, u.d.h3);
+      u.out3, y.out, u.out_w, y.lo.y_pitch, y.lo.frame_stride, u.d.w3, u.d.h3);
   return check_launch("swap_luma");
 }
 }  // namespace
@@ -1575,13 +1630,11 @@ int srcnn_upscale_yuv420_frames_host(srcnn_ctx* ctx, const srcnn_net* net,
                                      int out_w, int out_h, int filter, unsigned char* host_out) {
   SRCNN_REQUIRE(ctx && host_in && host_out, "null argument");
   SRCNN_ENTER(ctx);
-  SRCNN_TRY(check_upscale(net, w, h, out_w, out_h, filter));
-  SRCNN_REQUIRE(w % 2 == 0 && h % 2 == 0 && out_w % 2 == 0 && out_h % 2 == 0,
-                "4:2:0 frames need even sizes, got %dx%d -> %dx%d", w, h, out_w, out_h);
-  SRCNN_REQUIRE(n_frames > 0, "bad frame count %d", n_frames);
+  SRCNN_TRY(check_yuv420(net, w, h, n_frames, out_w, out_h, filter));
   srcnn_ctx::FramesStaging& st = ctx->yuv;
   const Dims d = net_dims(net, out_w, out_h);
-  const size_t in_frame = yuv420_frame(w, h), out_frame = yuv420_frame(out_w, out_h);
+  Yuv420 y{nullptr, 0, nullptr, nullptr, i420_dense(w, h), i420_dense(out_w, out_h)};
+  const size_t in_frame = y.li.frame_stride, out_frame = y.lo.frame_stride;
   // the device bytes a frame of a group holds: its input and result in each ring slot, its luma
   // and its network output (960x540 -> 1920x1080: 4 frames in ~128 MB); the frame and the plane
   // share the grid dimension of the resampling launch
@@ -1591,7 +1644,6 @@ int srcnn_upscale_yuv420_frames_host(srcnn_ctx* ctx, const srcnn_net* net,
                       65535 / 3};
   FramesCall fc;
   SRCNN_TRY(frames_prepare(ctx, net, st, w, h, n_frames, out_w, out_h, filter, fb, &fc));
-  Yuv420 y{nullptr, 0, nullptr, nullptr};
   SRCNN_TRY(resample::table_for(ctx, w / 2, h / 2, out_w / 2, out_h / 2, filter, &y.tab_c,
                                 &y.rows_max_c));
   unsigned char* ring_in = (unsigned char*)st.small;
@@ -1623,6 +1675,65 @@ int srcnn_upscale_yuv420_frames_host(srcnn_ctx* ctx, const srcnn_net* net,
                           SRCNN_TRY(launch_fused(ctx, fc.fn, u.luma, u.out3, u.out_w, u.out_h, S));
                           return yuv420_swap(ctx, u, y);
                         });
+}
+
+int srcnn_upscale_yuv420_frames(srcnn_ctx* ctx, const srcnn_net* net, srcnn_mem in,
+                                const srcnn_yuv420_layout* in_layout, int w, int h, int n_frames,
+                                srcnn_mem out, const srcnn_yuv420_layout* out_layout, int out_w,
+                                int out_h, int filter) {
+  SRCNN_ENTER(ctx);
+  SRCNN_TRY(check_yuv420(net, w, h, n_frames, out_w, out_h, filter));
+  SRCNN_REQUIRE(in_layout && out_layout, "null layout");
+  const int format = in_layout->format;
+  SRCNN_REQUIRE(format == SRCNN_YUV_I420 || format == SRCNN_YUV_NV12, "unknown 4:2:0 format %d",
+                format);
+  SRCNN_REQUIRE(out_layout->format == format, "input format %d and output format %d differ", format,
+                out_layout->format);
+  size_t in_need, out_need;
+  SRCNN_TRY(check_layout(*in_layout, w, h, n_frames, &in_need, "input"));
+  SRCNN_TRY(check_layout(*out_layout, out_w, out_h, n_frames, &out_need, "output"));
+  const unsigned char* pi;
+  unsigned char* po;
+  SRCNN_TRY(resolve(ctx, in, in_need, &pi, "input frames"));
+  SRCNN_TRY(resolve(ctx, out, out_need, &po, "output frames"));
+  const bool nv12 = format == SRCNN_YUV_NV12;
+  if (nv12) {
+    // the CbCr plane is read and written as uchar2: every frame's must start at an even address
+    SRCNN_REQUIRE(((uintptr_t)pi + in_layout->cb_offset) % 2 == 0 &&
+                      (n_frames == 1 || in_layout->frame_stride % 2 == 0),
+                  "input NV12 CbCr plane at an odd address");
+    SRCNN_REQUIRE(((uintptr_t)po + out_layout->cb_offset) % 2 == 0 &&
+                      (n_frames == 1 || out_layout->frame_stride % 2 == 0),
+                  "output NV12 CbCr plane at an odd address");
+  }
+  SRCNN_REQUIRE(pi + in_need <= po || po + out_need <= pi, "input and output bytes overlap");
+  ctx->note_write(out);
+  const Upscale job{w, h, out_w, out_h, filter, 1, net_dims(net, out_w, out_h), nullptr, 0};
+  // the scratch a frame of a group needs: its luma, its network output, its Q1 partials and sum;
+  // the frame (times the planes, I420) is a grid dimension of the group's launches
+  const FrameBytes fb{0, 0, 0,
+                      job.npx() * 4 + (size_t)job.d.w3 * job.d.h3 * 4 + job.red_frame(),
+                      nv12 ? 65535 : 65535 / 3};
+  FramesCall fc;
+  SRCNN_TRY(frames_prepare(ctx, net, ctx->yuv_dev, w, h, n_frames, out_w, out_h, filter, fb, &fc));
+  Yuv420 y{nullptr, 0, pi, po, *in_layout, *out_layout};
+  SRCNN_TRY(resample::table_for(ctx, w / 2, h / 2, out_w / 2, out_h / 2, filter, &y.tab_c,
+                                &y.rows_max_c));
+  // groups of frames (one frame without a fused kernel, for the reason forward_three_launch
+  // gives): enlargement + luma, Q1 mean, forward, Y write
+  Upscale& u = fc.u;
+  for (int f0 = 0; f0 < n_frames; f0 += fc.group) {
+    u.frames = std::min(fc.group, n_frames - f0);
+    y.in = pi + (size_t)f0 * y.li.frame_stride;
+    y.out = po + (size_t)f0 * y.lo.frame_stride;
+    SRCNN_TRY(yuv420_head(ctx, u, y));
+    if (fc.fused)
+      SRCNN_TRY(launch_fused(ctx, fc.fn, u.luma, u.out3, u.out_w, u.out_h, u.frames));
+    else
+      SRCNN_TRY(forward_three_launch(ctx, net, u, ctx->yuv_dev.s1, ctx->yuv_dev.s2));
+    SRCNN_TRY(yuv420_swap(ctx, u, y));
+  }
+  return SRCNN_OK;
 }
 
 int srcnn_infer_frames_host(srcnn_ctx* ctx, const srcnn_net* net, const float* host_in, int w,

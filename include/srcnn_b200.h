@@ -71,8 +71,11 @@ enum srcnn_kernel_id {
  * `profile` != 0 times every launch with a cudaEvent pair and blocks on it, like
  * CL_QUEUE_PROFILING_ENABLE + clWaitForEvents (src/opencl/Kernel.cpp:108-116). */
 int srcnn_ctx_create(int device, int profile, srcnn_ctx** out);
-/* Same, but enqueue on a caller-owned cudaStream_t (e.g. torch's current stream) so that
- * launches order with the caller's own work (NCCL all-reduce of the gradient). */
+/* Same, but enqueue on a caller-owned cudaStream_t (e.g. a torch.cuda.Stream()) so that
+ * launches order with the caller's own work (NCCL all-reduce of the gradient).  A null
+ * cuda_stream -- which is also what the legacy default stream, e.g. torch's current stream in a
+ * process that never switched streams, reports as its handle -- is not that stream: the context
+ * then creates a non-blocking stream of its own, which does not order with the default stream. */
 int srcnn_ctx_create_on_stream(int device, void* cuda_stream, int profile, srcnn_ctx** out);
 /* Context::~Context / _cleanup (src/opencl/Context.cpp:81-109): waits, frees everything. */
 int srcnn_ctx_destroy(srcnn_ctx* ctx);
@@ -333,6 +336,63 @@ int srcnn_upscale_frames_host(srcnn_ctx* ctx, const srcnn_net* net, const unsign
 int srcnn_upscale_yuv420_frames_host(srcnn_ctx* ctx, const srcnn_net* net,
                                      const unsigned char* host_in, int w, int h, int n_frames,
                                      int out_w, int out_h, int filter, unsigned char* host_out);
+
+/* Where the planes of 4:2:0 frames lie in a device buffer.  A frame's Y plane starts at the frame's
+ * first byte; every offset, pitch and stride is in bytes.  SRCNN_YUV_I420: Y, Cb and Cr planes
+ * (`yuv420p`); SRCNN_YUV_NV12: Y, then one plane of interleaved Cb, Cr pairs, Cb first (what
+ * hardware video decoders hand out and encoders take).  The dense I420 layout of
+ * srcnn_upscale_yuv420_frames_host is {I420, w*h*3/2, w, w/2, w*h, w*h*5/4}, the dense NV12 one
+ * {NV12, w*h*3/2, w, w, w*h, 0}. */
+enum { SRCNN_YUV_I420 = 0, SRCNN_YUV_NV12 = 1 };
+typedef struct srcnn_yuv420_layout {
+  int format;           /* SRCNN_YUV_I420 or SRCNN_YUV_NV12 */
+  size_t frame_stride;  /* from one frame's start to the next's */
+  size_t y_pitch;       /* from one Y row to the next, >= width */
+  size_t c_pitch;       /* from one chroma row to the next, >= width/2 (I420) or width (NV12) */
+  size_t cb_offset;     /* of the Cb plane (NV12: the CbCr plane) from the frame start */
+  size_t cr_offset;     /* I420: of the Cr plane; NV12: must be 0 */
+} srcnn_yuv420_layout;
+
+/* srcnn_upscale_yuv420_frames_host on frames that are already in device memory, in I420 or NV12
+ * with pitched rows: `in` holds n_frames frames of w x h in in_layout, `out` receives n_frames
+ * frames of out_w x out_h in out_layout, of the same format.  The Y, Cb and Cr bytes of a frame are
+ * those srcnn_upscale_yuv420_frames_host writes for it (NV12: the same Cb and Cr bytes,
+ * interleaved).  Bytes of `out` outside the planes' rows (pitch padding, gaps between planes or
+ * frames) are never written; bytes of `in` outside them never affect the result.
+ * Stream-ordered, like srcnn_forward_fused: the work is enqueued on the context stream and the
+ * call returns, without a copy or a host synchronisation (the caller orders its own work on that
+ * stream: create the context with srcnn_ctx_create_on_stream on a non-default stream, e.g. a
+ * torch.cuda.Stream(), and fill `in` and read `out` on it).  Once a call with the same sizes,
+ * layouts' formats and network has run, a call allocates nothing, so it can be captured into a
+ * CUDA graph on the context stream.  Such a graph reads the entry's scratch, which grows on
+ * demand: a later call on the context that needs more of it (larger frames, or more frames a
+ * group) reallocates it, and the graph must then be captured again.  It waits for
+ * srcnn_infer_rows_host_async calls in flight first; in profile mode every launch blocks.  Staging
+ * is the context's and apart from the other entries'.
+ * Networks with a fused kernel run groups of frames, one launch per step with every frame of the
+ * group in the grid: the enlargement of the planes straight into `out` + the luma of Y, the Q1 sum
+ * (2), minus the mean, the fused forward, the Y write.  A group holds as many frames as fit
+ * ~128 MB of device scratch (out_w*out_h*4 + h3*w3*4 bytes and the Q1 partials a frame: 8 frames
+ * of 1920x1080 with a 9-1-5 network), or SRCNN_FRAMES_GROUP frames when that is set (at most
+ * 21845 for I420, 65535 for NV12).  Networks without a fused kernel run frame by frame, for the
+ * reason srcnn_upscale_frames_host gives.
+ * Launches per call: n_groups * (5 + F) for I420 and n_groups * (6 + F) for NV12 (whose Y plane and
+ * CbCr plane are one enlargement launch each) with a fused kernel, n_frames * (4 + L + 1) without
+ * (plus n_frames for NV12), plus 1 when the network's packed operand image has to be rebuilt (F, L
+ * as for srcnn_upscale_frames_host).
+ * Errors, all before any launch (the output and the launch count stay untouched):
+ *   SRCNN_EINVAL: everything srcnn_upscale_yuv420_frames_host rejects; a null layout; an unknown
+ *     format, or formats that differ; a pitch below its row's bytes; a pitch, offset or stride of
+ *     2^31 bytes or more; planes of one frame whose byte ranges intersect; with n_frames > 1, a
+ *     frame_stride below the frame's extent (the end of its last plane's last row); NV12 with
+ *     cr_offset != 0, an odd c_pitch, or a CbCr plane at an odd address in any frame; input and
+ *     output byte ranges that overlap.
+ *   SRCNN_EHANDLE / SRCNN_ERANGE: an unknown buffer, or one smaller than
+ *     (n_frames - 1) * frame_stride + the frame's extent. */
+int srcnn_upscale_yuv420_frames(srcnn_ctx* ctx, const srcnn_net* net, srcnn_mem in,
+                                const srcnn_yuv420_layout* in_layout, int w, int h, int n_frames,
+                                srcnn_mem out, const srcnn_yuv420_layout* out_layout, int out_w,
+                                int out_h, int filter);
 
 /* srcnn_upscale_frames_host plus the quality of its results: host_ref holds n_frames reference
  * frames of out_w*out_h*4 bytes RGBA8 (the ground truth the small frames were made from).
