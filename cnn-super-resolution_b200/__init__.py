@@ -67,21 +67,32 @@ class CNet(C.Structure):
 
 
 YUV420_FORMATS = {"i420": 0, "nv12": 1}   # SRCNN_YUV_I420 / _NV12
+# SRCNN_CHROMA_CENTER / _LEFT / _TOPLEFT, by ffmpeg's chroma_location names
+CHROMA_SITINGS = {"center": 0, "left": 1, "topleft": 2}
 
 
 class CYuv420Layout(C.Structure):
     """struct srcnn_yuv420_layout of include/srcnn_b200.h"""
     _fields_ = [("format", _i), ("frame_stride", _sz), ("y_pitch", _sz), ("c_pitch", _sz),
-                ("cb_offset", _sz), ("cr_offset", _sz)]
+                ("cb_offset", _sz), ("cr_offset", _sz), ("chroma_siting", _i)]
 
 
-def yuv420_layout(fmt, w, h, y_pitch=None, c_pitch=None, cb_offset=None, frame_stride=None):
-    """Where the planes of w x h 4:2:0 frames ("i420" or "nv12") lie in a buffer, in bytes.  The
-    defaults are the dense layout; otherwise the chroma follows Y at cb_offset (default: right after
-    the Y plane's h rows), an I420 Cr plane follows Cb right after its h/2 rows, and a frame spans
-    frame_stride bytes (default: to the end of its last plane's last pitched row)."""
+def _siting_id(name):
+    if name not in CHROMA_SITINGS:
+        raise ValueError("unknown chroma siting %r (have %s)" % (name, sorted(CHROMA_SITINGS)))
+    return CHROMA_SITINGS[name]
+
+
+def yuv420_layout(fmt, w, h, y_pitch=None, c_pitch=None, cb_offset=None, frame_stride=None,
+                  chroma_siting="center"):
+    """Where the planes of w x h 4:2:0 frames ("i420" or "nv12") lie in a buffer, in bytes, and
+    where their chroma samples sit (CHROMA_SITINGS).  The defaults are the dense layout; otherwise
+    the chroma follows Y at cb_offset (default: right after the Y plane's h rows), an I420 Cr plane
+    follows Cb right after its h/2 rows, and a frame spans frame_stride bytes (default: to the end
+    of its last plane's last pitched row)."""
     if fmt not in YUV420_FORMATS:
         raise ValueError("unknown 4:2:0 format %r (have %s)" % (fmt, sorted(YUV420_FORMATS)))
+    siting = _siting_id(chroma_siting)
     nv12 = fmt == "nv12"
     y_pitch = w if y_pitch is None else y_pitch
     c_pitch = (w if nv12 else w // 2) if c_pitch is None else c_pitch
@@ -89,7 +100,7 @@ def yuv420_layout(fmt, w, h, y_pitch=None, c_pitch=None, cb_offset=None, frame_s
     cr_offset = 0 if nv12 else cb_offset + (h // 2) * c_pitch
     end = (cb_offset if nv12 else cr_offset) + (h // 2) * c_pitch
     return CYuv420Layout(YUV420_FORMATS[fmt], end if frame_stride is None else frame_stride,
-                         y_pitch, c_pitch, cb_offset, cr_offset)
+                         y_pitch, c_pitch, cb_offset, cr_offset, siting)
 
 
 _SIGS = {
@@ -131,6 +142,8 @@ _SIGS = {
     "srcnn_upscale_frames_host": (_i, [_vp, C.POINTER(CNet), _vp, _i, _i, _i, _i, _i, _i, _vp]),
     "srcnn_upscale_yuv420_frames_host": (_i, [_vp, C.POINTER(CNet), _vp, _i, _i, _i, _i, _i, _i,
                                               _vp]),
+    "srcnn_upscale_yuv420_frames_host_sited": (_i, [_vp, C.POINTER(CNet), _vp, _i, _i, _i, _i,
+                                                    _i, _i, _i, _i, _vp]),
     "srcnn_upscale_yuv420_frames": (_i, [_vp, C.POINTER(CNet), _u64, C.POINTER(CYuv420Layout), _i,
                                          _i, _i, _u64, C.POINTER(CYuv420Layout), _i, _i, _i]),
     "srcnn_image_quality": (_i, [_vp, _u64, _i, _u64, _i, _i, _i, _i, _u64]),
@@ -514,11 +527,15 @@ class Net:
                                                     _filter_id(resample), _np_ptr(out)))
         return out
 
-    def upscale_yuv420_frames_host(self, frames, w, h, out_w, out_h, resample="lanczos", out=None):
+    def upscale_yuv420_frames_host(self, frames, w, h, out_w, out_h, resample="lanczos", out=None,
+                                   chroma_siting="center", out_chroma_siting=None):
         """frames: uint8 [n][w*h*3//2] planar Y'CbCr 4:2:0 (I420: Y, then Cb, then Cr; w and h
         even) -> uint8 [n][out_w*out_h*3//2] I420: Y enlarged with Pillow's filter and its interior
-        replaced by the network's luma, Cb and Cr enlarged with the same filter (centre-sited
-        chroma).  `out` may be a preallocated (pinned) array."""
+        replaced by the network's luma, Cb and Cr enlarged with the same filter from chroma sited
+        at `chroma_siting` to chroma sited at `out_chroma_siting` (CHROMA_SITINGS; None: the
+        input's).  `out` may be a preallocated (pinned) array."""
+        s_in = _siting_id(chroma_siting)
+        s_out = s_in if out_chroma_siting is None else _siting_id(out_chroma_siting)
         n = frames.shape[0]
         assert frames.dtype == np.uint8 and frames.ndim == 2 and frames.shape[1] == w * h * 3 // 2
         frames = np.ascontiguousarray(frames)
@@ -526,9 +543,14 @@ class Net:
             out = np.empty((n, out_w * out_h * 3 // 2), np.uint8)
         assert out.dtype == np.uint8 and out.shape == (n, out_w * out_h * 3 // 2)
         assert out.flags.c_contiguous
-        _check(self.ctx.L.srcnn_upscale_yuv420_frames_host(self.ctx.h, C.byref(self.c),
-                                                           _np_ptr(frames), w, h, n, out_w, out_h,
-                                                           _filter_id(resample), _np_ptr(out)))
+        if s_in == s_out == CHROMA_SITINGS["center"]:
+            _check(self.ctx.L.srcnn_upscale_yuv420_frames_host(
+                self.ctx.h, C.byref(self.c), _np_ptr(frames), w, h, n, out_w, out_h,
+                _filter_id(resample), _np_ptr(out)))
+        else:
+            _check(self.ctx.L.srcnn_upscale_yuv420_frames_host_sited(
+                self.ctx.h, C.byref(self.c), _np_ptr(frames), w, h, n, out_w, out_h,
+                _filter_id(resample), s_in, s_out, _np_ptr(out)))
         return out
 
     def upscale_yuv420_frames(self, in_mem, w, h, n_frames, out_mem, out_w, out_h,
@@ -536,7 +558,8 @@ class Net:
         """upscale_yuv420_frames_host on device memory handles (Context.alloc, or Context.wrap of
         e.g. a torch CUDA tensor's data_ptr()): n_frames frames of w x h in in_mem -> out_w x out_h
         in out_mem, both in `fmt` ("i420" or "nv12") and laid out as in_layout / out_layout
-        (yuv420_layout; default: dense).  Enqueued on the context stream; returns at once, without a
+        (yuv420_layout, which also carries the chroma siting; default: dense, centre-sited).
+        Enqueued on the context stream; returns at once, without a
         copy or a host synchronisation."""
         li = yuv420_layout(fmt, w, h) if in_layout is None else in_layout
         lo = yuv420_layout(fmt, out_w, out_h) if out_layout is None else out_layout

@@ -22,9 +22,16 @@
 // launch with the frame in blockIdx.z (frame f reads in + f * in_frame, writes out / luma + f * W * H).
 // The same kernel with one byte a pixel enlarges the planes of Y'CbCr 4:2:0 frames: Pillow's "L"
 // path, and for the Y plane the luma Y' / 255; with two bytes a pixel NV12's interleaved CbCr plane,
-// each byte as its own "L" plane.  Plane rows may be pitched (the luma stays dense).  Pillow maps
-// pixel centres onto pixel centres, so the chroma planes come out right for centre-sited ("jpeg")
-// chroma.
+// each byte as its own "L" plane.  Plane rows may be pitched (the luma stays dense).
+//
+// Chroma siting lives in the tables alone.  Pillow maps pixel centres onto pixel centres, which is
+// right for centre-sited ("jpeg") chroma.  A chroma sample that sits at s (in chroma samples; 0.5
+// centred, 0.25 co-sited with the even luma column or row) is a shift of the sample centres on that
+// axis: the table of an axis from n_in samples sited at s_in to n_out sited at s_out is Pillow's
+// with a box that starts at
+//   in0 = (s_out - 0.5) * scale + (0.5 - s_in),  center = in0 + (i + 0.5) * scale,
+// which is exactly 0.0 for centre to centre (Pillow's plain enlargement, bit for bit); an axis of
+// ratio 1 whose in0 is not 0.0 is resampled, as Pillow resamples a box with a non-zero start.
 #pragma once
 #include <algorithm>
 #include <cmath>
@@ -61,15 +68,25 @@ inline double lanczos(double x) {
   return 0.0;
 }
 
-// one axis: bounds[n_out], counts[n_out], weights[n_out][taps] (int32, zero-padded)
-inline void axis_table(int n_in, int n_out, int filter, std::vector<int>& t) {
+// the offset of a siting inside its 2x2 luma cell, in chroma samples, per axis
+inline double siting_x(int siting) { return siting == SRCNN_CHROMA_CENTER ? 0.5 : 0.25; }
+inline double siting_y(int siting) { return siting == SRCNN_CHROMA_TOPLEFT ? 0.25 : 0.5; }
+// the box start of an axis from n_in samples sited at s_in to n_out sited at s_out
+inline double box_start(int n_in, int n_out, double s_in, double s_out) {
+  const double scale = (double)n_in / n_out;
+  return (s_out - 0.5) * scale + (0.5 - s_in);
+}
+
+// one axis from a box starting at in0: bounds[n_out], counts[n_out], weights[n_out][taps] (int32,
+// zero-padded)
+inline void axis_table(int n_in, int n_out, int filter, double in0, std::vector<int>& t) {
   const int taps = taps_of(filter);
   const size_t base = t.size();
   t.resize(base + (size_t)n_out * (2 + taps), 0);
   int* bounds = t.data() + base;
   int* counts = bounds + n_out;
   int* w = counts + n_out;
-  if (n_in == n_out) {   // not resampled
+  if (n_in == n_out && in0 == 0.0) {   // not resampled
     for (int i = 0; i < n_out; i++) {
       bounds[i] = i;
       counts[i] = 1;
@@ -80,7 +97,7 @@ inline void axis_table(int n_in, int n_out, int filter, std::vector<int>& t) {
   const double support = support_of(filter), scale = (double)n_in / n_out;
   std::vector<double> k((size_t)taps);
   for (int i = 0; i < n_out; i++) {
-    const double center = (i + 0.5) * scale;
+    const double center = in0 + (i + 0.5) * scale;
     int xmin = (int)(center - support + 0.5);
     if (xmin < 0) xmin = 0;
     int xmax = (int)(center + support + 0.5);
@@ -102,12 +119,13 @@ inline void axis_table(int n_in, int n_out, int filter, std::vector<int>& t) {
   }
 }
 
-// the host tables of (w, h) -> (W, H): horizontal axis first, then vertical, plus the most
-// input rows one CTA's vertical taps span
-inline std::vector<int> tables(int w, int h, int W, int H, int filter, int* rows_max) {
+// the host tables of (w, h) -> (W, H) with box starts x0 and y0: horizontal axis first, then
+// vertical, plus the most input rows one CTA's vertical taps span
+inline std::vector<int> tables(int w, int h, int W, int H, int filter, double x0, double y0,
+                               int* rows_max) {
   std::vector<int> t;
-  axis_table(w, W, filter, t);
-  axis_table(h, H, filter, t);
+  axis_table(w, W, filter, x0, t);
+  axis_table(h, H, filter, y0, t);
   const int* yb = t.data() + (size_t)W * (2 + taps_of(filter));
   const int* yn = yb + H;
   int m = 0;
@@ -121,7 +139,7 @@ inline std::vector<int> tables(int w, int h, int W, int H, int filter, int* rows
 
 // one plane of a launch: frame f reads in + f * in_frame and writes out + f * out_frame (pixels),
 // rows in_pitch and out_pitch pixels apart, and, with luma, the dense luma + f * W * H;
-// tab = table_for(w, h, W, H)
+// tab = table_for(w, h, W, H, ...)
 template <class Pix>
 struct Plane {
   const Pix* in;
@@ -235,10 +253,11 @@ __global__ void __launch_bounds__(kThreads) resample_kernel(const Planes<Pix> pl
   }
 }
 
-// the cached device tables of one shape and filter (uploaded on the context stream)
-inline int table_for(srcnn_ctx* ctx, int w, int h, int W, int H, int filter, const int** dev,
-                     int* rows_max) {
-  const srcnn_ctx::ResampleKey key{w, h, W, H, filter};
+// the cached device tables of one shape, filter and pair of chroma sitings (SRCNN_CHROMA_*; both
+// SRCNN_CHROMA_CENTER for RGBA8 and Y), uploaded on the context stream on first use
+inline int table_for(srcnn_ctx* ctx, int w, int h, int W, int H, int filter, int siting_in,
+                     int siting_out, const int** dev, int* rows_max) {
+  const srcnn_ctx::ResampleKey key{w, h, W, H, filter, siting_in, siting_out};
   for (const srcnn_ctx::ResampleTable& t : ctx->resample_tables)
     if (std::memcmp(&t.key, &key, sizeof(key)) == 0) {
       *dev = t.dev;
@@ -247,7 +266,8 @@ inline int table_for(srcnn_ctx* ctx, int w, int h, int W, int H, int filter, con
     }
   srcnn_ctx::ResampleTable t;
   t.key = key;
-  t.host = tables(w, h, W, H, filter, &t.rows_max);
+  t.host = tables(w, h, W, H, filter, box_start(w, W, siting_x(siting_in), siting_x(siting_out)),
+                  box_start(h, H, siting_y(siting_in), siting_y(siting_out)), &t.rows_max);
   void* p = nullptr;
   if (cudaMalloc(&p, t.host.size() * sizeof(int)) != cudaSuccess) {
     cudaGetLastError();
@@ -276,7 +296,9 @@ inline int launch_planes(srcnn_ctx* ctx, const Planes<Pix>& planes, int filter, 
   const dim3 grid((unsigned)((W + kTX - 1) / kTX), (unsigned)((H + kTY - 1) / kTY),
                   (unsigned)(frames * planes.n));
   const size_t smem = (size_t)rows_max * kTX * sizeof(Pix);
-  // at most (kTY - 1) + 2 * 3 + 1 rows for an enlargement: well under the default 48 KB
+  // at most (kTY - 1) + 2 * 3 + 1 rows for an enlargement: well under the default 48 KB.  A siting
+  // shifts a CTA's centres but not their spread, at most (kTY - 1) * scale <= kTY - 1 rows, and each
+  // output spans at most 2 * 3 + 1 taps (a conversion at ratio 1: 15 + 7 = 22 rows)
   if (filter == SRCNN_RESAMPLE_LANCZOS)
     resample_kernel<7, Pix><<<grid, kThreads, smem, ctx->stream>>>(planes);
   else

@@ -688,7 +688,8 @@ int srcnn_resample(srcnn_ctx* ctx, srcnn_mem rgba_in, int w, int h, srcnn_mem rg
   ctx->note_write(rgba_out);
   const int* tab;
   int rows_max;
-  SRCNN_TRY(resample::table_for(ctx, w, h, out_w, out_h, filter, &tab, &rows_max));
+  SRCNN_TRY(resample::table_for(ctx, w, h, out_w, out_h, filter, SRCNN_CHROMA_CENTER,
+                                SRCNN_CHROMA_CENTER, &tab, &rows_max));
   LaunchScope scope(ctx, SRCNN_K_RESAMPLE);
   SRCNN_TRY(resample::launch(ctx, pi, w, h, po, pl, out_w, out_h, filter, tab, rows_max));
   return check_launch("resample");
@@ -1261,7 +1262,8 @@ int srcnn_upscale_image_host(srcnn_ctx* ctx, const srcnn_net* net, const unsigne
     SRCNN_TRY(ensure_scratch(ctx, &st.s2, &st.s2_bytes, sizeof(float) * (size_t)d.w2 * d.h2 * net->n2));
   }
   Upscale u{w, h, out_w, out_h, filter, 1, d, nullptr, 0};
-  SRCNN_TRY(resample::table_for(ctx, w, h, out_w, out_h, filter, &u.tab, &u.rows_max));
+  SRCNN_TRY(resample::table_for(ctx, w, h, out_w, out_h, filter, SRCNN_CHROMA_CENTER,
+                                SRCNN_CHROMA_CENTER, &u.tab, &u.rows_max));
   fast::FusedNet fn;
   SRCNN_TRY(fused_net(ctx, net, &fn));
   u.small = (const uchar4*)st.small;
@@ -1420,7 +1422,8 @@ int frames_prepare(srcnn_ctx* ctx, const srcnn_net* net, srcnn_ctx::FramesStagin
     SRCNN_TRY(ensure_scratch(ctx, &st.s1, &st.s1_bytes, sizeof(float) * (size_t)d.w1 * d.h1 * net->n1));
     SRCNN_TRY(ensure_scratch(ctx, &st.s2, &st.s2_bytes, sizeof(float) * (size_t)d.w2 * d.h2 * net->n2));
   }
-  SRCNN_TRY(resample::table_for(ctx, w, h, out_w, out_h, filter, &u.tab, &u.rows_max));
+  SRCNN_TRY(resample::table_for(ctx, w, h, out_w, out_h, filter, SRCNN_CHROMA_CENTER,
+                                SRCNN_CHROMA_CENTER, &u.tab, &u.rows_max));
   SRCNN_TRY(fused_net(ctx, net, &fc->fn));
   u.rgba = (uchar4*)st.rgba;
   u.luma = (float*)st.luma;
@@ -1548,10 +1551,18 @@ int check_yuv420(const srcnn_net* net, int w, int h, int n_frames, int out_w, in
   return SRCNN_OK;
 }
 
+int check_sitings(int siting_in, int siting_out) {
+  for (int s : {siting_in, siting_out})
+    SRCNN_REQUIRE(s == SRCNN_CHROMA_CENTER || s == SRCNN_CHROMA_LEFT || s == SRCNN_CHROMA_TOPLEFT,
+                  "unknown chroma siting %d", s);
+  return SRCNN_OK;
+}
+
 // whole I420 frames of w x h back to back: the frames of srcnn_upscale_yuv420_frames_host
 srcnn_yuv420_layout i420_dense(int w, int h) {
   const size_t y = (size_t)w * h, c = y / 4;
-  return srcnn_yuv420_layout{SRCNN_YUV_I420, y + 2 * c, (size_t)w, (size_t)w / 2, y, y + c};
+  return srcnn_yuv420_layout{SRCNN_YUV_I420, y + 2 * c, (size_t)w, (size_t)w / 2, y, y + c,
+                             SRCNN_CHROMA_CENTER};
 }
 
 // the layout of n_frames frames of w x h (w, h even and > 0) holds them: *need = the bytes from
@@ -1628,9 +1639,19 @@ int yuv420_swap(srcnn_ctx* ctx, const Upscale& u, const Yuv420& y) {
 int srcnn_upscale_yuv420_frames_host(srcnn_ctx* ctx, const srcnn_net* net,
                                      const unsigned char* host_in, int w, int h, int n_frames,
                                      int out_w, int out_h, int filter, unsigned char* host_out) {
+  return srcnn_upscale_yuv420_frames_host_sited(ctx, net, host_in, w, h, n_frames, out_w, out_h,
+                                                filter, SRCNN_CHROMA_CENTER, SRCNN_CHROMA_CENTER,
+                                                host_out);
+}
+
+int srcnn_upscale_yuv420_frames_host_sited(srcnn_ctx* ctx, const srcnn_net* net,
+                                           const unsigned char* host_in, int w, int h, int n_frames,
+                                           int out_w, int out_h, int filter, int in_siting,
+                                           int out_siting, unsigned char* host_out) {
   SRCNN_REQUIRE(ctx && host_in && host_out, "null argument");
   SRCNN_ENTER(ctx);
   SRCNN_TRY(check_yuv420(net, w, h, n_frames, out_w, out_h, filter));
+  SRCNN_TRY(check_sitings(in_siting, out_siting));
   srcnn_ctx::FramesStaging& st = ctx->yuv;
   const Dims d = net_dims(net, out_w, out_h);
   Yuv420 y{nullptr, 0, nullptr, nullptr, i420_dense(w, h), i420_dense(out_w, out_h)};
@@ -1644,8 +1665,8 @@ int srcnn_upscale_yuv420_frames_host(srcnn_ctx* ctx, const srcnn_net* net,
                       65535 / 3};
   FramesCall fc;
   SRCNN_TRY(frames_prepare(ctx, net, st, w, h, n_frames, out_w, out_h, filter, fb, &fc));
-  SRCNN_TRY(resample::table_for(ctx, w / 2, h / 2, out_w / 2, out_h / 2, filter, &y.tab_c,
-                                &y.rows_max_c));
+  SRCNN_TRY(resample::table_for(ctx, w / 2, h / 2, out_w / 2, out_h / 2, filter, in_siting,
+                                out_siting, &y.tab_c, &y.rows_max_c));
   unsigned char* ring_in = (unsigned char*)st.small;
   unsigned char* ring_out = (unsigned char*)st.rgb;
   Upscale& u = fc.u;
@@ -1689,6 +1710,7 @@ int srcnn_upscale_yuv420_frames(srcnn_ctx* ctx, const srcnn_net* net, srcnn_mem 
                 format);
   SRCNN_REQUIRE(out_layout->format == format, "input format %d and output format %d differ", format,
                 out_layout->format);
+  SRCNN_TRY(check_sitings(in_layout->chroma_siting, out_layout->chroma_siting));
   size_t in_need, out_need;
   SRCNN_TRY(check_layout(*in_layout, w, h, n_frames, &in_need, "input"));
   SRCNN_TRY(check_layout(*out_layout, out_w, out_h, n_frames, &out_need, "output"));
@@ -1717,7 +1739,8 @@ int srcnn_upscale_yuv420_frames(srcnn_ctx* ctx, const srcnn_net* net, srcnn_mem 
   FramesCall fc;
   SRCNN_TRY(frames_prepare(ctx, net, ctx->yuv_dev, w, h, n_frames, out_w, out_h, filter, fb, &fc));
   Yuv420 y{nullptr, 0, pi, po, *in_layout, *out_layout};
-  SRCNN_TRY(resample::table_for(ctx, w / 2, h / 2, out_w / 2, out_h / 2, filter, &y.tab_c,
+  SRCNN_TRY(resample::table_for(ctx, w / 2, h / 2, out_w / 2, out_h / 2, filter,
+                                in_layout->chroma_siting, out_layout->chroma_siting, &y.tab_c,
                                 &y.rows_max_c));
   // groups of frames (one frame without a fused kernel, for the reason forward_three_launch
   // gives): enlargement + luma, Q1 mean, forward, Y write

@@ -64,10 +64,13 @@ class ConfigBasedDataPipeline : public DataPipeline {
                       size_t out_w, size_t out_h, int filter, unsigned char* out_rgb);
   /** upscale_frames for n_frames planar Y'CbCr 4:2:0 (I420) frames of w x h, back to back in
    * `in_yuv`; `out_yuv` receives n_frames I420 frames of out_w x out_h: Y enlarged and its
-   * interior replaced by the network's luma, Cb and Cr enlarged (srcnn_upscale_yuv420_frames_host) */
+   * interior replaced by the network's luma, Cb and Cr enlarged from chroma sited at in_siting to
+   * chroma sited at out_siting (SRCNN_CHROMA_*; srcnn_upscale_yuv420_frames_host_sited) */
   void upscale_yuv420_frames(LayerAllocationPool&, LayerAllocationPool&, LayerAllocationPool&,
                              const unsigned char* in_yuv, size_t w, size_t h, size_t n_frames,
-                             size_t out_w, size_t out_h, int filter, unsigned char* out_yuv);
+                             size_t out_w, size_t out_h, int filter, unsigned char* out_yuv,
+                             int in_siting = SRCNN_CHROMA_CENTER,
+                             int out_siting = SRCNN_CHROMA_CENTER);
   /** upscale_frames plus the quality of every result against its reference (n_frames frames of
    * out_w x out_h RGBA8 in `ref_rgba`): `metrics` receives 4 doubles a frame, {mse, ssim} of the
    * network's result and of the plain enlargement, over the region `border` pixels in from each

@@ -97,7 +97,11 @@ static std::runtime_error y4m_error(const std::string& path, const std::string& 
   return std::runtime_error("Y4M '" + path + "': " + what);
 }
 
-Y4mReader::Y4mReader(const char* path) : _path(path), _f(path, std::ios::binary) {
+// the colourspace tag (after 'C') and the XYSCSS= value of each SRCNN_CHROMA_* siting
+static const char* const kY4mSiting[3] = {"420jpeg", "420mpeg2", "420paldv"};
+static const char* const kY4mXyscss[3] = {"420JPEG", "420MPEG2", "420PALDV"};
+
+Y4mReader::Y4mReader(const char* path, bool any_siting) : _path(path), _f(path, std::ios::binary) {
   if (!_f.is_open()) throw y4m_error(_path, "could not open");
   std::string line;
   if (!std::getline(_f, line) || line.compare(0, 10, "YUV4MPEG2 ") != 0)
@@ -120,10 +124,13 @@ Y4mReader::Y4mReader(const char* path) : _path(path), _f(path, std::ios::binary)
         break;
       }
       case 'C':
-        if (v == "420mpeg2" || v == "420paldv")
-          throw y4m_error(_path, "chroma siting '" + t + "' is left-sited; only centre-sited 4:2:0 "
-                                 "(C420jpeg, C420) is supported");
-        if (v != "420jpeg" && v != "420")
+        if (v == "420mpeg2" || v == "420paldv") {
+          if (!any_siting)
+            throw y4m_error(_path, "chroma siting '" + t + "' is left-sited; only centre-sited 4:2:0 "
+                                   "(C420jpeg, C420) is supported; --chroma-siting keep enlarges it "
+                                   "at its own siting");
+          _header.chroma_siting = v == "420mpeg2" ? SRCNN_CHROMA_LEFT : SRCNN_CHROMA_TOPLEFT;
+        } else if (v != "420jpeg" && v != "420")
           throw y4m_error(_path, "colourspace '" + t + "' is not supported; only 8-bit 4:2:0 "
                                  "(C420jpeg, C420) is");
         break;
@@ -192,16 +199,24 @@ size_t Y4mReader::read_frames(size_t max, std::vector<unsigned char>& out) {
   return n;
 }
 
-void write_y4m_header(std::ostream& f, const Y4mHeader& in, int out_w, int out_h) {
+void write_y4m_header(std::ostream& f, const Y4mHeader& in, int out_w, int out_h, int out_siting) {
+  const bool resite = out_siting != in.chroma_siting;
+  bool has_c = false;
   f << "YUV4MPEG2";
   for (const std::string& t : in.tags) {
     if (t[0] == 'W')
       f << " W" << out_w;
     else if (t[0] == 'H')
       f << " H" << out_h;
+    else if (resite && t[0] == 'C')
+      f << " C" << kY4mSiting[out_siting];
+    else if (resite && t.compare(0, 7, "XYSCSS=") == 0)
+      f << " XYSCSS=" << kY4mXyscss[out_siting];
     else
       f << " " << t;
+    has_c = has_c || t[0] == 'C';
   }
+  if (resite && !has_c) f << " C" << kY4mSiting[out_siting];
   f << "\n";
 }
 

@@ -62,10 +62,12 @@ int write_image(const char* path, ImageData&);
 void write_image(const char* path, float* luma, size_t w, size_t h);
 
 /** The header of a YUV4MPEG2 (Y4M) stream: "YUV4MPEG2" and space-separated tags.  Only 8-bit
- * progressive 4:2:0 with centre-sited chroma (C420jpeg, the format's default, or C420) of even
- * size is accepted: the device layer resamples chroma by pixel centres. */
+ * progressive 4:2:0 of even size is accepted.  Its chroma siting is read as ffmpeg's reader maps
+ * the colourspace tag: C420jpeg (the format's default) and C420 centre-sited, C420mpeg2 left-sited,
+ * C420paldv top-left-sited. */
 struct Y4mHeader {
   int w = 0, h = 0;
+  int chroma_siting = SRCNN_CHROMA_CENTER;   // SRCNN_CHROMA_*
   std::vector<std::string> tags;   // every tag as read, in order ("W960", "F30000:1001", ...)
   size_t frame_bytes() const { return (size_t)w * h * 3 / 2; }
 };
@@ -73,7 +75,8 @@ struct Y4mHeader {
  * message: the constructor checks the header, check_frames() every frame marker and frame size. */
 class Y4mReader {
  public:
-  explicit Y4mReader(const char* path);
+  /** any_siting: accept chroma that is not centre-sited (refused otherwise) */
+  explicit Y4mReader(const char* path, bool any_siting = false);
   const Y4mHeader& header() const { return _header; }
   /** the number of frames; every frame starts with "FRAME[ params]\n" and is complete.  Leaves
    * the reader at the first frame. */
@@ -89,8 +92,10 @@ class Y4mReader {
   size_t _next = 0;
   Y4mHeader _header;
 };
-/** `in`'s header with W and H set to out_w x out_h and every other tag copied */
-void write_y4m_header(std::ostream&, const Y4mHeader& in, int out_w, int out_h);
+/** `in`'s header with W and H set to out_w x out_h and every other tag copied; for an out_siting
+ * (SRCNN_CHROMA_*) other than in's, the C tag names it (appended when `in` has none) and an
+ * XYSCSS= tag matches it */
+void write_y4m_header(std::ostream&, const Y4mHeader& in, int out_w, int out_h, int out_siting);
 /** n frames of `frame_bytes` bytes, each behind a bare "FRAME\n" */
 void write_y4m_frames(std::ostream&, const unsigned char* frames, size_t n, size_t frame_bytes);
 }  // namespace utils

@@ -1,5 +1,5 @@
 // `cnn [train | eval] [dry] [profile] --config CFG --in PATH [--out PATH] [--epochs N]
-//      [--scale N [--resample lanczos|bicubic]]`
+//      [--scale N [--resample lanczos|bicubic]] [--chroma-siting keep|420jpeg|420mpeg2|420paldv]`
 // Same grammar, flow and console output as the reference CLI (src/Main_cl.cpp:40-318):
 // forward mode = one image through the three layers, luma swapped back into the image (or every
 // image of a directory, see below);
@@ -13,9 +13,11 @@
 // srcnn_upscale_frames_host together, at most kDirBatch at a time; other files are skipped.
 // -i IN.y4m (forward mode) enlarges every frame of a YUV4MPEG2 video, 8-bit progressive 4:2:0 with
 // centre-sited chroma (C420jpeg / C420), into OUT.y4m (-o OUT.y4m): the header's W and H times
-// --scale, its other tags copied, kDirBatch frames per srcnn_upscale_yuv420_frames_host call; the
-// network replaces the luma, the chroma is only enlarged.  The header and every frame marker are
-// checked before any device work.
+// --scale, its other tags copied, kDirBatch frames per srcnn_upscale_yuv420_frames_host_sited call;
+// the network replaces the luma, the chroma is only enlarged.  The header and every frame marker are
+// checked before any device work.  Left- and top-left-sited chroma (C420mpeg2, C420paldv) is refused
+// unless --chroma-siting names the output's siting: `keep` (the input's, every tag copied) or a
+// colourspace tag, to which the chroma is converted (the C tag, and an XYSCSS= tag, then name it).
 // eval -i SAMPLES_DIR measures the network on the training mode's sample pairs: every `_small`
 // image, enlarged N times (--scale, default 1: the reference's `_small` images are already
 // enlarged), against its `_large` image, which must be exactly N times its size.  One line a pair
@@ -176,7 +178,8 @@ static void execute_directory(ConfigBasedDataPipeline& pipeline, GpuAllocationPo
 // every frame of a Y4M video through the I420 frames entry, `scale` times enlarged, kDirBatch
 // frames at a time; the result goes to out_path unless it is null (dry run)
 static void execute_y4m(ConfigBasedDataPipeline& pipeline, GpuAllocationPool& gpu_alloc,
-                        Y4mReader& video, const char* out_path, size_t scale, int filter) {
+                        Y4mReader& video, const char* out_path, size_t scale, int filter,
+                        int out_siting) {
   const Y4mHeader& hd = video.header();
   const size_t w = (size_t)hd.w, h = (size_t)hd.h, out_w = scale * w, out_h = scale * h;
   const size_t out_bytes = out_w * out_h * 3 / 2;
@@ -185,14 +188,15 @@ static void execute_y4m(ConfigBasedDataPipeline& pipeline, GpuAllocationPool& gp
     std::cout << "Saving result video to: '" << out_path << "'" << std::endl;
     out.open(out_path, std::ios::binary);
     if (!out.is_open()) throw std::runtime_error(std::string("Could not write video: ") + out_path);
-    write_y4m_header(out, hd, (int)out_w, (int)out_h);
+    write_y4m_header(out, hd, (int)out_w, (int)out_h, out_siting);
   }
   std::vector<unsigned char> in, result;
   size_t n;
   while ((n = video.read_frames(kDirBatch, in)) > 0) {
     result.resize(n * out_bytes);
     pipeline.upscale_yuv420_frames(gpu_alloc.layer_1, gpu_alloc.layer_2, gpu_alloc.layer_3,
-                                   in.data(), w, h, n, out_w, out_h, filter, result.data());
+                                   in.data(), w, h, n, out_w, out_h, filter, result.data(),
+                                   hd.chroma_siting, out_siting);
     if (out_path) write_y4m_frames(out, result.data(), n, out_bytes);
     in.clear();
   }
@@ -349,6 +353,7 @@ int main(int argc, char** argv) {
   argparse.add_argument("-e", "--epochs").help("Number of epochs during training");
   argparse.add_argument("-s", "--scale").help("Forward mode: enlarge the image N times first (default 1)");
   argparse.add_argument("-r", "--resample").help("Enlargement filter: lanczos (default) or bicubic");
+  argparse.add_argument("--chroma-siting").help("A .y4m input: the output's chroma siting, keep (the input's), 420jpeg, 420mpeg2 or 420paldv; accepts every siting the input may have");
   try {
     if (!argparse.parse((size_t)argc, argv)) return EXIT_SUCCESS;
   } catch (const std::exception& e) {
@@ -395,6 +400,23 @@ int main(int argc, char** argv) {
     std::cout << "A .y4m input applies to the forward mode only" << std::endl;
     return EXIT_FAILURE;
   }
+  // --chroma-siting: -1 = keep, else SRCNN_CHROMA_*
+  const char* siting_name = argparse.value("chroma-siting");
+  int out_siting = -1;
+  if (siting_name) {
+    const char* names[] = {"420jpeg", "420mpeg2", "420paldv"};
+    for (int s = 0; s < 3; s++)
+      if (std::strcmp(siting_name, names[s]) == 0) out_siting = s;
+    if (out_siting < 0 && std::strcmp(siting_name, "keep") != 0) {
+      std::cout << "--chroma-siting must be keep, 420jpeg, 420mpeg2 or 420paldv, got '"
+                << siting_name << "'" << std::endl;
+      return EXIT_FAILURE;
+    }
+    if (!in_y4m || train || eval) {
+      std::cout << "--chroma-siting applies to a .y4m input in the forward mode only" << std::endl;
+      return EXIT_FAILURE;
+    }
+  }
   const bool in_dir = !train && !eval && !in_y4m && is_directory(in_path);
   if ((in_dir || eval) && out_path && !is_directory(out_path)) {
     std::cout << "Output directory '" << out_path << "' does not exist or is not a directory"
@@ -430,7 +452,7 @@ int main(int argc, char** argv) {
     // a video is checked whole before the context exists
     std::unique_ptr<Y4mReader> video;
     if (in_y4m) {
-      video.reset(new Y4mReader(in_path));
+      video.reset(new Y4mReader(in_path, siting_name != nullptr));
       const size_t n_frames = video->check_frames();
       std::cout << "Video: " << video->header().w << "x" << video->header().h << ", " << n_frames
                 << " frames" << std::endl;
@@ -451,7 +473,8 @@ int main(int argc, char** argv) {
       return EXIT_SUCCESS;
     }
     if (video) {
-      execute_y4m(data_pipeline, gpu_alloc, *video, out_path, scale, filter);
+      execute_y4m(data_pipeline, gpu_alloc, *video, out_path, scale, filter,
+                  out_siting < 0 ? video->header().chroma_siting : out_siting);
       context.block();
       return EXIT_SUCCESS;
     }

@@ -313,9 +313,9 @@ int srcnn_upscale_frames_host(srcnn_ctx* ctx, const srcnn_net* net, const unsign
  *     clamp(luma * 255, 0, 255) truncated -- the byte swap_luma writes for a pixel with zero
  *     chroma -- and the border of (f1+f2+f3-3)/2 rows and columns keeps the enlarged Y, as
  *     swap_luma leaves it.
- *   - Cb and Cr are each enlarged (w/2, h/2) -> (out_w/2, out_h/2) with the same filter.  Pillow
- *     maps pixel centres onto pixel centres, which is right for centre-sited ("jpeg", Y4M's
- *     default 420jpeg) chroma; left-sited chroma (MPEG-2 and later codecs' default) would shift.
+ *   - Cb and Cr are each enlarged (w/2, h/2) -> (out_w/2, out_h/2) with the same filter, for
+ *     centre-sited chroma (SRCNN_CHROMA_CENTER; srcnn_upscale_yuv420_frames_host_sited takes
+ *     others): Pillow's enlargement, which maps pixel centres onto pixel centres.
  *   - The network sees the Y plane as stored: there is no range conversion, full or limited.
  * A frame's bytes do not depend on the other frames of the call or on the group size.
  * Synchronous; pageable buffers work, pinned ones give the overlap.  Waits for
@@ -332,17 +332,50 @@ int srcnn_upscale_frames_host(srcnn_ctx* ctx, const srcnn_net* net, const unsign
  * Launches per call: n_groups * (5 + F) with a fused kernel, n_frames * (4 + L + 1) without (F, L
  * as for srcnn_upscale_frames_host), plus 1 when the network's packed operand image has to be
  * rebuilt.  Everything srcnn_upscale_image_host rejects, an odd w, h, out_w or out_h, n_frames <= 0
- * and null pointers: SRCNN_EINVAL before any host buffer is read or written. */
+ * and null pointers: SRCNN_EINVAL before any host buffer is read or written.
+ * It is srcnn_upscale_yuv420_frames_host_sited with both sitings SRCNN_CHROMA_CENTER. */
 int srcnn_upscale_yuv420_frames_host(srcnn_ctx* ctx, const srcnn_net* net,
                                      const unsigned char* host_in, int w, int h, int n_frames,
                                      int out_w, int out_h, int filter, unsigned char* host_out);
+
+/* Where a 4:2:0 chroma sample sits inside its 2x2 luma cell, per axis in chroma samples: s = 0.5
+ * is centred, s = 0.25 co-sited with the even luma column or row.
+ *
+ *   siting                 s_x   s_y   Y4M tag (ffmpeg)   H.273 chroma_sample_loc_type
+ *   SRCNN_CHROMA_CENTER    0.5   0.5   C420jpeg, C420     1 (JPEG)
+ *   SRCNN_CHROMA_LEFT      0.25  0.5   C420mpeg2          0 (H.264 / HEVC without a signal)
+ *   SRCNN_CHROMA_TOPLEFT   0.25  0.25  C420paldv          2 (UHD / BT.2020, AV1 "colocated")
+ *
+ * A chroma axis from n_in samples sited at s_in to n_out samples sited at s_out is Pillow's
+ * enlargement of a box that starts at in0, computed in double in this order:
+ *   scale = (double)n_in / n_out;  in0 = (s_out - 0.5) * scale + (0.5 - s_in);
+ *   output i takes the taps around center = in0 + (i + 0.5) * scale
+ * (then the taps, weights, normalisation and 22-bit rounding of srcnn_resample).  Centre to centre
+ * gives in0 = 0.0 exactly, Pillow's plain enlargement.  An axis is copied only when n_in == n_out
+ * and in0 == 0.0; a siting conversion on an axis whose size does not change is resampled, as
+ * Pillow resamples a box with a non-zero start.  Luma is never affected. */
+enum { SRCNN_CHROMA_CENTER = 0, SRCNN_CHROMA_LEFT = 1, SRCNN_CHROMA_TOPLEFT = 2 };
+
+/* srcnn_upscale_yuv420_frames_host for chroma sited at in_siting in host_in, written sited at
+ * out_siting in host_out (SRCNN_CHROMA_*; they may differ, which converts the siting): Cb and Cr
+ * are enlarged as the definition above gives; Y, the launches, copies and groups are those of
+ * srcnn_upscale_yuv420_frames_host.  A siting pair's chroma table is built and uploaded on the
+ * pair's first call.  Everything srcnn_upscale_yuv420_frames_host rejects, and a siting outside
+ * SRCNN_CHROMA_*: SRCNN_EINVAL before any host buffer is read or written. */
+int srcnn_upscale_yuv420_frames_host_sited(srcnn_ctx* ctx, const srcnn_net* net,
+                                           const unsigned char* host_in, int w, int h, int n_frames,
+                                           int out_w, int out_h, int filter, int in_siting,
+                                           int out_siting, unsigned char* host_out);
 
 /* Where the planes of 4:2:0 frames lie in a device buffer.  A frame's Y plane starts at the frame's
  * first byte; every offset, pitch and stride is in bytes.  SRCNN_YUV_I420: Y, Cb and Cr planes
  * (`yuv420p`); SRCNN_YUV_NV12: Y, then one plane of interleaved Cb, Cr pairs, Cb first (what
  * hardware video decoders hand out and encoders take).  The dense I420 layout of
- * srcnn_upscale_yuv420_frames_host is {I420, w*h*3/2, w, w/2, w*h, w*h*5/4}, the dense NV12 one
- * {NV12, w*h*3/2, w, w, w*h, 0}. */
+ * srcnn_upscale_yuv420_frames_host is {I420, w*h*3/2, w, w/2, w*h, w*h*5/4, 0}, the dense NV12 one
+ * {NV12, w*h*3/2, w, w, w*h, 0, 0}.
+ * chroma_siting was appended as the last field so that the fields before it keep their offsets
+ * and a zero-initialised layout keeps its meaning (centre-sited chroma); a caller that declares
+ * the struct itself (a language binding) adds the field too. */
 enum { SRCNN_YUV_I420 = 0, SRCNN_YUV_NV12 = 1 };
 typedef struct srcnn_yuv420_layout {
   int format;           /* SRCNN_YUV_I420 or SRCNN_YUV_NV12 */
@@ -351,20 +384,22 @@ typedef struct srcnn_yuv420_layout {
   size_t c_pitch;       /* from one chroma row to the next, >= width/2 (I420) or width (NV12) */
   size_t cb_offset;     /* of the Cb plane (NV12: the CbCr plane) from the frame start */
   size_t cr_offset;     /* I420: of the Cr plane; NV12: must be 0 */
+  int chroma_siting;    /* SRCNN_CHROMA_*: where the frames' chroma samples sit; 0 = centre */
 } srcnn_yuv420_layout;
 
 /* srcnn_upscale_yuv420_frames_host on frames that are already in device memory, in I420 or NV12
  * with pitched rows: `in` holds n_frames frames of w x h in in_layout, `out` receives n_frames
  * frames of out_w x out_h in out_layout, of the same format.  The Y, Cb and Cr bytes of a frame are
- * those srcnn_upscale_yuv420_frames_host writes for it (NV12: the same Cb and Cr bytes,
- * interleaved).  Bytes of `out` outside the planes' rows (pitch padding, gaps between planes or
+ * those srcnn_upscale_yuv420_frames_host_sited writes for it with in_layout's chroma_siting as the
+ * input's and out_layout's as the output's (NV12: the same Cb and Cr bytes, interleaved).  Bytes of `out` outside the planes' rows (pitch padding, gaps between planes or
  * frames) are never written; bytes of `in` outside them never affect the result.
  * Stream-ordered, like srcnn_forward_fused: the work is enqueued on the context stream and the
  * call returns, without a copy or a host synchronisation (the caller orders its own work on that
  * stream: create the context with srcnn_ctx_create_on_stream on a non-default stream, e.g. a
  * torch.cuda.Stream(), and fill `in` and read `out` on it).  Once a call with the same sizes,
- * layouts' formats and network has run, a call allocates nothing, so it can be captured into a
- * CUDA graph on the context stream.  Such a graph reads the entry's scratch, which grows on
+ * layouts' formats, pair of chroma sitings and network has run, a call allocates nothing, so it can
+ * be captured into a CUDA graph on the context stream.  (A new siting pair is a new chroma table,
+ * allocated and uploaded on its first call: capture only a call whose pair has run before.)  Such a graph reads the entry's scratch, which grows on
  * demand: a later call on the context that needs more of it (larger frames, or more frames a
  * group) reallocates it, and the graph must then be captured again.  It waits for
  * srcnn_infer_rows_host_async calls in flight first; in profile mode every launch blocks.  Staging
@@ -382,7 +417,7 @@ typedef struct srcnn_yuv420_layout {
  * as for srcnn_upscale_frames_host).
  * Errors, all before any launch (the output and the launch count stay untouched):
  *   SRCNN_EINVAL: everything srcnn_upscale_yuv420_frames_host rejects; a null layout; an unknown
- *     format, or formats that differ; a pitch below its row's bytes; a pitch, offset or stride of
+ *     format, or formats that differ; a chroma_siting outside SRCNN_CHROMA_* in either layout; a pitch below its row's bytes; a pitch, offset or stride of
  *     2^31 bytes or more; planes of one frame whose byte ranges intersect; with n_frames > 1, a
  *     frame_stride below the frame's extent (the end of its last plane's last row); NV12 with
  *     cr_offset != 0, an odd c_pitch, or a CbCr plane at an odd address in any frame; input and

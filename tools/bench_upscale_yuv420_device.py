@@ -7,6 +7,9 @@ entry srcnn_upscale_yuv420_frames_host on the same content, all in one process o
                   CbCr plane after a 16-row-aligned Y plane (544 and 1088 rows)
   host entry      Net.upscale_yuv420_frames_host on pinned I420 buffers (upload, device work,
                   download; synchronous)
+  ... left, ... topleft   i420 dense, nv12 pitched and the host entry with left- and top-left-sited
+                  chroma kept as it is (chroma_siting of both layouts, of both host arguments):
+                  the same launches and kernel with other chroma taps, so the same time is expected
 
 for 9-1-5 128/64 and 64/32, Lanczos and bicubic (the frames of tools/bench_upscale_yuv420.py).
 The device entry is timed with CUDA events on the context stream around `--reps` calls after a
@@ -17,7 +20,7 @@ give the RGBA8 resampling kernel alone (ctx.resample, 2048^2 -> 4096^2, RGBA + l
 events), as tools/bench_upscale.py measures it, because the plane resampler took row pitches.
 
     python tools/bench_upscale_yuv420_device.py [--reps 20] [--seconds 2.0] \
-        > profiles/upscale_yuv420_device_b200.txt
+        > profiles/chroma_siting_b200.txt
 """
 import argparse
 import os
@@ -94,12 +97,19 @@ def main():
         yuv_out = pkg.PinnedBuffer((N, W * H * 3 // 2), np.uint8)
         frames(rng, yuv_in.array, np.empty((N, h, w, 4), np.uint8))
         Lay = pkg.yuv420_layout
+        def nv12_pitched(s):
+            return ("nv12", Lay("nv12", w, h, 1024, 1024, 544 * 1024, chroma_siting=s),
+                    Lay("nv12", W, H, 2048, 2048, 1088 * 2048, chroma_siting=s))
+
         layouts = {
             "i420 dense": ("i420", Lay("i420", w, h), Lay("i420", W, H)),
             "nv12 dense": ("nv12", Lay("nv12", w, h), Lay("nv12", W, H)),
-            "nv12 pitched": ("nv12", Lay("nv12", w, h, 1024, 1024, 544 * 1024),
-                             Lay("nv12", W, H, 2048, 2048, 1088 * 2048)),
+            "nv12 pitched": nv12_pitched("center"),
         }
+        for s in ("left", "topleft"):
+            layouts["i420 dense " + s] = ("i420", Lay("i420", w, h, chroma_siting=s),
+                                          Lay("i420", W, H, chroma_siting=s))
+            layouts["nv12 pitched " + s] = nv12_pitched(s)
         mems = {}
         for label, (fmt, li, lo) in layouts.items():
             src = yuv_in.array.reshape(-1) if fmt == "i420" else nv12_of(yuv_in.array, w, h, li)
@@ -111,8 +121,12 @@ def main():
             net = pkg.Net(ctx, *cfg, make_params(rng, *cfg))
             print("\n== %s ==" % name)
             for f in ("lanczos", "bicubic"):
-                host = net.upscale_yuv420_frames_host(yuv_in.array, w, h, W, H, f, out=yuv_out.array)
-                host = host.copy()
+                host = {}
+                for s in ("center", "left", "topleft"):
+                    host[s] = net.upscale_yuv420_frames_host(yuv_in.array, w, h, W, H, f,
+                                                             out=yuv_out.array,
+                                                             chroma_siting=s).copy()
+                sitings = {v: k for k, v in pkg.CHROMA_SITINGS.items()}
                 for label, (fmt, li, lo) in layouts.items():
                     m_in, m_out = mems[label]
 
@@ -124,12 +138,17 @@ def main():
                     same = ""
                     if fmt == "i420":   # the bytes are the host entry's
                         got = ctx.read(m_out, (N, W * H * 3 // 2), np.uint8)
-                        same = ", bytes == host entry: %s" % np.array_equal(got, host)
+                        same = ", bytes == host entry: %s" % np.array_equal(
+                            got, host[sitings[li.chroma_siting]])
                     print("%s, device entry %s: %.4f ms/frame, enqueue of one call %.3f ms%s"
                           % (f, label, ms / N, enq, same))
                 ms, n = timed(lambda: net.upscale_yuv420_frames_host(yuv_in.array, w, h, W, H, f,
                                                                      out=yuv_out.array), a.seconds)
                 print("%s, host entry (pinned): %.4f ms/frame (%d calls of %d frames)"
+                      % (f, ms / N, n, N))
+                ms, n = timed(lambda: net.upscale_yuv420_frames_host(
+                    yuv_in.array, w, h, W, H, f, out=yuv_out.array, chroma_siting="left"), a.seconds)
+                print("%s, host entry left (pinned): %.4f ms/frame (%d calls of %d frames)"
                       % (f, ms / N, n, N))
         for m_in, m_out in mems.values():
             ctx.release(m_in)
