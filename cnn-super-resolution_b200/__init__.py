@@ -74,7 +74,7 @@ CHROMA_SITINGS = {"center": 0, "left": 1, "topleft": 2}
 class CYuv420Layout(C.Structure):
     """struct srcnn_yuv420_layout of include/srcnn_b200.h"""
     _fields_ = [("format", _i), ("frame_stride", _sz), ("y_pitch", _sz), ("c_pitch", _sz),
-                ("cb_offset", _sz), ("cr_offset", _sz), ("chroma_siting", _i)]
+                ("cb_offset", _sz), ("cr_offset", _sz), ("chroma_siting", _i), ("bit_depth", _i)]
 
 
 def _siting_id(name):
@@ -84,23 +84,27 @@ def _siting_id(name):
 
 
 def yuv420_layout(fmt, w, h, y_pitch=None, c_pitch=None, cb_offset=None, frame_stride=None,
-                  chroma_siting="center"):
+                  chroma_siting="center", bit_depth=8):
     """Where the planes of w x h 4:2:0 frames ("i420" or "nv12") lie in a buffer, in bytes, and
-    where their chroma samples sit (CHROMA_SITINGS).  The defaults are the dense layout; otherwise
-    the chroma follows Y at cb_offset (default: right after the Y plane's h rows), an I420 Cr plane
-    follows Cb right after its h/2 rows, and a frame spans frame_stride bytes (default: to the end
-    of its last plane's last pitched row)."""
+    where their chroma samples sit (CHROMA_SITINGS).  bit_depth 10 makes them I010 ("i420") or
+    P010 ("nv12"), a 16-bit word a sample.  The defaults are the dense layout; otherwise the chroma
+    follows Y at cb_offset (default: right after the Y plane's h rows), an I420 Cr plane follows Cb
+    right after its h/2 rows, and a frame spans frame_stride bytes (default: to the end of its last
+    plane's last pitched row)."""
     if fmt not in YUV420_FORMATS:
         raise ValueError("unknown 4:2:0 format %r (have %s)" % (fmt, sorted(YUV420_FORMATS)))
+    if bit_depth not in (8, 10):
+        raise ValueError("bit depth %r is not 8 or 10" % (bit_depth,))
     siting = _siting_id(chroma_siting)
     nv12 = fmt == "nv12"
-    y_pitch = w if y_pitch is None else y_pitch
-    c_pitch = (w if nv12 else w // 2) if c_pitch is None else c_pitch
+    b = 2 if bit_depth == 10 else 1   # bytes a sample
+    y_pitch = w * b if y_pitch is None else y_pitch
+    c_pitch = (w if nv12 else w // 2) * b if c_pitch is None else c_pitch
     cb_offset = h * y_pitch if cb_offset is None else cb_offset
     cr_offset = 0 if nv12 else cb_offset + (h // 2) * c_pitch
     end = (cb_offset if nv12 else cr_offset) + (h // 2) * c_pitch
     return CYuv420Layout(YUV420_FORMATS[fmt], end if frame_stride is None else frame_stride,
-                         y_pitch, c_pitch, cb_offset, cr_offset, siting)
+                         y_pitch, c_pitch, cb_offset, cr_offset, siting, bit_depth)
 
 
 _SIGS = {
@@ -144,6 +148,8 @@ _SIGS = {
                                               _vp]),
     "srcnn_upscale_yuv420_frames_host_sited": (_i, [_vp, C.POINTER(CNet), _vp, _i, _i, _i, _i,
                                                     _i, _i, _i, _i, _vp]),
+    "srcnn_upscale_yuv420p10_frames_host": (_i, [_vp, C.POINTER(CNet), _vp, _i, _i, _i, _i, _i,
+                                                 _i, _i, _i, _vp]),
     "srcnn_upscale_yuv420_frames": (_i, [_vp, C.POINTER(CNet), _u64, C.POINTER(CYuv420Layout), _i,
                                          _i, _i, _u64, C.POINTER(CYuv420Layout), _i, _i, _i]),
     "srcnn_image_quality": (_i, [_vp, _u64, _i, _u64, _i, _i, _i, _i, _u64]),
@@ -553,16 +559,39 @@ class Net:
                 _filter_id(resample), s_in, s_out, _np_ptr(out)))
         return out
 
+    def upscale_yuv420p10_frames_host(self, frames, w, h, out_w, out_h, resample="lanczos",
+                                      out=None, chroma_siting="center", out_chroma_siting=None):
+        """upscale_yuv420_frames_host for 10-bit frames: uint16 [n][w*h*3//2] I010 (the samples of
+        I420 frames, each a value in its low 10 bits; the other bits are ignored) -> uint16
+        [n][out_w*out_h*3//2] I010 with the upper bits 0: every plane enlarged with Pillow's 16-bit
+        filter ("I;16") and capped at 1023, and the interior of Y replaced by the network's luma
+        (it reads v / 1023 and writes clamp(out * 1023) truncated).  `out` may be a preallocated
+        (pinned) array."""
+        s_in = _siting_id(chroma_siting)
+        s_out = s_in if out_chroma_siting is None else _siting_id(out_chroma_siting)
+        n = frames.shape[0]
+        assert frames.dtype == np.uint16 and frames.ndim == 2 and frames.shape[1] == w * h * 3 // 2
+        frames = np.ascontiguousarray(frames)
+        if out is None:
+            out = np.empty((n, out_w * out_h * 3 // 2), np.uint16)
+        assert out.dtype == np.uint16 and out.shape == (n, out_w * out_h * 3 // 2)
+        assert out.flags.c_contiguous
+        _check(self.ctx.L.srcnn_upscale_yuv420p10_frames_host(
+            self.ctx.h, C.byref(self.c), _np_ptr(frames), w, h, n, out_w, out_h,
+            _filter_id(resample), s_in, s_out, _np_ptr(out)))
+        return out
+
     def upscale_yuv420_frames(self, in_mem, w, h, n_frames, out_mem, out_w, out_h,
-                              resample="lanczos", fmt="i420", in_layout=None, out_layout=None):
+                              resample="lanczos", fmt="i420", in_layout=None, out_layout=None,
+                              bit_depth=8):
         """upscale_yuv420_frames_host on device memory handles (Context.alloc, or Context.wrap of
         e.g. a torch CUDA tensor's data_ptr()): n_frames frames of w x h in in_mem -> out_w x out_h
         in out_mem, both in `fmt` ("i420" or "nv12") and laid out as in_layout / out_layout
-        (yuv420_layout, which also carries the chroma siting; default: dense, centre-sited).
-        Enqueued on the context stream; returns at once, without a
-        copy or a host synchronisation."""
-        li = yuv420_layout(fmt, w, h) if in_layout is None else in_layout
-        lo = yuv420_layout(fmt, out_w, out_h) if out_layout is None else out_layout
+        (yuv420_layout, which also carries the chroma siting and the bit depth; default: dense,
+        centre-sited, `bit_depth` bits: 10 is I010 or P010).  Enqueued on the context stream;
+        returns at once, without a copy or a host synchronisation."""
+        li = yuv420_layout(fmt, w, h, bit_depth=bit_depth) if in_layout is None else in_layout
+        lo = yuv420_layout(fmt, out_w, out_h, bit_depth=bit_depth) if out_layout is None else out_layout
         _check(self.ctx.L.srcnn_upscale_yuv420_frames(self.ctx.h, C.byref(self.c), in_mem,
                                                       C.byref(li), w, h, n_frames, out_mem,
                                                       C.byref(lo), out_w, out_h,

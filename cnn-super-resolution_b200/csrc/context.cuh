@@ -162,10 +162,10 @@ struct srcnn_ctx {
   bool lanes_busy = false;
 
   cudaEvent_t lane_ev = nullptr;
-  // srcnn_resample weight tables, one per (w, h, W, H, filter, input and output chroma siting);
-  // the host copy stays alive because the upload that reads it is asynchronous
+  // srcnn_resample weight tables, one per (w, h, W, H, filter, input and output chroma siting,
+  // sample bit depth); the host copy stays alive because the upload that reads it is asynchronous
   struct ResampleKey {
-    int w, h, W, H, filter, siting_in, siting_out;
+    int w, h, W, H, filter, siting_in, siting_out, bit_depth;
   };
   struct ResampleTable {
     ResampleKey key;

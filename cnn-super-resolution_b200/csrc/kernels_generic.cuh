@@ -506,6 +506,9 @@ __global__ void swap_luma_kernel(const uchar4* __restrict__ rgba, const float* _
 // covers the luma_w x luma_h interior, written (gt_w - luma_w) / 2 pixels in from the left and top
 // edges of the gt_w-wide plane, whose rows are `pitch` bytes apart; the border keeps the enlarged
 // Y.  Frame blockIdx.z: target + blockIdx.z * frame_bytes, luma + blockIdx.z * luma_w * luma_h.
+// 10-bit planes (T = unsigned short, MAX = 1023) take the same rule with 1023 for 255, the value
+// written at bit SHIFT of its word (I010: 0, P010: 6).
+template <class T, int MAX, int SHIFT>
 __global__ void swap_luma_plane_kernel(const float* __restrict__ luma,
                                        unsigned char* __restrict__ target, int gt_w, size_t pitch,
                                        size_t frame_bytes, int luma_w, int luma_h) {
@@ -515,8 +518,9 @@ __global__ void swap_luma_plane_kernel(const float* __restrict__ luma,
   const int y = blockIdx.y * blockDim.y + threadIdx.y;
   if (x >= luma_w || y >= luma_h) return;
   const int pad = (gt_w - luma_w) / 2;
-  const float Y = __fmul_rn(luma[(size_t)y * luma_w + x], 255.0f);
-  target[(size_t)(y + pad) * pitch + x + pad] = (unsigned char)(unsigned int)fminf(fmaxf(Y, 0.f), 255.f);
+  const float Y = __fmul_rn(luma[(size_t)y * luma_w + x], (float)MAX);
+  *reinterpret_cast<T*>(target + (size_t)(y + pad) * pitch + x * sizeof(T) + pad * sizeof(T)) =
+      (T)((unsigned int)fminf(fmaxf(Y, 0.f), (float)MAX) << SHIFT);
 }
 
 }  // namespace generic

@@ -1401,9 +1401,10 @@ FrameBytes rgba_frame_bytes(const srcnn_net* net, int w, int h, int out_w, int o
 
 // staging in `st`, the resample table and the prepared network of a frames call whose arguments
 // have been checked
+// (`bit_depth` selects the resample table: 8, or 10 for the Y plane of 10-bit frames)
 int frames_prepare(srcnn_ctx* ctx, const srcnn_net* net, srcnn_ctx::FramesStaging& st, int w, int h,
                    int n_frames, int out_w, int out_h, int filter, const FrameBytes& fb,
-                   FramesCall* fc) {
+                   FramesCall* fc, int bit_depth = 8) {
   const Dims d = net_dims(net, out_w, out_h);
   const size_t npx = (size_t)out_w * out_h, out_px = (size_t)d.w3 * d.h3;
   SRCNN_CUDA(ctx->drain_lanes());
@@ -1423,7 +1424,7 @@ int frames_prepare(srcnn_ctx* ctx, const srcnn_net* net, srcnn_ctx::FramesStagin
     SRCNN_TRY(ensure_scratch(ctx, &st.s2, &st.s2_bytes, sizeof(float) * (size_t)d.w2 * d.h2 * net->n2));
   }
   SRCNN_TRY(resample::table_for(ctx, w, h, out_w, out_h, filter, SRCNN_CHROMA_CENTER,
-                                SRCNN_CHROMA_CENTER, &u.tab, &u.rows_max));
+                                SRCNN_CHROMA_CENTER, &u.tab, &u.rows_max, bit_depth));
   SRCNN_TRY(fused_net(ctx, net, &fc->fn));
   u.rgba = (uchar4*)st.rgba;
   u.luma = (float*)st.luma;
@@ -1558,27 +1559,41 @@ int check_sitings(int siting_in, int siting_out) {
   return SRCNN_OK;
 }
 
-// whole I420 frames of w x h back to back: the frames of srcnn_upscale_yuv420_frames_host
-srcnn_yuv420_layout i420_dense(int w, int h) {
-  const size_t y = (size_t)w * h, c = y / 4;
-  return srcnn_yuv420_layout{SRCNN_YUV_I420, y + 2 * c, (size_t)w, (size_t)w / 2, y, y + c,
-                             SRCNN_CHROMA_CENTER};
+// whole I420 (bit_depth 10: I010) frames of w x h back to back: the frames of
+// srcnn_upscale_yuv420_frames_host (srcnn_upscale_yuv420p10_frames_host)
+srcnn_yuv420_layout i420_dense(int w, int h, int bit_depth = 8) {
+  const size_t b = bit_depth == 10 ? 2 : 1, y = (size_t)w * h * b, c = y / 4;
+  return srcnn_yuv420_layout{SRCNN_YUV_I420, y + 2 * c, (size_t)w * b, (size_t)w / 2 * b, y, y + c,
+                             SRCNN_CHROMA_CENTER, bit_depth};
 }
 
 // the layout of n_frames frames of w x h (w, h even and > 0) holds them: *need = the bytes from
-// the first frame's start to the end of the last frame's last plane
+// the first frame's start to the end of the last frame's last plane.  Its bit_depth is 0, 8 or 10.
 int check_layout(const srcnn_yuv420_layout& l, int w, int h, int n_frames, size_t* need,
                  const char* what) {
   const bool nv12 = l.format == SRCNN_YUV_NV12;
-  const size_t big = (size_t)1 << 31, c_row = nv12 ? (size_t)w : (size_t)w / 2;
+  SRCNN_REQUIRE(l.bit_depth == 0 || l.bit_depth == 8 || l.bit_depth == 10,
+                "%s layout: bit depth %d is not 8 or 10", what, l.bit_depth);
+  const bool ten = l.bit_depth == 10;
+  const size_t big = (size_t)1 << 31, b = ten ? 2 : 1, y_row = (size_t)w * b,
+               c_row = (nv12 ? (size_t)w : (size_t)w / 2) * b;
   SRCNN_REQUIRE(l.frame_stride < big && l.y_pitch < big && l.c_pitch < big && l.cb_offset < big &&
                     l.cr_offset < big,
                 "%s layout: a pitch, offset or stride of 2^31 bytes or more", what);
-  SRCNN_REQUIRE(l.y_pitch >= (size_t)w && l.c_pitch >= c_row,
-                "%s layout: pitches %zu (Y) and %zu (chroma) below the rows' %d and %zu bytes", what,
-                l.y_pitch, l.c_pitch, w, c_row);
+  SRCNN_REQUIRE(l.y_pitch >= y_row && l.c_pitch >= c_row,
+                "%s layout: pitches %zu (Y) and %zu (chroma) below the rows' %zu and %zu bytes", what,
+                l.y_pitch, l.c_pitch, y_row, c_row);
+  if (ten) {
+    // every sample is a 16-bit word, every P010 CbCr pair a 32-bit one
+    SRCNN_REQUIRE(l.y_pitch % 2 == 0 && l.c_pitch % 2 == 0 && l.cb_offset % 2 == 0 &&
+                      l.cr_offset % 2 == 0 && (n_frames == 1 || l.frame_stride % 2 == 0),
+                  "%s layout: 10-bit samples need even pitches, offsets and frame_stride", what);
+    SRCNN_REQUIRE(!nv12 || (l.c_pitch % 4 == 0 && (n_frames == 1 || l.frame_stride % 4 == 0)),
+                  "%s layout: P010 needs a c_pitch and frame_stride that are multiples of 4, got "
+                  "%zu and %zu", what, l.c_pitch, l.frame_stride);
+  }
   // the planes' byte ranges from the frame start: Y [0, y_end), chroma [offset, offset + c_len)
-  const size_t y_end = (size_t)(h - 1) * l.y_pitch + w;
+  const size_t y_end = (size_t)(h - 1) * l.y_pitch + y_row;
   const size_t c_len = (size_t)(h / 2 - 1) * l.c_pitch + c_row;
   size_t extent = std::max(y_end, l.cb_offset + c_len);
   SRCNN_REQUIRE(l.cb_offset >= y_end, "%s layout: the %s plane at %zu intersects the Y plane [0, %zu)",
@@ -1616,11 +1631,16 @@ struct Yuv420 {
 // the luma of the Y plane, its Q1 mean.  4 launches (I420), 5 (NV12).
 int yuv420_head(srcnn_ctx* ctx, const Upscale& u, const Yuv420& y) {
   {
+    using namespace resample;
     const bool nv12 = y.li.format == SRCNN_YUV_NV12;
     LaunchScope scope(ctx, SRCNN_K_RESAMPLE, nv12 ? 2 : 1);
-    SRCNN_TRY((nv12 ? resample::launch_nv12 : resample::launch_yuv420)(
-        ctx, y.in, y.li, u.w, u.h, y.out, y.lo, u.luma, u.out_w, u.out_h, u.filter, u.tab,
-        u.rows_max, y.tab_c, y.rows_max_c, u.frames));
+    const auto launch =
+        y.li.bit_depth == 10
+            ? (nv12 ? launch_nv12<unsigned short, Words10<6>>
+                    : launch_yuv420<unsigned short, Words10<0>>)
+            : (nv12 ? launch_nv12<unsigned char, Bytes> : launch_yuv420<unsigned char, Bytes>);
+    SRCNN_TRY(launch(ctx, y.in, y.li, u.w, u.h, y.out, y.lo, u.luma, u.out_w, u.out_h, u.filter,
+                     u.tab, u.rows_max, y.tab_c, y.rows_max_c, u.frames));
     SRCNN_TRY(check_launch("resample"));
   }
   return q1_mean(ctx, u);
@@ -1630,8 +1650,12 @@ int yuv420_head(srcnn_ctx* ctx, const Upscale& u, const Yuv420& y) {
 int yuv420_swap(srcnn_ctx* ctx, const Upscale& u, const Yuv420& y) {
   LaunchScope scope(ctx, SRCNN_K_SWAP_LUMA);
   dim3 block(32, 8), grid((u.d.w3 + 31) / 32, (u.d.h3 + 7) / 8, u.frames);
-  generic::swap_luma_plane_kernel<<<grid, block, 0, ctx->stream>>>(
-      u.out3, y.out, u.out_w, y.lo.y_pitch, y.lo.frame_stride, u.d.w3, u.d.h3);
+  const auto kernel = y.lo.bit_depth != 10 ? generic::swap_luma_plane_kernel<unsigned char, 255, 0>
+                      : y.lo.format == SRCNN_YUV_NV12
+                          ? generic::swap_luma_plane_kernel<unsigned short, 1023, 6>
+                          : generic::swap_luma_plane_kernel<unsigned short, 1023, 0>;
+  kernel<<<grid, block, 0, ctx->stream>>>(u.out3, y.out, u.out_w, y.lo.y_pitch, y.lo.frame_stride,
+                                          u.d.w3, u.d.h3);
   return check_launch("swap_luma");
 }
 }  // namespace
@@ -1644,29 +1668,34 @@ int srcnn_upscale_yuv420_frames_host(srcnn_ctx* ctx, const srcnn_net* net,
                                                 host_out);
 }
 
-int srcnn_upscale_yuv420_frames_host_sited(srcnn_ctx* ctx, const srcnn_net* net,
-                                           const unsigned char* host_in, int w, int h, int n_frames,
-                                           int out_w, int out_h, int filter, int in_siting,
-                                           int out_siting, unsigned char* host_out) {
-  SRCNN_REQUIRE(ctx && host_in && host_out, "null argument");
+namespace {
+// srcnn_upscale_yuv420_frames_host_sited (bit_depth 8) and srcnn_upscale_yuv420p10_frames_host
+// (bit_depth 10) on dense frames
+int yuv420_frames_host(srcnn_ctx* ctx, const srcnn_net* net, const void* host_in_v, int w, int h,
+                       int n_frames, int out_w, int out_h, int filter, int in_siting,
+                       int out_siting, int bit_depth, void* host_out_v) {
+  SRCNN_REQUIRE(ctx && host_in_v && host_out_v, "null argument");
   SRCNN_ENTER(ctx);
   SRCNN_TRY(check_yuv420(net, w, h, n_frames, out_w, out_h, filter));
   SRCNN_TRY(check_sitings(in_siting, out_siting));
+  const unsigned char* host_in = static_cast<const unsigned char*>(host_in_v);
+  unsigned char* host_out = static_cast<unsigned char*>(host_out_v);
   srcnn_ctx::FramesStaging& st = ctx->yuv;
   const Dims d = net_dims(net, out_w, out_h);
-  Yuv420 y{nullptr, 0, nullptr, nullptr, i420_dense(w, h), i420_dense(out_w, out_h)};
+  Yuv420 y{nullptr, 0, nullptr, nullptr, i420_dense(w, h, bit_depth),
+           i420_dense(out_w, out_h, bit_depth)};
   const size_t in_frame = y.li.frame_stride, out_frame = y.lo.frame_stride;
   // the device bytes a frame of a group holds: its input and result in each ring slot, its luma
-  // and its network output (960x540 -> 1920x1080: 4 frames in ~128 MB); the frame and the plane
-  // share the grid dimension of the resampling launch
+  // and its network output (960x540 -> 1920x1080: 4 frames in ~128 MB, 3 with 10-bit samples);
+  // the frame and the plane share the grid dimension of the resampling launch
   const FrameBytes fb{in_frame, 0, out_frame,
                       (in_frame + out_frame) * kFrameRing + (size_t)out_w * out_h * 4 +
                           (size_t)d.w3 * d.h3 * 4,
                       65535 / 3};
   FramesCall fc;
-  SRCNN_TRY(frames_prepare(ctx, net, st, w, h, n_frames, out_w, out_h, filter, fb, &fc));
+  SRCNN_TRY(frames_prepare(ctx, net, st, w, h, n_frames, out_w, out_h, filter, fb, &fc, bit_depth));
   SRCNN_TRY(resample::table_for(ctx, w / 2, h / 2, out_w / 2, out_h / 2, filter, in_siting,
-                                out_siting, &y.tab_c, &y.rows_max_c));
+                                out_siting, &y.tab_c, &y.rows_max_c, bit_depth));
   unsigned char* ring_in = (unsigned char*)st.small;
   unsigned char* ring_out = (unsigned char*)st.rgb;
   Upscale& u = fc.u;
@@ -1697,6 +1726,23 @@ int srcnn_upscale_yuv420_frames_host_sited(srcnn_ctx* ctx, const srcnn_net* net,
                           return yuv420_swap(ctx, u, y);
                         });
 }
+}  // namespace
+
+int srcnn_upscale_yuv420_frames_host_sited(srcnn_ctx* ctx, const srcnn_net* net,
+                                           const unsigned char* host_in, int w, int h, int n_frames,
+                                           int out_w, int out_h, int filter, int in_siting,
+                                           int out_siting, unsigned char* host_out) {
+  return yuv420_frames_host(ctx, net, host_in, w, h, n_frames, out_w, out_h, filter, in_siting,
+                            out_siting, 8, host_out);
+}
+
+int srcnn_upscale_yuv420p10_frames_host(srcnn_ctx* ctx, const srcnn_net* net,
+                                        const uint16_t* host_in, int w, int h, int n_frames,
+                                        int out_w, int out_h, int filter, int in_siting,
+                                        int out_siting, uint16_t* host_out) {
+  return yuv420_frames_host(ctx, net, host_in, w, h, n_frames, out_w, out_h, filter, in_siting,
+                            out_siting, 10, host_out);
+}
 
 int srcnn_upscale_yuv420_frames(srcnn_ctx* ctx, const srcnn_net* net, srcnn_mem in,
                                 const srcnn_yuv420_layout* in_layout, int w, int h, int n_frames,
@@ -1711,6 +1757,10 @@ int srcnn_upscale_yuv420_frames(srcnn_ctx* ctx, const srcnn_net* net, srcnn_mem 
   SRCNN_REQUIRE(out_layout->format == format, "input format %d and output format %d differ", format,
                 out_layout->format);
   SRCNN_TRY(check_sitings(in_layout->chroma_siting, out_layout->chroma_siting));
+  const int bits = in_layout->bit_depth == 10 ? 10 : 8;
+  SRCNN_REQUIRE(bits == (out_layout->bit_depth == 10 ? 10 : 8),
+                "input bit depth %d and output bit depth %d differ", in_layout->bit_depth,
+                out_layout->bit_depth);
   size_t in_need, out_need;
   SRCNN_TRY(check_layout(*in_layout, w, h, n_frames, &in_need, "input"));
   SRCNN_TRY(check_layout(*out_layout, out_w, out_h, n_frames, &out_need, "output"));
@@ -1728,6 +1778,15 @@ int srcnn_upscale_yuv420_frames(srcnn_ctx* ctx, const srcnn_net* net, srcnn_mem 
                       (n_frames == 1 || out_layout->frame_stride % 2 == 0),
                   "output NV12 CbCr plane at an odd address");
   }
+  if (bits == 10) {
+    // 16-bit words, and P010 CbCr pairs read and written as 32-bit words (the strides and
+    // pitches are checked with the layouts)
+    const size_t a = nv12 ? 4 : 2;
+    SRCNN_REQUIRE((uintptr_t)pi % 2 == 0 && ((uintptr_t)pi + in_layout->cb_offset) % a == 0,
+                  "input 10-bit frames at an odd address, or a P010 CbCr plane off 4 bytes");
+    SRCNN_REQUIRE((uintptr_t)po % 2 == 0 && ((uintptr_t)po + out_layout->cb_offset) % a == 0,
+                  "output 10-bit frames at an odd address, or a P010 CbCr plane off 4 bytes");
+  }
   SRCNN_REQUIRE(pi + in_need <= po || po + out_need <= pi, "input and output bytes overlap");
   ctx->note_write(out);
   const Upscale job{w, h, out_w, out_h, filter, 1, net_dims(net, out_w, out_h), nullptr, 0};
@@ -1737,11 +1796,12 @@ int srcnn_upscale_yuv420_frames(srcnn_ctx* ctx, const srcnn_net* net, srcnn_mem 
                       job.npx() * 4 + (size_t)job.d.w3 * job.d.h3 * 4 + job.red_frame(),
                       nv12 ? 65535 : 65535 / 3};
   FramesCall fc;
-  SRCNN_TRY(frames_prepare(ctx, net, ctx->yuv_dev, w, h, n_frames, out_w, out_h, filter, fb, &fc));
+  SRCNN_TRY(frames_prepare(ctx, net, ctx->yuv_dev, w, h, n_frames, out_w, out_h, filter, fb, &fc,
+                           bits));
   Yuv420 y{nullptr, 0, pi, po, *in_layout, *out_layout};
   SRCNN_TRY(resample::table_for(ctx, w / 2, h / 2, out_w / 2, out_h / 2, filter,
                                 in_layout->chroma_siting, out_layout->chroma_siting, &y.tab_c,
-                                &y.rows_max_c));
+                                &y.rows_max_c, bits));
   // groups of frames (one frame without a fused kernel, for the reason forward_three_launch
   // gives): enlargement + luma, Q1 mean, forward, Y write
   Upscale& u = fc.u;

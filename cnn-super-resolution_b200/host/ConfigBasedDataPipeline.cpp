@@ -561,6 +561,24 @@ void ConfigBasedDataPipeline::upscale_yuv420_frames(LayerAllocationPool& l1, Lay
       "upscale_yuv420_frames");
 }
 
+void ConfigBasedDataPipeline::upscale_yuv420p10_frames(LayerAllocationPool& l1,
+                                                       LayerAllocationPool& l2,
+                                                       LayerAllocationPool& l3,
+                                                       const uint16_t* in_yuv, size_t w, size_t h,
+                                                       size_t n_frames, size_t out_w, size_t out_h,
+                                                       int filter, uint16_t* out_yuv,
+                                                       int in_siting, int out_siting) {
+  check_initialized(DataPipeline::LOAD_KERNEL_LUMA | DataPipeline::LOAD_KERNEL_MISC);
+  const srcnn_net net = device_net(l1, l2, l3, false, false);
+  opencl::ProfiledLaunch p1(*resample_kernel()), p2(*_sum_squared_kernel),
+      p3(*_subtract_from_all_kernel), p4(*_swap_luma_kernel);
+  _context->check_status(
+      srcnn_upscale_yuv420p10_frames_host(_context->c_ctx(), &net, in_yuv, (int)w, (int)h,
+                                          (int)n_frames, (int)out_w, (int)out_h, filter, in_siting,
+                                          out_siting, out_yuv),
+      "upscale_yuv420p10_frames");
+}
+
 void ConfigBasedDataPipeline::evaluate_frames(LayerAllocationPool& l1, LayerAllocationPool& l2,
                                               LayerAllocationPool& l3, const unsigned char* in_rgba,
                                               size_t w, size_t h, size_t n_frames, size_t out_w,

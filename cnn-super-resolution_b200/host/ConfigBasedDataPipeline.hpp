@@ -71,6 +71,14 @@ class ConfigBasedDataPipeline : public DataPipeline {
                              size_t out_w, size_t out_h, int filter, unsigned char* out_yuv,
                              int in_siting = SRCNN_CHROMA_CENTER,
                              int out_siting = SRCNN_CHROMA_CENTER);
+  /** upscale_yuv420_frames for 10-bit I010 frames (a little-endian 16-bit word a sample, the
+   * value in its low 10 bits): `out_yuv` receives n_frames I010 frames of out_w x out_h
+   * (srcnn_upscale_yuv420p10_frames_host) */
+  void upscale_yuv420p10_frames(LayerAllocationPool&, LayerAllocationPool&, LayerAllocationPool&,
+                                const uint16_t* in_yuv, size_t w, size_t h, size_t n_frames,
+                                size_t out_w, size_t out_h, int filter, uint16_t* out_yuv,
+                                int in_siting = SRCNN_CHROMA_CENTER,
+                                int out_siting = SRCNN_CHROMA_CENTER);
   /** upscale_frames plus the quality of every result against its reference (n_frames frames of
    * out_w x out_h RGBA8 in `ref_rgba`): `metrics` receives 4 doubles a frame, {mse, ssim} of the
    * network's result and of the plain enlargement, over the region `border` pixels in from each

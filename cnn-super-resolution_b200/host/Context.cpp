@@ -101,7 +101,8 @@ static std::runtime_error y4m_error(const std::string& path, const std::string& 
 static const char* const kY4mSiting[3] = {"420jpeg", "420mpeg2", "420paldv"};
 static const char* const kY4mXyscss[3] = {"420JPEG", "420MPEG2", "420PALDV"};
 
-Y4mReader::Y4mReader(const char* path, bool any_siting) : _path(path), _f(path, std::ios::binary) {
+Y4mReader::Y4mReader(const char* path, bool any_siting, bool ten_bit)
+    : _path(path), _f(path, std::ios::binary) {
   if (!_f.is_open()) throw y4m_error(_path, "could not open");
   std::string line;
   if (!std::getline(_f, line) || line.compare(0, 10, "YUV4MPEG2 ") != 0)
@@ -130,9 +131,12 @@ Y4mReader::Y4mReader(const char* path, bool any_siting) : _path(path), _f(path, 
                                    "(C420jpeg, C420) is supported; --chroma-siting keep enlarges it "
                                    "at its own siting");
           _header.chroma_siting = v == "420mpeg2" ? SRCNN_CHROMA_LEFT : SRCNN_CHROMA_TOPLEFT;
+        } else if (v == "420p10" && ten_bit) {
+          _header.bit_depth = 10;
         } else if (v != "420jpeg" && v != "420")
           throw y4m_error(_path, "colourspace '" + t + "' is not supported; only 8-bit 4:2:0 "
-                                 "(C420jpeg, C420) is");
+                                 "(C420jpeg, C420) is" +
+                                 (v == "420p10" ? "; --bit-depth 10 reads 10-bit 4:2:0" : ""));
         break;
       case 'I':
         if (v != "p")

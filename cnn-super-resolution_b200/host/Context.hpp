@@ -61,27 +61,31 @@ int write_image(const char* path, ImageData&);
 /** luma in [0,1] -> 8-bit binary PGM (reference: UtilsOpenCL.cpp write_image(float*)) */
 void write_image(const char* path, float* luma, size_t w, size_t h);
 
-/** The header of a YUV4MPEG2 (Y4M) stream: "YUV4MPEG2" and space-separated tags.  Only 8-bit
- * progressive 4:2:0 of even size is accepted.  Its chroma siting is read as ffmpeg's reader maps
- * the colourspace tag: C420jpeg (the format's default) and C420 centre-sited, C420mpeg2 left-sited,
- * C420paldv top-left-sited. */
+/** The header of a YUV4MPEG2 (Y4M) stream: "YUV4MPEG2" and space-separated tags.  Only
+ * progressive 4:2:0 of even size is accepted: 8-bit, or 10-bit (C420p10, ffmpeg's yuv420p10le:
+ * a little-endian 16-bit word a sample) when asked for.  Its chroma siting is read as ffmpeg's
+ * reader maps the colourspace tag: C420jpeg (the format's default), C420 and C420p10 centre-sited,
+ * C420mpeg2 left-sited, C420paldv top-left-sited. */
 struct Y4mHeader {
   int w = 0, h = 0;
   int chroma_siting = SRCNN_CHROMA_CENTER;   // SRCNN_CHROMA_*
+  int bit_depth = 8;                         // 8, or 10 for C420p10
   std::vector<std::string> tags;   // every tag as read, in order ("W960", "F30000:1001", ...)
-  size_t frame_bytes() const { return (size_t)w * h * 3 / 2; }
+  size_t frame_bytes() const { return (size_t)w * h * 3 / 2 * (bit_depth == 10 ? 2 : 1); }
 };
 /** Reads the frames of a Y4M file.  Every check throws std::runtime_error with a one-line
  * message: the constructor checks the header, check_frames() every frame marker and frame size. */
 class Y4mReader {
  public:
-  /** any_siting: accept chroma that is not centre-sited (refused otherwise) */
-  explicit Y4mReader(const char* path, bool any_siting = false);
+  /** any_siting: accept chroma that is not centre-sited; ten_bit: accept C420p10 (each refused
+   * otherwise) */
+  explicit Y4mReader(const char* path, bool any_siting = false, bool ten_bit = false);
   const Y4mHeader& header() const { return _header; }
   /** the number of frames; every frame starts with "FRAME[ params]\n" and is complete.  Leaves
    * the reader at the first frame. */
   size_t check_frames();
-  /** up to `max` next frames (I420, their parameters dropped) into `out`; returns how many */
+  /** up to `max` next frames (I420 or I010 bytes, their parameters dropped) into `out`; returns
+   * how many */
   size_t read_frames(size_t max, std::vector<unsigned char>& out);
 
  private:
@@ -96,7 +100,8 @@ class Y4mReader {
  * (SRCNN_CHROMA_*) other than in's, the C tag names it (appended when `in` has none) and an
  * XYSCSS= tag matches it */
 void write_y4m_header(std::ostream&, const Y4mHeader& in, int out_w, int out_h, int out_siting);
-/** n frames of `frame_bytes` bytes, each behind a bare "FRAME\n" */
+/** n frames of `frame_bytes` bytes, each behind a bare "FRAME\n" (10-bit frames as the
+ * little-endian words of a little-endian host, as they were read) */
 void write_y4m_frames(std::ostream&, const unsigned char* frames, size_t n, size_t frame_bytes);
 }  // namespace utils
 

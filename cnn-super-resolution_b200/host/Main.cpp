@@ -1,5 +1,6 @@
 // `cnn [train | eval] [dry] [profile] --config CFG --in PATH [--out PATH] [--epochs N]
-//      [--scale N [--resample lanczos|bicubic]] [--chroma-siting keep|420jpeg|420mpeg2|420paldv]`
+//      [--scale N [--resample lanczos|bicubic]] [--chroma-siting keep|420jpeg|420mpeg2|420paldv]
+//      [--bit-depth 8|10]`
 // Same grammar, flow and console output as the reference CLI (src/Main_cl.cpp:40-318):
 // forward mode = one image through the three layers, luma swapped back into the image (or every
 // image of a directory, see below);
@@ -18,6 +19,10 @@
 // checked before any device work.  Left- and top-left-sited chroma (C420mpeg2, C420paldv) is refused
 // unless --chroma-siting names the output's siting: `keep` (the input's, every tag copied) or a
 // colourspace tag, to which the chroma is converted (the C tag, and an XYSCSS= tag, then name it).
+// 10-bit video (C420p10, ffmpeg's yuv420p10le; centre-sited) is refused unless --bit-depth 10 asks
+// for it, and then goes through srcnn_upscale_yuv420p10_frames_host; --bit-depth 10 needs a
+// C420p10 header, and its output is centre-sited (--chroma-siting keep or 420jpeg), because a
+// C420p10 tag cannot state another siting.
 // eval -i SAMPLES_DIR measures the network on the training mode's sample pairs: every `_small`
 // image, enlarged N times (--scale, default 1: the reference's `_small` images are already
 // enlarged), against its `_large` image, which must be exactly N times its size.  One line a pair
@@ -175,14 +180,15 @@ static void execute_directory(ConfigBasedDataPipeline& pipeline, GpuAllocationPo
   flush();
 }
 
-// every frame of a Y4M video through the I420 frames entry, `scale` times enlarged, kDirBatch
-// frames at a time; the result goes to out_path unless it is null (dry run)
+// every frame of a Y4M video through the I420 (10-bit: I010) frames entry, `scale` times enlarged,
+// kDirBatch frames at a time; the result goes to out_path unless it is null (dry run)
 static void execute_y4m(ConfigBasedDataPipeline& pipeline, GpuAllocationPool& gpu_alloc,
                         Y4mReader& video, const char* out_path, size_t scale, int filter,
                         int out_siting) {
   const Y4mHeader& hd = video.header();
   const size_t w = (size_t)hd.w, h = (size_t)hd.h, out_w = scale * w, out_h = scale * h;
-  const size_t out_bytes = out_w * out_h * 3 / 2;
+  const bool ten = hd.bit_depth == 10;
+  const size_t out_bytes = out_w * out_h * 3 / 2 * (ten ? 2 : 1);
   std::ofstream out;
   if (out_path) {
     std::cout << "Saving result video to: '" << out_path << "'" << std::endl;
@@ -194,9 +200,17 @@ static void execute_y4m(ConfigBasedDataPipeline& pipeline, GpuAllocationPool& gp
   size_t n;
   while ((n = video.read_frames(kDirBatch, in)) > 0) {
     result.resize(n * out_bytes);
-    pipeline.upscale_yuv420_frames(gpu_alloc.layer_1, gpu_alloc.layer_2, gpu_alloc.layer_3,
-                                   in.data(), w, h, n, out_w, out_h, filter, result.data(),
-                                   hd.chroma_siting, out_siting);
+    // a 10-bit frame's bytes are its little-endian words; vector storage is aligned for them
+    if (ten)
+      pipeline.upscale_yuv420p10_frames(gpu_alloc.layer_1, gpu_alloc.layer_2, gpu_alloc.layer_3,
+                                        reinterpret_cast<const uint16_t*>(in.data()), w, h, n,
+                                        out_w, out_h, filter,
+                                        reinterpret_cast<uint16_t*>(result.data()),
+                                        hd.chroma_siting, out_siting);
+    else
+      pipeline.upscale_yuv420_frames(gpu_alloc.layer_1, gpu_alloc.layer_2, gpu_alloc.layer_3,
+                                     in.data(), w, h, n, out_w, out_h, filter, result.data(),
+                                     hd.chroma_siting, out_siting);
     if (out_path) write_y4m_frames(out, result.data(), n, out_bytes);
     in.clear();
   }
@@ -354,6 +368,7 @@ int main(int argc, char** argv) {
   argparse.add_argument("-s", "--scale").help("Forward mode: enlarge the image N times first (default 1)");
   argparse.add_argument("-r", "--resample").help("Enlargement filter: lanczos (default) or bicubic");
   argparse.add_argument("--chroma-siting").help("A .y4m input: the output's chroma siting, keep (the input's), 420jpeg, 420mpeg2 or 420paldv; accepts every siting the input may have");
+  argparse.add_argument("--bit-depth").help("A .y4m input: 8 (default) or 10, which reads 10-bit 4:2:0 (C420p10)");
   try {
     if (!argparse.parse((size_t)argc, argv)) return EXIT_SUCCESS;
   } catch (const std::exception& e) {
@@ -417,6 +432,19 @@ int main(int argc, char** argv) {
       return EXIT_FAILURE;
     }
   }
+  const char* depth_name = argparse.value("bit-depth");
+  int bit_depth = 8;
+  if (depth_name) {
+    if (std::strcmp(depth_name, "8") != 0 && std::strcmp(depth_name, "10") != 0) {
+      std::cout << "--bit-depth must be 8 or 10, got '" << depth_name << "'" << std::endl;
+      return EXIT_FAILURE;
+    }
+    bit_depth = std::atoi(depth_name);
+    if (!in_y4m || train || eval) {
+      std::cout << "--bit-depth applies to a .y4m input in the forward mode only" << std::endl;
+      return EXIT_FAILURE;
+    }
+  }
   const bool in_dir = !train && !eval && !in_y4m && is_directory(in_path);
   if ((in_dir || eval) && out_path && !is_directory(out_path)) {
     std::cout << "Output directory '" << out_path << "' does not exist or is not a directory"
@@ -452,7 +480,13 @@ int main(int argc, char** argv) {
     // a video is checked whole before the context exists
     std::unique_ptr<Y4mReader> video;
     if (in_y4m) {
-      video.reset(new Y4mReader(in_path, siting_name != nullptr));
+      video.reset(new Y4mReader(in_path, siting_name != nullptr, bit_depth == 10));
+      if (video->header().bit_depth != bit_depth)
+        throw std::runtime_error("--bit-depth 10 needs a 10-bit (C420p10) input; '" +
+                                 std::string(in_path) + "' is 8-bit");
+      if (bit_depth == 10 && out_siting > SRCNN_CHROMA_CENTER)
+        throw std::runtime_error("--chroma-siting must be keep or 420jpeg for a 10-bit input: a "
+                                 "C420p10 tag cannot state another siting");
       const size_t n_frames = video->check_frames();
       std::cout << "Video: " << video->header().w << "x" << video->header().h << ", " << n_frames
                 << " frames" << std::endl;

@@ -375,7 +375,15 @@ int srcnn_upscale_yuv420_frames_host_sited(srcnn_ctx* ctx, const srcnn_net* net,
  * {NV12, w*h*3/2, w, w, w*h, 0, 0}.
  * chroma_siting was appended as the last field so that the fields before it keep their offsets
  * and a zero-initialised layout keeps its meaning (centre-sited chroma); a caller that declares
- * the struct itself (a language binding) adds the field too. */
+ * the struct itself (a language binding) adds the field too.
+ * bit_depth was appended after it for the same reason: 0 or 8 is 8-bit samples, one byte each;
+ * 10 is 10-bit samples v in [0, 1023], one little-endian 16-bit word each, and then
+ * SRCNN_YUV_I420 means I010 (`yuv420p10le`, the frames of a C420p10 Y4M file: v in the low 10
+ * bits) and SRCNN_YUV_NV12 means P010 (what hardware decoders hand out for 10-bit streams: v in the
+ * high 10 bits, word = v << 6).  The other 6 bits of an input word never affect a result and are
+ * written as 0.  A 10-bit row is twice the bytes of an 8-bit one: the dense I010 layout is {I420,
+ * w*h*3, 2*w, w, 2*w*h, 2*w*h*5/4, 0, 10}, the dense P010 one {NV12, w*h*3, 2*w, 2*w, 2*w*h, 0, 0,
+ * 10}. */
 enum { SRCNN_YUV_I420 = 0, SRCNN_YUV_NV12 = 1 };
 typedef struct srcnn_yuv420_layout {
   int format;           /* SRCNN_YUV_I420 or SRCNN_YUV_NV12 */
@@ -385,13 +393,17 @@ typedef struct srcnn_yuv420_layout {
   size_t cb_offset;     /* of the Cb plane (NV12: the CbCr plane) from the frame start */
   size_t cr_offset;     /* I420: of the Cr plane; NV12: must be 0 */
   int chroma_siting;    /* SRCNN_CHROMA_*: where the frames' chroma samples sit; 0 = centre */
+  int bit_depth;        /* 0 or 8: 8-bit samples; 10: 10-bit samples in 16-bit words (I010, P010) */
 } srcnn_yuv420_layout;
 
 /* srcnn_upscale_yuv420_frames_host on frames that are already in device memory, in I420 or NV12
  * with pitched rows: `in` holds n_frames frames of w x h in in_layout, `out` receives n_frames
  * frames of out_w x out_h in out_layout, of the same format.  The Y, Cb and Cr bytes of a frame are
  * those srcnn_upscale_yuv420_frames_host_sited writes for it with in_layout's chroma_siting as the
- * input's and out_layout's as the output's (NV12: the same Cb and Cr bytes, interleaved).  Bytes of `out` outside the planes' rows (pitch padding, gaps between planes or
+ * input's and out_layout's as the output's (NV12: the same Cb and Cr bytes, interleaved).  With
+ * bit_depth 10 in both layouts the frames are I010 or P010, and a frame's samples are those
+ * srcnn_upscale_yuv420p10_frames_host writes for it (P010: the same Cb and Cr, interleaved, each
+ * value at bit 6 of its word); the groups, scratch and launches are those of 8-bit frames.  Bytes of `out` outside the planes' rows (pitch padding, gaps between planes or
  * frames) are never written; bytes of `in` outside them never affect the result.
  * Stream-ordered, like srcnn_forward_fused: the work is enqueued on the context stream and the
  * call returns, without a copy or a host synchronisation (the caller orders its own work on that
@@ -417,7 +429,11 @@ typedef struct srcnn_yuv420_layout {
  * as for srcnn_upscale_frames_host).
  * Errors, all before any launch (the output and the launch count stay untouched):
  *   SRCNN_EINVAL: everything srcnn_upscale_yuv420_frames_host rejects; a null layout; an unknown
- *     format, or formats that differ; a chroma_siting outside SRCNN_CHROMA_* in either layout; a pitch below its row's bytes; a pitch, offset or stride of
+ *     format, or formats that differ; a chroma_siting outside SRCNN_CHROMA_* in either layout; a
+ *     bit_depth other than 0, 8 or 10, or input and output bit depths that differ; 10-bit with an
+ *     odd pitch, offset, buffer start or (n_frames > 1) frame_stride, or P010 with a CbCr plane
+ *     or c_pitch that is not a multiple of 4 bytes in any frame; a pitch below its row's bytes
+ *     (10-bit: 2*w for Y and P010 CbCr, w for I010 chroma); a pitch, offset or stride of
  *     2^31 bytes or more; planes of one frame whose byte ranges intersect; with n_frames > 1, a
  *     frame_stride below the frame's extent (the end of its last plane's last row); NV12 with
  *     cr_offset != 0, an odd c_pitch, or a CbCr plane at an odd address in any frame; input and
@@ -428,6 +444,30 @@ int srcnn_upscale_yuv420_frames(srcnn_ctx* ctx, const srcnn_net* net, srcnn_mem 
                                 const srcnn_yuv420_layout* in_layout, int w, int h, int n_frames,
                                 srcnn_mem out, const srcnn_yuv420_layout* out_layout, int out_w,
                                 int out_h, int filter);
+
+/* srcnn_upscale_yuv420_frames_host_sited for 10-bit frames: host_in holds n_frames dense I010
+ * frames of w x h (Y, then Cb, then Cr, one little-endian 16-bit word a sample with the value v in
+ * its low 10 bits: w*h*3 bytes a frame, the frames of a C420p10 Y4M file), host_out receives
+ * n_frames frames of out_w*out_h*3 bytes.  The bits above the low 10 of an input word never
+ * affect a result; every output word is v in [0, 1023], its upper bits 0.  Per frame:
+ *   - every plane is enlarged with Pillow's 16-bit path (Image.fromarray(plane, "I;16").resize):
+ *     the coefficients of the 8-bit path kept as normalised doubles (not rounded to 22 bits), each
+ *     output the sum of v * k in double in tap order, rounded half away from zero and clipped to
+ *     [0, 65535]; the horizontal pass first into a 16-bit intermediate, an axis copied when its
+ *     size does not change and its box starts at 0.0.  The final samples are capped at 1023.  The
+ *     chroma planes take the box starts of the sitings as in the 8-bit entry.
+ *   - the luma v / 1023 of the enlarged Y, minus the Q1 mean, goes through the three layers;
+ *     inside the network's output region the Y sample is clamp(luma * 1023, 0, 1023) truncated,
+ *     and the border keeps the enlarged Y.
+ * A frame's words do not depend on the other frames of the call or on the group size.  The ring,
+ * groups and launches are those of srcnn_upscale_yuv420_frames_host with every frame twice the
+ * bytes (3 frames a group for 960x540 -> 1920x1080 with a 9-1-5 network).  Everything
+ * srcnn_upscale_yuv420_frames_host_sited rejects: SRCNN_EINVAL before any host buffer is read or
+ * written. */
+int srcnn_upscale_yuv420p10_frames_host(srcnn_ctx* ctx, const srcnn_net* net,
+                                        const uint16_t* host_in, int w, int h, int n_frames,
+                                        int out_w, int out_h, int filter, int in_siting,
+                                        int out_siting, uint16_t* host_out);
 
 /* srcnn_upscale_frames_host plus the quality of its results: host_ref holds n_frames reference
  * frames of out_w*out_h*4 bytes RGBA8 (the ground truth the small frames were made from).
